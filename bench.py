@@ -23,6 +23,9 @@ A "step" is one pass of the hot path (pre-pass -> entropy decode -> IDCT/colour)
              (oracle/_ref) where it decodes the file, else against the non-strict oracle port.
   cpu_baseline  the reference CPU path on the host cores of this box, bounded sample. The parity check, this
              leg and --impl reference are the only places oracle/ is executed by this file.
+
+--dump-outputs DIR writes what the last timed step computed (see dump_outputs) so that two builds can be compared
+output for output: the inputs are synthetic and seeded, identical from run to run for the same arguments.
 """
 import argparse
 import hashlib
@@ -34,6 +37,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (which may be read-only)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -364,6 +368,30 @@ def check_parity(batch, idx, digests):
     return out
 
 
+DUMP_VALUES = 4 << 20      # values per dumped array and job: 16 MiB of pixels and 32 MiB of coefficients
+
+
+def dump_outputs(out_dir, batch, rank, world):
+    """Writes the batch's outputs as a caller reads them after the last timed step, flat and image after image: the
+    BGRA pixels (uint8 [H, W, 4] per image) to pixels.npy as float32 and the coefficient tap (int32 [blocks, 64] per
+    image) to coefs.npy as float64 (with 16-bit quantisers a coefficient can exceed what float32 holds exactly). An
+    image whose output is larger than its share of DUMP_VALUES contributes a fixed sample: flat indices drawn by numpy's
+    default_rng seeded with (image index, array number), sorted. With several ranks every rank writes its own files
+    (suffix _rank<r>) and the share shrinks with the rank count."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = max(1, DUMP_VALUES // (world * batch.n))
+    suffix = "_rank%d" % rank if world > 1 else ""
+    for k, (name, read, dtype) in enumerate((("pixels", batch.pixels, np.float32), ("coefs", batch.coefs, np.float64))):
+        parts = []
+        for i in range(batch.n):
+            a = read(i).reshape(-1)
+            if a.size > share:
+                a = a[np.sort(np.random.default_rng((i, k)).integers(0, a.size, share))]
+            parts.append(a.astype(dtype))
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.concatenate(parts))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -375,7 +403,10 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=0, help="images in the cpu_baseline sample (0 = about 8 per core)")
     ap.add_argument("--no-parity", action="store_true", help="skip the comparison with the reference (measurement scripts)")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the pixels and coefficients of the last timed step to DIR/pixels.npy and DIR/coefs.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b2j" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -473,6 +504,8 @@ def main():
     barrier()
     st = batch.status()
     assert not st.any(), "decode status not clean: %s" % st[st != 0][:8]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, batch, rank, world)
     ms_per_step = allmax(total_ms) / args.steps
     pix_job = allsum(float(info.total_pixels))
     value = pix_job / (ms_per_step * 1e-3) / 1e6

@@ -2,6 +2,7 @@
 the host LUT builder, exercised through tests/native/libb2jcheck.so (same header, built with g++),
 against the oracle. This is not a CPU decode path: it checks formulas before GPU time is spent."""
 import ctypes
+import hashlib
 import os
 
 import numpy as np
@@ -42,13 +43,20 @@ def test_idct_matches_oracle(chk, oracle):
         assert np.array_equal(got, oracle.idct(a))
 
 
-def test_idct_matches_reference_build(chk, reference):
+def idct_blocks():
     rng = np.random.RandomState(2)
-    for _ in range(100):
-        a = np.ascontiguousarray(rng.randint(-255, 255, 64) * (rng.rand(64) < 0.4), dtype=np.int32)
+    return [np.ascontiguousarray(rng.randint(-255, 255, 64) * (rng.rand(64) < 0.4), dtype=np.int32) for _ in range(100)]
+
+
+def test_idct_matches_reference_build(chk, reference_digests):
+    want = reference_digests["idct"]
+    blocks = idct_blocks()
+    assert len(blocks) == len(want)
+    for k, (a, w) in enumerate(zip(blocks, want)):
+        assert hashlib.sha256(a.tobytes()).hexdigest() == w["block_sha256"], k
         got = a.copy()
         chk.chk_idct(got.ctypes.data)
-        assert np.array_equal(got, reference.fast_idct(a))
+        assert hashlib.sha256(got.tobytes()).hexdigest() == w["idct_sha256"], k
 
 
 def test_colour_exhaustive_against_double_formula(chk):
@@ -57,14 +65,20 @@ def test_colour_exhaustive_against_double_formula(chk):
     assert chk.chk_csc_exhaustive(first) == 0, list(first)
 
 
-def test_colour_spot_against_oracle_and_reference(chk, oracle, reference):
+def colour_triples():
     rng = np.random.RandomState(3)
     trip = [(-256, -256, -256), (255, 255, 255), (0, 0, 0), (188, -200, 200), (201, -200, 200), (187, -200, 200), (202, -200, 200)]
     trip += [tuple(int(v) for v in rng.randint(-256, 256, 3)) for _ in range(2000)]
-    for y, u, v in trip:
-        got = chk.chk_csc_pixel(y, u, v)
-        assert got == oracle.yuv_to_rgb32(y, u, v)
-        assert got == reference.yuv_to_rgb32(y, u, v)
+    return trip
+
+
+def test_colour_spot_against_oracle_and_reference(chk, oracle, reference_digests):
+    """Every triple against the oracle; all of them at once against the digest of the reference's uint32 results."""
+    got = []
+    for y, u, v in colour_triples():
+        got.append(chk.chk_csc_pixel(y, u, v))
+        assert got[-1] == oracle.yuv_to_rgb32(y, u, v)
+    assert hashlib.sha256(np.array(got, np.uint32).tobytes()).hexdigest() == reference_digests["colour_spot_sha256"]
 
 
 def test_extend(chk):

@@ -1,5 +1,5 @@
 """CPU: pins the oracle (oracle/oracle.c) against the reference's own fixture hashes, the committed
-golden vectors, and -- where it was built -- the unmodified reference compiled from source."""
+golden vectors, and the stored digests of the unmodified reference's output (tests/golden/reference_digests.json)."""
 import hashlib
 import json
 import os
@@ -61,42 +61,62 @@ CASES = [(64, 48, "444", 75, 0, False), (67, 45, "420", 90, 0, False), (67, 45, 
          (640, 360, "420", 90, 16, False)]
 
 
-@pytest.mark.parametrize("case", CASES)
-def test_oracle_matches_reference_build(oracle, reference, case):
+def _sha(a):
+    return hashlib.sha256(a if isinstance(a, bytes) else a.tobytes()).hexdigest()
+
+
+def case_key(case):
+    return "%dx%d_%s_q%d_ri%d%s" % (case[0], case[1], case[2], case[3], case[4], "_opt" if case[5] else "")
+
+
+def case_jpeg(case):
     w, h, ss, q, ri, opt = case
-    data = synth.synth_jpeg(w, h, 500 + w + h, q, ss, ri, opt)
-    ok, info, rcoef, rbgra, _ = reference.decode(data, skip_gate=(ss == "422"))
+    return synth.synth_jpeg(w, h, 500 + w + h, q, ss, ri, opt)
+
+
+@pytest.mark.parametrize("case", CASES)
+def test_oracle_matches_reference_build(oracle, reference_digests, case):
+    want = reference_digests["oracle_cases"][case_key(case)]
+    data = case_jpeg(case)
+    assert _sha(data) == want["file_sha256"]
     rc, img, coef, bgra = oracle.decode(data, gate=1)
-    assert ok == (rc == 0)
-    if ok:
-        assert np.array_equal(coef, rcoef)
-        assert np.array_equal(bgra, rbgra)
+    assert want["ok"] == (rc == 0)
+    if want["ok"]:
+        assert _sha(coef) == want["coef_sha256"]
+        assert _sha(bgra) == want["pixel_sha256"]
 
 
-def test_oracle_reproduces_reference_rst_defect(oracle, reference):
+def rst_defect_jpegs():
+    return [synth.synth_jpeg(640, 480, 900 + i, 90, "420", 1) for i in range(24)]   # 1200 restart markers per image
+
+
+def test_oracle_reproduces_reference_rst_defect(oracle, reference_digests):
     """The reference drops an RSTn whose FF is the last byte of one of its 2 KiB reads and then
     aborts (decoder.cpp:118-131). strict mode predicts exactly those files; non-strict decodes them."""
+    want = reference_digests["rst_defect"]
+    files = rst_defect_jpegs()
+    assert len(files) == len(want)
     n_fail = 0
-    for i in range(24):
-        data = synth.synth_jpeg(640, 480, 900 + i, 90, "420", 1)   # 1200 restart markers per image
-        ok, _, rcoef, _, _ = reference.decode(data, want_pixels=False)
+    for data, w in zip(files, want):
+        assert _sha(data) == w["file_sha256"]
         oracle.set_strict(True)
         rc_s, _, coef_s, _ = oracle.decode(data, want_pixels=False)
         oracle.set_strict(False)
         rc_n, _, coef_n, _ = oracle.decode(data, want_pixels=False)
         oracle.set_strict(True)
-        assert ok == (rc_s == 0)
+        assert w["ok"] == (rc_s == 0)
         assert rc_n == 0
-        if ok:
-            assert np.array_equal(coef_s, rcoef) and np.array_equal(coef_n, rcoef)
+        if w["ok"]:
+            assert _sha(coef_s) == w["coef_sha256"] and _sha(coef_n) == w["coef_sha256"]
         else:
             n_fail += 1
     assert n_fail > 0   # with 1200 markers per image the defect shows up in this sample
 
 
-def test_crafted_streams_oracle_vs_reference(oracle, reference):
+def crafted_streams():
+    """[(jpeg, blocks, quantisers, blocks per MCU, luma blocks per MCU)] in a fixed order."""
     rng = np.random.RandomState(5)
-    zz = oracle.zigzag()
+    out = []
     for sampling, (w, h) in (((2, 2), (48, 32)), ((1, 1), (24, 16)), ((2, 1), (48, 16))):
         ny = sampling[0] * sampling[1]
         tot = ny + 2
@@ -118,15 +138,25 @@ def test_crafted_streams_oracle_vs_reference(oracle, reference):
         q = [[1 + (i % 7) for i in range(64)], [2 + (i % 5) for i in range(64)]]
         for ri, fill in ((0, 0), (1, 0), (2, 3)):
             data = jpegcraft.build_jpeg(w, h, sampling, blocks, q, restart_interval=ri, fill_before_rst=fill)
-            rc, img, coef, _ = oracle.decode(data, gate=1, want_pixels=False)
-            ok, _, rcoef, _, _ = reference.decode(data, skip_gate=True, want_pixels=False)
-            assert rc == 0 and ok
-            assert np.array_equal(coef, rcoef)
-            exp = np.zeros_like(coef)
-            for b in range(len(blocks)):
-                qq = np.array(q[0] if b % tot < ny else q[1])
-                exp[b, zz] = blocks[b] * qq
-            assert np.array_equal(coef, exp)
+            out.append((data, blocks, q, tot, ny))
+    return out
+
+
+def test_crafted_streams_oracle_vs_reference(oracle, reference_digests):
+    want = reference_digests["crafted"]
+    streams = crafted_streams()
+    assert len(streams) == len(want)
+    zz = oracle.zigzag()
+    for (data, blocks, q, tot, ny), w in zip(streams, want):
+        assert _sha(data) == w["file_sha256"]
+        rc, img, coef, _ = oracle.decode(data, gate=1, want_pixels=False)
+        assert rc == 0 and w["ok"]
+        assert _sha(coef) == w["coef_sha256"]
+        exp = np.zeros_like(coef)
+        for b in range(len(blocks)):
+            qq = np.array(q[0] if b % tot < ny else q[1])
+            exp[b, zz] = blocks[b] * qq
+        assert np.array_equal(coef, exp)
 
 
 def test_grayscale_extension_against_pillow(oracle):
@@ -172,25 +202,33 @@ def _random_blocks(n, seed):
     return blocks
 
 
-@pytest.mark.parametrize("samp", GENERIC_LAYOUTS, ids=lambda s: "%d%d" % s[0])
-def test_generic_luma_sampling_oracle_vs_reference(oracle, reference, samp):
-    """Luma h x v beyond the four everyday layouts (4:1:1 = 41, 14, 31, 42, ...) with 1x1 chroma: the reference's gate
-    refuses them, its CPU loops decode them as they are (decoder.cpp:429-495). Oracle (extended gate) against the
-    unmodified reference with the gate skipped: coefficients and pixels bit-exact, with and without restart markers."""
-    import jpegcraft
-    from oracle import GATE_EXTENDED
+def generic_luma_key(samp, ri):
+    return "%d%d_ri%d" % (samp[0] + (ri,))
+
+
+def generic_luma_jpeg(samp, ri):
     (h, v) = samp[0]
     w, hgt = 8 * h * 3 - 3, 8 * v * 2 - 1            # 3 x 2 MCUs, ragged right and bottom edges
     n = 6 * (h * v + 2)
+    return jpegcraft.build_jpeg(w, hgt, samp, _random_blocks(n, 7 * h + v + ri), [[2 + (i % 5) for i in range(64)], [3] * 64], restart_interval=ri)
+
+
+@pytest.mark.parametrize("samp", GENERIC_LAYOUTS, ids=lambda s: "%d%d" % s[0])
+def test_generic_luma_sampling_oracle_vs_reference(oracle, reference_digests, samp):
+    """Luma h x v beyond the four everyday layouts (4:1:1 = 41, 14, 31, 42, ...) with 1x1 chroma: the reference's gate
+    refuses them, its CPU loops decode them as they are (decoder.cpp:429-495). Oracle (extended gate) against the
+    unmodified reference with the gate skipped: coefficients and pixels bit-exact, with and without restart markers."""
+    from oracle import GATE_EXTENDED
     for ri in (0, 2):
-        data = jpegcraft.build_jpeg(w, hgt, samp, _random_blocks(n, 7 * h + v + ri), [[2 + (i % 5) for i in range(64)], [3] * 64], restart_interval=ri)
+        want = reference_digests["generic_luma"][generic_luma_key(samp, ri)]
+        data = generic_luma_jpeg(samp, ri)
+        assert _sha(data) == want["file_sha256"]
         assert oracle.parse(data, 0)[0] != 0         # the reference gate refuses it
         rc, img, coef, bgra = oracle.decode(data, gate=GATE_EXTENDED)
         assert rc == 0
-        ok, info, rcoef, rbgra, _ = reference.decode(data, skip_gate=True)
-        assert ok
-        assert np.array_equal(coef, rcoef)
-        assert np.array_equal(bgra, rbgra)
+        assert want["ok"]
+        assert _sha(coef) == want["coef_sha256"]
+        assert _sha(bgra) == want["pixel_sha256"]
 
 
 def test_multi_block_chroma_is_plain_replication(oracle):
