@@ -163,7 +163,15 @@ const char *b2j_last_error(void);
 
 /* Parse SOI .. SOS of a baseline JFIF file held in memory. Same accept/reject behaviour as
  * the reference's load_jpg() + is_supported_file() (gate = B2J_GATE_REFERENCE), or with
- * 4:2:2 / 4:4:0 admitted (B2J_GATE_EXTENDED). */
+ * 4:2:2 / 4:4:0 admitted (B2J_GATE_EXTENDED).
+ * Deviation, under every gate: B2J_E_UNSUPPORTED for a file whose Huffman tables need more than 12288 entries of
+ * two-level decode tables together (16 header entries, then per distinct table 64 (DC) or 1024 (AC) first-level entries
+ * plus 2^(L - 6) resp. 2^(L - 10) entries for every first-level prefix whose longest code has length L, each sub-table
+ * starting on a multiple of 8). The decode kernels keep them in 24 KB of shared memory. The Annex K tables need 2536
+ * entries; tables with at most the 12 DC and 162 AC symbols a baseline encoder uses need at most 11656 (the largest a
+ * search over code lengths finds, three components on distinct tables). Only tables of about 256 codes up to 16 bits
+ * long pass the limit, e.g. three DC and two AC tables of that kind. The reference decodes such files. The check is per
+ * file, so that such a file cannot make b2j_batch_create fail for the whole batch. */
 int b2j_parse_header(const uint8_t *file, size_t len, int gate, b2j_image_desc *out);
 
 /* ------------------------------------------------------------------ device -------------- */

@@ -151,6 +151,13 @@ struct TileDev
 // (code space overflow) or needs more than `max_entries` entries.
 bool build_huff_lut(const uint8_t counts[16], const uint8_t *symbols, bool is_dc, std::vector<uint16_t> &out, size_t max_entries);
 
+// Entries build_huff_lut() makes for this table (no limit applied).
+size_t huff_lut_entries(const uint8_t counts[16], bool is_dc);
+
+// Entries of the decode part of an image's LUT set (header + the decode tables of its distinct table slots), the
+// part that must fit kLutMaxDecode.
+size_t lut_set_decode_entries(const b2j_image_desc &d);
+
 // Canonical Huffman table -> walk table (1 << kWalkBits 32-bit entries as pairs of u16, format above).
 bool build_walk_lut(const uint8_t counts[16], const uint8_t *symbols, bool is_dc, std::vector<uint16_t> &out);
 

@@ -137,6 +137,10 @@ int check_gate(const b2j_image_desc &d, int gate)
         const int td = d.huff_id[c] >> 4, ta = d.huff_id[c] & 0xF;
         if (td > 3 || ta > 3 || !d.huff_present[td] || !d.huff_present[4 + ta]) return B2J_E_UNSUPPORTED;
     }
+    // the decode kernels hold an image's decode tables in shared memory: tables whose two-level decode tables do not
+    // fit together (three components with tables of 256 codes up to 16 bits long) are refused here, per file, rather
+    // than when the batch that holds the file is built (documented deviation, include/b2j.h)
+    if (b2j::lut_set_decode_entries(d) > (size_t)b2j::kLutMaxDecode) return B2J_E_UNSUPPORTED;
     if (d.color_space == B2J_CS_GRAY) return B2J_OK;   // admitted by parse_sof0 under B2J_GATE_GRAY only
     const int y = d.sampling[0];
     if (d.sampling[1] == 0x11 && d.sampling[2] == 0x11 && (y == 0x22 || y == 0x11)) return B2J_OK;   // decoder.cpp:58-69

@@ -88,6 +88,53 @@ bool build_huff_lut(const uint8_t counts[16], const uint8_t *symbols, bool is_dc
     return out.size() <= max_entries;
 }
 
+size_t huff_lut_entries(const uint8_t counts[16], bool is_dc)
+{
+    // what build_huff_lut() builds, counted: canonical codes come in increasing order, so the primary prefixes with long
+    // codes come in increasing order too, and the last code below a prefix is its longest
+    const int K = is_dc ? kLutBitsDc : kLutBits;
+    size_t rel = 0;
+    uint32_t code = 0, prefix = 0;
+    int longest = 0;
+    auto close = [&]() {
+        if (!longest) return;
+        while (rel % kLutSubAlign) rel++;
+        rel += (size_t)1 << (longest - K);
+    };
+    for (int l = 1; l <= 16; l++)
+    {
+        for (int i = 0; i < counts[l - 1]; i++, code++)
+        {
+            if (l <= K) continue;
+            const uint32_t p = code >> (l - K);
+            if (longest && p != prefix) close();
+            prefix = p;
+            longest = l;
+        }
+        code <<= 1;
+    }
+    close();
+    return ((size_t)1 << K) + rel;
+}
+
+size_t lut_set_decode_entries(const b2j_image_desc &d)
+{
+    // build_lut_set(): the header, then one decode table per distinct table slot, padded to 16 bytes
+    size_t n = kLutHeader;
+    bool seen[8] = {false, false, false, false, false, false, false, false};
+    for (int c = 0; c < 3; c++)
+        for (int kind = 0; kind < 2; kind++)
+        {
+            const int th = kind == 0 ? (d.huff_id[c] >> 4) : (d.huff_id[c] & 0xF);
+            if (th > 3) continue;
+            const int slot = kind * 4 + th;
+            if (seen[slot]) continue;
+            seen[slot] = true;
+            n += huff_lut_entries(d.huff_counts[slot], kind == 0);
+        }
+    return (n + 7) & ~(size_t)7;
+}
+
 bool build_walk_lut(const uint8_t counts[16], const uint8_t *symbols, bool is_dc, std::vector<uint16_t> &out)
 {
     const int K = is_dc ? kWalkBitsDc : kWalkBits;
