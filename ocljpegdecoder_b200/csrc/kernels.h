@@ -26,7 +26,6 @@ struct DecodeArgs
     // scratch
     uint8_t *clean;
     uint64_t *chunk_state;   // pre-pass: look-back words, zeroed before every decode
-    uint32_t *scan_ticket;   // pre-pass: one chunk-ticket counter per part (launch), zeroed with them
     uint32_t *clean_len, *seg_start;
     SubRec *recs;           // self-synchronising path: one record per sub-sequence
     uint4 *sync_cta_base;   // per chunk (= decode CTA) of the self-synchronising path: (blocks started, DC sums), then their prefix
@@ -38,25 +37,22 @@ struct DecodeArgs
     uint8_t *pixels;
     int32_t *status;
     // sizes
-    uint32_t n_images, n_chunks, n_huff_ctas, n_tiles, max_lut_len, max_lut_dec_len, max_lut_walk_len;   // LUT set lengths: whole / decode part / walk part
+    uint32_t n_images, n_chunks, n_huff_ctas, n_sync_ctas, n_sync_imgs, max_lut_len, max_lut_dec_len, max_lut_walk_len;   // LUT set lengths: whole / decode part / walk part
+    // tiles, sorted by kind: [0, gray_tile0) the four everyday colour layouts, [gray_tile0, generic_tile0) one-component
+    // images, [generic_tile0, n_tiles) every other layout (kModeGeneric)
+    uint32_t gray_tile0, generic_tile0, n_tiles;
     int out_format;          // B2J_OUT_*: layout of the pixel plane (b2j_batch_set_output_format)
-    bool use_tma;
     bool any_wide_q;         // some quantiser of the batch exceeds 255 (16-bit DQT): generic dequantisation
 };
-
-// A contiguous group of images of a batch: the unit the two-stream pipeline works on.
-// Tiles of a part, sorted by kind: [tile0, tile_mid) the four everyday colour layouts, [tile_mid, tile_gen) one-component images,
-// [tile_gen, tile1) every other layout (kModeGeneric).
-struct PartRange { uint32_t img0, img1, chunk0, chunk1, cta0, cta1, tile0, tile1, scta0, scta1, simg0, simg1, tile_mid, tile_gen; };
 
 cudaError_t init_constants();
 cudaError_t configure_kernels(uint32_t max_lut_len);
 size_t huff_smem_bytes(uint32_t max_lut_len);
-void launch_prepass(const DecodeArgs &a, const PartRange &r, uint32_t part, cudaStream_t s);   // 1 kernel
-void launch_huffman(const DecodeArgs &a, const PartRange &r, cudaStream_t s);   // 1 kernel
-void launch_huffman_sync(const DecodeArgs &a, const PartRange &r, cudaStream_t s);   // 4 kernels
+void launch_prepass(const DecodeArgs &a, cudaStream_t s);   // 1 kernel
+void launch_huffman(const DecodeArgs &a, cudaStream_t s);   // 1 kernel
+void launch_huffman_sync(const DecodeArgs &a, cudaStream_t s);   // 4 kernels
 constexpr int kSyncLaunches = 4;
-void launch_idct(const DecodeArgs &a, const PartRange &r, cudaStream_t s);      // 1 kernel
+void launch_idct(const DecodeArgs &a, cudaStream_t s);      // 1 kernel per tile kind present
 void launch_downscale(const uint8_t *pix, const ImgDev *imgs, const uint64_t *out_off, uint8_t *out, uint32_t n_images, uint32_t max_out_samples,
                       uint32_t factor, int fmt, cudaStream_t s);   // box-filter reduction of the pixel plane
 void launch_pack(const int32_t *in, int16_t *coef, size_t n_values, cudaStream_t s);   // int32 dequantised coefficients -> the int16 plane

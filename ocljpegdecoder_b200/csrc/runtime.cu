@@ -92,10 +92,8 @@ struct b2j_ctx
 {
     int device;
     cudaStream_t stream;
-    cudaStream_t stream2;   // the IDCT/colour stage of part p runs here while part p+1 is entropy-decoded
-    int n_parts;
+    cudaStream_t stream2;   // host feed: the downloads of a group run here while the next group decodes on `stream`
     PFN_cuTensorMapEncodeTiled_v12000 encode_tiled;
-    bool use_tma;
     int sm_count;
     Pool dev_pool{false};
     Pool pin_pool{true};
@@ -118,7 +116,7 @@ struct b2j_batch
 
     // scratch + outputs
     uint8_t *d_scratch; size_t d_scratch_cap;
-    size_t off_clean, off_clean_end, off_clean_len, off_seg_start, off_status, off_recs, off_pres, off_sync_stats, off_chunk_state, off_chunk_states, off_zero_end, off_ticket;
+    size_t off_clean, off_clean_end, off_clean_len, off_seg_start, off_status, off_recs, off_pres, off_sync_stats, off_chunk_state, off_chunk_states, off_zero_end;
     size_t scratch_bytes;
     int16_t *d_coef; size_t d_coef_cap; size_t coef_rows;
     uint8_t *d_pix; size_t d_pix_cap; size_t pix_bytes;
@@ -130,8 +128,6 @@ struct b2j_batch
     CUtensorMap tmap;
     DecodeArgs args;
     uint32_t n_segs_total;
-    std::vector<PartRange> parts;
-    std::vector<cudaEvent_t> ev_huff, ev_idct;   // per part: entropy decode done / pixels done
     bool uploaded;
     cudaStream_t last_stream;   // the stream the batch was last uploaded / decoded / read on
 };
@@ -141,7 +137,6 @@ namespace {
 int make_tensor_map(b2j_ctx *ctx, b2j_batch *b)
 {
     memset(&b->tmap, 0, sizeof(b->tmap));
-    if (!ctx->encode_tiled) return B2J_OK;
     // coefficient plane as a 2-D tensor [rows][64] of int16; box = one tile, 128-byte swizzle
     const cuuint64_t dims[2] = {64, (cuuint64_t)b->coef_rows};
     const cuuint64_t strides[1] = {128};
@@ -202,13 +197,6 @@ bool geometry_ok(const b2j_image_desc &d)
 }
 
 cudaStream_t pick_stream(b2j_batch *b, void *stream) { return b->last_stream = (stream ? (cudaStream_t)stream : b->ctx->stream); }
-
-void destroy_events(b2j_batch *b)
-{
-    for (auto &e : b->ev_huff) if (e) cudaEventDestroy(e);
-    for (auto &e : b->ev_idct) if (e) cudaEventDestroy(e);
-    b->ev_huff.clear(); b->ev_idct.clear();
-}
 
 void release_batch_buffers(b2j_batch *b)
 {
@@ -281,12 +269,6 @@ extern "C" int b2j_create(int device, b2j_ctx **out)
     ctx->sm_count = prop.multiProcessorCount;
     ctx->encode_tiled = nullptr;
     ctx->stream = ctx->stream2 = nullptr;
-    {
-        const char *pe = getenv("B2J_PARTS");
-        ctx->n_parts = pe ? atoi(pe) : 1;   // > 1 was measured slower on B200 (DESIGN.md): the entropy decoder is one wave
-        if (ctx->n_parts < 1) ctx->n_parts = 1;
-        if (ctx->n_parts > 16) ctx->n_parts = 16;
-    }
     cudaError_t ce = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking);
     if (ce == cudaSuccess) ce = cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking);
     if (ce == cudaSuccess) ce = init_constants();
@@ -306,15 +288,13 @@ extern "C" int b2j_create(int device, b2j_ctx **out)
         cudaGetLastError();
     if (!ctx->encode_tiled)
     {
-        // every colour kernel but the BGRA measurement variant loads its tile through a tensor map
+        // the colour kernel loads its tiles through a tensor map
         cudaStreamDestroy(ctx->stream);
         cudaStreamDestroy(ctx->stream2);
         delete ctx;
         t_last_error = "the driver does not export cuTensorMapEncodeTiled (needed for the TMA tile loads)";
         return B2J_E_CUDA;
     }
-    const char *env = getenv("B2J_USE_TMA");
-    ctx->use_tma = !(env && env[0] == '0');
     *out = ctx;
     return B2J_OK;
 }
@@ -362,11 +342,9 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     b->last_stream = nullptr;
 
     std::vector<uint32_t> chunk_img;
-    std::vector<uint32_t> img_cta0((size_t)n + 1), img_tile0((size_t)n + 1), img_chunk0((size_t)n + 1);
     std::vector<HuffCtaDev> ctas;    // restart-interval path
     std::vector<HuffCtaDev> sctas;   // self-synchronising path (no DRI)
     std::vector<uint32_t> simgs;
-    std::vector<uint32_t> img_scta0((size_t)n + 1), img_simg0((size_t)n + 1);
     uint32_t sub_total = 0;
     std::vector<TileDev> tiles;
     std::vector<uint16_t> luts;
@@ -389,8 +367,6 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
         if (coef_only) { if (!geometry_ok(d)) { rc = B2J_E_ARG; break; } }
         else if (d.scan_offset > lens[i] || d.scan_size > lens[i] - d.scan_offset || d.scan_size == 0 || d.scan_size >= 0x1FFFFFFFull || !geometry_ok(d))
         { rc = d.scan_size == 0 && d.scan_offset <= lens[i] ? B2J_E_DATA : B2J_E_ARG; break; }
-        img_cta0[(size_t)i] = (uint32_t)ctas.size(); img_tile0[(size_t)i] = (uint32_t)tiles.size(); img_chunk0[(size_t)i] = (uint32_t)chunk_img.size();
-        img_scta0[(size_t)i] = (uint32_t)sctas.size(); img_simg0[(size_t)i] = (uint32_t)simgs.size();
         im.raw_off = raw_total;
         im.raw_len = coef_only ? 0u : (uint32_t)d.scan_size;
         raw_total += align_up((size_t)im.raw_len + 32, 16);
@@ -483,40 +459,9 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     }
     if (rc != B2J_OK) { delete b; return rc; }
     if (blk_total + kTileBlocks >= 0xFFFFFFF0ull) { delete b; return B2J_E_ARG; }
-    img_cta0[(size_t)n] = (uint32_t)ctas.size(); img_tile0[(size_t)n] = (uint32_t)tiles.size(); img_chunk0[(size_t)n] = (uint32_t)chunk_img.size();
-    img_scta0[(size_t)n] = (uint32_t)sctas.size(); img_simg0[(size_t)n] = (uint32_t)simgs.size();
-    {
-        // contiguous groups of images with similar block counts: the units of the two-stream pipeline
-        const int np = ctx->n_parts < n ? ctx->n_parts : n;
-        int i0 = 0;
-        for (int p = 0; p < np; p++)
-        {
-            int i1 = i0;
-            const size_t target = blk_total * (size_t)(p + 1) / (size_t)np;
-            while (i1 < n && (i1 == i0 || (size_t)b->imgs[(size_t)i1].blk_first + b->imgs[(size_t)i1].blk_count <= target) && n - i1 > np - p - 1) i1++;
-            if (p == np - 1) i1 = n;
-            b->parts.push_back({(uint32_t)i0, (uint32_t)i1, img_chunk0[(size_t)i0], img_chunk0[(size_t)i1], img_cta0[(size_t)i0], img_cta0[(size_t)i1],
-                                img_tile0[(size_t)i0], img_tile0[(size_t)i1], img_scta0[(size_t)i0], img_scta0[(size_t)i1],
-                                img_simg0[(size_t)i0], img_simg0[(size_t)i1], 0u, 0u});
-            // the tiles of one-component images go behind the others: they have a kernel of their own
-            PartRange &pr = b->parts.back();
-            auto mid = std::stable_partition(tiles.begin() + pr.tile0, tiles.begin() + pr.tile1,
-                                             [](const TileDev &t) { return (t.info & 0xFFu) < kModeGray; });
-            auto gen = std::stable_partition(mid, tiles.begin() + pr.tile1, [](const TileDev &t) { return (t.info & 0xFFu) == kModeGray; });
-            pr.tile_mid = (uint32_t)(mid - tiles.begin());
-            pr.tile_gen = (uint32_t)(gen - tiles.begin());
-            i0 = i1;
-        }
-        b->ev_huff.resize(b->parts.size());
-        b->ev_idct.resize(b->parts.size());
-        for (size_t p = 0; p < b->parts.size(); p++) b->ev_huff[p] = b->ev_idct[p] = nullptr;
-        for (size_t p = 0; p < b->parts.size(); p++)
-        {
-            cudaError_t e = cudaEventCreateWithFlags(&b->ev_huff[p], cudaEventDisableTiming);
-            if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->ev_idct[p], cudaEventDisableTiming);
-            if (e != cudaSuccess) { destroy_events(b); delete b; return fail_cuda(e, "cudaEventCreateWithFlags"); }
-        }
-    }
+    // tiles sorted by kind, each kind a kernel of its own: the four everyday colour layouts, one-component images, the rest
+    const auto gray0 = std::stable_partition(tiles.begin(), tiles.end(), [](const TileDev &t) { return (t.info & 0xFFu) < kModeGray; });
+    const auto generic0 = std::stable_partition(gray0, tiles.end(), [](const TileDev &t) { return (t.info & 0xFFu) == kModeGray; });
 
     // ---- input blob layout
     size_t off = 0;
@@ -545,7 +490,6 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     b->off_status = place(4 * (size_t)n);
     b->off_sync_stats = place(4 * 8);
     b->off_chunk_state = place(8 * chunk_img.size());
-    b->off_ticket = place(4 * 16);   // one counter per part (at most 16)
     b->off_zero_end = off;
     b->scratch_bytes = off;
     b->n_segs_total = seg_total;
@@ -565,7 +509,7 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
             cudaGetLastError();
         }
     }
-    if (rc != B2J_OK) { destroy_events(b); release_batch_buffers(b); delete b; return rc == B2J_E_CUDA ? B2J_E_NOMEM : rc; }
+    if (rc != B2J_OK) { release_batch_buffers(b); delete b; return rc == B2J_E_CUDA ? B2J_E_NOMEM : rc; }
 
     // ---- fill the pinned blob
     memcpy(b->h_blob + b->off_imgs, b->imgs.data(), sizeof(ImgDev) * (size_t)n);
@@ -587,7 +531,7 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     }
 
     rc = make_tensor_map(ctx, b);
-    if (rc != B2J_OK) { destroy_events(b); release_batch_buffers(b); delete b; return rc; }
+    if (rc != B2J_OK) { release_batch_buffers(b); delete b; return rc; }
 
     DecodeArgs &a = b->args;
     a.raw = b->d_blob + b->off_raw;
@@ -606,7 +550,6 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     a.tmap = &b->tmap;
     a.clean = b->d_scratch + b->off_clean;
     a.chunk_state = reinterpret_cast<uint64_t *>(b->d_scratch + b->off_chunk_state);
-    a.scan_ticket = reinterpret_cast<uint32_t *>(b->d_scratch + b->off_ticket);
     a.clean_len = reinterpret_cast<uint32_t *>(b->d_scratch + b->off_clean_len);
     a.seg_start = reinterpret_cast<uint32_t *>(b->d_scratch + b->off_seg_start);
     a.status = reinterpret_cast<int32_t *>(b->d_scratch + b->off_status);
@@ -615,11 +558,14 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     a.n_images = (uint32_t)n;
     a.n_chunks = (uint32_t)chunk_img.size();
     a.n_huff_ctas = (uint32_t)ctas.size();
+    a.n_sync_ctas = (uint32_t)sctas.size();
+    a.n_sync_imgs = (uint32_t)simgs.size();
+    a.gray_tile0 = (uint32_t)(gray0 - tiles.begin());
+    a.generic_tile0 = (uint32_t)(generic0 - tiles.begin());
     a.n_tiles = (uint32_t)tiles.size();
     a.max_lut_len = max_lut_len;
     a.max_lut_dec_len = max_lut_dec_len;
     a.max_lut_walk_len = max_lut_walk_len;
-    a.use_tma = ctx->use_tma;
     a.out_format = B2J_OUT_BGRA;
     a.any_wide_q = false;
     for (const ImgDev &im : b->imgs) a.any_wide_q = a.any_wide_q || im.wide_q != 0;
@@ -631,9 +577,8 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     b2j_batch_info &inf = b->info;
     memset(&inf, 0, sizeof(inf));
     inf.n_images = n;
-    int idct_launches = 0;
-    for (const PartRange &pr : b->parts) idct_launches += (pr.tile_mid > pr.tile0 ? 1 : 0) + (pr.tile_gen > pr.tile_mid ? 1 : 0) + (pr.tile1 > pr.tile_gen ? 1 : 0);
-    inf.kernel_launches = idct_launches + (int32_t)b->parts.size() * (1 + (ctas.empty() ? 0 : 1) + (sctas.empty() ? 0 : kSyncLaunches));
+    const int idct_launches = (a.gray_tile0 > 0 ? 1 : 0) + (a.generic_tile0 > a.gray_tile0 ? 1 : 0) + (a.n_tiles > a.generic_tile0 ? 1 : 0);
+    inf.kernel_launches = idct_launches + 1 + (ctas.empty() ? 0 : 1) + (sctas.empty() ? 0 : kSyncLaunches);
     inf.total_pixels = pixels;
     inf.total_blocks = (int64_t)blk_total;
     inf.scan_bytes = scan_bytes;
@@ -651,10 +596,8 @@ extern "C" void b2j_batch_destroy(b2j_batch *b)
     if (!b) return;
     cudaSetDevice(b->ctx->device);
     // the buffers go back to the pool: nothing enqueued on them may still be in flight, including work on a caller's stream
-    if (b->last_stream && b->last_stream != b->ctx->stream && b->last_stream != b->ctx->stream2) cudaStreamSynchronize(b->last_stream);
+    if (b->last_stream && b->last_stream != b->ctx->stream) cudaStreamSynchronize(b->last_stream);
     cudaStreamSynchronize(b->ctx->stream);
-    cudaStreamSynchronize(b->ctx->stream2);
-    destroy_events(b);
     release_batch_buffers(b);
     delete b;
 }
@@ -682,67 +625,37 @@ extern "C" int b2j_batch_upload(b2j_batch *b, void *stream)
     return B2J_OK;
 }
 
-// Events of one timed step: [0] start, [1] end, then 5 per part: before pre-pass, after pre-pass, after
-// Huffman (stream 1), before IDCT, after IDCT (stream 2).
-static size_t events_per_step(const b2j_batch *b) { return 2 + 5 * b->parts.size(); }
+// Events of one timed step: start (before the memsets), before the pre-pass, after it, after the entropy stage,
+// after the IDCT/colour stage (= end of the step).
+constexpr size_t kStepEvents = 5;
 
-// One decode of the whole batch. The batch is split into parts; part p's IDCT/colour kernel runs on the
-// context's second stream while part p+1 is still in the pre-pass / entropy decoder on `s`: the two
-// stages stress different resources (shared-memory LUT gathers vs. ALU + HBM) and overlap well.
-// On return everything is ordered behind `s` again.
-static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* events_per_step() or NULL */)
+// One decode of the whole batch: the pre-pass, the entropy stage and the IDCT/colour stage, in order on `s`.
+static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStepEvents or NULL */)
 {
     if (!b->uploaded) { t_last_error = "b2j_batch_decode before b2j_batch_upload"; return B2J_E_ARG; }
     const DecodeArgs &a = b->args;
-    cudaStream_t s2 = b->ctx->stream2;
     if (ev) CU_TRY(cudaEventRecord(ev[0], s));
     if (a.n_huff_ctas) CU_TRY(cudaMemsetAsync(a.seg_start, 0xFF, 4 * (size_t)b->n_segs_total, s));   // read by the restart-interval decoder only
     CU_TRY(cudaMemsetAsync(b->d_scratch + b->off_status, 0, b->off_zero_end - b->off_status, s));   // status words, sync stats, look-back words
-    const size_t np = b->parts.size();
-    for (size_t p = 0; p < np; p++)
-    {
-        const PartRange &r = b->parts[p];
-        cudaEvent_t *pe = ev ? ev + 2 + 5 * p : nullptr;
-        if (pe) CU_TRY(cudaEventRecord(pe[0], s));
-        launch_prepass(a, r, (uint32_t)p, s);
-        if (pe) CU_TRY(cudaEventRecord(pe[1], s));
-        launch_huffman(a, r, s);
-        launch_huffman_sync(a, r, s);
-        if (pe) CU_TRY(cudaEventRecord(pe[2], s));
-        if (np == 1)
-        {
-            if (pe) CU_TRY(cudaEventRecord(pe[3], s));
-            launch_idct(a, r, s);
-            if (pe) CU_TRY(cudaEventRecord(pe[4], s));
-        }
-        else
-        {
-            CU_TRY(cudaEventRecord(b->ev_huff[p], s));
-            CU_TRY(cudaStreamWaitEvent(s2, b->ev_huff[p], 0));
-            if (pe) CU_TRY(cudaEventRecord(pe[3], s2));
-            launch_idct(a, r, s2);
-            if (pe) CU_TRY(cudaEventRecord(pe[4], s2));
-            CU_TRY(cudaEventRecord(b->ev_idct[p], s2));
-        }
-    }
-    if (np > 1) CU_TRY(cudaStreamWaitEvent(s, b->ev_idct[np - 1], 0));   // stream 2 is in order: the last part covers all
     if (ev) CU_TRY(cudaEventRecord(ev[1], s));
+    launch_prepass(a, s);
+    if (ev) CU_TRY(cudaEventRecord(ev[2], s));
+    launch_huffman(a, s);
+    launch_huffman_sync(a, s);
+    if (ev) CU_TRY(cudaEventRecord(ev[3], s));
+    launch_idct(a, s);
+    if (ev) CU_TRY(cudaEventRecord(ev[4], s));
     CU_TRY(cudaGetLastError());
     return B2J_OK;
 }
 
-static void collect_times(const b2j_batch *b, cudaEvent_t *ev, b2j_stage_times *t)
+static void collect_times(cudaEvent_t *ev, b2j_stage_times *t)
 {
     t->prepass_ms = t->huffman_ms = t->idct_ms = 0.f;
-    for (size_t p = 0; p < b->parts.size(); p++)
-    {
-        cudaEvent_t *pe = ev + 2 + 5 * p;
-        float x = 0.f;
-        cudaEventElapsedTime(&x, pe[0], pe[1]); t->prepass_ms += x;
-        cudaEventElapsedTime(&x, pe[1], pe[2]); t->huffman_ms += x;
-        cudaEventElapsedTime(&x, pe[3], pe[4]); t->idct_ms += x;
-    }
-    cudaEventElapsedTime(&t->total_ms, ev[0], ev[1]);
+    cudaEventElapsedTime(&t->prepass_ms, ev[1], ev[2]);
+    cudaEventElapsedTime(&t->huffman_ms, ev[2], ev[3]);
+    cudaEventElapsedTime(&t->idct_ms, ev[3], ev[4]);
+    cudaEventElapsedTime(&t->total_ms, ev[0], ev[4]);
 }
 
 extern "C" int b2j_batch_decode(b2j_batch *b, void *stream)
@@ -762,7 +675,7 @@ extern "C" int b2j_batch_decode_steps(b2j_batch *b, void *stream, int steps, b2j
     if (!b || steps <= 0) return B2J_E_ARG;
     CU_TRY(cudaSetDevice(b->ctx->device));
     cudaStream_t s = pick_stream(b, stream);
-    const size_t per = events_per_step(b);
+    const size_t per = kStepEvents;
     std::vector<cudaEvent_t> ev((size_t)steps * per, nullptr);
     int rc = B2J_OK;
     for (auto &e : ev)
@@ -778,8 +691,8 @@ extern "C" int b2j_batch_decode_steps(b2j_batch *b, void *stream, int steps, b2j
     }
     if (rc == B2J_OK)
     {
-        for (int k = 0; k < steps && per_step; k++) collect_times(b, &ev[(size_t)k * per], &per_step[k]);
-        if (total_ms) cudaEventElapsedTime(total_ms, ev[0], ev[(size_t)(steps - 1) * per + 1]);
+        for (int k = 0; k < steps && per_step; k++) collect_times(&ev[(size_t)k * per], &per_step[k]);
+        if (total_ms) cudaEventElapsedTime(total_ms, ev[0], ev[(size_t)steps * per - 1]);
     }
     for (auto &e : ev) if (e) cudaEventDestroy(e);
     return rc;
@@ -976,7 +889,6 @@ namespace {
 // Buffers back to the pools without a stream synchronisation: the caller has seen the event that closes the batch's work.
 void destroy_batch_done(b2j_batch *b)
 {
-    destroy_events(b);
     release_batch_buffers(b);
     delete b;
 }
@@ -1387,7 +1299,7 @@ extern "C" int b2j_idct_run(b2j_idct *p)
     CU_TRY(cudaSetDevice(b->ctx->device));
     cudaStream_t s = pick_stream(b, nullptr);
     CU_TRY(cudaMemsetAsync(b->args.status, 0, 4, s));
-    launch_idct(b->args, b->parts[0], s);
+    launch_idct(b->args, s);
     CU_TRY(cudaGetLastError());
     CU_TRY(cudaStreamSynchronize(s));
     return B2J_OK;

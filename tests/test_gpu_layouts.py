@@ -1,6 +1,6 @@
-"""GPU: generic sampling layouts, per-component tables, long Huffman codes, the kernel-choice knobs and the largest decode
-tables, against the oracle (extended gate, non-strict) and against the blocks the streams were written from
-(tests/test_layout_streams.py). Coefficients bit-exact, pixels exact, status clean."""
+"""GPU: generic sampling layouts, per-component tables, long Huffman codes and the largest decode tables, against the
+oracle (extended gate, non-strict) and against the blocks the streams were written from (tests/test_layout_streams.py).
+Coefficients bit-exact, pixels exact, status clean."""
 import hashlib
 import io
 import os
@@ -118,32 +118,6 @@ def test_generic_layouts_other_output_formats(mixed_default):
             assert np.array_equal(batch.pixels(i), np.moveaxis(b[..., 2::-1], 2, 0)), MIXED[i][0]
     finally:
         batch.set_output_format(b2j.OUT_BGRA)
-
-
-@pytest.mark.parametrize("env", [("B2J_PARTS", "2"), ("B2J_PARTS", "3"), ("B2J_USE_TMA", "0")], ids=lambda e: "%s=%s" % e)
-def test_kernel_choice_knobs_give_identical_output(mixed_default, env):
-    """The per-part tile partition (three tile kinds per part, per-part sync offsets) and the plain-load colour kernel:
-    the variables are read when the decoder is created."""
-    import ocljpegdecoder_b200 as b2j
-    _, st0, c0, p0 = mixed_default
-    old = os.environ.get(env[0])
-    os.environ[env[0]] = env[1]
-    try:
-        dec = b2j.Decoder(0)
-    finally:
-        if old is None:
-            del os.environ[env[0]]
-        else:
-            os.environ[env[0]] = old
-    try:
-        batch, st, coefs, pix = _decode(dec, [m[1] for m in MIXED], gray=True)
-        batch.close()
-    finally:
-        dec.close()
-    assert np.array_equal(st, st0)
-    for i in range(len(MIXED)):
-        assert np.array_equal(coefs[i], c0[i]), MIXED[i][0]
-        assert np.array_equal(pix[i], p0[i]), MIXED[i][0]
 
 
 @pytest.mark.parametrize("luma", [(4, 1), (1, 4), (3, 1), (4, 2), (2, 4)], ids=lambda s: "%d%d" % s)
