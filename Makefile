@@ -48,12 +48,3 @@ clean:
 	$(MAKE) -s -C oracle clean
 
 .PHONY: all oracle clean mathcheck
-
-# measurement variants: make variant NAME=x DEFS="-DB2J_...=..." -> build/var_x/libb2j.so (load with B2J_LIBRARY=...)
-variant:
-	@mkdir -p build/var_$(NAME)
-	$(NVCC) $(NVFLAGS) $(DEFS) -c $(CSRC)/kernels.cu -o build/var_$(NAME)/kernels.o 2> build/var_$(NAME)/kernels.ptxas.log
-	$(NVCC) $(NVFLAGS) $(DEFS) -c $(CSRC)/runtime.cu -o build/var_$(NAME)/runtime.o 2> build/var_$(NAME)/runtime.ptxas.log
-	$(CXX) -O2 -std=c++17 -fPIC $(DEFS) -c $(CSRC)/huff_lut.cpp -o build/var_$(NAME)/huff_lut.o
-	$(CXX) -O2 -std=c++17 -fPIC $(DEFS) -c $(CSRC)/host_parse.cpp -o build/var_$(NAME)/host_parse.o
-	$(NVCC) $(ARCH) -shared -o build/var_$(NAME)/libb2j.so build/var_$(NAME)/kernels.o build/var_$(NAME)/runtime.o build/var_$(NAME)/host_parse.o build/var_$(NAME)/huff_lut.o

@@ -11,26 +11,14 @@
 namespace b2j {
 
 // ---------------------------------------------------------------- constants ------------
-#ifndef B2J_SCAN_GROUPS
-#define B2J_SCAN_GROUPS 4
-#endif
-constexpr int kScanGroups = B2J_SCAN_GROUPS;           // 16-byte groups per thread in the pre-pass (4 loads in flight per thread)
+constexpr int kScanGroups = 4;           // 16-byte groups per thread in the pre-pass (4 loads in flight per thread)
 constexpr int kScanThreads = 256;
 constexpr int kScanChunkBytes = kScanThreads * kScanGroups * 16;   // bytes of raw scan one CTA of the pre-pass handles
 constexpr int kHuffThreads = 128;        // decode lanes (= segments) per Huffman CTA
-#ifndef B2J_SUB_BYTES
-#define B2J_SUB_BYTES 128
-#endif
-constexpr int kSubBytes = B2J_SUB_BYTES; // self-synchronising decode: bytes of clean stream per sub-sequence (one lane each); 64 and 32 were measured slower (DESIGN.md)
-#ifndef B2J_SYNC_PRE_LANES
-#define B2J_SYNC_PRE_LANES 2
-#endif
-constexpr int kSyncPre = B2J_SYNC_PRE_LANES;   // chunk-wise synchronisation (b2j_sync.h): sub-sequences walked in front of a chunk
+constexpr int kSubBytes = 128;           // self-synchronising decode: bytes of clean stream per sub-sequence (one lane each); 64 and 32 were measured slower (DESIGN.md)
+constexpr int kSyncPre = 2;              // chunk-wise synchronisation (b2j_sync.h): sub-sequences walked in front of a chunk
 constexpr int kSyncLanes = kHuffThreads - kSyncPre;   // output sub-sequences per chunk
-#ifndef B2J_LUT_BITS
-#define B2J_LUT_BITS 10
-#endif
-constexpr int kLutBits = B2J_LUT_BITS;   // primary Huffman LUT width, AC tables (one lookup per coefficient)
+constexpr int kLutBits = 10;             // primary Huffman LUT width, AC tables (one lookup per coefficient)
 constexpr int kLutBitsDc = 6;            // DC tables (one lookup per block): small, the shared memory goes to the stream rings
 constexpr int kLutHeader = 16;           // u16 words of header in front of a LUT set:
                                          //   [0..2] DC table of component c, [3..5] AC table (decode tables, entry format below)
@@ -38,14 +26,8 @@ constexpr int kLutHeader = 16;           // u16 words of header in front of a LU
                                          //   [12]   length of the decode part of the set (header + decode tables), a multiple of 8
 constexpr int kLutMaxDecode = 12288;     // u16 entries of the decode part of a LUT set (24 KB of shared memory)
 constexpr int kLutMaxEntries = 32768;    // u16 entries of a whole LUT set, walk tables included (64 KB)
-#ifndef B2J_WALK_BITS
-#define B2J_WALK_BITS 10
-#endif
-constexpr int kWalkBits = B2J_WALK_BITS; // index width of the AC walk tables (several AC symbols per lookup)
-#ifndef B2J_WALK_BITS_DC
-#define B2J_WALK_BITS_DC 8
-#endif
-constexpr int kWalkBitsDc = B2J_WALK_BITS_DC;   // index width of the DC walk tables: small, shared memory decides how many CTAs an SM holds
+constexpr int kWalkBits = 10;            // index width of the AC walk tables (several AC symbols per lookup)
+constexpr int kWalkBitsDc = 8;           // index width of the DC walk tables: small, shared memory decides how many CTAs an SM holds
 constexpr int kTileBlocks = 192;         // 8x8 blocks per IDCT/colour tile (= threads per CTA)
 constexpr uint32_t kSegInvalid = 0xFFFFFFFFu;
 constexpr uint32_t kChunkDead = 0xFFFFFFFFu;

@@ -42,7 +42,7 @@ cudaError_t init_constants()
 }
 
 // =====================================================================================
-// Pre-pass: byte classification shared by the count and the write kernel.
+// Pre-pass: byte classification.
 // For byte b with predecessor p and successor n (all inside one image's scan):
 //   b == FF : kept iff n == 00 (stuffed data byte). Otherwise it is a marker prefix / fill byte
 //             and is dropped; if n is none of 00, FF, D0..D7 the scan ends here (EOI or any
@@ -184,9 +184,7 @@ __device__ __forceinline__ uint32_t local_limit(uint32_t chunk_term, uint32_t ti
 // CHUNK-LOCAL offsets (which need no base), warp 0 probes its predecessors half-way through its squeezing and
 // evaluates the probe afterwards; only the copy-out (shifted to the alignment of the global destination)
 // and the restart-interval table wait for the base.
-#ifndef B2J_PROBE_AT
-#define B2J_PROBE_AT (kScanGroups - 1)   // the 16-byte group in front of whose squeeze warp 0 sends its look-back probe
-#endif
+constexpr int kProbeAt = kScanGroups - 1;   // the 16-byte group in front of whose squeeze warp 0 sends its look-back probe
 constexpr uint64_t kStAgg = 1ull << 62, kStIncl = 2ull << 62, kStTerm = 1ull << 61;
 __device__ __forceinline__ uint64_t st_pack(uint64_t flag, uint32_t keep, uint32_t mark, bool term)
 {
@@ -282,10 +280,8 @@ __device__ __forceinline__ void mark_group(const uint32_t w[4], const ScanFlags 
     }
 }
 
-#ifndef B2J_SCAN_MIN_CTAS
-#define B2J_SCAN_MIN_CTAS 4   // 64 registers (92 B of spills), 4 CTAs per SM: 0.162 vs 0.164 ms (256 x 1080p), 0.459 vs 0.474 ms (64 x 4K)
-#endif
-__global__ void __launch_bounds__(kScanThreads, B2J_SCAN_MIN_CTAS)
+constexpr int kScanMinCtas = 4;   // 64 registers (92 B of spills), 4 CTAs per SM: 0.162 vs 0.164 ms (256 x 1080p), 0.459 vs 0.474 ms (64 x 4K)
+__global__ void __launch_bounds__(kScanThreads, kScanMinCtas)
 k_unstuff_fused(const uint8_t *__restrict__ raw, uint8_t *__restrict__ clean, const ImgDev *__restrict__ imgs,
                 const uint32_t *__restrict__ chunk_img, uint64_t *__restrict__ chunk_state, uint32_t *__restrict__ clean_len,
                 uint32_t *__restrict__ seg_start, int32_t *__restrict__ status)
@@ -358,7 +354,7 @@ k_unstuff_fused(const uint8_t *__restrict__ raw, uint8_t *__restrict__ clean, co
         {
             // the probe leaves late in the squeeze (measured: before group 1 / 2 / 3 of 4: 0.167 / 0.164 / 0.162 ms): the neighbouring chunks, which started together with this one,
             // have published their aggregates by then, and the answer is back when the squeeze is finished
-            if (g == B2J_PROBE_AT && warp == 0 && k != 0 && lane < k) probe = st_load(probe_p);
+            if (g == kProbeAt && warp == 0 && k != 0 && lane < k) probe = st_load(probe_p);
             squeeze_group(s_out, lo, st.w[g], st.f[g], nkeep[g]);
             lo += nkeep[g];
         }
@@ -469,7 +465,6 @@ struct BitReader
     uint32_t cur, nxt;     // big-endian words: `cur` holds the bit at `bitpos`
     uint32_t raw[DEPTH];   // look-ahead, memory byte order; raw[0] enters the window next
     uint32_t bitpos;       // 0..31 after refill()
-    uint32_t nref;         // words shifted into the window since init()
     uint32_t wi;           // index (from wbase) of the next word to fetch: a fixed per-lane base and a 32-bit index
     const uint32_t *wbase; // cost one IMAD.WIDE per fetch; a moving 64-bit pointer costs two more instructions
 
@@ -483,11 +478,8 @@ struct BitReader
         for (int k = 0; k < DEPTH; k++) raw[k] = __ldg(wbase + 2 + k);
         wi = 2 + DEPTH;
         bitpos = (off & 3u) * 8u;
-        nref = 0u;
     }
-    // words shifted into the window since init(): nref, or the same number from the fetch index for loops
-    // that never read nref (its updates are then dead code)
-    __device__ __forceinline__ uint32_t words_consumed() const { return nref; }
+    // words shifted into the window since init()
     __device__ __forceinline__ uint32_t words_fetched() const { return wi - (2u + DEPTH); }
     __device__ __forceinline__ uint32_t peek() const { return __funnelshift_l(nxt, cur, bitpos); }
     __device__ __forceinline__ void refill()
@@ -500,7 +492,6 @@ struct BitReader
             for (int k = 0; k + 1 < DEPTH; k++) raw[k] = raw[k + 1];
             raw[DEPTH - 1] = __ldg(wbase + wi);
             wi++;
-            nref++;
             bitpos -= 32u;
         }
     }
@@ -985,10 +976,8 @@ k_sync_sweep(const uint8_t *__restrict__ clean, const ImgDev *__restrict__ imgs,
              uint4 *chunk_state, uint4 *cta_tot, uint32_t *__restrict__ stats)
 {
     extern __shared__ __align__(16) uint8_t smem[];
-    __shared__ uint4 s_wtot[kHuffThreads / 32];
     __shared__ __align__(16) WalkCtab s_ctab[16];
     __shared__ uint32_t s_min;
-    SyncShared &sh = *reinterpret_cast<SyncShared *>(smem);
     uint16_t *s_lut = reinterpret_cast<uint16_t *>(smem + kSyncSharedBytes);
     const uint32_t tid = threadIdx.x;
     const uint32_t img = sync_imgs[blockIdx.x];
@@ -1081,15 +1070,13 @@ k_sync_cta_scan(const ImgDev *__restrict__ imgs, const uint32_t *__restrict__ sy
 
 // =====================================================================================
 // IDCT + upsample + colour.
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
 __device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count)
 {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr(bar)), "r"(count));
 }
 __device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes)
 {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(bar)), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ bool mbar_try_wait(uint64_t *bar, uint32_t parity)
 {
@@ -1098,14 +1085,14 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t *bar, uint32_t parity)
         "{\n\t.reg .pred p;\n\t"
         "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
         "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
+        : "=r"(ok) : "r"(smem_addr(bar)), "r"(parity) : "memory");
     return ok != 0;
 }
 __device__ __forceinline__ void tma_load_2d(void *dst, const CUtensorMap *map, int x, int y, uint64_t *bar)
 {
     asm volatile(
         "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(x), "r"(y), "r"(smem_u32(bar)) : "memory");
+        ::"r"(smem_addr(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(x), "r"(y), "r"(smem_addr(bar)) : "memory");
 }
 
 // Packed clamp(a + b, 0, 255) on two int16 lanes.
@@ -1140,8 +1127,8 @@ struct TileGeom
 constexpr uint32_t kQtStride = 68;       // words between the per-component quantiser tables: 64 + 4, so that
                                          // the three tables start in different 16-byte bank groups
 
-// What the transform and the colour phase need to know about a tile, staged in shared memory one
-// iteration ahead (persistent kernel) so that no global load sits between two tiles.
+// What the transform and the colour phase need to know about a tile, staged in shared memory while the
+// tile's coefficients arrive.
 struct TileSide
 {
     alignas(16) uint32_t qt[3 * kQtStride];   // quantisers, natural order, widened to 32 bit
@@ -1156,9 +1143,9 @@ struct TileSmem
 {
     // coefficient tile: kTileBlocks rows of 128 B each; the 16-byte chunk c of row r sits at chunk
     // c ^ (r & 7) (the TMA SWIZZLE_128B pattern)
-    alignas(1024) uint8_t tile[1][kTileBlocks * 128];
-    TileSide side[1];
-    alignas(8) uint64_t bar[1];
+    alignas(1024) uint8_t tile[kTileBlocks * 128];
+    TileSide side;
+    alignas(8) uint64_t bar;
 };
 
 // Chroma offsets of one pixel pair, packed as two int16: the pair shares one sample when RH == 2.
@@ -1506,7 +1493,7 @@ __device__ __forceinline__ void csc_generic(const uint8_t *__restrict__ s_tile, 
     const uint32_t width = sd.width, height = sd.height;
     const bool vec_ok = (width & 3u) == 0u;
     constexpr uint32_t bpp = FMT == B2J_OUT_BGRA ? 4u : (FMT == B2J_OUT_RGB24 ? 3u : 1u);
-    const size_t pitch = (size_t)width * bpp, plane = (size_t)width * height;
+    const size_t plane = (size_t)width * height;
     for (uint32_t it = tid; it < sd.n_mcus * items; it += kTileBlocks)
     {
         const uint32_t m = it / items, r = it % items, y = r / xg, x = (r % xg) * 4u;
@@ -1552,66 +1539,54 @@ __device__ __forceinline__ void csc_dispatch(const uint8_t *tilep, const TileSid
     }
 }
 
-// Side data of a tile, in two halves so that the global loads of the first half can fly while the
-// previous tile is being transformed.
-struct SideRegs { uint32_t q, width, height, mcu_count_w, samp; uint64_t pix_off; };
-
-__device__ __forceinline__ SideRegs side_load(const ImgDev *__restrict__ imgs, const uint16_t *__restrict__ qtabs, const TileDev d)
-{
-    SideRegs r;
-    const ImgDev *im = imgs + d.img;
-    r.q = threadIdx.x < 96 ? __ldg(reinterpret_cast<const uint32_t *>(qtabs + (size_t)d.img * 192) + threadIdx.x) : 0u;   // a pair
-    r.width = __ldg(&im->width);
-    r.height = __ldg(&im->height);
-    r.mcu_count_w = __ldg(&im->mcu_count_w);
-    r.samp = __ldg(&im->samp);
-    r.pix_off = __ldg(reinterpret_cast<const unsigned long long *>(&im->pix_off));
-    return r;
-}
-
+// Side data of a tile: every global load first, then the stores to shared memory.
 template <bool NARROWQ>
-__device__ __forceinline__ void side_store(TileSide &sd, const TileDev d, const SideRegs &r, uint8_t *__restrict__ pix)
+__device__ __forceinline__ void side_stage(TileSide &sd, const ImgDev *__restrict__ imgs, const uint16_t *__restrict__ qtabs, const TileDev d,
+                                           uint8_t *__restrict__ pix)
 {
     const uint32_t tid = threadIdx.x;
+    const ImgDev *im = imgs + d.img;
+    const uint32_t q = tid < 96 ? __ldg(reinterpret_cast<const uint32_t *>(qtabs + (size_t)d.img * 192) + tid) : 0u;   // a pair
+    const uint32_t width = __ldg(&im->width);
+    const uint32_t height = __ldg(&im->height);
+    const uint32_t mcu_count_w = __ldg(&im->mcu_count_w);
+    const uint32_t samp = __ldg(&im->samp);
+    const uint64_t pix_off = __ldg(reinterpret_cast<const unsigned long long *>(&im->pix_off));
     const uint32_t n_mcus = d.info >> 8;
     if (tid < 96)
     {
         const uint32_t comp = tid >> 5, k = tid & 31u;   // quantiser pair k of component comp
-        if (NARROWQ) sd.qt[comp * kQtStride + k] = (r.q & 0xFFu) | ((r.q >> 16) << 24);
-        else { sd.qt[comp * kQtStride + 2 * k] = r.q & 0xFFFFu; sd.qt[comp * kQtStride + 2 * k + 1] = r.q >> 16; }
+        if (NARROWQ) sd.qt[comp * kQtStride + k] = (q & 0xFFu) | ((q >> 16) << 24);
+        else { sd.qt[comp * kQtStride + 2 * k] = q & 0xFFFFu; sd.qt[comp * kQtStride + 2 * k + 1] = q >> 16; }
     }
     if (tid < n_mcus)
     {
         const uint32_t gm = d.mcu_first + tid;
-        const uint32_t my = gm / r.mcu_count_w;
-        sd.mcu_xy[tid] = make_uint2(gm - my * r.mcu_count_w, my);
+        const uint32_t my = gm / mcu_count_w;
+        sd.mcu_xy[tid] = make_uint2(gm - my * mcu_count_w, my);
     }
     if (tid == 0)
     {
-        sd.pix = pix + r.pix_off;
-        sd.width = r.width; sd.height = r.height;
+        sd.pix = pix + pix_off;
+        sd.width = width; sd.height = height;
         sd.mode = d.info & 0xFFu; sd.n_mcus = n_mcus;
-        sd.samp = r.samp;
+        sd.samp = samp;
     }
 }
-
-__device__ __forceinline__ uint32_t mode_tot(uint32_t mode) { return mode == kMode444 ? 3u : (mode == kMode420 ? 6u : 4u); }
 
 // One tile per CTA. The 24 KB coefficient tile arrives by one TMA tensor load (128-byte swizzle,
 // mbarrier completion) issued by thread 0 while the other threads fetch the side data.
 // Measured on B200 (profiles/): a persistent double-buffered variant and a warp-autonomous variant of
 // this kernel were both slower -- the kernel is bound by dependent-issue latency at 24 warps per SM,
 // not by the latency in front of a tile, so the simplest structure wins.
-#ifndef B2J_IDCT_MIN_CTAS
-#define B2J_IDCT_MIN_CTAS 5   // measured on B200: 64 registers with ~220 B of spills beats 80 registers at 4 CTAs per SM
-#endif
-// GRAY: the kernel for the tiles of one-component images (B2J_GATE_GRAY). A kernel of its own over a tile range of
-// its own (the host sorts the batch's tiles by kind), because merely carrying the extra paths, or a test for them at
-// the top of the kernel, slows the colour kernel down by 2 % (measured).
-// KIND: kTileColour (the four everyday layouts), kTileGray, kTileGeneric (any other layout: csc_generic).
+constexpr int kIdctMinCtas = 5;   // measured on B200: 64 registers with ~220 B of spills beats 80 registers at 4 CTAs per SM
+// KIND: kTileColour (the four everyday layouts), kTileGray (one-component images, B2J_GATE_GRAY) or kTileGeneric (any
+// other layout: csc_generic). Each kind is a kernel of its own over a tile range of its own (the host sorts the batch's
+// tiles by kind), because merely carrying the extra paths, or a test for them at the top of the kernel, slows the
+// colour kernel down by 2 % (measured).
 constexpr int kTileColour = 0, kTileGray = 1, kTileGeneric = 2;
 template <bool NARROWQ, int FMT, int KIND>
-__global__ void __launch_bounds__(kTileBlocks, B2J_IDCT_MIN_CTAS)
+__global__ void __launch_bounds__(kTileBlocks, kIdctMinCtas)
 k_idct_csc(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
            const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ pix, int32_t *__restrict__ status)
 {
@@ -1620,35 +1595,35 @@ k_idct_csc(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ 
     const TileDev d = tiles[blockIdx.x];
     if (tid == 0)
     {
-        mbar_init(&sm.bar[0], 1);
+        mbar_init(&sm.bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        mbar_expect_tx(&sm.bar[0], kTileBlocks * 128);
-        tma_load_2d(sm.tile[0], &tmap, 0, (int)d.row_first, &sm.bar[0]);
+        mbar_expect_tx(&sm.bar, kTileBlocks * 128);
+        tma_load_2d(sm.tile, &tmap, 0, (int)d.row_first, &sm.bar);
     }
-    side_store<NARROWQ>(sm.side[0], d, side_load(imgs, qtabs, d), pix);
+    side_stage<NARROWQ>(sm.side, imgs, qtabs, d, pix);
     __syncthreads();   // barrier initialisation + side data visible
     uint32_t spins = 0;
-    while (!mbar_try_wait(&sm.bar[0], 0))
+    while (!mbar_try_wait(&sm.bar, 0))
     {
         if (++spins > (1u << 22)) { if (tid == 0) atomicOr(&status[d.img], B2J_ST_INTERNAL); break; }   // never hang the GPU
     }
     if (KIND == kTileGray)
     {
-        idct_phase<0, 0, NARROWQ>(sm.tile[0], sm.side[0]);
+        idct_phase<0, 0, NARROWQ>(sm.tile, sm.side);
         __syncthreads();
-        csc_gray<FMT>(sm.tile[0], sm.side[0], tid);
+        csc_gray<FMT>(sm.tile, sm.side, tid);
     }
     else if (KIND == kTileGeneric)
     {
-        idct_phase<-1, -1, NARROWQ>(sm.tile[0], sm.side[0]);
+        idct_phase<-1, -1, NARROWQ>(sm.tile, sm.side);
         __syncthreads();
-        csc_generic<FMT>(sm.tile[0], sm.side[0], tid);
+        csc_generic<FMT>(sm.tile, sm.side, tid);
     }
     else
     {
-        idct_dispatch<NARROWQ>(sm.tile[0], sm.side[0]);
+        idct_dispatch<NARROWQ>(sm.tile, sm.side);
         __syncthreads();
-        csc_dispatch<FMT>(sm.tile[0], sm.side[0]);
+        csc_dispatch<FMT>(sm.tile, sm.side);
     }
 }
 

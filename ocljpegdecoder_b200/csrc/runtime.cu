@@ -6,7 +6,8 @@
 //   b2j_batch_create   lays out every buffer of a batch once (compressed scans, tables, segment
 //                      and tile descriptors, coefficient plane, pixel plane)
 //   b2j_batch_upload   one host->device copy of the packed input blob
-//   b2j_batch_decode   5 kernel launches on one stream, no host synchronisation
+//   b2j_batch_decode   the pre-pass, entropy and IDCT/colour kernels in order on one stream, no host
+//                      synchronisation
 // There is no CPU fallback anywhere in this file: without a device every call fails.
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -817,7 +818,6 @@ extern "C" int b2j_batch_downscale(b2j_batch *b, void *stream, int factor)
     CU_TRY(cudaSetDevice(b->ctx->device));
     cudaStream_t s = pick_stream(b, stream);
     const int fmt = b->args.out_format;
-    const size_t bpp = fmt == B2J_OUT_BGRA ? 4 : 3;
     const size_t table = align_up(8 * (size_t)b->n, 256);
     if (b->small_factor != factor || b->small_off.size() != (size_t)b->n)
     {
@@ -850,7 +850,6 @@ extern "C" int b2j_batch_downscale(b2j_batch *b, void *stream, int factor)
         const uint32_t ns = ow * oh * (fmt == B2J_OUT_RGB_PLANAR ? 3u : 1u);
         if (ns > max_samples) max_samples = ns;
     }
-    (void)bpp;
     launch_downscale(b->d_pix, b->args.imgs, reinterpret_cast<const uint64_t *>(b->d_small), b->d_small, (uint32_t)b->n, max_samples, (uint32_t)factor, fmt, s);
     CU_TRY(cudaGetLastError());
     return B2J_OK;
@@ -1230,9 +1229,6 @@ extern "C" int b2j_decode_host(b2j_ctx *ctx, int n, const uint8_t *const *files,
     memset(&o, 0, sizeof(o));
     o.gate = gate;
     o.out_format = B2J_OUT_BGRA;
-    if (const char *ge = getenv("B2J_HOST_GROUP")) o.group = atoi(ge);
-    if (const char *te = getenv("B2J_HOST_THREADS")) o.n_threads = atoi(te);
-    if (const char *me = getenv("B2J_HOST_GROUP_MB")) o.group_mb = atoi(me);
     return b2j_decode_host_ex(ctx, n, files, lens, &o, out_bgra, status);
 }
 
