@@ -96,6 +96,22 @@ extern "C" {
 #define B2J_OUT_RGB24 1      /* R,G,B bytes interleaved, pitch W*3 (SURVEY.md 8f rank 3: what image consumers want)     */
 #define B2J_OUT_RGB_PLANAR 2 /* three planes R, G, B of W*H bytes each (a CHW uint8 tensor left on the device)          */
 
+/* ---- which pixels a decode computes from the coefficients (b2j_batch_set_pixel_model) ---- */
+#define B2J_PIXELS_REFERENCE 0 /* the reference's: Chen-Wang IDCT, chroma replication, exact integer colour (default) */
+#define B2J_PIXELS_LIBJPEG 1   /* libjpeg-turbo's default decode, what Pillow, OpenCV and torchvision's CPU decoder give:
+                                * ISLOW IDCT (jidctint.c), "fancy" chroma upsampling (jdsample.c: triangle filter for
+                                * chroma at half the luma's width, height or both, replication for every other ratio and
+                                * for chroma 1 or 2 samples wide), SCALEBITS-16 fixed-point YCbCr -> RGB (jdcolor.c).
+                                * The pixels equal libjpeg-turbo's C code paths for every decodable input, and default
+                                * Pillow for encoder-produced files. Caveats:
+                                *  - with extreme coefficients (random AC up to +-300 and beyond) libjpeg-turbo's SIMD IDCT,
+                                *    which Pillow uses by default, overflows 16-bit lanes and differs from its own C code;
+                                *    this model follows the C code (JSIMD_FORCENONE=1);
+                                *  - equality is claimed for 8-bit DQTs. A 16-bit DQT entry is used as parsed under the
+                                *    batch's gate: without B2J_PARSE_ROBUST it is byte-swapped relative to libjpeg;
+                                *  - files libjpeg would treat as RGB (Adobe transform 0, component ids 'R', 'G', 'B') are
+                                *    still converted as YCbCr. */
+
 /* reference enum ColorSpace (macro.h:114-119) */
 #define B2J_CS_YUV444 0
 #define B2J_CS_YUV411 1
@@ -203,6 +219,11 @@ int b2j_batch_sync(b2j_batch *batch, void *stream);
  * in every format -- exact integer colour of decoder.cpp:367-370 -- only their arrangement differs. b2j_decode_host()
  * and the reference-API shim always produce the reference's BGRA. */
 int b2j_batch_set_output_format(b2j_batch *batch, int format);
+/* Pixel model for the decodes that follow (B2J_PIXELS_*; default B2J_PIXELS_REFERENCE), with every output format and
+ * with b2j_batch_downscale(). The coefficients and the status words are the same in both models; only the stage after
+ * the coefficient plane differs. B2J_PIXELS_LIBJPEG runs two kernels instead of one per tile kind, and the first decode
+ * in it allocates a sample plane of 64 bytes per block (b2j_batch_info counts both). B2J_E_ARG for an unknown model. */
+int b2j_batch_set_pixel_model(b2j_batch *batch, int model);
 
 /* Per-image status words (B2J_ST_* bits). Synchronises the stream. */
 int b2j_batch_status(b2j_batch *batch, void *stream, int32_t *status /* n */);
@@ -249,12 +270,14 @@ typedef struct b2j_host_opts
                           * the machine offers, at most 8                                                        */
     int32_t group;       /* images per pipeline group (0 = 32): a group is uploaded, decoded and read back as one */
     int32_t group_mb;    /* and at most this many MiB of files per group (0 = 12): one host thread stages a group  */
-    int32_t reserved[3]; /* 0                                                                                     */
+    int32_t pixel_model; /* B2J_PIXELS_* (0 = the reference's pixels)                                             */
+    int32_t reserved[2]; /* 0                                                                                     */
 } b2j_host_opts;
 
 /* b2j_decode_host() with options: the pixels arrive in opts->out_format (RGB24 moves 25 % fewer bytes over PCIe,
- * which is what bounds this call), headers are parsed and scans staged by opts->n_threads host threads while the
- * calling thread only enqueues uploads, decodes and downloads. out[i]: w*h*4 or w*h*3 bytes. */
+ * which is what bounds this call) and opts->pixel_model (B2J_E_ARG for an unknown one), headers are parsed and scans
+ * staged by opts->n_threads host threads while the calling thread only enqueues uploads, decodes and downloads.
+ * out[i]: w*h*4 or w*h*3 bytes. */
 int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *files, const size_t *lens, const b2j_host_opts *opts,
                        uint8_t *const *out, int32_t *status);
 

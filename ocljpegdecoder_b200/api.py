@@ -11,6 +11,8 @@ GATE_EXTENDED = 1
 PARSE_ROBUST = 2     # OR-able: skip COM / late APPn / unknown segments, big-endian 16-bit DQT
 GATE_GRAY = 4        # OR-able: one-component (grayscale) frames
 OUT_BGRA, OUT_RGB24, OUT_RGB_PLANAR = 0, 1, 2
+PIXELS_REFERENCE = 0   # the reference's pixels (default)
+PIXELS_LIBJPEG = 1     # libjpeg-turbo's default decode: ISLOW IDCT, fancy chroma upsampling, fixed-point colour (Pillow's pixels)
 
 B2J_OK = 0
 B2J_E_NODEVICE = -7
@@ -19,7 +21,7 @@ B2J_E_NODEVICE = -7
 EXPORTED_SYMBOLS = [
     "b2j_abi_version", "b2j_strerror", "b2j_last_error", "b2j_parse_header", "b2j_device_count",
     "b2j_create", "b2j_destroy", "b2j_batch_create", "b2j_batch_destroy", "b2j_batch_get_info",
-    "b2j_batch_upload", "b2j_batch_set_output_format", "b2j_batch_decode", "b2j_batch_decode_timed", "b2j_batch_decode_steps", "b2j_batch_sync", "b2j_batch_status", "b2j_batch_sync_stats",
+    "b2j_batch_upload", "b2j_batch_set_output_format", "b2j_batch_set_pixel_model", "b2j_batch_decode", "b2j_batch_decode_timed", "b2j_batch_decode_steps", "b2j_batch_sync", "b2j_batch_status", "b2j_batch_sync_stats",
     "b2j_batch_pixels_device", "b2j_batch_coefs_device", "b2j_batch_read_pixels", "b2j_batch_read_all_pixels",
     "b2j_batch_read_coefs", "b2j_decode_host", "b2j_decode_host_ex", "b2j_decode_host_multi", "b2j_host_alloc", "b2j_host_free",
     "b2j_read_files", "b2j_idct_create", "b2j_idct_blk_count", "b2j_idct_upload", "b2j_idct_run", "b2j_idct_read_pixels", "b2j_idct_read_coefs",
@@ -64,7 +66,7 @@ class BatchInfo(ctypes.Structure):
 class HostOpts(ctypes.Structure):
     """b2j_host_opts"""
     _fields_ = [("gate", ctypes.c_int32), ("out_format", ctypes.c_int32), ("n_threads", ctypes.c_int32), ("group", ctypes.c_int32),
-                ("group_mb", ctypes.c_int32), ("reserved", ctypes.c_int32 * 3)]
+                ("group_mb", ctypes.c_int32), ("pixel_model", ctypes.c_int32), ("reserved", ctypes.c_int32 * 2)]
 
 
 class StageTimes(ctypes.Structure):
@@ -106,6 +108,7 @@ def load_library():
     L.b2j_batch_get_info.argtypes = [vp, ctypes.POINTER(BatchInfo)]
     L.b2j_batch_upload.argtypes = [vp, vp]
     L.b2j_batch_set_output_format.argtypes = [vp, ci]
+    L.b2j_batch_set_pixel_model.argtypes = [vp, ci]
     L.b2j_batch_decode.argtypes = [vp, vp]
     L.b2j_batch_decode_timed.argtypes = [vp, vp, ctypes.POINTER(StageTimes)]
     L.b2j_batch_decode_steps.argtypes = [vp, vp, ci, ctypes.POINTER(StageTimes), ctypes.POINTER(ctypes.c_float)]
@@ -177,13 +180,14 @@ class HostArgs:
     """The argument arrays of a b2j_decode_host* call, marshalled once (8192 small files cost tens of milliseconds of
     ctypes work per call otherwise): files / lens / outs as for Decoder.decode_host_ex."""
 
-    def __init__(self, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0, group_mb=0):
+    def __init__(self, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0, group_mb=0,
+                 pixel_model=PIXELS_REFERENCE):
         self.n = len(files)
         self.files = files                      # keeps the bytes objects alive
         lens = lens if lens is not None else [len(f) for f in files]
         self.outs, self.fp, self.op = _host_call_args(files, outs, gate, out_format)
         self.ln = (ctypes.c_size_t * self.n)(*lens)
-        self.opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, group_mb=group_mb)
+        self.opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, group_mb=group_mb, pixel_model=pixel_model)
         self.status = np.zeros(self.n, np.int32)
 
 
@@ -230,14 +234,15 @@ def host_free(address):
     load_library().b2j_host_free(ctypes.c_void_p(address))
 
 
-def decode_host_multi(decoders, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0):
+def decode_host_multi(decoders, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0,
+                      pixel_model=PIXELS_REFERENCE):
     """b2j_decode_host_multi over the given Decoder objects (one per GPU). files: bytes objects or addresses (then `lens`)."""
     L = load_library()
     n = len(files)
     lens = lens if lens is not None else [len(f) for f in files]
     outs, fp, op = _host_call_args(files, outs, gate, out_format)
     ln = (ctypes.c_size_t * n)(*lens)
-    opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group)
+    opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, pixel_model=pixel_model)
     cx = (ctypes.c_void_p * len(decoders))(*[d._h.value for d in decoders])
     status = np.zeros(n, np.int32)
     _check(L.b2j_decode_host_multi(cx, len(decoders), n, fp, ln, ctypes.byref(opts), op, status.ctypes.data), "b2j_decode_host_multi")
@@ -294,14 +299,15 @@ class Decoder:
                "b2j_decode_host_ex")
         return args.outs, args.status
 
-    def decode_host_ex(self, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0):
-        """b2j_decode_host_ex: like decode_host with an output layout and host threads. files: bytes objects or addresses
-        (then `lens`); outs: numpy arrays or addresses."""
+    def decode_host_ex(self, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0,
+                       pixel_model=PIXELS_REFERENCE):
+        """b2j_decode_host_ex: like decode_host with an output layout, a pixel model and host threads. files: bytes objects
+        or addresses (then `lens`); outs: numpy arrays or addresses."""
         n = len(files)
         lens = lens if lens is not None else [len(f) for f in files]
         outs, fp, op = _host_call_args(files, outs, gate, out_format)
         ln = (ctypes.c_size_t * n)(*lens)
-        opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group)
+        opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, pixel_model=pixel_model)
         status = np.zeros(n, np.int32)
         _check(self.lib.b2j_decode_host_ex(self._h, n, fp, ln, ctypes.byref(opts), op, status.ctypes.data), "b2j_decode_host_ex")
         return outs, status
@@ -411,6 +417,12 @@ class Batch:
         """OUT_BGRA (reference layout, default), OUT_RGB24 (H,W,3) or OUT_RGB_PLANAR (3,H,W) for the decodes that follow."""
         _check(self.lib.b2j_batch_set_output_format(self._h, fmt), "b2j_batch_set_output_format")
         self.out_format = fmt
+
+    def set_pixel_model(self, model):
+        """PIXELS_REFERENCE (the reference's pixels, default) or PIXELS_LIBJPEG (libjpeg-turbo's, what Pillow decodes) for
+        the decodes that follow; combines with every output format and with downscale()."""
+        _check(self.lib.b2j_batch_set_pixel_model(self._h, model), "b2j_batch_set_pixel_model")
+        self.pixel_model = model
 
     def pixels(self, i, stream=None):
         d = self.descs[i]

@@ -17,6 +17,9 @@
 //       replication + exact integer YCbCr->BGRA and 128-bit coalesced stores. Replaces
 //       Fast_IDCT (cpuIDCT8x8.cpp:25-127), the upsample/colour loop of decode_mcu_data()
 //       (decoder.cpp:429-495) and the OpenCL kernels idct8x8.cl:157-222.
+//   k_idct_islow, k_upsample_ycc
+//       the libjpeg pixel model (B2J_PIXELS_LIBJPEG) instead of k_idct_csc: libjpeg-turbo's ISLOW IDCT into a sample
+//       plane, then its fancy chroma upsampling and fixed-point colour.
 //   k_expand_coefs
 //       the reference's coefficient tap (int32, dequantised) from the int16 plane, for parity.
 #include <cuda.h>
@@ -1628,6 +1631,214 @@ k_idct_csc(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ 
 }
 
 // =====================================================================================
+// The libjpeg pixel model (B2J_PIXELS_LIBJPEG): libjpeg-turbo's default decode of the same coefficients, in two kernels
+// of their own so that the reference model's colour kernel keeps its code and its instruction cache (DESIGN.md §3).
+//   k_idct_islow      per tile, one thread per block: dequantise, ISLOW IDCT (jidctint.c), range limit; 64 sample bytes
+//                     per block into the sample plane
+//   k_upsample_ycc    per 4-pixel group: chroma upsampling as jdsample.c chooses it (fancy triangle filter for 2x1, 2x2
+//                     and 1x2, replication otherwise), fixed-point YCbCr -> RGB (jdcolor.c), store in the output format
+// Sample plane: image i at byte 64 * blk_first, its components one after another, each an MCU-padded plane of
+// (mcu_count_w * h * 8) x (mcu_count_h * v * 8) bytes -- 64 bytes per block, so the image's share is 64 * blk_count.
+
+// One 1-D pass of jpeg_idct_islow (CONST_BITS 13) over d[0..7] (a column, then a row), in place, descaled by N bits.
+// The arithmetic is 64-bit, like libjpeg's JLONG: a dequantised coefficient reaches 32767 * 65535 < 2^31, and the
+// constants reach 2^14.7, so 32-bit products would overflow for the large coefficients valid files may carry.
+template <int N>
+__device__ __forceinline__ void islow_1d(int64_t d[8])
+{
+    int64_t z1 = (d[2] + d[6]) * 4433;                      // FIX(0.541196100)
+    const int64_t tmp2 = z1 - d[6] * 15137;                 // FIX(1.847759065)
+    const int64_t tmp3 = z1 + d[2] * 6270;                  // FIX(0.765366865)
+    const int64_t tmp0 = (d[0] + d[4]) * 8192, tmp1 = (d[0] - d[4]) * 8192;
+    const int64_t e10 = tmp0 + tmp3, e13 = tmp0 - tmp3, e11 = tmp1 + tmp2, e12 = tmp1 - tmp2;
+    int64_t t0 = d[7], t1 = d[5], t2 = d[3], t3 = d[1];
+    z1 = t0 + t3;
+    int64_t z2 = t1 + t2, z3 = t0 + t2, z4 = t1 + t3;
+    const int64_t z5 = (z3 + z4) * 9633;                    // FIX(1.175875602)
+    t0 *= 2446; t1 *= 16819; t2 *= 25172; t3 *= 12299;      // FIX(0.298631336), FIX(2.053119869), FIX(3.072711026), FIX(1.501321110)
+    z1 *= -7373; z2 *= -20995;                              // FIX(0.899976223), FIX(2.562915447)
+    z3 = z3 * -16069 + z5; z4 = z4 * -3196 + z5;            // FIX(1.961570560), FIX(0.390180644)
+    t0 += z1 + z3; t1 += z2 + z4; t2 += z2 + z3; t3 += z1 + z4;
+    constexpr int64_t r = 1ll << (N - 1);
+    d[0] = (e10 + t3 + r) >> N; d[7] = (e10 - t3 + r) >> N;
+    d[1] = (e11 + t2 + r) >> N; d[6] = (e11 - t2 + r) >> N;
+    d[2] = (e12 + t1 + r) >> N; d[5] = (e12 - t1 + r) >> N;
+    d[3] = (e13 + t0 + r) >> N; d[4] = (e13 - t0 + r) >> N;
+}
+
+// libjpeg's range limit of an IDCT output (sample_range_limit[] indexed with y & 1023): it wraps, it does not clamp.
+__device__ __forceinline__ uint32_t islow_limit(int64_t y)
+{
+    const uint32_t m = ((uint32_t)y + 128u) & 1023u;
+    return m < 256u ? m : (m < 640u ? 255u : 0u);
+}
+
+// Every tile kind in one kernel: the component of a block comes from the image's sampling factors (gray: 0x11, one block).
+__global__ void __launch_bounds__(kTileBlocks)
+k_idct_islow(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
+             const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ samples, int32_t *__restrict__ status)
+{
+    TileSmem &sm = *tile_smem();
+    const uint32_t tid = threadIdx.x;
+    const TileDev d = tiles[blockIdx.x];
+    if (tid == 0)
+    {
+        mbar_init(&sm.bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_expect_tx(&sm.bar, kTileBlocks * 128);
+        tma_load_2d(sm.tile, &tmap, 0, (int)d.row_first, &sm.bar);
+    }
+    side_stage<false>(sm.side, imgs, qtabs, d, samples);   // 32-bit quantisers; sd.pix is not used
+    __syncthreads();
+    uint32_t spins = 0;
+    while (!mbar_try_wait(&sm.bar, 0))
+    {
+        if (++spins > (1u << 22)) { if (tid == 0) atomicOr(&status[d.img], B2J_ST_INTERNAL); break; }   // never hang the GPU
+    }
+    const ImgDev *im = imgs + d.img;
+    const uint32_t sp = sm.side.samp;
+    const uint32_t yh = sp & 15u, yv = (sp >> 4) & 15u, uh = (sp >> 8) & 15u, uv = (sp >> 12) & 15u, vh = (sp >> 16) & 15u;
+    const uint32_t ny = yh * yv, nu = uh * uv, tot = ny + nu + vh * ((sp >> 20) & 15u);
+    if (tid >= sm.side.n_mcus * tot) return;
+    const uint32_t m = tid / tot, bi = tid % tot;
+    const uint32_t comp = (bi >= ny ? 1u : 0u) + (bi >= ny + nu ? 1u : 0u);
+    const uint32_t k = bi - (comp > 0 ? ny : 0u) - (comp > 1 ? nu : 0u);   // block inside the component's part of the MCU
+    const uint32_t h = comp == 0 ? yh : (comp == 1 ? uh : vh);
+    const uint32_t v = comp == 0 ? yv : (comp == 1 ? uv : (sp >> 20) & 15u);
+    const uint32_t mcu_count = __ldg(&im->mcu_count), mcw = __ldg(&im->mcu_count_w), blk_first = __ldg(&im->blk_first);
+    const size_t pitch = (size_t)mcw * h * 8u;
+    const uint2 mxy = sm.side.mcu_xy[m];
+    uint8_t *dst = samples + 64ull * ((size_t)blk_first + (size_t)mcu_count * ((comp > 0 ? ny : 0u) + (comp > 1 ? nu : 0u))) +
+                   (size_t)((mxy.y * v + k / h) * 8u) * pitch + (mxy.x * h + k % h) * 8u;
+    const uint32_t *q = sm.side.qt + comp * kQtStride;
+    const uint8_t *rowp = sm.tile + tid * 128u;
+    const uint32_t sw = tid & 7u;
+    int32_t ws[64];   // jidctint.c's int workspace: the pass-1 results are stored as 32-bit ints
+#pragma unroll
+    for (int c = 0; c < 8; c++)
+    {
+        int64_t col[8];
+#pragma unroll
+        for (int r = 0; r < 8; r++)
+        {
+            const int32_t coef = *reinterpret_cast<const int16_t *>(rowp + (((uint32_t)r ^ sw) << 4) + c * 2);
+            col[r] = (int64_t)(coef * (int32_t)q[8 * r + c]);   // DEQUANTIZE: an int product (fits, see islow_1d)
+        }
+        islow_1d<13 - 2>(col);
+#pragma unroll
+        for (int r = 0; r < 8; r++) ws[8 * r + c] = (int32_t)col[r];
+    }
+#pragma unroll
+    for (int r = 0; r < 8; r++)
+    {
+        int64_t row[8];
+#pragma unroll
+        for (int c = 0; c < 8; c++) row[c] = ws[8 * r + c];
+        islow_1d<13 + 2 + 3>(row);
+        uint2 o;
+        o.x = islow_limit(row[0]) | islow_limit(row[1]) << 8 | islow_limit(row[2]) << 16 | islow_limit(row[3]) << 24;
+        o.y = islow_limit(row[4]) | islow_limit(row[5]) << 8 | islow_limit(row[6]) << 16 | islow_limit(row[7]) << 24;
+        *reinterpret_cast<uint2 *>(dst + (size_t)r * pitch) = o;   // pitch and offsets are multiples of 8
+    }
+}
+
+// One component of an image in the sample plane, and how it becomes full resolution.
+struct UpComp
+{
+    const uint8_t *p;     // first sample of the component's plane
+    uint32_t pitch;       // bytes per row of the plane
+    uint32_t dw, dh;      // samples that belong to the image: ceil(W * h / hmax) x ceil(H * v / vmax)
+    uint32_t rh, rv;      // upsampling ratio hmax / h, vmax / v
+};
+
+__device__ __forceinline__ UpComp up_comp(const uint8_t *p, uint32_t h, uint32_t v, uint32_t hmax, uint32_t vmax, uint32_t mcw, uint32_t width,
+                                          uint32_t height)
+{
+    UpComp c;
+    c.p = p; c.pitch = mcw * h * 8u;
+    c.dw = (width * h + hmax - 1u) / hmax; c.dh = (height * v + vmax - 1u) / vmax;
+    c.rh = hmax / h; c.rv = vmax / v;
+    return c;
+}
+
+// The component's value at output pixel (x, y), as jdsample.c computes it. Neighbours outside [0, dw) x [0, dh) are
+// clamped, which is libjpeg's edge replication; the first and last columns of its loops are that case.
+__device__ __forceinline__ uint32_t up_sample(const UpComp &c, uint32_t x, uint32_t y)
+{
+    const bool fancy_h = c.rh == 2u && c.dw > 2u;
+    if (c.rh == 1u && c.rv == 1u) return __ldg(c.p + (size_t)y * c.pitch + x);
+    if (c.rh == 1u && c.rv == 2u)                                      // h1v2_fancy_upsample
+    {
+        const uint32_t r = y >> 1, n = (y & 1u) ? min(r + 1u, c.dh - 1u) : (r ? r - 1u : 0u);
+        return (3u * __ldg(c.p + (size_t)r * c.pitch + x) + __ldg(c.p + (size_t)n * c.pitch + x) + 1u + (y & 1u)) >> 2;
+    }
+    if (fancy_h && c.rv == 1u)                                         // h2v1_fancy_upsample
+    {
+        const uint8_t *row = c.p + (size_t)y * c.pitch;
+        const uint32_t sx = x >> 1, nx = (x & 1u) ? min(sx + 1u, c.dw - 1u) : (sx ? sx - 1u : 0u);
+        return (3u * __ldg(row + sx) + __ldg(row + nx) + 1u + (x & 1u)) >> 2;
+    }
+    if (fancy_h && c.rv == 2u)                                         // h2v2_fancy_upsample
+    {
+        const uint32_t r = y >> 1, n = (y & 1u) ? min(r + 1u, c.dh - 1u) : (r ? r - 1u : 0u);
+        const uint32_t sx = x >> 1, nx = (x & 1u) ? min(sx + 1u, c.dw - 1u) : (sx ? sx - 1u : 0u);
+        const uint8_t *r0 = c.p + (size_t)r * c.pitch, *r1 = c.p + (size_t)n * c.pitch;
+        const uint32_t cs = 3u * __ldg(r0 + sx) + __ldg(r1 + sx), cn = 3u * __ldg(r0 + nx) + __ldg(r1 + nx);
+        return (3u * cs + cn + 8u - (x & 1u)) >> 4;
+    }
+    return __ldg(c.p + (size_t)(y / c.rv) * c.pitch + x / c.rh);      // int_upsample / h2v1 / h2v2: replication
+}
+
+// jdcolor.c ycc_rgb_convert (SCALEBITS 16): R | G << 8 | B << 16
+__device__ __forceinline__ uint32_t ycc_rgb_libjpeg(int32_t y, int32_t cb, int32_t cr)
+{
+    cb -= 128; cr -= 128;
+    const int32_t r = y + ((91881 * cr + 32768) >> 16);
+    const int32_t g = y + ((-22554 * cb - 46802 * cr + 32768) >> 16);
+    const int32_t b = y + ((116130 * cb + 32768) >> 16);
+    return (uint32_t)min(max(r, 0), 255) | (uint32_t)min(max(g, 0), 255) << 8 | (uint32_t)min(max(b, 0), 255) << 16;
+}
+
+// One thread per 4-pixel group of a row; blockIdx.y (strided by gridDim.y) = image.
+template <int FMT>
+__global__ void __launch_bounds__(256)
+k_upsample_ycc(const uint8_t *__restrict__ samples, const ImgDev *__restrict__ imgs, uint32_t n_images, uint8_t *__restrict__ pix)
+{
+    for (uint32_t img = blockIdx.y; img < n_images; img += gridDim.y)
+    {
+        const ImgDev &im = imgs[img];
+        const uint32_t width = im.width, height = im.height, gw = (width + 3u) / 4u;
+        const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+        if (i >= gw * height) continue;
+        const uint32_t py = i / gw, px = (i % gw) * 4u;
+        const uint32_t sp = im.samp, mcw = im.mcu_count_w;
+        const uint32_t yh = sp & 15u, yv = (sp >> 4) & 15u, uh = (sp >> 8) & 15u, uv = (sp >> 12) & 15u, vh = (sp >> 16) & 15u, vv = (sp >> 20) & 15u;
+        const uint8_t *p0 = samples + 64ull * im.blk_first;
+        const bool gray = im.mode == kModeGray;
+        // the chroma factors divide the luma's (geometry_ok), so the luma's are the maxima
+        const UpComp cy = up_comp(p0, yh, yv, yh, yv, mcw, width, height);
+        UpComp cu = cy, cv = cy;
+        if (!gray)
+        {
+            cu = up_comp(p0 + 64ull * im.mcu_count * (yh * yv), uh, uv, yh, yv, mcw, width, height);
+            cv = up_comp(p0 + 64ull * im.mcu_count * (yh * yv + uh * uv), vh, vv, yh, yv, mcw, width, height);
+        }
+        uint32_t R[2] = {0u, 0u}, Gc[2] = {0u, 0u}, B[2] = {0u, 0u};
+#pragma unroll
+        for (uint32_t k = 0; k < 4u; k++)
+        {
+            const uint32_t x = min(px + k, width - 1u);   // the stores skip pixels behind the last column
+            const uint32_t Y = up_sample(cy, x, py);
+            const uint32_t rgb = gray ? Y * 0x10101u : ycc_rgb_libjpeg((int32_t)Y, (int32_t)up_sample(cu, x, py), (int32_t)up_sample(cv, x, py));
+            const uint32_t sh = 16u * (k & 1u);
+            R[k >> 1] |= (rgb & 0xFFu) << sh; Gc[k >> 1] |= ((rgb >> 8) & 0xFFu) << sh; B[k >> 1] |= (rgb >> 16) << sh;
+        }
+        constexpr uint32_t bpp = FMT == B2J_OUT_BGRA ? 4u : (FMT == B2J_OUT_RGB24 ? 3u : 1u);
+        store_pixels4<FMT>(pix + im.pix_off + ((size_t)py * width + px) * bpp, (size_t)width * height, px, width, (width & 3u) == 0u, R, Gc, B);
+    }
+}
+
+// =====================================================================================
 // Coefficient tap: int16 quantised plane -> the reference's int32 dequantised mcu_data layout.
 __global__ void __launch_bounds__(256)
 k_expand_coefs(const int16_t *__restrict__ coef, const uint16_t *__restrict__ qtab, uint32_t blk_count,
@@ -1752,8 +1963,32 @@ static void launch_idct_format(const DecodeArgs &a, cudaStream_t s)
     launch_idct_kind<FMT, kTileGeneric>(a, a.generic_tile0, a.n_tiles - a.generic_tile0, s);
 }
 
+// The libjpeg model: the IDCT over every tile into the sample plane, then the upsampling / colour pass over every image.
+template <int FMT>
+static void launch_libjpeg_format(const DecodeArgs &a, cudaStream_t s)
+{
+    k_idct_islow<<<a.n_tiles, kTileBlocks, kTileSmemBytes, s>>>(*a.tmap, a.imgs, a.tiles, a.qtabs, a.samples, a.status);
+    const dim3 grid((a.max_px_groups + 255u) / 256u, a.n_images < 65535u ? a.n_images : 65535u);
+    k_upsample_ycc<FMT><<<grid, 256, 0, s>>>(a.samples, a.imgs, a.n_images, a.pixels);
+}
+
+int idct_launches(const DecodeArgs &a)
+{
+    if (a.n_tiles == 0) return 0;
+    if (a.pixel_model == B2J_PIXELS_LIBJPEG) return 2;
+    return (a.gray_tile0 > 0 ? 1 : 0) + (a.generic_tile0 > a.gray_tile0 ? 1 : 0) + (a.n_tiles > a.generic_tile0 ? 1 : 0);
+}
+
 void launch_idct(const DecodeArgs &a, cudaStream_t s)
 {
+    if (a.pixel_model == B2J_PIXELS_LIBJPEG)
+    {
+        if (a.n_tiles == 0) return;
+        if (a.out_format == B2J_OUT_RGB24) launch_libjpeg_format<B2J_OUT_RGB24>(a, s);
+        else if (a.out_format == B2J_OUT_RGB_PLANAR) launch_libjpeg_format<B2J_OUT_RGB_PLANAR>(a, s);
+        else launch_libjpeg_format<B2J_OUT_BGRA>(a, s);
+        return;
+    }
     if (a.out_format == B2J_OUT_RGB24) launch_idct_format<B2J_OUT_RGB24>(a, s);
     else if (a.out_format == B2J_OUT_RGB_PLANAR) launch_idct_format<B2J_OUT_RGB_PLANAR>(a, s);
     else launch_idct_format<B2J_OUT_BGRA>(a, s);

@@ -123,6 +123,7 @@ struct b2j_batch
     uint8_t *d_pix; size_t d_pix_cap; size_t pix_bytes;
     int32_t *d_expand; size_t d_expand_cap;   // lazily allocated for the coefficient tap
     uint8_t *d_small; size_t d_small_cap;     // lazily allocated: the reduced pixels of b2j_batch_downscale() behind a table of offsets
+    uint8_t *d_samples; size_t d_samples_cap; // lazily allocated by the first decode in the libjpeg pixel model: its sample plane
     int small_factor;                         // 0 = none yet
     std::vector<uint64_t> small_off;          // byte offset of every image's reduced pixels behind the offset table
 
@@ -210,8 +211,9 @@ void release_batch_buffers(b2j_batch *b)
     c->dev_pool.put(b->d_pix, b->d_pix_cap);
     c->dev_pool.put(b->d_expand, b->d_expand_cap);
     c->dev_pool.put(b->d_small, b->d_small_cap);
+    c->dev_pool.put(b->d_samples, b->d_samples_cap);
     b->h_blob = b->d_blob = b->d_scratch = b->d_pix = nullptr;
-    b->d_coef = nullptr; b->d_expand = nullptr; b->d_small = nullptr;
+    b->d_coef = nullptr; b->d_expand = nullptr; b->d_small = nullptr; b->d_samples = nullptr;
 }
 
 } // namespace
@@ -338,6 +340,7 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     b->imgs.resize((size_t)n);
     b->h_blob = b->d_blob = b->d_scratch = b->d_pix = nullptr;
     b->d_coef = nullptr; b->d_expand = nullptr; b->d_small = nullptr; b->d_small_cap = 0; b->small_factor = 0;
+    b->d_samples = nullptr; b->d_samples_cap = 0;
     b->h_blob_cap = b->d_blob_cap = b->d_scratch_cap = b->d_coef_cap = b->d_pix_cap = b->d_expand_cap = 0;
     b->uploaded = false;
     b->last_stream = nullptr;
@@ -355,6 +358,7 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     static const uint8_t zz[64] = B2J_ZIGZAG_TABLE;
 
     size_t raw_total = 0, pix_total = 0, blk_total = 0;
+    uint32_t max_px_groups = 0;   // largest ceil(W / 4) * H
     uint32_t seg_total = 0, max_lut_len = 0, max_lut_dec_len = 0, max_lut_walk_len = 0;
     int64_t pixels = 0, scan_bytes = 0;
     int rc = B2J_OK;
@@ -406,8 +410,12 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
         im.tot_blks = (uint32_t)d.tot_blks_per_mcu;
         im.ny_blks = (uint32_t)d.blks_per_mcu[0];
         im.nu_blks = (uint32_t)d.blks_per_mcu[1];
-        im.samp = (uint32_t)(d.sampling[0] >> 4) | (uint32_t)(d.sampling[0] & 0xF) << 4 | (uint32_t)(d.sampling[1] >> 4) << 8 |
-                  (uint32_t)(d.sampling[1] & 0xF) << 12 | (uint32_t)(d.sampling[2] >> 4) << 16 | (uint32_t)(d.sampling[2] & 0xF) << 20;
+        im.samp = (uint32_t)(d.sampling[0] >> 4) | (uint32_t)(d.sampling[0] & 0xF) << 4;
+        // a gray frame has no chroma: geometry_ok() does not look at sampling[1..2] then, and the kernels that derive the
+        // block layout from samp (the generic and the libjpeg-model ones) must see zero blocks there
+        if (im.mode != kModeGray)
+            im.samp |= (uint32_t)(d.sampling[1] >> 4) << 8 | (uint32_t)(d.sampling[1] & 0xF) << 12 | (uint32_t)(d.sampling[2] >> 4) << 16 |
+                       (uint32_t)(d.sampling[2] & 0xF) << 20;
         im.yh = (uint32_t)(d.sampling[0] >> 4);
         const uint32_t mcus_per_tile = kTileBlocks / im.tot_blks;
         for (uint32_t m = 0; m < im.mcu_count; m += mcus_per_tile)
@@ -424,6 +432,7 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
                 if (q > 255) im.wide_q = 1;
             }
         pixels += (int64_t)d.width * d.height;
+        max_px_groups = std::max(max_px_groups, (uint32_t)((d.width + 3) / 4) * (uint32_t)d.height);
         if (coef_only) continue;
         scan_bytes += (int64_t)d.scan_size;
         // decode tables, shared between images that carry identical DHT payloads
@@ -570,6 +579,9 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     a.out_format = B2J_OUT_BGRA;
     a.any_wide_q = false;
     for (const ImgDev &im : b->imgs) a.any_wide_q = a.any_wide_q || im.wide_q != 0;
+    a.pixel_model = B2J_PIXELS_REFERENCE;
+    a.samples = nullptr;
+    a.max_px_groups = max_px_groups;
     {
         const char *sp = getenv("B2J_SYNC_PRE");
         a.sync_use_pre = !(sp && atoi(sp) == 0);
@@ -578,8 +590,7 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     b2j_batch_info &inf = b->info;
     memset(&inf, 0, sizeof(inf));
     inf.n_images = n;
-    const int idct_launches = (a.gray_tile0 > 0 ? 1 : 0) + (a.generic_tile0 > a.gray_tile0 ? 1 : 0) + (a.n_tiles > a.generic_tile0 ? 1 : 0);
-    inf.kernel_launches = idct_launches + 1 + (ctas.empty() ? 0 : 1) + (sctas.empty() ? 0 : kSyncLaunches);
+    inf.kernel_launches = idct_launches(a) + 1 + (ctas.empty() ? 0 : 1) + (sctas.empty() ? 0 : kSyncLaunches);
     inf.total_pixels = pixels;
     inf.total_blocks = (int64_t)blk_total;
     inf.scan_bytes = scan_bytes;
@@ -634,6 +645,17 @@ constexpr size_t kStepEvents = 5;
 static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStepEvents or NULL */)
 {
     if (!b->uploaded) { t_last_error = "b2j_batch_decode before b2j_batch_upload"; return B2J_E_ARG; }
+    if (b->args.pixel_model == B2J_PIXELS_LIBJPEG && !b->d_samples)
+    {
+        // the sample plane: 64 bytes per block, image by image at 64 * blk_first
+        {
+            std::lock_guard<std::mutex> lk(b->ctx->mu);
+            cudaError_t e = b->ctx->dev_pool.get((size_t)b->info.total_blocks * 64, (void **)&b->d_samples, &b->d_samples_cap);
+            if (e != cudaSuccess) { fail_cuda(e, "sample plane allocation"); cudaGetLastError(); b->d_samples = nullptr; b->d_samples_cap = 0; return B2J_E_NOMEM; }
+        }
+        b->args.samples = b->d_samples;
+        b->info.device_bytes += (int64_t)b->d_samples_cap;
+    }
     const DecodeArgs &a = b->args;
     if (ev) CU_TRY(cudaEventRecord(ev[0], s));
     if (a.n_huff_ctas) CU_TRY(cudaMemsetAsync(a.seg_start, 0xFF, 4 * (size_t)b->n_segs_total, s));   // read by the restart-interval decoder only
@@ -736,6 +758,15 @@ extern "C" int b2j_batch_set_output_format(b2j_batch *b, int format)
 {
     if (!b || (format != B2J_OUT_BGRA && format != B2J_OUT_RGB24 && format != B2J_OUT_RGB_PLANAR)) return B2J_E_ARG;
     b->args.out_format = format;   // the pixel plane is sized for 4 bytes per pixel: every format fits
+    return B2J_OK;
+}
+
+extern "C" int b2j_batch_set_pixel_model(b2j_batch *b, int model)
+{
+    if (!b || (model != B2J_PIXELS_REFERENCE && model != B2J_PIXELS_LIBJPEG)) return B2J_E_ARG;
+    b->info.kernel_launches -= idct_launches(b->args);
+    b->args.pixel_model = model;   // the sample plane, once allocated, stays with the batch
+    b->info.kernel_launches += idct_launches(b->args);
     return B2J_OK;
 }
 
@@ -939,6 +970,8 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
     if (!ctx || n <= 0 || !files || !lens || !out || !status || !opts) return B2J_E_ARG;
     const int fmt = opts->out_format;
     if (fmt != B2J_OUT_BGRA && fmt != B2J_OUT_RGB24 && fmt != B2J_OUT_RGB_PLANAR) return B2J_E_ARG;
+    const int model = opts->pixel_model;
+    if (model != B2J_PIXELS_REFERENCE && model != B2J_PIXELS_LIBJPEG) return B2J_E_ARG;
     CU_TRY(cudaSetDevice(ctx->device));
     const int gate = opts->gate;
     const int group = opts->group > 0 ? opts->group : 32;
@@ -1006,7 +1039,11 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
             {
                 G.rc = b2j_batch_create(ctx, (int)d.size(), d.data(), f.data(), l.data(), &G.b);
                 if (G.rc != B2J_OK) G.err = t_last_error;
-                else pack_pixel_plane(G.b, fmt);
+                else
+                {
+                    pack_pixel_plane(G.b, fmt);
+                    b2j_batch_set_pixel_model(G.b, model);
+                }
             }
             {
                 std::lock_guard<std::mutex> lk(mu);
