@@ -55,31 +55,44 @@ int fail_cuda(cudaError_t e, const char *what)
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// A buffer held from a Pool; empty (null, capacity 0) when none is held.
+struct PoolBuf
+{
+    void *p = nullptr;
+    size_t cap = 0;
+};
+
 // A grow-only cache of device / pinned allocations so that repeated batches (the e2e path) do
 // not pay cudaMalloc / cudaHostAlloc every call.
 struct Pool
 {
-    struct Buf { void *p; size_t cap; };
-    std::vector<Buf> free_list;
+    std::vector<PoolBuf> free_list;
     bool pinned;
     explicit Pool(bool pin) : pinned(pin) {}
-    cudaError_t get(size_t n, void **out, size_t *cap)
+    // fills the empty `b` with at least n bytes; leaves it empty on failure
+    cudaError_t get(size_t n, PoolBuf &b)
     {
         size_t best = (size_t)-1;
         for (size_t i = 0; i < free_list.size(); i++)
             if (free_list[i].cap >= n && (best == (size_t)-1 || free_list[i].cap < free_list[best].cap)) best = i;
         if (best != (size_t)-1)
         {
-            *out = free_list[best].p; *cap = free_list[best].cap;
+            b = free_list[best];
             free_list.erase(free_list.begin() + (long)best);
             return cudaSuccess;
         }
         n = align_up(n ? n : 1, 1 << 20);
-        cudaError_t e = pinned ? cudaHostAlloc(out, n, cudaHostAllocDefault) : cudaMalloc(out, n);
-        *cap = n;
+        void *p = nullptr;
+        const cudaError_t e = pinned ? cudaHostAlloc(&p, n, cudaHostAllocDefault) : cudaMalloc(&p, n);
+        if (e == cudaSuccess) b = {p, n};
         return e;
     }
-    void put(void *p, size_t cap) { if (p) free_list.push_back({p, cap}); }
+    // hands `b` back and leaves it empty
+    void put(PoolBuf &b)
+    {
+        if (b.p) free_list.push_back(b);
+        b = {};
+    }
     void drain()
     {
         for (auto &b : free_list) { if (pinned) cudaFreeHost(b.p); else cudaFree(b.p); }
@@ -92,8 +105,8 @@ struct Pool
 struct b2j_ctx
 {
     int device;
-    cudaStream_t stream;
-    cudaStream_t stream2;   // host feed: the downloads of a group run here while the next group decodes on `stream`
+    cudaStream_t stream = nullptr;
+    cudaStream_t stream2 = nullptr;   // host feed: the downloads of a group run here while the next group decodes on `stream`
     PFN_cuTensorMapEncodeTiled_v12000 encode_tiled;
     int sm_count;
     Pool dev_pool{false};
@@ -105,33 +118,30 @@ struct b2j_batch
 {
     b2j_ctx *ctx;
     int n;
-    std::vector<b2j_image_desc> descs;
     std::vector<ImgDev> imgs;
     b2j_batch_info info;
 
     // packed input blob: host (pinned) and device copies share one layout
-    uint8_t *h_blob; size_t h_blob_cap;
-    uint8_t *d_blob; size_t d_blob_cap;
+    PoolBuf h_blob, d_blob;
     size_t blob_bytes;
-    size_t off_imgs, off_chunk_img, off_ctas, off_sctas, off_simgs, off_tiles, off_luts, off_qtabs, off_raw;
+    ImgDev *h_imgs;      // the image table in the pinned blob
 
-    // scratch + outputs
-    uint8_t *d_scratch; size_t d_scratch_cap;
-    size_t off_clean, off_clean_end, off_clean_len, off_seg_start, off_status, off_recs, off_pres, off_sync_stats, off_chunk_state, off_chunk_states, off_zero_end;
-    size_t scratch_bytes;
-    int16_t *d_coef; size_t d_coef_cap; size_t coef_rows;
-    uint8_t *d_pix; size_t d_pix_cap; size_t pix_bytes;
-    int32_t *d_expand; size_t d_expand_cap;   // lazily allocated for the coefficient tap
-    uint8_t *d_small; size_t d_small_cap;     // lazily allocated: the reduced pixels of b2j_batch_downscale() behind a table of offsets
-    uint8_t *d_samples; size_t d_samples_cap; // lazily allocated by the first decode in the libjpeg pixel model: its sample plane
-    int small_factor;                         // 0 = none yet
+    // scratch + outputs; the DecodeArgs pointers lead into them
+    PoolBuf d_scratch, d_coef, d_pix;
+    size_t clean_bytes;  // the clean stream and its tail, from args.clean: defined by the first upload
+    size_t zero_bytes;   // the status words, sync stats and look-back words, from args.status: zeroed by every decode
+    size_t coef_rows;
+    uint32_t n_segs_total;
+    PoolBuf d_expand;    // lazily allocated for the coefficient tap
+    PoolBuf d_small;     // lazily allocated: the reduced pixels of b2j_batch_downscale() behind a table of offsets
+    PoolBuf d_samples;   // lazily allocated by the first decode in the libjpeg pixel model: its sample plane
+    int small_factor = 0;                     // 0 = none
     std::vector<uint64_t> small_off;          // byte offset of every image's reduced pixels behind the offset table
 
     CUtensorMap tmap;
     DecodeArgs args;
-    uint32_t n_segs_total;
-    bool uploaded;
-    cudaStream_t last_stream;   // the stream the batch was last uploaded / decoded / read on
+    bool uploaded = false;
+    cudaStream_t last_stream = nullptr;   // the stream the batch was last uploaded / decoded / read on
 };
 
 namespace {
@@ -144,7 +154,7 @@ int make_tensor_map(b2j_ctx *ctx, b2j_batch *b)
     const cuuint64_t strides[1] = {128};
     const cuuint32_t box[2] = {64, (cuuint32_t)kTileBlocks};
     const cuuint32_t estr[2] = {1, 1};
-    CUresult r = ctx->encode_tiled(&b->tmap, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, b->d_coef, dims, strides, box, estr,
+    CUresult r = ctx->encode_tiled(&b->tmap, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, b->d_coef.p, dims, strides, box, estr,
                                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS)
@@ -200,20 +210,58 @@ bool geometry_ok(const b2j_image_desc &d)
 
 cudaStream_t pick_stream(b2j_batch *b, void *stream) { return b->last_stream = (stream ? (cudaStream_t)stream : b->ctx->stream); }
 
+// Grows the device buffer `buf` to at least n bytes from the context's pool; its contents are not kept. On failure the
+// buffer is left empty and CUDA's last error is cleared, so that it cannot fail the next, unrelated call on this thread.
+cudaError_t grow(b2j_ctx *ctx, PoolBuf &buf, size_t n)
+{
+    if (buf.cap >= n) return cudaSuccess;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->dev_pool.put(buf);
+    const cudaError_t e = ctx->dev_pool.get(n, buf);
+    if (e != cudaSuccess) cudaGetLastError();
+    return e;
+}
+
 void release_batch_buffers(b2j_batch *b)
 {
     b2j_ctx *c = b->ctx;
     std::lock_guard<std::mutex> lk(c->mu);
-    c->pin_pool.put(b->h_blob, b->h_blob_cap);
-    c->dev_pool.put(b->d_blob, b->d_blob_cap);
-    c->dev_pool.put(b->d_scratch, b->d_scratch_cap);
-    c->dev_pool.put(b->d_coef, b->d_coef_cap);
-    c->dev_pool.put(b->d_pix, b->d_pix_cap);
-    c->dev_pool.put(b->d_expand, b->d_expand_cap);
-    c->dev_pool.put(b->d_small, b->d_small_cap);
-    c->dev_pool.put(b->d_samples, b->d_samples_cap);
-    b->h_blob = b->d_blob = b->d_scratch = b->d_pix = nullptr;
-    b->d_coef = nullptr; b->d_expand = nullptr; b->d_small = nullptr; b->d_samples = nullptr;
+    c->pin_pool.put(b->h_blob);
+    for (PoolBuf *d : {&b->d_blob, &b->d_scratch, &b->d_coef, &b->d_pix, &b->d_expand, &b->d_small, &b->d_samples}) c->dev_pool.put(*d);
+}
+
+// b2j_batch_info::device_bytes: the buffers a decode uses (the read-back buffers of the coefficient tap and of
+// b2j_batch_downscale() are not counted)
+int64_t device_bytes(const b2j_batch *b)
+{
+    return (int64_t)(b->d_blob.cap + b->d_scratch.cap + b->d_coef.cap + b->d_pix.cap + b->d_samples.cap);
+}
+
+// The image `image` of the batch, or nullptr when the batch has no such image.
+const ImgDev *image_of(const b2j_batch *b, int image) { return b && image >= 0 && image < b->n ? &b->imgs[(size_t)image] : nullptr; }
+
+// Bytes per pixel of an output format (B2J_OUT_*).
+size_t format_bpp(int fmt) { return fmt == B2J_OUT_BGRA ? 4 : 3; }
+
+size_t image_bytes(const b2j_batch *b, const ImgDev &im) { return (size_t)im.width * im.height * format_bpp(b->args.out_format); }
+
+// One device->host copy on the call's stream, waited for.
+int read_back(b2j_batch *b, void *stream, void *dst, const void *src, size_t bytes)
+{
+    CU_TRY(cudaSetDevice(b->ctx->device));
+    const cudaStream_t s = pick_stream(b, stream);
+    CU_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s));
+    CU_TRY(cudaStreamSynchronize(s));
+    return B2J_OK;
+}
+
+template <class T> T *at(const PoolBuf &buf, size_t off) { return reinterpret_cast<T *>((uint8_t *)buf.p + off); }
+
+// Copies a host-built array to its place in the pinned blob; returns where it lands on the device.
+template <class T> const T *stage(const b2j_batch *b, size_t off, const std::vector<T> &v)
+{
+    memcpy(at<T>(b->h_blob, off), v.data(), sizeof(T) * v.size());
+    return at<const T>(b->d_blob, off);
 }
 
 } // namespace
@@ -267,11 +315,19 @@ extern "C" int b2j_create(int device, b2j_ctx **out)
         t_last_error = std::string("device ") + prop.name + " is not sm_100-class; kernels are built for sm_100a only";
         return B2J_E_NODEVICE;
     }
+    // the colour kernel loads its tiles through a tensor map
+    void *fn = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || qres != cudaDriverEntryPointSuccess || !fn)
+    {
+        cudaGetLastError();
+        t_last_error = "the driver does not export cuTensorMapEncodeTiled (needed for the TMA tile loads)";
+        return B2J_E_CUDA;
+    }
     b2j_ctx *ctx = new b2j_ctx;
     ctx->device = device;
     ctx->sm_count = prop.multiProcessorCount;
-    ctx->encode_tiled = nullptr;
-    ctx->stream = ctx->stream2 = nullptr;
+    ctx->encode_tiled = (PFN_cuTensorMapEncodeTiled_v12000)fn;
     cudaError_t ce = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking);
     if (ce == cudaSuccess) ce = cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking);
     if (ce == cudaSuccess) ce = init_constants();
@@ -282,21 +338,6 @@ extern "C" int b2j_create(int device, b2j_ctx **out)
         if (ctx->stream2) cudaStreamDestroy(ctx->stream2);
         delete ctx;
         return fail_cuda(ce, "b2j_create");
-    }
-    void *fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-        ctx->encode_tiled = (PFN_cuTensorMapEncodeTiled_v12000)fn;
-    else
-        cudaGetLastError();
-    if (!ctx->encode_tiled)
-    {
-        // the colour kernel loads its tiles through a tensor map
-        cudaStreamDestroy(ctx->stream);
-        cudaStreamDestroy(ctx->stream2);
-        delete ctx;
-        t_last_error = "the driver does not export cuTensorMapEncodeTiled (needed for the TMA tile loads)";
-        return B2J_E_CUDA;
     }
     *out = ctx;
     return B2J_OK;
@@ -336,14 +377,7 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     b2j_batch *b = new b2j_batch();
     b->ctx = ctx;
     b->n = n;
-    b->descs.assign(descs, descs + n);
     b->imgs.resize((size_t)n);
-    b->h_blob = b->d_blob = b->d_scratch = b->d_pix = nullptr;
-    b->d_coef = nullptr; b->d_expand = nullptr; b->d_small = nullptr; b->d_small_cap = 0; b->small_factor = 0;
-    b->d_samples = nullptr; b->d_samples_cap = 0;
-    b->h_blob_cap = b->d_blob_cap = b->d_scratch_cap = b->d_coef_cap = b->d_pix_cap = b->d_expand_cap = 0;
-    b->uploaded = false;
-    b->last_stream = nullptr;
 
     std::vector<uint32_t> chunk_img;
     std::vector<HuffCtaDev> ctas;    // restart-interval path
@@ -473,98 +507,89 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     const auto gray0 = std::stable_partition(tiles.begin(), tiles.end(), [](const TileDev &t) { return (t.info & 0xFFu) < kModeGray; });
     const auto generic0 = std::stable_partition(gray0, tiles.end(), [](const TileDev &t) { return (t.info & 0xFFu) == kModeGray; });
 
-    // ---- input blob layout
+    // ---- input blob layout: regions 256-byte aligned, in this order; a region of no bytes shares its offset with the next
     size_t off = 0;
     auto place = [&](size_t bytes) { const size_t o = off; off = align_up(off + bytes, 256); return o; };
-    b->off_imgs = place(sizeof(ImgDev) * (size_t)n);
-    b->off_chunk_img = place(sizeof(uint32_t) * chunk_img.size());
-    b->off_ctas = place(sizeof(HuffCtaDev) * ctas.size());
-    b->off_sctas = place(sizeof(HuffCtaDev) * sctas.size());
-    b->off_simgs = place(sizeof(uint32_t) * simgs.size());
-    b->off_tiles = place(sizeof(TileDev) * tiles.size());
-    b->off_luts = place(sizeof(uint16_t) * luts.size());
-    b->off_qtabs = place(sizeof(uint16_t) * qtabs.size());
-    b->off_raw = place(raw_total + kScanChunkBytes + 64);   // the pre-pass reads whole chunks
+    auto place_array = [&](const auto &v) { return place(sizeof(v[0]) * v.size()); };
+    const size_t o_imgs = place_array(b->imgs);
+    const size_t o_chunk_img = place_array(chunk_img);
+    const size_t o_ctas = place_array(ctas);
+    const size_t o_sctas = place_array(sctas);
+    const size_t o_simgs = place_array(simgs);
+    const size_t o_tiles = place_array(tiles);
+    const size_t o_luts = place_array(luts);
+    const size_t o_qtabs = place_array(qtabs);
+    const size_t o_raw = place(raw_total + kScanChunkBytes + 64);   // the pre-pass reads whole chunks
     b->blob_bytes = off;
 
     // ---- scratch layout
     off = 0;
-    b->off_clean = place(raw_total + 256);   // the bit readers prefetch up to 48 bytes past a segment
-    b->off_clean_end = off;
-    b->off_clean_len = place(4 * (size_t)n);
-    b->off_seg_start = place(4 * (size_t)seg_total);
-    b->off_recs = place(sizeof(SubRec) * (size_t)sub_total);
-    b->off_pres = place(sizeof(uint4) * (sctas.size() + 1));
-    b->off_chunk_states = place(sizeof(uint4) * (sctas.size() + 1));
+    const size_t o_clean = place(raw_total + 256);   // the bit readers prefetch up to 48 bytes past a segment
+    b->clean_bytes = off - o_clean;
+    const size_t o_clean_len = place(4 * (size_t)n);
+    const size_t o_seg_start = place(4 * (size_t)seg_total);
+    const size_t o_recs = place(sizeof(SubRec) * (size_t)sub_total);
+    const size_t o_pres = place(sizeof(uint4) * (sctas.size() + 1));
+    const size_t o_chunk_states = place(sizeof(uint4) * (sctas.size() + 1));
     // what every decode starts from zero, side by side: one memset
-    b->off_status = place(4 * (size_t)n);
-    b->off_sync_stats = place(4 * 8);
-    b->off_chunk_state = place(8 * chunk_img.size());
-    b->off_zero_end = off;
-    b->scratch_bytes = off;
+    const size_t o_status = place(4 * (size_t)n);
+    const size_t o_sync_stats = place(4 * 8);
+    const size_t o_chunk_state = place(8 * chunk_img.size());
+    b->zero_bytes = off - o_status;
+    const size_t scratch_bytes = off;
     b->n_segs_total = seg_total;
     b->coef_rows = blk_total + kTileBlocks;   // one tile of padding: the last tile may read past the last block
-    b->pix_bytes = pix_total;
 
     {
         std::lock_guard<std::mutex> lk(ctx->mu);
         cudaError_t e;
-        if ((e = ctx->pin_pool.get(b->blob_bytes, (void **)&b->h_blob, &b->h_blob_cap)) != cudaSuccess ||
-            (e = ctx->dev_pool.get(b->blob_bytes, (void **)&b->d_blob, &b->d_blob_cap)) != cudaSuccess ||
-            (e = ctx->dev_pool.get(b->scratch_bytes, (void **)&b->d_scratch, &b->d_scratch_cap)) != cudaSuccess ||
-            (e = ctx->dev_pool.get(b->coef_rows * 128, (void **)&b->d_coef, &b->d_coef_cap)) != cudaSuccess ||
-            (e = ctx->dev_pool.get(b->pix_bytes, (void **)&b->d_pix, &b->d_pix_cap)) != cudaSuccess)
+        if ((e = ctx->pin_pool.get(b->blob_bytes, b->h_blob)) != cudaSuccess ||
+            (e = ctx->dev_pool.get(b->blob_bytes, b->d_blob)) != cudaSuccess ||
+            (e = ctx->dev_pool.get(scratch_bytes, b->d_scratch)) != cudaSuccess ||
+            (e = ctx->dev_pool.get(b->coef_rows * 128, b->d_coef)) != cudaSuccess ||
+            (e = ctx->dev_pool.get(pix_total, b->d_pix)) != cudaSuccess)
         {
             rc = fail_cuda(e, "batch allocation");
             cudaGetLastError();
         }
     }
     if (rc != B2J_OK) { release_batch_buffers(b); delete b; return rc == B2J_E_CUDA ? B2J_E_NOMEM : rc; }
+    rc = make_tensor_map(ctx, b);
+    if (rc != B2J_OK) { release_batch_buffers(b); delete b; return rc; }
 
-    // ---- fill the pinned blob
-    memcpy(b->h_blob + b->off_imgs, b->imgs.data(), sizeof(ImgDev) * (size_t)n);
-    memcpy(b->h_blob + b->off_chunk_img, chunk_img.data(), sizeof(uint32_t) * chunk_img.size());
-    memcpy(b->h_blob + b->off_ctas, ctas.data(), sizeof(HuffCtaDev) * ctas.size());
-    memcpy(b->h_blob + b->off_sctas, sctas.data(), sizeof(HuffCtaDev) * sctas.size());
-    memcpy(b->h_blob + b->off_simgs, simgs.data(), sizeof(uint32_t) * simgs.size());
-    memcpy(b->h_blob + b->off_tiles, tiles.data(), sizeof(TileDev) * tiles.size());
-    memcpy(b->h_blob + b->off_luts, luts.data(), sizeof(uint16_t) * luts.size());
-    memcpy(b->h_blob + b->off_qtabs, qtabs.data(), sizeof(uint16_t) * qtabs.size());
+    // ---- the pinned blob, and where the kernels find each region on the device
+    DecodeArgs &a = b->args;
+    a.imgs = stage(b, o_imgs, b->imgs);
+    b->h_imgs = at<ImgDev>(b->h_blob, o_imgs);
+    a.chunk_img = stage(b, o_chunk_img, chunk_img);
+    a.huff_ctas = stage(b, o_ctas, ctas);
+    a.sync_ctas = stage(b, o_sctas, sctas);
+    a.sync_imgs = stage(b, o_simgs, simgs);
+    a.tiles = stage(b, o_tiles, tiles);
+    a.luts = stage(b, o_luts, luts);
+    a.qtabs = stage(b, o_qtabs, qtabs);
     for (int i = 0; i < n; i++)
     {
         const ImgDev &im = b->imgs[(size_t)i];
-        uint8_t *dst = b->h_blob + b->off_raw + im.raw_off;
+        uint8_t *dst = at<uint8_t>(b->h_blob, o_raw + im.raw_off);
         if (im.raw_len) memcpy(dst, files[i] + descs[i].scan_offset, im.raw_len);
         // pad with FF D9 D9 ...: running off the end of a scan then looks like EOI to the pre-pass
         memset(dst + im.raw_len, 0xD9, align_up((size_t)im.raw_len + 32, 16) - im.raw_len);
         dst[im.raw_len] = 0xFF;
     }
-
-    rc = make_tensor_map(ctx, b);
-    if (rc != B2J_OK) { release_batch_buffers(b); delete b; return rc; }
-
-    DecodeArgs &a = b->args;
-    a.raw = b->d_blob + b->off_raw;
-    a.imgs = reinterpret_cast<const ImgDev *>(b->d_blob + b->off_imgs);
-    a.chunk_img = reinterpret_cast<const uint32_t *>(b->d_blob + b->off_chunk_img);
-    a.huff_ctas = reinterpret_cast<const HuffCtaDev *>(b->d_blob + b->off_ctas);
-    a.sync_ctas = reinterpret_cast<const HuffCtaDev *>(b->d_blob + b->off_sctas);
-    a.sync_imgs = reinterpret_cast<const uint32_t *>(b->d_blob + b->off_simgs);
-    a.recs = reinterpret_cast<SubRec *>(b->d_scratch + b->off_recs);
-    a.sync_cta_base = reinterpret_cast<uint4 *>(b->d_scratch + b->off_pres);
-    a.sync_stats = reinterpret_cast<uint32_t *>(b->d_scratch + b->off_sync_stats);
-    a.sync_chunk_state = reinterpret_cast<uint4 *>(b->d_scratch + b->off_chunk_states);
-    a.tiles = reinterpret_cast<const TileDev *>(b->d_blob + b->off_tiles);
-    a.luts = reinterpret_cast<const uint16_t *>(b->d_blob + b->off_luts);
-    a.qtabs = reinterpret_cast<const uint16_t *>(b->d_blob + b->off_qtabs);
+    a.raw = at<const uint8_t>(b->d_blob, o_raw);
+    a.clean = at<uint8_t>(b->d_scratch, o_clean);
+    a.clean_len = at<uint32_t>(b->d_scratch, o_clean_len);
+    a.seg_start = at<uint32_t>(b->d_scratch, o_seg_start);
+    a.recs = at<SubRec>(b->d_scratch, o_recs);
+    a.sync_cta_base = at<uint4>(b->d_scratch, o_pres);
+    a.sync_chunk_state = at<uint4>(b->d_scratch, o_chunk_states);
+    a.status = at<int32_t>(b->d_scratch, o_status);
+    a.sync_stats = at<uint32_t>(b->d_scratch, o_sync_stats);
+    a.chunk_state = at<uint64_t>(b->d_scratch, o_chunk_state);
     a.tmap = &b->tmap;
-    a.clean = b->d_scratch + b->off_clean;
-    a.chunk_state = reinterpret_cast<uint64_t *>(b->d_scratch + b->off_chunk_state);
-    a.clean_len = reinterpret_cast<uint32_t *>(b->d_scratch + b->off_clean_len);
-    a.seg_start = reinterpret_cast<uint32_t *>(b->d_scratch + b->off_seg_start);
-    a.status = reinterpret_cast<int32_t *>(b->d_scratch + b->off_status);
-    a.coef = b->d_coef;
-    a.pixels = b->d_pix;
+    a.coef = at<int16_t>(b->d_coef, 0);
+    a.pixels = at<uint8_t>(b->d_pix, 0);
     a.n_images = (uint32_t)n;
     a.n_chunks = (uint32_t)chunk_img.size();
     a.n_huff_ctas = (uint32_t)ctas.size();
@@ -597,7 +622,7 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     inf.coef_plane_bytes = 128 * (int64_t)blk_total;
     inf.pixel_bytes = 4 * pixels;
     inf.algorithmic_bytes = inf.scan_bytes + 2 * inf.coef_plane_bytes + inf.pixel_bytes;
-    inf.device_bytes = (int64_t)(b->d_blob_cap + b->d_scratch_cap + b->d_coef_cap + b->d_pix_cap);
+    inf.device_bytes = device_bytes(b);
     inf.h2d_bytes = (int64_t)b->blob_bytes;
     *out = b;
     return B2J_OK;
@@ -626,12 +651,12 @@ extern "C" int b2j_batch_upload(b2j_batch *b, void *stream)
     if (!b) return B2J_E_ARG;
     CU_TRY(cudaSetDevice(b->ctx->device));
     cudaStream_t s = pick_stream(b, stream);
-    CU_TRY(cudaMemcpyAsync(b->d_blob, b->h_blob, b->blob_bytes, cudaMemcpyHostToDevice, s));
+    CU_TRY(cudaMemcpyAsync(b->d_blob.p, b->h_blob.p, b->blob_bytes, cudaMemcpyHostToDevice, s));
     if (!b->uploaded)
     {
         // padding rows of the plane and the tail of the clean stream are read (never used); define them once
-        CU_TRY(cudaMemsetAsync(b->d_coef + (b->coef_rows - kTileBlocks) * 64, 0, (size_t)kTileBlocks * 128, s));
-        CU_TRY(cudaMemsetAsync(b->d_scratch + b->off_clean, 0, b->off_clean_end - b->off_clean, s));
+        CU_TRY(cudaMemsetAsync(b->args.coef + (b->coef_rows - kTileBlocks) * 64, 0, (size_t)kTileBlocks * 128, s));
+        CU_TRY(cudaMemsetAsync(b->args.clean, 0, b->clean_bytes, s));
         b->uploaded = true;
     }
     return B2J_OK;
@@ -645,21 +670,18 @@ constexpr size_t kStepEvents = 5;
 static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStepEvents or NULL */)
 {
     if (!b->uploaded) { t_last_error = "b2j_batch_decode before b2j_batch_upload"; return B2J_E_ARG; }
-    if (b->args.pixel_model == B2J_PIXELS_LIBJPEG && !b->d_samples)
+    if (b->args.pixel_model == B2J_PIXELS_LIBJPEG && !b->d_samples.p)
     {
         // the sample plane: 64 bytes per block, image by image at 64 * blk_first
-        {
-            std::lock_guard<std::mutex> lk(b->ctx->mu);
-            cudaError_t e = b->ctx->dev_pool.get((size_t)b->info.total_blocks * 64, (void **)&b->d_samples, &b->d_samples_cap);
-            if (e != cudaSuccess) { fail_cuda(e, "sample plane allocation"); cudaGetLastError(); b->d_samples = nullptr; b->d_samples_cap = 0; return B2J_E_NOMEM; }
-        }
-        b->args.samples = b->d_samples;
-        b->info.device_bytes += (int64_t)b->d_samples_cap;
+        const cudaError_t e = grow(b->ctx, b->d_samples, (size_t)b->info.total_blocks * 64);
+        if (e != cudaSuccess) { fail_cuda(e, "sample plane allocation"); return B2J_E_NOMEM; }
+        b->args.samples = at<uint8_t>(b->d_samples, 0);
+        b->info.device_bytes = device_bytes(b);
     }
     const DecodeArgs &a = b->args;
     if (ev) CU_TRY(cudaEventRecord(ev[0], s));
     if (a.n_huff_ctas) CU_TRY(cudaMemsetAsync(a.seg_start, 0xFF, 4 * (size_t)b->n_segs_total, s));   // read by the restart-interval decoder only
-    CU_TRY(cudaMemsetAsync(b->d_scratch + b->off_status, 0, b->off_zero_end - b->off_status, s));   // status words, sync stats, look-back words
+    CU_TRY(cudaMemsetAsync(a.status, 0, b->zero_bytes, s));   // status words, sync stats, look-back words
     if (ev) CU_TRY(cudaEventRecord(ev[1], s));
     launch_prepass(a, s);
     if (ev) CU_TRY(cudaEventRecord(ev[2], s));
@@ -732,26 +754,13 @@ extern "C" int b2j_batch_sync(b2j_batch *b, void *stream)
 extern "C" int b2j_batch_status(b2j_batch *b, void *stream, int32_t *status)
 {
     if (!b || !status) return B2J_E_ARG;
-    CU_TRY(cudaSetDevice(b->ctx->device));
-    cudaStream_t s = pick_stream(b, stream);
-    CU_TRY(cudaMemcpyAsync(status, b->args.status, 4 * (size_t)b->n, cudaMemcpyDeviceToHost, s));
-    CU_TRY(cudaStreamSynchronize(s));
-    return B2J_OK;
+    return read_back(b, stream, status, b->args.status, 4 * (size_t)b->n);
 }
 
 extern "C" int b2j_batch_sync_stats(b2j_batch *b, void *stream, uint32_t *out8)
 {
     if (!b || !out8) return B2J_E_ARG;
-    CU_TRY(cudaSetDevice(b->ctx->device));
-    cudaStream_t s = pick_stream(b, stream);
-    CU_TRY(cudaMemcpyAsync(out8, b->args.sync_stats, 4 * 8, cudaMemcpyDeviceToHost, s));
-    CU_TRY(cudaStreamSynchronize(s));
-    return B2J_OK;
-}
-
-static size_t image_bytes(const b2j_batch *b, const ImgDev &im)
-{
-    return (size_t)im.width * im.height * (b->args.out_format == B2J_OUT_BGRA ? 4u : 3u);
+    return read_back(b, stream, out8, b->args.sync_stats, 4 * 8);
 }
 
 extern "C" int b2j_batch_set_output_format(b2j_batch *b, int format)
@@ -772,29 +781,27 @@ extern "C" int b2j_batch_set_pixel_model(b2j_batch *b, int model)
 
 extern "C" int b2j_batch_pixels_device(const b2j_batch *b, int image, void **dptr, size_t *nbytes)
 {
-    if (!b || image < 0 || image >= b->n || !dptr) return B2J_E_ARG;
-    *dptr = b->d_pix + b->imgs[(size_t)image].pix_off;
-    if (nbytes) *nbytes = image_bytes(b, b->imgs[(size_t)image]);
+    const ImgDev *im = image_of(b, image);
+    if (!im || !dptr) return B2J_E_ARG;
+    *dptr = b->args.pixels + im->pix_off;
+    if (nbytes) *nbytes = image_bytes(b, *im);
     return B2J_OK;
 }
 
 extern "C" int b2j_batch_coefs_device(const b2j_batch *b, int image, void **dptr, size_t *nbytes)
 {
-    if (!b || image < 0 || image >= b->n || !dptr) return B2J_E_ARG;
-    *dptr = b->d_coef + (size_t)b->imgs[(size_t)image].blk_first * 64;
-    if (nbytes) *nbytes = (size_t)b->imgs[(size_t)image].blk_count * 128;
+    const ImgDev *im = image_of(b, image);
+    if (!im || !dptr) return B2J_E_ARG;
+    *dptr = b->args.coef + (size_t)im->blk_first * 64;
+    if (nbytes) *nbytes = (size_t)im->blk_count * 128;
     return B2J_OK;
 }
 
 extern "C" int b2j_batch_read_pixels(b2j_batch *b, void *stream, int image, uint8_t *dst)
 {
-    if (!b || image < 0 || image >= b->n || !dst) return B2J_E_ARG;
-    CU_TRY(cudaSetDevice(b->ctx->device));
-    cudaStream_t s = pick_stream(b, stream);
-    const ImgDev &im = b->imgs[(size_t)image];
-    CU_TRY(cudaMemcpyAsync(dst, b->d_pix + im.pix_off, image_bytes(b, im), cudaMemcpyDeviceToHost, s));
-    CU_TRY(cudaStreamSynchronize(s));
-    return B2J_OK;
+    const ImgDev *im = image_of(b, image);
+    if (!im || !dst) return B2J_E_ARG;
+    return read_back(b, stream, dst, b->args.pixels + im->pix_off, image_bytes(b, *im));
 }
 
 extern "C" int b2j_batch_read_all_pixels(b2j_batch *b, void *stream, uint8_t *const *dsts)
@@ -806,7 +813,7 @@ extern "C" int b2j_batch_read_all_pixels(b2j_batch *b, void *stream, uint8_t *co
     {
         const ImgDev &im = b->imgs[(size_t)i];
         if (!dsts[i]) continue;
-        CU_TRY(cudaMemcpyAsync(dsts[i], b->d_pix + im.pix_off, image_bytes(b, im), cudaMemcpyDeviceToHost, s));
+        CU_TRY(cudaMemcpyAsync(dsts[i], b->args.pixels + im.pix_off, image_bytes(b, im), cudaMemcpyDeviceToHost, s));
     }
     CU_TRY(cudaStreamSynchronize(s));
     return B2J_OK;
@@ -814,25 +821,17 @@ extern "C" int b2j_batch_read_all_pixels(b2j_batch *b, void *stream, uint8_t *co
 
 extern "C" int b2j_batch_read_coefs(b2j_batch *b, void *stream, int image, int32_t *dst)
 {
-    if (!b || image < 0 || image >= b->n || !dst) return B2J_E_ARG;
+    const ImgDev *im = image_of(b, image);
+    if (!im || !dst) return B2J_E_ARG;
     CU_TRY(cudaSetDevice(b->ctx->device));
     cudaStream_t s = pick_stream(b, stream);
-    const ImgDev &im = b->imgs[(size_t)image];
-    const size_t bytes = (size_t)im.blk_count * 256;
-    if (b->d_expand_cap < bytes)
-    {
-        std::lock_guard<std::mutex> lk(b->ctx->mu);
-        b->ctx->dev_pool.put(b->d_expand, b->d_expand_cap);
-        b->d_expand = nullptr; b->d_expand_cap = 0;
-        cudaError_t e = b->ctx->dev_pool.get(bytes, (void **)&b->d_expand, &b->d_expand_cap);
-        if (e != cudaSuccess) return fail_cuda(e, "coefficient tap allocation");
-    }
-    launch_expand(b->d_coef + (size_t)im.blk_first * 64, b->args.qtabs + (size_t)image * 192, im.blk_count, im.tot_blks, im.ny_blks, im.nu_blks,
-                  b->d_expand, s);
+    const size_t bytes = (size_t)im->blk_count * 256;
+    const cudaError_t e = grow(b->ctx, b->d_expand, bytes);
+    if (e != cudaSuccess) return fail_cuda(e, "coefficient tap allocation");
+    launch_expand(b->args.coef + (size_t)im->blk_first * 64, b->args.qtabs + (size_t)image * 192, im->blk_count, im->tot_blks, im->ny_blks, im->nu_blks,
+                  at<int32_t>(b->d_expand, 0), s);
     CU_TRY(cudaGetLastError());
-    CU_TRY(cudaMemcpyAsync(dst, b->d_expand, bytes, cudaMemcpyDeviceToHost, s));
-    CU_TRY(cudaStreamSynchronize(s));
-    return B2J_OK;
+    return read_back(b, stream, dst, b->d_expand.p, bytes);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -849,29 +848,22 @@ extern "C" int b2j_batch_downscale(b2j_batch *b, void *stream, int factor)
     CU_TRY(cudaSetDevice(b->ctx->device));
     cudaStream_t s = pick_stream(b, stream);
     const int fmt = b->args.out_format;
-    const size_t table = align_up(8 * (size_t)b->n, 256);
-    if (b->small_factor != factor || b->small_off.size() != (size_t)b->n)
+    if (b->small_factor != factor)
     {
+        b->small_factor = 0;   // no reduced copy until the buffer and its offset table are in place
         b->small_off.resize((size_t)b->n);
-        size_t off = table;
+        size_t off = align_up(8 * (size_t)b->n, 256);   // behind the offset table
         for (int i = 0; i < b->n; i++)
         {
             uint32_t ow, oh;
             small_dims(b->imgs[(size_t)i], factor, &ow, &oh);
             b->small_off[(size_t)i] = off;
-            off += align_up((size_t)ow * oh * 4, 16);   // sized for BGRA: every format fits
+            off += align_up((size_t)ow * oh * format_bpp(B2J_OUT_BGRA), 16);   // sized for BGRA: every format fits
         }
-        if (b->d_small_cap < off)
-        {
-            std::lock_guard<std::mutex> lk(b->ctx->mu);
-            b->ctx->dev_pool.put(b->d_small, b->d_small_cap);
-            b->d_small = nullptr; b->d_small_cap = 0;
-            cudaError_t e = b->ctx->dev_pool.get(off, (void **)&b->d_small, &b->d_small_cap);
-            if (e != cudaSuccess) { cudaGetLastError(); return B2J_E_NOMEM; }
-        }
-        b->small_factor = factor;
-        CU_TRY(cudaMemcpyAsync(b->d_small, b->small_off.data(), 8 * (size_t)b->n, cudaMemcpyHostToDevice, s));
+        if (grow(b->ctx, b->d_small, off) != cudaSuccess) return B2J_E_NOMEM;
+        CU_TRY(cudaMemcpyAsync(b->d_small.p, b->small_off.data(), 8 * (size_t)b->n, cudaMemcpyHostToDevice, s));
         CU_TRY(cudaStreamSynchronize(s));   // the table is a pageable vector that may be rebuilt
+        b->small_factor = factor;
     }
     uint32_t max_samples = 0;
     for (int i = 0; i < b->n; i++)
@@ -881,18 +873,20 @@ extern "C" int b2j_batch_downscale(b2j_batch *b, void *stream, int factor)
         const uint32_t ns = ow * oh * (fmt == B2J_OUT_RGB_PLANAR ? 3u : 1u);
         if (ns > max_samples) max_samples = ns;
     }
-    launch_downscale(b->d_pix, b->args.imgs, reinterpret_cast<const uint64_t *>(b->d_small), b->d_small, (uint32_t)b->n, max_samples, (uint32_t)factor, fmt, s);
+    launch_downscale(b->args.pixels, b->args.imgs, at<const uint64_t>(b->d_small, 0), at<uint8_t>(b->d_small, 0), (uint32_t)b->n, max_samples,
+                     (uint32_t)factor, fmt, s);
     CU_TRY(cudaGetLastError());
     return B2J_OK;
 }
 
 extern "C" int b2j_batch_downscaled_device(const b2j_batch *b, int image, void **dptr, size_t *nbytes, int *width, int *height)
 {
-    if (!b || image < 0 || image >= b->n || !dptr || !b->small_factor) return B2J_E_ARG;
+    const ImgDev *im = image_of(b, image);
+    if (!im || !dptr || !b->small_factor) return B2J_E_ARG;
     uint32_t ow, oh;
-    small_dims(b->imgs[(size_t)image], b->small_factor, &ow, &oh);
-    *dptr = b->d_small + b->small_off[(size_t)image];
-    if (nbytes) *nbytes = (size_t)ow * oh * (b->args.out_format == B2J_OUT_BGRA ? 4u : 3u);
+    small_dims(*im, b->small_factor, &ow, &oh);
+    *dptr = at<uint8_t>(b->d_small, b->small_off[(size_t)image]);
+    if (nbytes) *nbytes = (size_t)ow * oh * format_bpp(b->args.out_format);
     if (width) *width = (int)ow;
     if (height) *height = (int)oh;
     return B2J_OK;
@@ -903,12 +897,7 @@ extern "C" int b2j_batch_read_downscaled(b2j_batch *b, void *stream, int image, 
     void *p = nullptr; size_t nb = 0;
     if (!dst) return B2J_E_ARG;
     const int rc = b2j_batch_downscaled_device(b, image, &p, &nb, nullptr, nullptr);
-    if (rc != B2J_OK) return rc;
-    CU_TRY(cudaSetDevice(b->ctx->device));
-    cudaStream_t s = pick_stream(b, stream);
-    CU_TRY(cudaMemcpyAsync(dst, p, nb, cudaMemcpyDeviceToHost, s));
-    CU_TRY(cudaStreamSynchronize(s));
-    return B2J_OK;
+    return rc != B2J_OK ? rc : read_back(b, stream, dst, p, nb);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -929,16 +918,14 @@ void destroy_batch_done(b2j_batch *b)
 void pack_pixel_plane(b2j_batch *b, int fmt)
 {
     const size_t a = fmt == B2J_OUT_BGRA ? 16 : 4;
-    size_t off = 0;
-    for (int i = 0; i < b->n; i++)
-    {
-        ImgDev &im = b->imgs[(size_t)i];
-        off = align_up(off, a);
-        im.pix_off = off;
-        off += (size_t)im.width * im.height * (fmt == B2J_OUT_BGRA ? 4u : 3u);
-    }
     b->args.out_format = fmt;
-    memcpy(b->h_blob + b->off_imgs, b->imgs.data(), sizeof(ImgDev) * (size_t)b->n);
+    size_t off = 0;
+    for (ImgDev &im : b->imgs)
+    {
+        im.pix_off = off = align_up(off, a);
+        off += image_bytes(b, im);
+    }
+    memcpy(b->h_imgs, b->imgs.data(), sizeof(ImgDev) * (size_t)b->n);
 }
 
 int auto_threads(int asked, int cap)
@@ -997,12 +984,12 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
     const int ng = (int)groups.size();
 
     // per-image status words come back through one pinned array, copied behind each group's pixels
-    int32_t *h_status = nullptr; size_t h_status_cap = 0;
+    PoolBuf h_status_buf;
     {
         std::lock_guard<std::mutex> lk(ctx->mu);
-        cudaError_t e = ctx->pin_pool.get(4 * (size_t)n, (void **)&h_status, &h_status_cap);
-        if (e != cudaSuccess) { cudaGetLastError(); return B2J_E_NOMEM; }
+        if (ctx->pin_pool.get(4 * (size_t)n, h_status_buf) != cudaSuccess) { cudaGetLastError(); return B2J_E_NOMEM; }
     }
+    int32_t *const h_status = at<int32_t>(h_status_buf, 0);
 
     std::mutex mu;
     std::condition_variable cv;
@@ -1106,7 +1093,7 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
             if (!dst) { k = k1; continue; }
             while (k1 < G.idx.size() && out[G.idx[k1]] == dst + bytes && G.b->imgs[k1].pix_off == im.pix_off + bytes)
                 bytes += image_bytes(G.b, G.b->imgs[k1++]);
-            e = cudaMemcpyAsync(dst, G.b->d_pix + im.pix_off, bytes, cudaMemcpyDeviceToHost, ctx->stream2);
+            e = cudaMemcpyAsync(dst, G.b->args.pixels + im.pix_off, bytes, cudaMemcpyDeviceToHost, ctx->stream2);
             k = k1;
         }
         // the status words of the group's images land at their file indices (consecutive only when no file was refused)
@@ -1153,7 +1140,7 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
     }
     {
         std::lock_guard<std::mutex> lk(ctx->mu);
-        ctx->pin_pool.put(h_status, h_status_cap);
+        ctx->pin_pool.put(h_status_buf);
     }
     return rc;
 }
@@ -1274,10 +1261,9 @@ extern "C" int b2j_decode_host(b2j_ctx *ctx, int n, const uint8_t *const *files,
 
 struct b2j_idct
 {
-    b2j_batch *b;          // a coefficient-only batch of one image: tiles, unit quantisers, plane, pixels
-    int32_t *d_in;         // the uploaded int32 coefficients (kept: clidct_retrieve_data_from_device reads them back)
-    size_t d_in_cap;
-    int blk_count;
+    b2j_batch *b = nullptr;   // a coefficient-only batch of one image: tiles, unit quantisers, plane, pixels
+    PoolBuf d_in;             // the uploaded int32 coefficients (kept: clidct_retrieve_data_from_device reads them back)
+    int blk_count = 0;
 };
 
 extern "C" int b2j_idct_create(b2j_ctx *ctx, int width, int height, int luma_h, int luma_v, b2j_idct **out)
@@ -1296,14 +1282,9 @@ extern "C" int b2j_idct_create(b2j_ctx *ctx, int width, int height, int luma_h, 
     d.tot_blks_per_mcu = luma_h * luma_v + 2;
     d.blk_count = d.mcu_count * d.tot_blks_per_mcu;
     b2j_idct *p = new b2j_idct;
-    p->b = nullptr; p->d_in = nullptr; p->d_in_cap = 0; p->blk_count = d.blk_count;
+    p->blk_count = d.blk_count;
     int rc = batch_create_impl(ctx, 1, &d, nullptr, nullptr, true, &p->b);
-    if (rc == B2J_OK)
-    {
-        std::lock_guard<std::mutex> lk(ctx->mu);
-        cudaError_t e = ctx->dev_pool.get((size_t)d.blk_count * 256, (void **)&p->d_in, &p->d_in_cap);
-        if (e != cudaSuccess) { cudaGetLastError(); rc = B2J_E_NOMEM; }
-    }
+    if (rc == B2J_OK && grow(ctx, p->d_in, (size_t)d.blk_count * 256) != cudaSuccess) rc = B2J_E_NOMEM;
     if (rc == B2J_OK) rc = b2j_batch_upload(p->b, nullptr);   // descriptors, tiles, quantisers
     if (rc != B2J_OK) { b2j_idct_destroy(p); return rc; }
     *out = p;
@@ -1318,8 +1299,9 @@ extern "C" int b2j_idct_upload(b2j_idct *p, const int32_t *coefs, int offset, in
     b2j_batch *b = p->b;
     CU_TRY(cudaSetDevice(b->ctx->device));
     cudaStream_t s = pick_stream(b, nullptr);
-    CU_TRY(cudaMemcpyAsync(p->d_in + (size_t)offset * 64, coefs, (size_t)count * 256, cudaMemcpyHostToDevice, s));
-    launch_pack(p->d_in + (size_t)offset * 64, b->d_coef + (size_t)offset * 64, (size_t)count * 64, s);
+    int32_t *in = at<int32_t>(p->d_in, (size_t)offset * 256);
+    CU_TRY(cudaMemcpyAsync(in, coefs, (size_t)count * 256, cudaMemcpyHostToDevice, s));
+    launch_pack(in, b->args.coef + (size_t)offset * 64, (size_t)count * 64, s);
     CU_TRY(cudaGetLastError());
     CU_TRY(cudaStreamSynchronize(s));   // the caller's buffer may be pageable and reused
     return B2J_OK;
@@ -1347,11 +1329,7 @@ extern "C" int b2j_idct_read_pixels(b2j_idct *p, uint8_t *dst)
 extern "C" int b2j_idct_read_coefs(b2j_idct *p, int32_t *dst)
 {
     if (!p || !dst) return B2J_E_ARG;
-    CU_TRY(cudaSetDevice(p->b->ctx->device));
-    cudaStream_t s = pick_stream(p->b, nullptr);
-    CU_TRY(cudaMemcpyAsync(dst, p->d_in, (size_t)p->blk_count * 256, cudaMemcpyDeviceToHost, s));
-    CU_TRY(cudaStreamSynchronize(s));
-    return B2J_OK;
+    return read_back(p->b, nullptr, dst, p->d_in.p, (size_t)p->blk_count * 256);
 }
 
 extern "C" void b2j_idct_destroy(b2j_idct *p)
@@ -1364,7 +1342,7 @@ extern "C" void b2j_idct_destroy(b2j_idct *p)
         cudaStreamSynchronize(ctx->stream);
         {
             std::lock_guard<std::mutex> lk(ctx->mu);
-            ctx->dev_pool.put(p->d_in, p->d_in_cap);
+            ctx->dev_pool.put(p->d_in);
         }
         b2j_batch_destroy(p->b);
     }
