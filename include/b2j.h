@@ -34,6 +34,8 @@
  *   b2j_decode_host_multi   main.cpp:17-37      one call over several GPUs: images are sharded by compressed bytes,
  *                                               one host thread and one context per GPU, no exchange between them
  *   b2j_batch_downscale     (none)              reduced copies of the decoded pixels for consumers (SURVEY.md 8f rank 3)
+ *   b2j_batch_set_scale     (none)              libjpeg's scaled decode (scale_num / scale_denom, Pillow's draft()):
+ *                                               1/2, 1/4 or 1/8 size straight from the coefficients
  *   b2j_idct_*              idct.h:9-18         the device backend as the reference's own decoder.cpp drives it
  *                                               (coefficients in, pixels out): see "secondary boundary" below
  *   b2j_read_files          decoder.cpp:94-101  the 2 KiB fread() loop (and main.cpp's fopen): whole files read with
@@ -224,6 +226,15 @@ int b2j_batch_set_output_format(b2j_batch *batch, int format);
  * the coefficient plane differs. B2J_PIXELS_LIBJPEG runs two kernels instead of one per tile kind, and the first decode
  * in it allocates a sample plane of 64 bytes per block (b2j_batch_info counts both). B2J_E_ARG for an unknown model. */
 int b2j_batch_set_pixel_model(b2j_batch *batch, int model);
+/* Scale of the decodes that follow: denom 1 (default), 2, 4 or 8, B2J_E_ARG for any other value. Reduced size:
+ * ceil(w/denom) x ceil(h/denom), in the batch's output format, at the image's usual place with tight pitch (the reads,
+ * b2j_batch_pixels_device and the host calls follow it). This is libjpeg-turbo's scaled decode (scale_num = 1,
+ * scale_denom = denom; Pillow's Image.draft()): the reduced IDCTs of jidctred.c, each component at the DCT size
+ * jdmaster.c chooses, then jdsample.c's upsampling (no fancy filter at 1/8) and the same colour conversion. It needs
+ * B2J_PIXELS_LIBJPEG: a decode with denom != 1 in the reference model fails with B2J_E_ARG (b2j_last_error() says why),
+ * and so does b2j_batch_downscale() while denom != 1. The coefficients, the status words and b2j_batch_info do not
+ * change; the sample plane keeps its size. */
+int b2j_batch_set_scale(b2j_batch *batch, int denom);
 
 /* Per-image status words (B2J_ST_* bits). Synchronises the stream. */
 int b2j_batch_status(b2j_batch *batch, void *stream, int32_t *status /* n */);
@@ -233,13 +244,15 @@ int b2j_batch_status(b2j_batch *batch, void *stream, int32_t *status /* n */);
  * sub-sequences the sequential sweep had to re-walk. Synchronises. */
 int b2j_batch_sync_stats(b2j_batch *batch, void *stream, uint32_t *out8);
 
-/* Device-resident results. Pixels: top-down, tight pitch, in the batch's output format (BGRA: width*4 per row, A = 0). */
+/* Device-resident results. Pixels: top-down, tight pitch, in the batch's output format (BGRA: width*4 per row, A = 0),
+ * at the batch's scale (b2j_batch_set_scale: width and height are then the reduced ones). */
 int b2j_batch_pixels_device(const b2j_batch *batch, int image, void **dptr, size_t *nbytes);
 /* Coefficient plane: int16[blk_count][64], natural order, QUANTISED (dequantisation happens
  * at IDCT load), MCU-interleaved block order. */
 int b2j_batch_coefs_device(const b2j_batch *batch, int image, void **dptr, size_t *nbytes);
 
-/* D2H of one image (synchronises). dst: width*height*4 bytes (BGRA) or width*height*3 (RGB24, planar RGB). */
+/* D2H of one image (synchronises). dst: width*height*4 bytes (BGRA) or width*height*3 (RGB24, planar RGB), of the size at
+ * the batch's scale. */
 int b2j_batch_read_pixels(b2j_batch *batch, void *stream, int image, uint8_t *dst);
 /* D2H of every image into dsts[i] (pinned staging, one copy per image; synchronises). */
 int b2j_batch_read_all_pixels(b2j_batch *batch, void *stream, uint8_t *const *dsts);
@@ -250,7 +263,7 @@ int b2j_batch_read_coefs(b2j_batch *batch, void *stream, int image, int32_t *dst
 /* Output stage for consumers that want smaller images (SURVEY.md 8f rank 3): box-filter reduction of the decoded pixels by
  * factor 2, 4 or 8 per axis, after b2j_batch_decode(), in the batch's output format. Reduced size: ceil(w/f) x ceil(h/f);
  * every value is the rounded mean (sum + n/2) / n of the n input values it covers (at the right / bottom edge: of those that
- * exist). The full-size pixels stay where they are. */
+ * exist). The full-size pixels stay where they are. B2J_E_ARG while the batch's scale (b2j_batch_set_scale) is not 1. */
 int b2j_batch_downscale(b2j_batch *batch, void *stream, int factor);
 int b2j_batch_downscaled_device(const b2j_batch *batch, int image, void **dptr, size_t *nbytes, int *width, int *height);
 int b2j_batch_read_downscaled(b2j_batch *batch, void *stream, int image, uint8_t *dst);   /* synchronises */
@@ -271,13 +284,15 @@ typedef struct b2j_host_opts
     int32_t group;       /* images per pipeline group (0 = 32): a group is uploaded, decoded and read back as one */
     int32_t group_mb;    /* and at most this many MiB of files per group (0 = 12): one host thread stages a group  */
     int32_t pixel_model; /* B2J_PIXELS_* (0 = the reference's pixels)                                             */
-    int32_t reserved[2]; /* 0                                                                                     */
+    int32_t scale;       /* 1, 2, 4 or 8 (0 = 1): b2j_batch_set_scale(); needs B2J_PIXELS_LIBJPEG                     */
+    int32_t reserved[1]; /* 0                                                                                     */
 } b2j_host_opts;
 
 /* b2j_decode_host() with options: the pixels arrive in opts->out_format (RGB24 moves 25 % fewer bytes over PCIe,
  * which is what bounds this call) and opts->pixel_model (B2J_E_ARG for an unknown one), headers are parsed and scans
  * staged by opts->n_threads host threads while the calling thread only enqueues uploads, decodes and downloads.
- * out[i]: w*h*4 or w*h*3 bytes. */
+ * out[i]: w*h*4 or w*h*3 bytes, with w = ceil(width/scale) and h = ceil(height/scale) for opts->scale (B2J_E_ARG for a
+ * scale other than 0, 1, 2, 4 and 8, and for a scale other than 1 in the reference pixel model). */
 int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *files, const size_t *lens, const b2j_host_opts *opts,
                        uint8_t *const *out, int32_t *status);
 

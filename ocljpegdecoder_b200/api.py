@@ -21,7 +21,7 @@ B2J_E_NODEVICE = -7
 EXPORTED_SYMBOLS = [
     "b2j_abi_version", "b2j_strerror", "b2j_last_error", "b2j_parse_header", "b2j_device_count",
     "b2j_create", "b2j_destroy", "b2j_batch_create", "b2j_batch_destroy", "b2j_batch_get_info",
-    "b2j_batch_upload", "b2j_batch_set_output_format", "b2j_batch_set_pixel_model", "b2j_batch_decode", "b2j_batch_decode_timed", "b2j_batch_decode_steps", "b2j_batch_sync", "b2j_batch_status", "b2j_batch_sync_stats",
+    "b2j_batch_upload", "b2j_batch_set_output_format", "b2j_batch_set_pixel_model", "b2j_batch_set_scale", "b2j_batch_decode", "b2j_batch_decode_timed", "b2j_batch_decode_steps", "b2j_batch_sync", "b2j_batch_status", "b2j_batch_sync_stats",
     "b2j_batch_pixels_device", "b2j_batch_coefs_device", "b2j_batch_read_pixels", "b2j_batch_read_all_pixels",
     "b2j_batch_read_coefs", "b2j_decode_host", "b2j_decode_host_ex", "b2j_decode_host_multi", "b2j_host_alloc", "b2j_host_free",
     "b2j_read_files", "b2j_idct_create", "b2j_idct_blk_count", "b2j_idct_upload", "b2j_idct_run", "b2j_idct_read_pixels", "b2j_idct_read_coefs",
@@ -66,7 +66,7 @@ class BatchInfo(ctypes.Structure):
 class HostOpts(ctypes.Structure):
     """b2j_host_opts"""
     _fields_ = [("gate", ctypes.c_int32), ("out_format", ctypes.c_int32), ("n_threads", ctypes.c_int32), ("group", ctypes.c_int32),
-                ("group_mb", ctypes.c_int32), ("pixel_model", ctypes.c_int32), ("reserved", ctypes.c_int32 * 2)]
+                ("group_mb", ctypes.c_int32), ("pixel_model", ctypes.c_int32), ("scale", ctypes.c_int32), ("reserved", ctypes.c_int32 * 1)]
 
 
 class StageTimes(ctypes.Structure):
@@ -109,6 +109,7 @@ def load_library():
     L.b2j_batch_upload.argtypes = [vp, vp]
     L.b2j_batch_set_output_format.argtypes = [vp, ci]
     L.b2j_batch_set_pixel_model.argtypes = [vp, ci]
+    L.b2j_batch_set_scale.argtypes = [vp, ci]
     L.b2j_batch_decode.argtypes = [vp, vp]
     L.b2j_batch_decode_timed.argtypes = [vp, vp, ctypes.POINTER(StageTimes)]
     L.b2j_batch_decode_steps.argtypes = [vp, vp, ci, ctypes.POINTER(StageTimes), ctypes.POINTER(ctypes.c_float)]
@@ -159,18 +160,20 @@ def parse_header(data, gate=GATE_EXTENDED):
     return rc, d
 
 
-def _out_shape(d, fmt):
-    return (d.height, d.width, 4) if fmt == OUT_BGRA else ((d.height, d.width, 3) if fmt == OUT_RGB24 else (3, d.height, d.width))
+def _out_shape(d, fmt, scale=1):
+    """Shape of an image's pixels in output format fmt, at 1/scale of its size (ceil(W/scale) x ceil(H/scale))."""
+    w, h = -(-d.width // scale), -(-d.height // scale)
+    return (h, w, 4) if fmt == OUT_BGRA else ((h, w, 3) if fmt == OUT_RGB24 else (3, h, w))
 
 
-def _host_call_args(files, outs, gate, fmt):
+def _host_call_args(files, outs, gate, fmt, scale=1):
     """Argument arrays of the b2j_decode_host* calls; allocates the outputs when none are given."""
     n = len(files)
     if outs is None:
         outs = []
         for f in files:
             rc, d = parse_header(f, gate)
-            outs.append(np.zeros(_out_shape(d, fmt), np.uint8) if rc == 0 else np.zeros((0, 0, 4), np.uint8))
+            outs.append(np.zeros(_out_shape(d, fmt, scale or 1), np.uint8) if rc == 0 else np.zeros((0, 0, 4), np.uint8))
     ptrs = [f if isinstance(f, int) else ctypes.cast(ctypes.c_char_p(f), ctypes.c_void_p).value for f in files]
     fp = ctypes.cast((ctypes.c_void_p * n)(*ptrs), ctypes.POINTER(ctypes.c_char_p))
     return outs, fp, (ctypes.c_void_p * n)(*[o if isinstance(o, int) else o.ctypes.data for o in outs])
@@ -181,13 +184,14 @@ class HostArgs:
     ctypes work per call otherwise): files / lens / outs as for Decoder.decode_host_ex."""
 
     def __init__(self, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0, group_mb=0,
-                 pixel_model=PIXELS_REFERENCE):
+                 pixel_model=PIXELS_REFERENCE, scale=1):
         self.n = len(files)
         self.files = files                      # keeps the bytes objects alive
         lens = lens if lens is not None else [len(f) for f in files]
-        self.outs, self.fp, self.op = _host_call_args(files, outs, gate, out_format)
+        self.outs, self.fp, self.op = _host_call_args(files, outs, gate, out_format, scale)
         self.ln = (ctypes.c_size_t * self.n)(*lens)
-        self.opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, group_mb=group_mb, pixel_model=pixel_model)
+        self.opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, group_mb=group_mb, pixel_model=pixel_model,
+                             scale=scale)
         self.status = np.zeros(self.n, np.int32)
 
 
@@ -235,14 +239,14 @@ def host_free(address):
 
 
 def decode_host_multi(decoders, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0,
-                      pixel_model=PIXELS_REFERENCE):
+                      pixel_model=PIXELS_REFERENCE, scale=1):
     """b2j_decode_host_multi over the given Decoder objects (one per GPU). files: bytes objects or addresses (then `lens`)."""
     L = load_library()
     n = len(files)
     lens = lens if lens is not None else [len(f) for f in files]
-    outs, fp, op = _host_call_args(files, outs, gate, out_format)
+    outs, fp, op = _host_call_args(files, outs, gate, out_format, scale)
     ln = (ctypes.c_size_t * n)(*lens)
-    opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, pixel_model=pixel_model)
+    opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, pixel_model=pixel_model, scale=scale)
     cx = (ctypes.c_void_p * len(decoders))(*[d._h.value for d in decoders])
     status = np.zeros(n, np.int32)
     _check(L.b2j_decode_host_multi(cx, len(decoders), n, fp, ln, ctypes.byref(opts), op, status.ctypes.data), "b2j_decode_host_multi")
@@ -300,14 +304,15 @@ class Decoder:
         return args.outs, args.status
 
     def decode_host_ex(self, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0,
-                       pixel_model=PIXELS_REFERENCE):
-        """b2j_decode_host_ex: like decode_host with an output layout, a pixel model and host threads. files: bytes objects
-        or addresses (then `lens`); outs: numpy arrays or addresses."""
+                       pixel_model=PIXELS_REFERENCE, scale=1):
+        """b2j_decode_host_ex: like decode_host with an output layout, a pixel model, a scale (1, 2, 4 or 8: the libjpeg
+        model's scaled decode) and host threads. files: bytes objects or addresses (then `lens`); outs: numpy arrays or
+        addresses."""
         n = len(files)
         lens = lens if lens is not None else [len(f) for f in files]
-        outs, fp, op = _host_call_args(files, outs, gate, out_format)
+        outs, fp, op = _host_call_args(files, outs, gate, out_format, scale)
         ln = (ctypes.c_size_t * n)(*lens)
-        opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, pixel_model=pixel_model)
+        opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, pixel_model=pixel_model, scale=scale)
         status = np.zeros(n, np.int32)
         _check(self.lib.b2j_decode_host_ex(self._h, n, fp, ln, ctypes.byref(opts), op, status.ctypes.data), "b2j_decode_host_ex")
         return outs, status
@@ -424,17 +429,28 @@ class Batch:
         _check(self.lib.b2j_batch_set_pixel_model(self._h, model), "b2j_batch_set_pixel_model")
         self.pixel_model = model
 
+    def set_scale(self, denom):
+        """1 (default), 2, 4 or 8: the decodes that follow give ceil(W/denom) x ceil(H/denom) pixels, libjpeg-turbo's scaled
+        decode (Pillow's draft()). Needs PIXELS_LIBJPEG when decoding; downscale() is refused while denom != 1."""
+        _check(self.lib.b2j_batch_set_scale(self._h, denom), "b2j_batch_set_scale")
+        self.scale = denom
+
+    def pixel_shape(self, i):
+        """Shape of image i's pixels in the batch's output format and scale."""
+        return _out_shape(self.descs[i], getattr(self, "out_format", OUT_BGRA), getattr(self, "scale", 1))
+
     def pixels(self, i, stream=None):
-        d = self.descs[i]
-        fmt = getattr(self, "out_format", OUT_BGRA)
-        shape = (d.height, d.width, 4) if fmt == OUT_BGRA else ((d.height, d.width, 3) if fmt == OUT_RGB24 else (3, d.height, d.width))
-        out = np.zeros(shape, np.uint8)
+        out = np.zeros(self.pixel_shape(i), np.uint8)
         _check(self.lib.b2j_batch_read_pixels(self._h, stream, i, out.ctypes.data), "b2j_batch_read_pixels")
         return out
 
-    def read_all_pixels(self, outs, stream=None):
+    def read_all_pixels(self, outs=None, stream=None):
+        """Every image's pixels into outs (arrays or addresses; allocated at pixel_shape() when None). Returns outs."""
+        if outs is None:
+            outs = [np.zeros(self.pixel_shape(i), np.uint8) for i in range(self.n)]
         op = (ctypes.c_void_p * self.n)(*[o if isinstance(o, int) else o.ctypes.data for o in outs])
         _check(self.lib.b2j_batch_read_all_pixels(self._h, stream, op), "b2j_batch_read_all_pixels")
+        return outs
 
     def coefs(self, i, stream=None):
         """The reference's coefficient tap: int32 [blk_count, 64], natural order, dequantised."""

@@ -20,6 +20,9 @@
 //   k_idct_islow, k_upsample_ycc
 //       the libjpeg pixel model (B2J_PIXELS_LIBJPEG) instead of k_idct_csc: libjpeg-turbo's ISLOW IDCT into a sample
 //       plane, then its fancy chroma upsampling and fixed-point colour.
+//   k_idct_scaled, k_upsample_scaled
+//       the same model's scaled decode (1/2, 1/4, 1/8): jidctred.c's reduced IDCTs, then upsampling and colour at the
+//       reduced size.
 //   k_expand_coefs
 //       the reference's coefficient tap (int32, dequantised) from the int16 plane, for parity.
 #include <cuda.h>
@@ -1639,6 +1642,8 @@ k_idct_csc(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ 
 //                     and 1x2, replication otherwise), fixed-point YCbCr -> RGB (jdcolor.c), store in the output format
 // Sample plane: image i at byte 64 * blk_first, its components one after another, each an MCU-padded plane of
 // (mcu_count_w * h * 8) x (mcu_count_h * v * 8) bytes -- 64 bytes per block, so the image's share is 64 * blk_count.
+// The scaled decode keeps the component offsets; a component of DCT size ss fills (mcu_count_w * h * ss) x
+// (mcu_count_h * v * ss) bytes at the start of its share.
 
 // One 1-D pass of jpeg_idct_islow (CONST_BITS 13) over d[0..7] (a column, then a row), in place, descaled by N bits.
 // The arithmetic is 64-bit, like libjpeg's JLONG: a dequantised coefficient reaches 32767 * 65535 < 2^31, and the
@@ -1742,6 +1747,195 @@ k_idct_islow(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict_
     }
 }
 
+// ---- the scaled decode (b2j_batch_set_scale: 1/2, 1/4, 1/8), libjpeg-turbo's rules for scale_denom 2, 4, 8
+// Dequantised coefficient (r, c) of the block in tile row `rowp` (swizzle sw): DEQUANTIZE, an int product (fits, see islow_1d).
+__device__ __forceinline__ int64_t tile_coef(const uint8_t *rowp, uint32_t sw, const uint32_t *q, int r, int c)
+{
+    const int32_t coef = *reinterpret_cast<const int16_t *>(rowp + (((uint32_t)r ^ sw) << 4) + c * 2);
+    return (int64_t)(coef * (int32_t)q[8 * r + c]);
+}
+
+// jpeg_idct_islow of the block in row `row` of the tile: 8 rows of 8 samples at dst, `pitch` bytes apart (pitch and dst
+// multiples of 8). k_idct_islow's transform; that kernel keeps its own copy of it and of the tile load below, so that
+// its machine code stays as it was measured.
+__device__ __forceinline__ void islow_block(const uint8_t *tile, uint32_t row, const uint32_t *q, uint8_t *dst, size_t pitch)
+{
+    const uint8_t *rowp = tile + row * 128u;
+    const uint32_t sw = row & 7u;
+    int32_t ws[64];   // jidctint.c's int workspace: the pass-1 results are stored as 32-bit ints
+#pragma unroll
+    for (int c = 0; c < 8; c++)
+    {
+        int64_t col[8];
+#pragma unroll
+        for (int r = 0; r < 8; r++) col[r] = tile_coef(rowp, sw, q, r, c);
+        islow_1d<13 - 2>(col);
+#pragma unroll
+        for (int r = 0; r < 8; r++) ws[8 * r + c] = (int32_t)col[r];
+    }
+#pragma unroll
+    for (int r = 0; r < 8; r++)
+    {
+        int64_t row8[8];
+#pragma unroll
+        for (int c = 0; c < 8; c++) row8[c] = ws[8 * r + c];
+        islow_1d<13 + 2 + 3>(row8);
+        uint2 o;
+        o.x = islow_limit(row8[0]) | islow_limit(row8[1]) << 8 | islow_limit(row8[2]) << 16 | islow_limit(row8[3]) << 24;
+        o.y = islow_limit(row8[4]) | islow_limit(row8[5]) << 8 | islow_limit(row8[6]) << 16 | islow_limit(row8[7]) << 24;
+        *reinterpret_cast<uint2 *>(dst + (size_t)r * pitch) = o;
+    }
+}
+
+// The tile's coefficients arrive by TMA while its side data is staged, as in k_idct_islow.
+__device__ __forceinline__ void libjpeg_tile_load(TileSmem &sm, const CUtensorMap *tmap, const ImgDev *__restrict__ imgs, const TileDev d,
+                                                  const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ samples, int32_t *__restrict__ status)
+{
+    const uint32_t tid = threadIdx.x;
+    if (tid == 0)
+    {
+        mbar_init(&sm.bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_expect_tx(&sm.bar, kTileBlocks * 128);
+        tma_load_2d(sm.tile, tmap, 0, (int)d.row_first, &sm.bar);
+    }
+    side_stage<false>(sm.side, imgs, qtabs, d, samples);   // 32-bit quantisers; sd.pix is not used
+    __syncthreads();
+    uint32_t spins = 0;
+    while (!mbar_try_wait(&sm.bar, 0))
+    {
+        if (++spins > (1u << 22)) { if (tid == 0) atomicOr(&status[d.img], B2J_ST_INTERNAL); break; }   // never hang the GPU
+    }
+}
+
+// A component's DCT size ss as jdmaster.c chooses it for the smallest size mins = 8 / scale: doubled from mins while
+// both of its factors still divide the maxima evenly. Its blocks become ss x ss samples; 4:2:0 at 1/2: luma 4, chroma 8.
+__device__ __forceinline__ uint32_t dct_size(uint32_t h, uint32_t v, uint32_t hmax, uint32_t vmax, uint32_t mins)
+{
+    uint32_t ss = mins;
+    while (ss < 8u && (hmax * mins) % (h * ss * 2u) == 0u && (vmax * mins) % (v * ss * 2u) == 0u) ss *= 2u;
+    return ss;
+}
+
+// One 1-D pass of jidctred.c's jpeg_idct_4x4 over d[0..7] (d[4] is not used): 4 outputs, descaled by N bits.
+template <int N>
+__device__ __forceinline__ void red4_1d(const int64_t d[8], int64_t o[4])
+{
+    const int64_t t0 = d[0] * (1ll << 14);                   // << (CONST_BITS + 1)
+    const int64_t t2 = d[2] * 15137 - d[6] * 6270;           // FIX(1.847759065), FIX(0.765366865)
+    const int64_t t10 = t0 + t2, t12 = t0 - t2;
+    const int64_t a = d[7] * -1730 + d[5] * 11893 + d[3] * -17799 + d[1] * 8697;   // FIX(0.211164243), FIX(1.451774981), FIX(2.172734803), FIX(1.061594337)
+    const int64_t b = d[7] * -4176 + d[5] * -4926 + d[3] * 7373 + d[1] * 20995;    // FIX(0.509795579), FIX(0.601344887), FIX(0.899976223), FIX(2.562915447)
+    constexpr int64_t r = 1ll << (N - 1);
+    o[0] = (t10 + b + r) >> N; o[3] = (t10 - b + r) >> N;
+    o[1] = (t12 + a + r) >> N; o[2] = (t12 - a + r) >> N;
+}
+
+// One 1-D pass of jpeg_idct_2x2 over d[0], d[1], d[3], d[5], d[7]: 2 outputs, descaled by N bits.
+template <int N>
+__device__ __forceinline__ void red2_1d(const int64_t d[8], int64_t o[2])
+{
+    const int64_t t10 = d[0] * (1ll << 15);                  // << (CONST_BITS + 2)
+    const int64_t t0 = d[7] * -5906 + d[5] * 6967 + d[3] * -10426 + d[1] * 29692;  // FIX(0.720959822), FIX(0.850430095), FIX(1.272758580), FIX(3.624509785)
+    constexpr int64_t r = 1ll << (N - 1);
+    o[0] = (t10 + t0 + r) >> N; o[1] = (t10 - t0 + r) >> N;
+}
+
+// jpeg_idct_4x4: 4 rows of 4 samples at dst (pitch and dst multiples of 4). Like islow_block, 64-bit products and a
+// 32-bit workspace; column 4 contributes nothing.
+__device__ __forceinline__ void red4_block(const uint8_t *tile, uint32_t row, const uint32_t *q, uint8_t *dst, size_t pitch)
+{
+    const uint8_t *rowp = tile + row * 128u;
+    const uint32_t sw = row & 7u;
+    int32_t ws[4][8];
+#pragma unroll
+    for (int c = 0; c < 8; c++)
+    {
+        if (c == 4) continue;
+        int64_t col[8], o[4];
+#pragma unroll
+        for (int r = 0; r < 8; r++) col[r] = r == 4 ? 0 : tile_coef(rowp, sw, q, r, c);
+        red4_1d<13 - 2 + 1>(col, o);
+#pragma unroll
+        for (int r = 0; r < 4; r++) ws[r][c] = (int32_t)o[r];
+    }
+#pragma unroll
+    for (int r = 0; r < 4; r++)
+    {
+        int64_t d[8], o[4];
+#pragma unroll
+        for (int c = 0; c < 8; c++) d[c] = c == 4 ? 0 : ws[r][c];
+        red4_1d<13 + 2 + 3 + 1>(d, o);
+        *reinterpret_cast<uint32_t *>(dst + (size_t)r * pitch) =
+            islow_limit(o[0]) | islow_limit(o[1]) << 8 | islow_limit(o[2]) << 16 | islow_limit(o[3]) << 24;
+    }
+}
+
+// jpeg_idct_2x2: 2 rows of 2 samples at dst (pitch and dst even); only rows and columns 0, 1, 3, 5 and 7 contribute.
+__device__ __forceinline__ void red2_block(const uint8_t *tile, uint32_t row, const uint32_t *q, uint8_t *dst, size_t pitch)
+{
+    const uint8_t *rowp = tile + row * 128u;
+    const uint32_t sw = row & 7u;
+    constexpr uint32_t kUsed = 0xABu;   // bits 0, 1, 3, 5, 7
+    int32_t ws[2][8];
+#pragma unroll
+    for (int c = 0; c < 8; c++)
+    {
+        if (!((kUsed >> c) & 1u)) continue;
+        int64_t col[8], o[2];
+#pragma unroll
+        for (int r = 0; r < 8; r++) col[r] = ((kUsed >> r) & 1u) ? tile_coef(rowp, sw, q, r, c) : 0;
+        red2_1d<13 - 2 + 2>(col, o);
+        ws[0][c] = (int32_t)o[0]; ws[1][c] = (int32_t)o[1];
+    }
+#pragma unroll
+    for (int r = 0; r < 2; r++)
+    {
+        int64_t d[8], o[2];
+#pragma unroll
+        for (int c = 0; c < 8; c++) d[c] = ((kUsed >> c) & 1u) ? ws[r][c] : 0;
+        red2_1d<13 + 2 + 3 + 2>(d, o);
+        *reinterpret_cast<uint16_t *>(dst + (size_t)r * pitch) = (uint16_t)(islow_limit(o[0]) | islow_limit(o[1]) << 8);
+    }
+}
+
+// The scaled decode's IDCT: every block becomes ss x ss samples of its component's plane (pitch mcu_count_w * h * ss),
+// by jidctred.c's reduced transforms or by jpeg_idct_islow (ss 8), jpeg_idct_1x1: (DC * q + 4) >> 3. The plane keeps
+// its 64 bytes per block. Threads take the tile's blocks component by component (the luma blocks of all its MCUs,
+// then Cb's, then Cr's), so that a warp mixes transform sizes only where one component's run ends inside it: never in
+// a full 4:2:0 tile (128 luma, 32 + 32 chroma blocks).
+__global__ void __launch_bounds__(kTileBlocks)
+k_idct_scaled(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
+              const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ samples, int32_t *__restrict__ status, uint32_t mins)
+{
+    TileSmem &sm = *tile_smem();
+    const uint32_t tid = threadIdx.x;
+    const TileDev d = tiles[blockIdx.x];
+    libjpeg_tile_load(sm, &tmap, imgs, d, qtabs, samples, status);
+    const ImgDev *im = imgs + d.img;
+    const uint32_t sp = sm.side.samp, n = sm.side.n_mcus;
+    const uint32_t yh = sp & 15u, yv = (sp >> 4) & 15u, uh = (sp >> 8) & 15u, uv = (sp >> 12) & 15u, vh = (sp >> 16) & 15u, vv = (sp >> 20) & 15u;
+    const uint32_t ny = yh * yv, nu = uh * uv, tot = ny + nu + vh * vv;
+    if (tid >= n * tot) return;
+    const uint32_t comp = (tid >= n * ny ? 1u : 0u) + (tid >= n * (ny + nu) ? 1u : 0u);
+    const uint32_t before = (comp > 0 ? ny : 0u) + (comp > 1 ? nu : 0u);   // blocks of the earlier components per MCU
+    const uint32_t nc = comp == 0 ? ny : (comp == 1 ? nu : vh * vv);
+    const uint32_t j = tid - n * before, m = j / nc, k = j % nc;        // MCU m of the tile, block k of the component in it
+    const uint32_t h = comp == 0 ? yh : (comp == 1 ? uh : vh), v = comp == 0 ? yv : (comp == 1 ? uv : vv);
+    const uint32_t ss = dct_size(h, v, yh, yv, mins);   // the chroma factors divide the luma's (geometry_ok): those are the maxima
+    const uint32_t mcu_count = __ldg(&im->mcu_count), mcw = __ldg(&im->mcu_count_w), blk_first = __ldg(&im->blk_first);
+    const size_t pitch = (size_t)mcw * h * ss;
+    const uint2 mxy = sm.side.mcu_xy[m];
+    uint8_t *dst = samples + 64ull * ((size_t)blk_first + (size_t)mcu_count * before) + (size_t)((mxy.y * v + k / h) * ss) * pitch +
+                   (mxy.x * h + k % h) * ss;
+    const uint32_t row = m * tot + before + k;   // the block's row in the tile (MCU-interleaved)
+    const uint32_t *q = sm.side.qt + comp * kQtStride;
+    if (ss == 8u) islow_block(sm.tile, row, q, dst, pitch);
+    else if (ss == 4u) red4_block(sm.tile, row, q, dst, pitch);
+    else if (ss == 2u) red2_block(sm.tile, row, q, dst, pitch);
+    else *dst = (uint8_t)islow_limit((tile_coef(sm.tile + row * 128u, row & 7u, q, 0, 0) + 4) >> 3);
+}
+
 // One component of an image in the sample plane, and how it becomes full resolution.
 struct UpComp
 {
@@ -1830,6 +2024,67 @@ k_upsample_ycc(const uint8_t *__restrict__ samples, const ImgDev *__restrict__ i
             const uint32_t x = min(px + k, width - 1u);   // the stores skip pixels behind the last column
             const uint32_t Y = up_sample(cy, x, py);
             const uint32_t rgb = gray ? Y * 0x10101u : ycc_rgb_libjpeg((int32_t)Y, (int32_t)up_sample(cu, x, py), (int32_t)up_sample(cv, x, py));
+            const uint32_t sh = 16u * (k & 1u);
+            R[k >> 1] |= (rgb & 0xFFu) << sh; Gc[k >> 1] |= ((rgb >> 8) & 0xFFu) << sh; B[k >> 1] |= (rgb >> 16) << sh;
+        }
+        constexpr uint32_t bpp = FMT == B2J_OUT_BGRA ? 4u : (FMT == B2J_OUT_RGB24 ? 3u : 1u);
+        store_pixels4<FMT>(pix + im.pix_off + ((size_t)py * width + px) * bpp, (size_t)width * height, px, width, (width & 3u) == 0u, R, Gc, B);
+    }
+}
+
+// ---- upsampling and colour of the scaled decode, at the output size ceil(W / s) x ceil(H / s), s = 8 / mins
+// A component of DCT size ss (dct_size) has ceil(W * h * ss / (hmax * 8)) x ceil(H * v * ss / (vmax * 8)) samples (jdmaster.c's
+// downsampled_width / _height) and is upsampled by hmax * mins / (h * ss) x vmax * mins / (v * ss).
+__device__ __forceinline__ UpComp up_comp_scaled(const uint8_t *p, uint32_t h, uint32_t v, uint32_t hmax, uint32_t vmax, uint32_t mcw,
+                                                 uint32_t width, uint32_t height, uint32_t mins)
+{
+    const uint32_t ss = dct_size(h, v, hmax, vmax, mins);
+    UpComp c;
+    c.p = p; c.pitch = mcw * h * ss;
+    c.dw = (width * h * ss + hmax * 8u - 1u) / (hmax * 8u); c.dh = (height * v * ss + vmax * 8u - 1u) / (vmax * 8u);
+    c.rh = hmax * mins / (h * ss); c.rv = vmax * mins / (v * ss);
+    return c;
+}
+
+// jdsample.c applies its fancy filters only while the smallest DCT size exceeds 1: at 1/8 every ratio replicates.
+__device__ __forceinline__ uint32_t up_sample_scaled(const UpComp &c, uint32_t x, uint32_t y, bool fancy)
+{
+    return fancy ? up_sample(c, x, y) : __ldg(c.p + (size_t)(y / c.rv) * c.pitch + x / c.rh);
+}
+
+// k_upsample_ycc at the output size; its own copy, so that k_upsample_ycc keeps its code.
+template <int FMT>
+__global__ void __launch_bounds__(256)
+k_upsample_scaled(const uint8_t *__restrict__ samples, const ImgDev *__restrict__ imgs, uint32_t n_images, uint8_t *__restrict__ pix, uint32_t mins)
+{
+    const uint32_t s = 8u / mins;
+    const bool fancy = mins > 1u;
+    for (uint32_t img = blockIdx.y; img < n_images; img += gridDim.y)
+    {
+        const ImgDev &im = imgs[img];
+        const uint32_t width = (im.width + s - 1u) / s, height = (im.height + s - 1u) / s, gw = (width + 3u) / 4u;
+        const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+        if (i >= gw * height) continue;
+        const uint32_t py = i / gw, px = (i % gw) * 4u;
+        const uint32_t sp = im.samp, mcw = im.mcu_count_w;
+        const uint32_t yh = sp & 15u, yv = (sp >> 4) & 15u, uh = (sp >> 8) & 15u, uv = (sp >> 12) & 15u, vh = (sp >> 16) & 15u, vv = (sp >> 20) & 15u;
+        const uint8_t *p0 = samples + 64ull * im.blk_first;
+        const bool gray = im.mode == kModeGray;
+        const UpComp cy = up_comp_scaled(p0, yh, yv, yh, yv, mcw, im.width, im.height, mins);
+        UpComp cu = cy, cv = cy;
+        if (!gray)
+        {
+            cu = up_comp_scaled(p0 + 64ull * im.mcu_count * (yh * yv), uh, uv, yh, yv, mcw, im.width, im.height, mins);
+            cv = up_comp_scaled(p0 + 64ull * im.mcu_count * (yh * yv + uh * uv), vh, vv, yh, yv, mcw, im.width, im.height, mins);
+        }
+        uint32_t R[2] = {0u, 0u}, Gc[2] = {0u, 0u}, B[2] = {0u, 0u};
+#pragma unroll
+        for (uint32_t k = 0; k < 4u; k++)
+        {
+            const uint32_t x = min(px + k, width - 1u);   // the stores skip pixels behind the last column
+            const uint32_t Y = up_sample_scaled(cy, x, py, fancy);
+            const uint32_t rgb = gray ? Y * 0x10101u
+                                      : ycc_rgb_libjpeg((int32_t)Y, (int32_t)up_sample_scaled(cu, x, py, fancy), (int32_t)up_sample_scaled(cv, x, py, fancy));
             const uint32_t sh = 16u * (k & 1u);
             R[k >> 1] |= (rgb & 0xFFu) << sh; Gc[k >> 1] |= ((rgb >> 8) & 0xFFu) << sh; B[k >> 1] |= (rgb >> 16) << sh;
         }
@@ -1963,13 +2218,21 @@ static void launch_idct_format(const DecodeArgs &a, cudaStream_t s)
     launch_idct_kind<FMT, kTileGeneric>(a, a.generic_tile0, a.n_tiles - a.generic_tile0, s);
 }
 
-// The libjpeg model: the IDCT over every tile into the sample plane, then the upsampling / colour pass over every image.
+// The libjpeg model: the IDCT over every tile into the sample plane, then the upsampling / colour pass over every image;
+// the scaled decode has a pair of its own.
 template <int FMT>
 static void launch_libjpeg_format(const DecodeArgs &a, cudaStream_t s)
 {
-    k_idct_islow<<<a.n_tiles, kTileBlocks, kTileSmemBytes, s>>>(*a.tmap, a.imgs, a.tiles, a.qtabs, a.samples, a.status);
     const dim3 grid((a.max_px_groups + 255u) / 256u, a.n_images < 65535u ? a.n_images : 65535u);
-    k_upsample_ycc<FMT><<<grid, 256, 0, s>>>(a.samples, a.imgs, a.n_images, a.pixels);
+    if (a.scale == 1)
+    {
+        k_idct_islow<<<a.n_tiles, kTileBlocks, kTileSmemBytes, s>>>(*a.tmap, a.imgs, a.tiles, a.qtabs, a.samples, a.status);
+        k_upsample_ycc<FMT><<<grid, 256, 0, s>>>(a.samples, a.imgs, a.n_images, a.pixels);
+        return;
+    }
+    const uint32_t mins = 8u / a.scale;   // the smallest DCT size
+    k_idct_scaled<<<a.n_tiles, kTileBlocks, kTileSmemBytes, s>>>(*a.tmap, a.imgs, a.tiles, a.qtabs, a.samples, a.status, mins);
+    k_upsample_scaled<FMT><<<grid, 256, 0, s>>>(a.samples, a.imgs, a.n_images, a.pixels, mins);
 }
 
 int idct_launches(const DecodeArgs &a)

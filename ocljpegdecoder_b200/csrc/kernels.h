@@ -45,7 +45,8 @@ struct DecodeArgs
     bool any_wide_q;         // some quantiser of the batch exceeds 255 (16-bit DQT): generic dequantisation
     int pixel_model;         // B2J_PIXELS_*: which pixels the IDCT/colour stage computes (b2j_batch_set_pixel_model)
     uint8_t *samples;        // B2J_PIXELS_LIBJPEG: the sample plane, 64 B per block (allocated by the first decode in that model)
-    uint32_t max_px_groups;  // largest ceil(W / 4) * H of the batch: the grid of the libjpeg model's upsampling kernel
+    uint32_t max_px_groups;  // largest ceil(OW / 4) * OH of the batch's output sizes: the grid of the libjpeg model's upsampling kernel
+    uint32_t scale;          // B2J_PIXELS_LIBJPEG: the output is ceil(W / scale) x ceil(H / scale); 1, 2, 4 or 8 (b2j_batch_set_scale)
 };
 
 cudaError_t init_constants();

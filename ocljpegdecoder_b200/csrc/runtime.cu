@@ -243,7 +243,13 @@ const ImgDev *image_of(const b2j_batch *b, int image) { return b && image >= 0 &
 // Bytes per pixel of an output format (B2J_OUT_*).
 size_t format_bpp(int fmt) { return fmt == B2J_OUT_BGRA ? 4 : 3; }
 
-size_t image_bytes(const b2j_batch *b, const ImgDev &im) { return (size_t)im.width * im.height * format_bpp(b->args.out_format); }
+// An image's output size at the batch's scale: ceil(W / scale) x ceil(H / scale).
+uint32_t out_width(const b2j_batch *b, const ImgDev &im) { return (im.width + b->args.scale - 1) / b->args.scale; }
+uint32_t out_height(const b2j_batch *b, const ImgDev &im) { return (im.height + b->args.scale - 1) / b->args.scale; }
+
+size_t image_bytes(const b2j_batch *b, const ImgDev &im) { return (size_t)out_width(b, im) * out_height(b, im) * format_bpp(b->args.out_format); }
+
+bool scale_ok(int denom) { return denom == 1 || denom == 2 || denom == 4 || denom == 8; }
 
 // One device->host copy on the call's stream, waited for.
 int read_back(b2j_batch *b, void *stream, void *dst, const void *src, size_t bytes)
@@ -607,6 +613,7 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     a.pixel_model = B2J_PIXELS_REFERENCE;
     a.samples = nullptr;
     a.max_px_groups = max_px_groups;
+    a.scale = 1;
     {
         const char *sp = getenv("B2J_SYNC_PRE");
         a.sync_use_pre = !(sp && atoi(sp) == 0);
@@ -670,6 +677,11 @@ constexpr size_t kStepEvents = 5;
 static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStepEvents or NULL */)
 {
     if (!b->uploaded) { t_last_error = "b2j_batch_decode before b2j_batch_upload"; return B2J_E_ARG; }
+    if (b->args.scale != 1 && b->args.pixel_model != B2J_PIXELS_LIBJPEG)
+    {
+        t_last_error = "a scaled decode (b2j_batch_set_scale) needs the libjpeg pixel model: the reference has none";
+        return B2J_E_ARG;
+    }
     if (b->args.pixel_model == B2J_PIXELS_LIBJPEG && !b->d_samples.p)
     {
         // the sample plane: 64 bytes per block, image by image at 64 * blk_first
@@ -779,6 +791,16 @@ extern "C" int b2j_batch_set_pixel_model(b2j_batch *b, int model)
     return B2J_OK;
 }
 
+extern "C" int b2j_batch_set_scale(b2j_batch *b, int denom)
+{
+    if (!b || !scale_ok(denom)) return B2J_E_ARG;
+    b->args.scale = (uint32_t)denom;
+    uint32_t groups = 0;   // the upsampling kernel's grid: one thread per 4 output pixels of a row
+    for (const ImgDev &im : b->imgs) groups = std::max(groups, (out_width(b, im) + 3) / 4 * out_height(b, im));
+    b->args.max_px_groups = groups;
+    return B2J_OK;
+}
+
 extern "C" int b2j_batch_pixels_device(const b2j_batch *b, int image, void **dptr, size_t *nbytes)
 {
     const ImgDev *im = image_of(b, image);
@@ -845,6 +867,7 @@ static void small_dims(const ImgDev &im, int f, uint32_t *ow, uint32_t *oh)
 extern "C" int b2j_batch_downscale(b2j_batch *b, void *stream, int factor)
 {
     if (!b || (factor != 2 && factor != 4 && factor != 8)) return B2J_E_ARG;
+    if (b->args.scale != 1) { t_last_error = "b2j_batch_downscale of a scaled decode"; return B2J_E_ARG; }
     CU_TRY(cudaSetDevice(b->ctx->device));
     cudaStream_t s = pick_stream(b, stream);
     const int fmt = b->args.out_format;
@@ -959,6 +982,13 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
     if (fmt != B2J_OUT_BGRA && fmt != B2J_OUT_RGB24 && fmt != B2J_OUT_RGB_PLANAR) return B2J_E_ARG;
     const int model = opts->pixel_model;
     if (model != B2J_PIXELS_REFERENCE && model != B2J_PIXELS_LIBJPEG) return B2J_E_ARG;
+    const int scale = opts->scale ? opts->scale : 1;
+    if (!scale_ok(scale)) return B2J_E_ARG;
+    if (scale != 1 && model != B2J_PIXELS_LIBJPEG)
+    {
+        t_last_error = "a scaled decode (b2j_host_opts.scale) needs the libjpeg pixel model: the reference has none";
+        return B2J_E_ARG;
+    }
     CU_TRY(cudaSetDevice(ctx->device));
     const int gate = opts->gate;
     const int group = opts->group > 0 ? opts->group : 32;
@@ -1028,6 +1058,7 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
                 if (G.rc != B2J_OK) G.err = t_last_error;
                 else
                 {
+                    b2j_batch_set_scale(G.b, scale);   // before the packing: it sizes the images
                     pack_pixel_plane(G.b, fmt);
                     b2j_batch_set_pixel_model(G.b, model);
                 }
