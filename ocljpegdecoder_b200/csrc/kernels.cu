@@ -17,12 +17,9 @@
 //       replication + exact integer YCbCr->BGRA and 128-bit coalesced stores. Replaces
 //       Fast_IDCT (cpuIDCT8x8.cpp:25-127), the upsample/colour loop of decode_mcu_data()
 //       (decoder.cpp:429-495) and the OpenCL kernels idct8x8.cl:157-222.
-//   k_idct_islow, k_upsample_ycc
-//       the libjpeg pixel model (B2J_PIXELS_LIBJPEG) instead of k_idct_csc: libjpeg-turbo's ISLOW IDCT into a sample
-//       plane, then its fancy chroma upsampling and fixed-point colour.
-//   k_idct_scaled, k_upsample_scaled
-//       the same model's scaled decode (1/2, 1/4, 1/8): jidctred.c's reduced IDCTs, then upsampling and colour at the
-//       reduced size.
+//   k_idct_libjpeg, k_upsample_libjpeg
+//       the libjpeg pixel model (B2J_PIXELS_LIBJPEG) instead of k_idct_csc, at every scale (1, 1/2, 1/4, 1/8):
+//       libjpeg-turbo's ISLOW or reduced IDCTs into a sample plane, then its chroma upsampling and fixed-point colour.
 //   k_expand_coefs
 //       the reference's coefficient tap (int32, dequantised) from the int16 plane, for parity.
 #include <cuda.h>
@@ -1580,8 +1577,33 @@ __device__ __forceinline__ void side_stage(TileSide &sd, const ImgDev *__restric
     }
 }
 
-// One tile per CTA. The 24 KB coefficient tile arrives by one TMA tensor load (128-byte swizzle,
-// mbarrier completion) issued by thread 0 while the other threads fetch the side data.
+// The CTA's tile (tiles[blockIdx.x], returned): its 24 KB of coefficients arrive in sm.tile by one TMA tensor load
+// (128-byte swizzle, mbarrier completion) issued by thread 0 while the other threads stage the side data. The wait is
+// bounded: a load that never completes flags the image with B2J_ST_INTERNAL.
+template <bool NARROWQ>
+__device__ __forceinline__ TileDev tile_load(TileSmem &sm, const CUtensorMap *tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
+                                             const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ pix, int32_t *__restrict__ status)
+{
+    const uint32_t tid = threadIdx.x;
+    const TileDev d = tiles[blockIdx.x];
+    if (tid == 0)
+    {
+        mbar_init(&sm.bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_expect_tx(&sm.bar, kTileBlocks * 128);
+        tma_load_2d(sm.tile, tmap, 0, (int)d.row_first, &sm.bar);
+    }
+    side_stage<NARROWQ>(sm.side, imgs, qtabs, d, pix);
+    __syncthreads();   // barrier initialisation + side data visible
+    uint32_t spins = 0;
+    while (!mbar_try_wait(&sm.bar, 0))
+    {
+        if (++spins > (1u << 22)) { if (tid == 0) atomicOr(&status[d.img], B2J_ST_INTERNAL); break; }   // never hang the GPU
+    }
+    return d;
+}
+
+// One tile per CTA, loaded by tile_load.
 // Measured on B200 (profiles/): a persistent double-buffered variant and a warp-autonomous variant of
 // this kernel were both slower -- the kernel is bound by dependent-issue latency at 24 warps per SM,
 // not by the latency in front of a tile, so the simplest structure wins.
@@ -1598,21 +1620,7 @@ k_idct_csc(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ 
 {
     TileSmem &sm = *tile_smem();
     const uint32_t tid = threadIdx.x;
-    const TileDev d = tiles[blockIdx.x];
-    if (tid == 0)
-    {
-        mbar_init(&sm.bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        mbar_expect_tx(&sm.bar, kTileBlocks * 128);
-        tma_load_2d(sm.tile, &tmap, 0, (int)d.row_first, &sm.bar);
-    }
-    side_stage<NARROWQ>(sm.side, imgs, qtabs, d, pix);
-    __syncthreads();   // barrier initialisation + side data visible
-    uint32_t spins = 0;
-    while (!mbar_try_wait(&sm.bar, 0))
-    {
-        if (++spins > (1u << 22)) { if (tid == 0) atomicOr(&status[d.img], B2J_ST_INTERNAL); break; }   // never hang the GPU
-    }
+    tile_load<NARROWQ>(sm, &tmap, imgs, tiles, qtabs, pix, status);
     if (KIND == kTileGray)
     {
         idct_phase<0, 0, NARROWQ>(sm.tile, sm.side);
@@ -1634,16 +1642,18 @@ k_idct_csc(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ 
 }
 
 // =====================================================================================
-// The libjpeg pixel model (B2J_PIXELS_LIBJPEG): libjpeg-turbo's default decode of the same coefficients, in two kernels
-// of their own so that the reference model's colour kernel keeps its code and its instruction cache (DESIGN.md §3).
-//   k_idct_islow      per tile, one thread per block: dequantise, ISLOW IDCT (jidctint.c), range limit; 64 sample bytes
-//                     per block into the sample plane
-//   k_upsample_ycc    per 4-pixel group: chroma upsampling as jdsample.c chooses it (fancy triangle filter for 2x1, 2x2
-//                     and 1x2, replication otherwise), fixed-point YCbCr -> RGB (jdcolor.c), store in the output format
-// Sample plane: image i at byte 64 * blk_first, its components one after another, each an MCU-padded plane of
-// (mcu_count_w * h * 8) x (mcu_count_h * v * 8) bytes -- 64 bytes per block, so the image's share is 64 * blk_count.
-// The scaled decode keeps the component offsets; a component of DCT size ss fills (mcu_count_w * h * ss) x
-// (mcu_count_h * v * ss) bytes at the start of its share.
+// The libjpeg pixel model (B2J_PIXELS_LIBJPEG): libjpeg-turbo's default decode of the same coefficients at scale_denom
+// s = 1, 2, 4 or 8 (b2j_batch_set_scale), in two kernels of their own so that the reference model's colour kernel keeps
+// its code and its instruction cache (DESIGN.md §3). Both take the smallest DCT size MINS = 8 / s as a template parameter.
+//   k_idct_libjpeg      per tile, one thread per block: dequantise, then at the component's DCT size ss (jdmaster.c)
+//                       the ISLOW IDCT (jidctint.c, ss 8) or a reduced one (jidctred.c), range limit; ss x ss samples
+//                       per block into the sample plane
+//   k_upsample_libjpeg  per 4-pixel group of the ceil(W / s) x ceil(H / s) output: chroma upsampling as jdsample.c
+//                       chooses it (fancy triangle filter for 2x1, 2x2 and 1x2 while MINS > 1, replication otherwise),
+//                       fixed-point YCbCr -> RGB (jdcolor.c), store in the output format
+// Sample plane: image i at byte 64 * blk_first, its components one after another, each with a share of 64 bytes per
+// block, so the image's share is 64 * blk_count. A component of DCT size ss fills (mcu_count_w * h * ss) x
+// (mcu_count_h * v * ss) bytes at the start of its share: at ss 8, all of it.
 
 // One 1-D pass of jpeg_idct_islow (CONST_BITS 13) over d[0..7] (a column, then a row), in place, descaled by N bits.
 // The arithmetic is 64-bit, like libjpeg's JLONG: a dequantised coefficient reaches 32767 * 65535 < 2^31, and the
@@ -1678,76 +1688,6 @@ __device__ __forceinline__ uint32_t islow_limit(int64_t y)
     return m < 256u ? m : (m < 640u ? 255u : 0u);
 }
 
-// Every tile kind in one kernel: the component of a block comes from the image's sampling factors (gray: 0x11, one block).
-__global__ void __launch_bounds__(kTileBlocks)
-k_idct_islow(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
-             const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ samples, int32_t *__restrict__ status)
-{
-    TileSmem &sm = *tile_smem();
-    const uint32_t tid = threadIdx.x;
-    const TileDev d = tiles[blockIdx.x];
-    if (tid == 0)
-    {
-        mbar_init(&sm.bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        mbar_expect_tx(&sm.bar, kTileBlocks * 128);
-        tma_load_2d(sm.tile, &tmap, 0, (int)d.row_first, &sm.bar);
-    }
-    side_stage<false>(sm.side, imgs, qtabs, d, samples);   // 32-bit quantisers; sd.pix is not used
-    __syncthreads();
-    uint32_t spins = 0;
-    while (!mbar_try_wait(&sm.bar, 0))
-    {
-        if (++spins > (1u << 22)) { if (tid == 0) atomicOr(&status[d.img], B2J_ST_INTERNAL); break; }   // never hang the GPU
-    }
-    const ImgDev *im = imgs + d.img;
-    const uint32_t sp = sm.side.samp;
-    const uint32_t yh = sp & 15u, yv = (sp >> 4) & 15u, uh = (sp >> 8) & 15u, uv = (sp >> 12) & 15u, vh = (sp >> 16) & 15u;
-    const uint32_t ny = yh * yv, nu = uh * uv, tot = ny + nu + vh * ((sp >> 20) & 15u);
-    if (tid >= sm.side.n_mcus * tot) return;
-    const uint32_t m = tid / tot, bi = tid % tot;
-    const uint32_t comp = (bi >= ny ? 1u : 0u) + (bi >= ny + nu ? 1u : 0u);
-    const uint32_t k = bi - (comp > 0 ? ny : 0u) - (comp > 1 ? nu : 0u);   // block inside the component's part of the MCU
-    const uint32_t h = comp == 0 ? yh : (comp == 1 ? uh : vh);
-    const uint32_t v = comp == 0 ? yv : (comp == 1 ? uv : (sp >> 20) & 15u);
-    const uint32_t mcu_count = __ldg(&im->mcu_count), mcw = __ldg(&im->mcu_count_w), blk_first = __ldg(&im->blk_first);
-    const size_t pitch = (size_t)mcw * h * 8u;
-    const uint2 mxy = sm.side.mcu_xy[m];
-    uint8_t *dst = samples + 64ull * ((size_t)blk_first + (size_t)mcu_count * ((comp > 0 ? ny : 0u) + (comp > 1 ? nu : 0u))) +
-                   (size_t)((mxy.y * v + k / h) * 8u) * pitch + (mxy.x * h + k % h) * 8u;
-    const uint32_t *q = sm.side.qt + comp * kQtStride;
-    const uint8_t *rowp = sm.tile + tid * 128u;
-    const uint32_t sw = tid & 7u;
-    int32_t ws[64];   // jidctint.c's int workspace: the pass-1 results are stored as 32-bit ints
-#pragma unroll
-    for (int c = 0; c < 8; c++)
-    {
-        int64_t col[8];
-#pragma unroll
-        for (int r = 0; r < 8; r++)
-        {
-            const int32_t coef = *reinterpret_cast<const int16_t *>(rowp + (((uint32_t)r ^ sw) << 4) + c * 2);
-            col[r] = (int64_t)(coef * (int32_t)q[8 * r + c]);   // DEQUANTIZE: an int product (fits, see islow_1d)
-        }
-        islow_1d<13 - 2>(col);
-#pragma unroll
-        for (int r = 0; r < 8; r++) ws[8 * r + c] = (int32_t)col[r];
-    }
-#pragma unroll
-    for (int r = 0; r < 8; r++)
-    {
-        int64_t row[8];
-#pragma unroll
-        for (int c = 0; c < 8; c++) row[c] = ws[8 * r + c];
-        islow_1d<13 + 2 + 3>(row);
-        uint2 o;
-        o.x = islow_limit(row[0]) | islow_limit(row[1]) << 8 | islow_limit(row[2]) << 16 | islow_limit(row[3]) << 24;
-        o.y = islow_limit(row[4]) | islow_limit(row[5]) << 8 | islow_limit(row[6]) << 16 | islow_limit(row[7]) << 24;
-        *reinterpret_cast<uint2 *>(dst + (size_t)r * pitch) = o;   // pitch and offsets are multiples of 8
-    }
-}
-
-// ---- the scaled decode (b2j_batch_set_scale: 1/2, 1/4, 1/8), libjpeg-turbo's rules for scale_denom 2, 4, 8
 // Dequantised coefficient (r, c) of the block in tile row `rowp` (swizzle sw): DEQUANTIZE, an int product (fits, see islow_1d).
 __device__ __forceinline__ int64_t tile_coef(const uint8_t *rowp, uint32_t sw, const uint32_t *q, int r, int c)
 {
@@ -1756,8 +1696,7 @@ __device__ __forceinline__ int64_t tile_coef(const uint8_t *rowp, uint32_t sw, c
 }
 
 // jpeg_idct_islow of the block in row `row` of the tile: 8 rows of 8 samples at dst, `pitch` bytes apart (pitch and dst
-// multiples of 8). k_idct_islow's transform; that kernel keeps its own copy of it and of the tile load below, so that
-// its machine code stays as it was measured.
+// multiples of 8).
 __device__ __forceinline__ void islow_block(const uint8_t *tile, uint32_t row, const uint32_t *q, uint8_t *dst, size_t pitch)
 {
     const uint8_t *rowp = tile + row * 128u;
@@ -1784,27 +1723,6 @@ __device__ __forceinline__ void islow_block(const uint8_t *tile, uint32_t row, c
         o.x = islow_limit(row8[0]) | islow_limit(row8[1]) << 8 | islow_limit(row8[2]) << 16 | islow_limit(row8[3]) << 24;
         o.y = islow_limit(row8[4]) | islow_limit(row8[5]) << 8 | islow_limit(row8[6]) << 16 | islow_limit(row8[7]) << 24;
         *reinterpret_cast<uint2 *>(dst + (size_t)r * pitch) = o;
-    }
-}
-
-// The tile's coefficients arrive by TMA while its side data is staged, as in k_idct_islow.
-__device__ __forceinline__ void libjpeg_tile_load(TileSmem &sm, const CUtensorMap *tmap, const ImgDev *__restrict__ imgs, const TileDev d,
-                                                  const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ samples, int32_t *__restrict__ status)
-{
-    const uint32_t tid = threadIdx.x;
-    if (tid == 0)
-    {
-        mbar_init(&sm.bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        mbar_expect_tx(&sm.bar, kTileBlocks * 128);
-        tma_load_2d(sm.tile, tmap, 0, (int)d.row_first, &sm.bar);
-    }
-    side_stage<false>(sm.side, imgs, qtabs, d, samples);   // 32-bit quantisers; sd.pix is not used
-    __syncthreads();
-    uint32_t spins = 0;
-    while (!mbar_try_wait(&sm.bar, 0))
-    {
-        if (++spins > (1u << 22)) { if (tid == 0) atomicOr(&status[d.img], B2J_ST_INTERNAL); break; }   // never hang the GPU
     }
 }
 
@@ -1899,19 +1817,20 @@ __device__ __forceinline__ void red2_block(const uint8_t *tile, uint32_t row, co
     }
 }
 
-// The scaled decode's IDCT: every block becomes ss x ss samples of its component's plane (pitch mcu_count_w * h * ss),
-// by jidctred.c's reduced transforms or by jpeg_idct_islow (ss 8), jpeg_idct_1x1: (DC * q + 4) >> 3. The plane keeps
-// its 64 bytes per block. Threads take the tile's blocks component by component (the luma blocks of all its MCUs,
-// then Cb's, then Cr's), so that a warp mixes transform sizes only where one component's run ends inside it: never in
-// a full 4:2:0 tile (128 luma, 32 + 32 chroma blocks).
+// Every tile kind in one kernel: the component of a block comes from the image's sampling factors (gray: 0x11, one
+// block). Every block becomes ss x ss samples of its component's plane (pitch mcu_count_w * h * ss), by jpeg_idct_islow
+// (ss 8), jidctred.c's reduced transforms or jpeg_idct_1x1: (DC * q + 4) >> 3. Threads take the tile's blocks component
+// by component (the luma blocks of all its MCUs, then Cb's, then Cr's), so that a warp mixes transform sizes only where
+// one component's run ends inside it: never in a full 4:2:0 tile (128 luma, 32 + 32 chroma blocks). MINS, the smallest
+// DCT size, is a template parameter so that the full-size decode (MINS 8) carries no reduced transform.
+template <uint32_t MINS>
 __global__ void __launch_bounds__(kTileBlocks)
-k_idct_scaled(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
-              const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ samples, int32_t *__restrict__ status, uint32_t mins)
+k_idct_libjpeg(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
+               const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ samples, int32_t *__restrict__ status)
 {
     TileSmem &sm = *tile_smem();
     const uint32_t tid = threadIdx.x;
-    const TileDev d = tiles[blockIdx.x];
-    libjpeg_tile_load(sm, &tmap, imgs, d, qtabs, samples, status);
+    const TileDev d = tile_load<false>(sm, &tmap, imgs, tiles, qtabs, samples, status);   // 32-bit quantisers; sd.pix is not used
     const ImgDev *im = imgs + d.img;
     const uint32_t sp = sm.side.samp, n = sm.side.n_mcus;
     const uint32_t yh = sp & 15u, yv = (sp >> 4) & 15u, uh = (sp >> 8) & 15u, uv = (sp >> 12) & 15u, vh = (sp >> 16) & 15u, vv = (sp >> 20) & 15u;
@@ -1922,7 +1841,7 @@ k_idct_scaled(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict
     const uint32_t nc = comp == 0 ? ny : (comp == 1 ? nu : vh * vv);
     const uint32_t j = tid - n * before, m = j / nc, k = j % nc;        // MCU m of the tile, block k of the component in it
     const uint32_t h = comp == 0 ? yh : (comp == 1 ? uh : vh), v = comp == 0 ? yv : (comp == 1 ? uv : vv);
-    const uint32_t ss = dct_size(h, v, yh, yv, mins);   // the chroma factors divide the luma's (geometry_ok): those are the maxima
+    const uint32_t ss = dct_size(h, v, yh, yv, MINS);   // the chroma factors divide the luma's (geometry_ok): those are the maxima
     const uint32_t mcu_count = __ldg(&im->mcu_count), mcw = __ldg(&im->mcu_count_w), blk_first = __ldg(&im->blk_first);
     const size_t pitch = (size_t)mcw * h * ss;
     const uint2 mxy = sm.side.mcu_xy[m];
@@ -1936,51 +1855,58 @@ k_idct_scaled(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict
     else *dst = (uint8_t)islow_limit((tile_coef(sm.tile + row * 128u, row & 7u, q, 0, 0) + 4) >> 3);
 }
 
-// One component of an image in the sample plane, and how it becomes full resolution.
+// One component of an image in the sample plane, and how it becomes output resolution.
 struct UpComp
 {
     const uint8_t *p;     // first sample of the component's plane
     uint32_t pitch;       // bytes per row of the plane
-    uint32_t dw, dh;      // samples that belong to the image: ceil(W * h / hmax) x ceil(H * v / vmax)
-    uint32_t rh, rv;      // upsampling ratio hmax / h, vmax / v
+    uint32_t dw, dh;      // samples that belong to the image (up_comp)
+    uint32_t rh, rv;      // upsampling ratios (up_comp)
 };
 
-__device__ __forceinline__ UpComp up_comp(const uint8_t *p, uint32_t h, uint32_t v, uint32_t hmax, uint32_t vmax, uint32_t mcw, uint32_t width,
-                                          uint32_t height)
+// A component of DCT size ss (dct_size) has ceil(W * h * ss / (hmax * 8)) x ceil(H * v * ss / (vmax * 8)) samples (jdmaster.c's
+// downsampled_width / _height) and is upsampled by hmax * mins / (h * ss) x vmax * mins / (v * ss).
+__device__ __forceinline__ UpComp up_comp(const uint8_t *p, uint32_t h, uint32_t v, uint32_t hmax, uint32_t vmax, uint32_t mcw,
+                                          uint32_t width, uint32_t height, uint32_t mins)
 {
+    const uint32_t ss = dct_size(h, v, hmax, vmax, mins);
     UpComp c;
-    c.p = p; c.pitch = mcw * h * 8u;
-    c.dw = (width * h + hmax - 1u) / hmax; c.dh = (height * v + vmax - 1u) / vmax;
-    c.rh = hmax / h; c.rv = vmax / v;
+    c.p = p; c.pitch = mcw * h * ss;
+    c.dw = (width * h * ss + hmax * 8u - 1u) / (hmax * 8u); c.dh = (height * v * ss + vmax * 8u - 1u) / (vmax * 8u);
+    c.rh = hmax * mins / (h * ss); c.rv = vmax * mins / (v * ss);
     return c;
 }
 
 // The component's value at output pixel (x, y), as jdsample.c computes it. Neighbours outside [0, dw) x [0, dh) are
-// clamped, which is libjpeg's edge replication; the first and last columns of its loops are that case.
-__device__ __forceinline__ uint32_t up_sample(const UpComp &c, uint32_t x, uint32_t y)
+// clamped, which is libjpeg's edge replication; the first and last columns of its loops are that case. jdsample.c
+// applies its fancy filters only while the smallest DCT size exceeds 1 (`fancy`): at 1/8 every ratio replicates.
+__device__ __forceinline__ uint32_t up_sample(const UpComp &c, uint32_t x, uint32_t y, bool fancy)
 {
-    const bool fancy_h = c.rh == 2u && c.dw > 2u;
-    if (c.rh == 1u && c.rv == 1u) return __ldg(c.p + (size_t)y * c.pitch + x);
-    if (c.rh == 1u && c.rv == 2u)                                      // h1v2_fancy_upsample
+    if (fancy)
     {
-        const uint32_t r = y >> 1, n = (y & 1u) ? min(r + 1u, c.dh - 1u) : (r ? r - 1u : 0u);
-        return (3u * __ldg(c.p + (size_t)r * c.pitch + x) + __ldg(c.p + (size_t)n * c.pitch + x) + 1u + (y & 1u)) >> 2;
+        const bool fancy_h = c.rh == 2u && c.dw > 2u;
+        if (c.rh == 1u && c.rv == 1u) return __ldg(c.p + (size_t)y * c.pitch + x);
+        if (c.rh == 1u && c.rv == 2u)                                      // h1v2_fancy_upsample
+        {
+            const uint32_t r = y >> 1, n = (y & 1u) ? min(r + 1u, c.dh - 1u) : (r ? r - 1u : 0u);
+            return (3u * __ldg(c.p + (size_t)r * c.pitch + x) + __ldg(c.p + (size_t)n * c.pitch + x) + 1u + (y & 1u)) >> 2;
+        }
+        if (fancy_h && c.rv == 1u)                                         // h2v1_fancy_upsample
+        {
+            const uint8_t *row = c.p + (size_t)y * c.pitch;
+            const uint32_t sx = x >> 1, nx = (x & 1u) ? min(sx + 1u, c.dw - 1u) : (sx ? sx - 1u : 0u);
+            return (3u * __ldg(row + sx) + __ldg(row + nx) + 1u + (x & 1u)) >> 2;
+        }
+        if (fancy_h && c.rv == 2u)                                         // h2v2_fancy_upsample
+        {
+            const uint32_t r = y >> 1, n = (y & 1u) ? min(r + 1u, c.dh - 1u) : (r ? r - 1u : 0u);
+            const uint32_t sx = x >> 1, nx = (x & 1u) ? min(sx + 1u, c.dw - 1u) : (sx ? sx - 1u : 0u);
+            const uint8_t *r0 = c.p + (size_t)r * c.pitch, *r1 = c.p + (size_t)n * c.pitch;
+            const uint32_t cs = 3u * __ldg(r0 + sx) + __ldg(r1 + sx), cn = 3u * __ldg(r0 + nx) + __ldg(r1 + nx);
+            return (3u * cs + cn + 8u - (x & 1u)) >> 4;
+        }
     }
-    if (fancy_h && c.rv == 1u)                                         // h2v1_fancy_upsample
-    {
-        const uint8_t *row = c.p + (size_t)y * c.pitch;
-        const uint32_t sx = x >> 1, nx = (x & 1u) ? min(sx + 1u, c.dw - 1u) : (sx ? sx - 1u : 0u);
-        return (3u * __ldg(row + sx) + __ldg(row + nx) + 1u + (x & 1u)) >> 2;
-    }
-    if (fancy_h && c.rv == 2u)                                         // h2v2_fancy_upsample
-    {
-        const uint32_t r = y >> 1, n = (y & 1u) ? min(r + 1u, c.dh - 1u) : (r ? r - 1u : 0u);
-        const uint32_t sx = x >> 1, nx = (x & 1u) ? min(sx + 1u, c.dw - 1u) : (sx ? sx - 1u : 0u);
-        const uint8_t *r0 = c.p + (size_t)r * c.pitch, *r1 = c.p + (size_t)n * c.pitch;
-        const uint32_t cs = 3u * __ldg(r0 + sx) + __ldg(r1 + sx), cn = 3u * __ldg(r0 + nx) + __ldg(r1 + nx);
-        return (3u * cs + cn + 8u - (x & 1u)) >> 4;
-    }
-    return __ldg(c.p + (size_t)(y / c.rv) * c.pitch + x / c.rh);      // int_upsample / h2v1 / h2v2: replication
+    return __ldg(c.p + (size_t)(y / c.rv) * c.pitch + x / c.rh);          // int_upsample / h2v1 / h2v2: replication
 }
 
 // jdcolor.c ycc_rgb_convert (SCALEBITS 16): R | G << 8 | B << 16
@@ -1993,72 +1919,14 @@ __device__ __forceinline__ uint32_t ycc_rgb_libjpeg(int32_t y, int32_t cb, int32
     return (uint32_t)min(max(r, 0), 255) | (uint32_t)min(max(g, 0), 255) << 8 | (uint32_t)min(max(b, 0), 255) << 16;
 }
 
-// One thread per 4-pixel group of a row; blockIdx.y (strided by gridDim.y) = image.
-template <int FMT>
+// One thread per 4-pixel group of a row of the ceil(W / s) x ceil(H / s) output, s = 8 / MINS; blockIdx.y (strided by
+// gridDim.y) = image.
+template <int FMT, uint32_t MINS>
 __global__ void __launch_bounds__(256)
-k_upsample_ycc(const uint8_t *__restrict__ samples, const ImgDev *__restrict__ imgs, uint32_t n_images, uint8_t *__restrict__ pix)
+k_upsample_libjpeg(const uint8_t *__restrict__ samples, const ImgDev *__restrict__ imgs, uint32_t n_images, uint8_t *__restrict__ pix)
 {
-    for (uint32_t img = blockIdx.y; img < n_images; img += gridDim.y)
-    {
-        const ImgDev &im = imgs[img];
-        const uint32_t width = im.width, height = im.height, gw = (width + 3u) / 4u;
-        const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-        if (i >= gw * height) continue;
-        const uint32_t py = i / gw, px = (i % gw) * 4u;
-        const uint32_t sp = im.samp, mcw = im.mcu_count_w;
-        const uint32_t yh = sp & 15u, yv = (sp >> 4) & 15u, uh = (sp >> 8) & 15u, uv = (sp >> 12) & 15u, vh = (sp >> 16) & 15u, vv = (sp >> 20) & 15u;
-        const uint8_t *p0 = samples + 64ull * im.blk_first;
-        const bool gray = im.mode == kModeGray;
-        // the chroma factors divide the luma's (geometry_ok), so the luma's are the maxima
-        const UpComp cy = up_comp(p0, yh, yv, yh, yv, mcw, width, height);
-        UpComp cu = cy, cv = cy;
-        if (!gray)
-        {
-            cu = up_comp(p0 + 64ull * im.mcu_count * (yh * yv), uh, uv, yh, yv, mcw, width, height);
-            cv = up_comp(p0 + 64ull * im.mcu_count * (yh * yv + uh * uv), vh, vv, yh, yv, mcw, width, height);
-        }
-        uint32_t R[2] = {0u, 0u}, Gc[2] = {0u, 0u}, B[2] = {0u, 0u};
-#pragma unroll
-        for (uint32_t k = 0; k < 4u; k++)
-        {
-            const uint32_t x = min(px + k, width - 1u);   // the stores skip pixels behind the last column
-            const uint32_t Y = up_sample(cy, x, py);
-            const uint32_t rgb = gray ? Y * 0x10101u : ycc_rgb_libjpeg((int32_t)Y, (int32_t)up_sample(cu, x, py), (int32_t)up_sample(cv, x, py));
-            const uint32_t sh = 16u * (k & 1u);
-            R[k >> 1] |= (rgb & 0xFFu) << sh; Gc[k >> 1] |= ((rgb >> 8) & 0xFFu) << sh; B[k >> 1] |= (rgb >> 16) << sh;
-        }
-        constexpr uint32_t bpp = FMT == B2J_OUT_BGRA ? 4u : (FMT == B2J_OUT_RGB24 ? 3u : 1u);
-        store_pixels4<FMT>(pix + im.pix_off + ((size_t)py * width + px) * bpp, (size_t)width * height, px, width, (width & 3u) == 0u, R, Gc, B);
-    }
-}
-
-// ---- upsampling and colour of the scaled decode, at the output size ceil(W / s) x ceil(H / s), s = 8 / mins
-// A component of DCT size ss (dct_size) has ceil(W * h * ss / (hmax * 8)) x ceil(H * v * ss / (vmax * 8)) samples (jdmaster.c's
-// downsampled_width / _height) and is upsampled by hmax * mins / (h * ss) x vmax * mins / (v * ss).
-__device__ __forceinline__ UpComp up_comp_scaled(const uint8_t *p, uint32_t h, uint32_t v, uint32_t hmax, uint32_t vmax, uint32_t mcw,
-                                                 uint32_t width, uint32_t height, uint32_t mins)
-{
-    const uint32_t ss = dct_size(h, v, hmax, vmax, mins);
-    UpComp c;
-    c.p = p; c.pitch = mcw * h * ss;
-    c.dw = (width * h * ss + hmax * 8u - 1u) / (hmax * 8u); c.dh = (height * v * ss + vmax * 8u - 1u) / (vmax * 8u);
-    c.rh = hmax * mins / (h * ss); c.rv = vmax * mins / (v * ss);
-    return c;
-}
-
-// jdsample.c applies its fancy filters only while the smallest DCT size exceeds 1: at 1/8 every ratio replicates.
-__device__ __forceinline__ uint32_t up_sample_scaled(const UpComp &c, uint32_t x, uint32_t y, bool fancy)
-{
-    return fancy ? up_sample(c, x, y) : __ldg(c.p + (size_t)(y / c.rv) * c.pitch + x / c.rh);
-}
-
-// k_upsample_ycc at the output size; its own copy, so that k_upsample_ycc keeps its code.
-template <int FMT>
-__global__ void __launch_bounds__(256)
-k_upsample_scaled(const uint8_t *__restrict__ samples, const ImgDev *__restrict__ imgs, uint32_t n_images, uint8_t *__restrict__ pix, uint32_t mins)
-{
-    const uint32_t s = 8u / mins;
-    const bool fancy = mins > 1u;
+    constexpr uint32_t s = 8u / MINS;
+    constexpr bool fancy = MINS > 1u;
     for (uint32_t img = blockIdx.y; img < n_images; img += gridDim.y)
     {
         const ImgDev &im = imgs[img];
@@ -2070,21 +1938,22 @@ k_upsample_scaled(const uint8_t *__restrict__ samples, const ImgDev *__restrict_
         const uint32_t yh = sp & 15u, yv = (sp >> 4) & 15u, uh = (sp >> 8) & 15u, uv = (sp >> 12) & 15u, vh = (sp >> 16) & 15u, vv = (sp >> 20) & 15u;
         const uint8_t *p0 = samples + 64ull * im.blk_first;
         const bool gray = im.mode == kModeGray;
-        const UpComp cy = up_comp_scaled(p0, yh, yv, yh, yv, mcw, im.width, im.height, mins);
+        // the chroma factors divide the luma's (geometry_ok), so the luma's are the maxima
+        const UpComp cy = up_comp(p0, yh, yv, yh, yv, mcw, im.width, im.height, MINS);
         UpComp cu = cy, cv = cy;
         if (!gray)
         {
-            cu = up_comp_scaled(p0 + 64ull * im.mcu_count * (yh * yv), uh, uv, yh, yv, mcw, im.width, im.height, mins);
-            cv = up_comp_scaled(p0 + 64ull * im.mcu_count * (yh * yv + uh * uv), vh, vv, yh, yv, mcw, im.width, im.height, mins);
+            cu = up_comp(p0 + 64ull * im.mcu_count * (yh * yv), uh, uv, yh, yv, mcw, im.width, im.height, MINS);
+            cv = up_comp(p0 + 64ull * im.mcu_count * (yh * yv + uh * uv), vh, vv, yh, yv, mcw, im.width, im.height, MINS);
         }
         uint32_t R[2] = {0u, 0u}, Gc[2] = {0u, 0u}, B[2] = {0u, 0u};
 #pragma unroll
         for (uint32_t k = 0; k < 4u; k++)
         {
             const uint32_t x = min(px + k, width - 1u);   // the stores skip pixels behind the last column
-            const uint32_t Y = up_sample_scaled(cy, x, py, fancy);
+            const uint32_t Y = up_sample(cy, x, py, fancy);
             const uint32_t rgb = gray ? Y * 0x10101u
-                                      : ycc_rgb_libjpeg((int32_t)Y, (int32_t)up_sample_scaled(cu, x, py, fancy), (int32_t)up_sample_scaled(cv, x, py, fancy));
+                                      : ycc_rgb_libjpeg((int32_t)Y, (int32_t)up_sample(cu, x, py, fancy), (int32_t)up_sample(cv, x, py, fancy));
             const uint32_t sh = 16u * (k & 1u);
             R[k >> 1] |= (rgb & 0xFFu) << sh; Gc[k >> 1] |= ((rgb >> 8) & 0xFFu) << sh; B[k >> 1] |= (rgb >> 16) << sh;
         }
@@ -2218,21 +2087,22 @@ static void launch_idct_format(const DecodeArgs &a, cudaStream_t s)
     launch_idct_kind<FMT, kTileGeneric>(a, a.generic_tile0, a.n_tiles - a.generic_tile0, s);
 }
 
-// The libjpeg model: the IDCT over every tile into the sample plane, then the upsampling / colour pass over every image;
-// the scaled decode has a pair of its own.
+// The libjpeg model: the IDCT over every tile into the sample plane, then the upsampling / colour pass over every image.
+template <int FMT, uint32_t MINS>
+static void launch_libjpeg_scale(const DecodeArgs &a, cudaStream_t s)
+{
+    const dim3 grid((a.max_px_groups + 255u) / 256u, a.n_images < 65535u ? a.n_images : 65535u);
+    k_idct_libjpeg<MINS><<<a.n_tiles, kTileBlocks, kTileSmemBytes, s>>>(*a.tmap, a.imgs, a.tiles, a.qtabs, a.samples, a.status);
+    k_upsample_libjpeg<FMT, MINS><<<grid, 256, 0, s>>>(a.samples, a.imgs, a.n_images, a.pixels);
+}
+
 template <int FMT>
 static void launch_libjpeg_format(const DecodeArgs &a, cudaStream_t s)
 {
-    const dim3 grid((a.max_px_groups + 255u) / 256u, a.n_images < 65535u ? a.n_images : 65535u);
-    if (a.scale == 1)
-    {
-        k_idct_islow<<<a.n_tiles, kTileBlocks, kTileSmemBytes, s>>>(*a.tmap, a.imgs, a.tiles, a.qtabs, a.samples, a.status);
-        k_upsample_ycc<FMT><<<grid, 256, 0, s>>>(a.samples, a.imgs, a.n_images, a.pixels);
-        return;
-    }
-    const uint32_t mins = 8u / a.scale;   // the smallest DCT size
-    k_idct_scaled<<<a.n_tiles, kTileBlocks, kTileSmemBytes, s>>>(*a.tmap, a.imgs, a.tiles, a.qtabs, a.samples, a.status, mins);
-    k_upsample_scaled<FMT><<<grid, 256, 0, s>>>(a.samples, a.imgs, a.n_images, a.pixels, mins);
+    if (a.scale == 1) launch_libjpeg_scale<FMT, 8>(a, s);   // MINS = 8 / scale, the smallest DCT size
+    else if (a.scale == 2) launch_libjpeg_scale<FMT, 4>(a, s);
+    else if (a.scale == 4) launch_libjpeg_scale<FMT, 2>(a, s);
+    else launch_libjpeg_scale<FMT, 1>(a, s);
 }
 
 int idct_launches(const DecodeArgs &a)

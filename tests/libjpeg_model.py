@@ -1,9 +1,11 @@
 """The libjpeg pixel model (B2J_PIXELS_LIBJPEG) in numpy: what libjpeg-turbo's C code computes from a baseline file's
-dequantised coefficients with its default decompression settings (jidctint.c ISLOW IDCT, jdsample.c "fancy" chroma
-upsampling, jdcolor.c fixed-point YCbCr -> RGB).
+dequantised coefficients with its default decompression settings at scale_denom 1, 2, 4 or 8 (b2j_batch_set_scale,
+Pillow's draft()): jidctint.c's ISLOW IDCT or jidctred.c's reduced IDCTs at the DCT size jdmaster.c chooses per
+component, jdsample.c's upsampling ("fancy" chroma filters, none at 1/8), jdcolor.c's fixed-point YCbCr -> RGB.
 
 Test tooling. It is fed the oracle's coefficients (int32 [blk_count, 64], natural order, dequantised, MCU-interleaved) and
-is the reference the GPU tests compare the kernels with. tests/test_libjpeg_model.py checks it against Pillow.
+is the reference the GPU tests compare the kernels with. tests/test_libjpeg_model.py (full size) and
+tests/test_scaled_model.py (1/2, 1/4, 1/8) check it against Pillow and libjpeg-turbo's C code.
 """
 import numpy as np
 
@@ -15,6 +17,17 @@ F1501, F1847, F1961, F2053, F2562, F3072 = 12299, 15137, 16069, 16819, 20995, 25
 
 def _descale(x, n):
     return (x + (1 << (n - 1))) >> n
+
+
+def _range_limit(y):
+    """range_limit[y & RANGE_MASK] of an IDCT output: wraps, does not clamp."""
+    m = (y + 128) & 1023
+    return np.where(m < 256, m, np.where(m < 640, 255, 0)).astype(np.uint8)
+
+
+def _wrap32(w):
+    """The pass-1 results are stored in the IDCTs' int workspace: 32 bits."""
+    return ((w + (1 << 31)) & 0xFFFFFFFF) - (1 << 31)
 
 
 def _pass(d, n):
@@ -44,12 +57,49 @@ def idct_islow(blocks):
     """Dequantised coefficients int [n, 64] (natural order) -> samples uint8 [n, 8, 8]. 64-bit arithmetic like libjpeg's
     JLONG; the pass-1 results are stored as C int (32 bits), so they wrap the way the C code's workspace does."""
     x = np.asarray(blocks, np.int64).reshape(-1, 8, 8)
-    ws = _pass([x[:, k, :] for k in range(8)], CONST_BITS - PASS1_BITS)          # columns: out[k] = row k
-    ws = [((w + (1 << 31)) & 0xFFFFFFFF) - (1 << 31) for w in ws]
-    ws = np.stack(ws, axis=1)                                                     # [n, row, col]
-    y = np.stack(_pass([ws[:, :, k] for k in range(8)], CONST_BITS + PASS1_BITS + 3), axis=2)
-    m = (y + 128) & 1023                                                          # range_limit[y & RANGE_MASK]
-    return np.where(m < 256, m, np.where(m < 640, 255, 0)).astype(np.uint8)
+    ws = np.stack([_wrap32(w) for w in _pass([x[:, k, :] for k in range(8)], CONST_BITS - PASS1_BITS)], axis=1)   # [n, r, c]
+    return _range_limit(np.stack(_pass([ws[:, :, k] for k in range(8)], CONST_BITS + PASS1_BITS + 3), axis=2))
+
+
+def _pass4(d, n):
+    """One 1-D pass of jpeg_idct_4x4 over d[0..7] (d[4] unused): 4 outputs DESCALE(., n)."""
+    tmp0 = d[0] << (CONST_BITS + 1)
+    tmp2 = d[2] * 15137 + d[6] * -6270
+    t10, t12 = tmp0 + tmp2, tmp0 - tmp2
+    z1, z2, z3, z4 = d[7], d[5], d[3], d[1]
+    a = z1 * -1730 + z2 * 11893 + z3 * -17799 + z4 * 8697
+    b = z1 * -4176 + z2 * -4926 + z3 * 7373 + z4 * 20995
+    return [_descale(o, n) for o in (t10 + b, t12 + a, t12 - a, t10 - b)]
+
+
+def idct_4x4(blocks):
+    """jpeg_idct_4x4: int [n, 64] -> uint8 [n, 4, 4], 64-bit products, 32-bit workspace like idct_islow."""
+    x = np.asarray(blocks, np.int64).reshape(-1, 8, 8)
+    ws = np.stack([_wrap32(w) for w in _pass4([x[:, k, :] for k in range(8)], CONST_BITS - PASS1_BITS + 1)], axis=1)
+    return _range_limit(np.stack(_pass4([ws[:, :, k] for k in range(8)], CONST_BITS + PASS1_BITS + 3 + 1), axis=2))
+
+
+def _pass2(d, n):
+    """One 1-D pass of jpeg_idct_2x2 over d[0], d[1], d[3], d[5], d[7]: 2 outputs DESCALE(., n)."""
+    t10 = d[0] << (CONST_BITS + 2)
+    t0 = d[7] * -5906 + d[5] * 6967 + d[3] * -10426 + d[1] * 29692
+    return [_descale(t10 + t0, n), _descale(t10 - t0, n)]
+
+
+def idct_2x2(blocks):
+    """jpeg_idct_2x2: int [n, 64] -> uint8 [n, 2, 2]."""
+    x = np.asarray(blocks, np.int64).reshape(-1, 8, 8)
+    ws = np.stack([_wrap32(w) for w in _pass2([x[:, k, :] for k in range(8)], CONST_BITS - PASS1_BITS + 2)], axis=1)
+    return _range_limit(np.stack(_pass2([ws[:, :, k] for k in range(8)], CONST_BITS + PASS1_BITS + 3 + 2), axis=2))
+
+
+def idct_1x1(blocks):
+    """jpeg_idct_1x1: (DC * q + 4) >> 3 -> uint8 [n, 1, 1]."""
+    x = np.asarray(blocks, np.int64).reshape(-1, 64)
+    return _range_limit((x[:, 0] + 4) >> 3).reshape(-1, 1, 1)
+
+
+IDCT_BY_SIZE = {8: idct_islow, 4: idct_4x4, 2: idct_2x2, 1: idct_1x1}
 
 
 def layout(sampling):
@@ -57,31 +107,26 @@ def layout(sampling):
     return [(s >> 4, s & 15) for s in sampling if s]
 
 
-def component_planes(coef, sampling, mcu_count_w, mcu_count_h):
-    """IDCT of every block, assembled into one MCU-padded sample plane per component (uint8 [rows, cols])."""
-    samp = layout(sampling)
-    nblk = [h * v for h, v in samp]
-    tot = sum(nblk)
-    px = idct_islow(coef).reshape(mcu_count_h, mcu_count_w, tot, 8, 8)
-    planes, first = [], 0
-    for (h, v), n in zip(samp, nblk):
-        b = px[:, :, first:first + n].reshape(mcu_count_h, mcu_count_w, v, h, 8, 8)
-        planes.append(b.transpose(0, 2, 4, 1, 3, 5).reshape(mcu_count_h * v * 8, mcu_count_w * h * 8))
-        first += n
-    return planes
+def dct_size(h, v, hmax, vmax, min_size):
+    """jdmaster.c: a component's DCT size, doubled from min_size = 8 / scale while both factors still divide evenly."""
+    ss = min_size
+    while ss < 8 and (hmax * min_size) % (h * ss * 2) == 0 and (vmax * min_size) % (v * ss * 2) == 0:
+        ss *= 2
+    return ss
 
 
 def _clamp_idx(i, n):
     return np.clip(i, 0, n - 1)
 
 
-def upsample(plane, rh, rv, dw, dh, width, height):
-    """One component's samples (the dw x dh top-left part of its plane) -> width x height, jdsample.c's choice of method."""
+def upsample(plane, rh, rv, dw, dh, width, height, fancy=True):
+    """One component's samples (the dw x dh top-left part of its plane) -> width x height, jdsample.c's choice of method.
+    jdsample.c has no fancy filter when the smallest DCT size is 1 (fancy=False): every ratio replicates."""
     s = plane[:dh, :dw].astype(np.int32)
     xs = np.arange(width)
     ys = np.arange(height)
-    if (rh, rv) == (1, 1):
-        return s[:height, :width]
+    if not fancy or (rh, rv) == (1, 1):
+        return s[(ys // rv)[:, None], (xs // rh)[None, :]]
     if (rh, rv) == (2, 1) and dw > 2:
         sx = xs >> 1
         near = s[:, sx] * 3
@@ -112,30 +157,38 @@ def ycc_to_rgb(y, cb, cr):
     return np.clip(np.stack([r, g, b], axis=-1), 0, 255).astype(np.uint8)
 
 
-def decode_rgb(coef, width, height, sampling, mcu_count_w, mcu_count_h):
-    """Dequantised coefficients -> RGB uint8 [height, width, 3] in the libjpeg model (gray: R = G = B = Y)."""
+def decode_rgb(coef, width, height, sampling, mcu_count_w, mcu_count_h, scale=1):
+    """Dequantised coefficients -> RGB uint8 [ceil(height/scale), ceil(width/scale), 3] in the libjpeg model (gray:
+    R = G = B = Y)."""
     samp = layout(sampling)
-    planes = component_planes(coef, sampling, mcu_count_w, mcu_count_h)
     hmax, vmax = max(h for h, _ in samp), max(v for _, v in samp)
-    comps = []
-    for (h, v), p in zip(samp, planes):
-        dw, dh = -(-width * h // hmax), -(-height * v // vmax)
-        comps.append(upsample(p, hmax // h, vmax // v, dw, dh, width, height))
+    mins = 8 // scale
+    ow, oh = -(-width // scale), -(-height // scale)
+    coef = np.asarray(coef).reshape(mcu_count_h, mcu_count_w, sum(h * v for h, v in samp), 64)
+    first, comps = 0, []
+    for h, v in samp:
+        ss = dct_size(h, v, hmax, vmax, mins)
+        px = IDCT_BY_SIZE[ss](coef[:, :, first:first + h * v].reshape(-1, 64)).reshape(mcu_count_h, mcu_count_w, v, h, ss, ss)
+        plane = px.transpose(0, 2, 4, 1, 3, 5).reshape(mcu_count_h * v * ss, mcu_count_w * h * ss)   # MCU-padded
+        first += h * v
+        dw, dh = -(-width * h * ss // (hmax * 8)), -(-height * v * ss // (vmax * 8))
+        rh, rv = hmax * mins // (h * ss), vmax * mins // (v * ss)
+        comps.append(upsample(plane, rh, rv, dw, dh, ow, oh, fancy=mins > 1))
     if len(comps) == 1:
         g = comps[0].astype(np.uint8)
         return np.stack([g, g, g], axis=-1)
     return ycc_to_rgb(*comps)
 
 
-def decode_oracle(oracle, data, gate):
-    """The model's RGB pixels of one file, from the oracle's coefficients (non-strict: the intended decode)."""
+def decode_oracle(oracle, data, gate, scale=1):
+    """The model's RGB pixels of one file at 1/scale, from the oracle's coefficients (non-strict: the intended decode)."""
     oracle.set_strict(False)
     try:
         rc, img, coef, _ = oracle.decode(data, gate=gate, want_pixels=False)
     finally:
         oracle.set_strict(True)
     assert rc == 0, rc
-    return decode_rgb(coef, img.width, img.height, list(img.sampling), img.mcu_count_w, img.mcu_count_h)
+    return decode_rgb(coef, img.width, img.height, list(img.sampling), img.mcu_count_w, img.mcu_count_h, scale)
 
 
 def box_filter(px, factor):

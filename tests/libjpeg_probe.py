@@ -2,8 +2,8 @@
 
 For each config one batch is decoded with b2j_batch_decode_steps, the two models alternating (reference, libjpeg,
 reference, libjpeg), and the median per-stage milliseconds of every run are printed with the traffic the libjpeg model
-adds (the sample plane is written by k_idct_islow and read back by k_upsample_ycc: at least 128 bytes per block), the
-card's name and its power limit. A separate profiled run per model (torch.profiler, CUDA activities) splits the device
+adds (the sample plane is written by k_idct_libjpeg and read back by k_upsample_libjpeg: at least 128 bytes per block),
+the card's name and its power limit. A separate profiled run per model (torch.profiler, CUDA activities) splits the device
 time of one step by kernel. The libjpeg model's pixels of the first images are checked against the numpy model.
 usage: python tests/libjpeg_probe.py [--steps K] [--warmup W] [--configs 1,4] [--out FILE]"""
 import argparse

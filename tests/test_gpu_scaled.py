@@ -7,7 +7,7 @@ import io
 import numpy as np
 import pytest
 
-import libjpeg_scaled_model
+import libjpeg_model
 from test_gpu_libjpeg import ITEMS, _as_rgb, _gate
 
 pytestmark = pytest.mark.gpu
@@ -37,7 +37,7 @@ def expected(oracle):
     for name, data, _ in ITEMS:
         for s in SCALES:
             pil = None if name.startswith("x") else _draft(data, s)
-            px[s].append((libjpeg_scaled_model.decode_oracle_scaled(oracle, data, gate, s), pil))
+            px[s].append((libjpeg_model.decode_oracle(oracle, data, gate, s), pil))
         oracle.set_strict(False)
         try:
             rc, _, coef, _ = oracle.decode(data, gate=gate, want_pixels=False)

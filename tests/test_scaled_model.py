@@ -1,4 +1,4 @@
-"""CPU: the numpy model of the libjpeg pixel model's scaled decode (tests/libjpeg_scaled_model.py) against
+"""CPU: the numpy model of the libjpeg pixel model's scaled decode (tests/libjpeg_model.py) against
 Pillow's draft() (libjpeg-turbo's scale_denom 2, 4, 8) on Pillow-written 4:4:4, 4:2:2, 4:2:0 and gray files with and without
 restart markers and on jpegcraft layouts, and against libjpeg-turbo's C code (JSIMD_FORCENONE=1) on streams of extreme
 coefficients. The GPU tests of the scaled decode take this model as their reference."""
@@ -13,7 +13,6 @@ import pytest
 
 import jpegcraft
 import libjpeg_model
-import libjpeg_scaled_model
 import synth
 from test_libjpeg_model import _gray_jpeg, _ijg_tables, extreme_streams
 
@@ -46,17 +45,11 @@ def _check(oracle, data, scales=SCALES):
     from PIL import Image
     w, h = Image.open(io.BytesIO(data)).size
     for s in scales:
-        got = libjpeg_scaled_model.decode_oracle_scaled(oracle, data, _gate(), s)
+        got = libjpeg_model.decode_oracle(oracle, data, _gate(), s)
         assert got.shape == (-(-h // s), -(-w // s), 3), (s, got.shape)
         want = _draft_rgb(data, s)
         if want is not None:
             assert np.array_equal(got, want), (s, w, h, int((got != want).any(axis=2).sum()))
-
-
-def test_scale_one_is_the_full_size_model(oracle):
-    data = synth.synth_jpeg(131, 77, 1, 85, "420", 3)
-    full = libjpeg_model.decode_oracle(oracle, data, _gate())
-    assert np.array_equal(libjpeg_scaled_model.decode_oracle_scaled(oracle, data, _gate(), 1), full)
 
 
 @pytest.mark.parametrize("ri", [0, 2])
@@ -105,7 +98,7 @@ def test_scaled_model_equals_libjpeg_c_code_on_extreme_coefficients(oracle, tmp_
     for k, data in enumerate(streams):
         for s in SCALES:
             want = np.load("%s.%d.npy" % (str(tmp_path / ("x%d.jpg" % k)), s))
-            got = libjpeg_scaled_model.decode_oracle_scaled(oracle, data, _gate(), s)
+            got = libjpeg_model.decode_oracle(oracle, data, _gate(), s)
             assert np.array_equal(got, want), (k, s, int((got != want).any(axis=2).sum()))
 
 
