@@ -7,6 +7,6 @@ fails, and if no B200 is visible, ``Decoder()`` raises.
 """
 from .api import (  # noqa: F401
     B2JError, BatchInfo, Decoder, Batch, Idct, ImageDesc, StageTimes, HostOpts, HostArgs, PinnedBuffer, parse_header, read_files, host_free, decode_host_multi, library_path, load_library,
-    GATE_REFERENCE, GATE_EXTENDED, PARSE_ROBUST, GATE_GRAY, OUT_BGRA, OUT_RGB24, OUT_RGB_PLANAR, PIXELS_REFERENCE, PIXELS_LIBJPEG,
+    GATE_REFERENCE, GATE_EXTENDED, PARSE_ROBUST, GATE_GRAY, OUT_BGRA, OUT_RGB24, OUT_RGB_PLANAR, OUT_GRAY8, PIXELS_REFERENCE, PIXELS_LIBJPEG,
     EXPORTED_SYMBOLS,
 )

@@ -10,7 +10,7 @@ GATE_REFERENCE = 0
 GATE_EXTENDED = 1
 PARSE_ROBUST = 2     # OR-able: skip COM / late APPn / unknown segments, big-endian 16-bit DQT
 GATE_GRAY = 4        # OR-able: one-component (grayscale) frames
-OUT_BGRA, OUT_RGB24, OUT_RGB_PLANAR = 0, 1, 2
+OUT_BGRA, OUT_RGB24, OUT_RGB_PLANAR, OUT_GRAY8 = 0, 1, 2, 3
 PIXELS_REFERENCE = 0   # the reference's pixels (default)
 PIXELS_LIBJPEG = 1     # libjpeg-turbo's default decode: ISLOW IDCT, fancy chroma upsampling, fixed-point colour (Pillow's pixels)
 
@@ -163,6 +163,8 @@ def parse_header(data, gate=GATE_EXTENDED):
 def _out_shape(d, fmt, scale=1):
     """Shape of an image's pixels in output format fmt, at 1/scale of its size (ceil(W/scale) x ceil(H/scale))."""
     w, h = -(-d.width // scale), -(-d.height // scale)
+    if fmt == OUT_GRAY8:
+        return (h, w)
     return (h, w, 4) if fmt == OUT_BGRA else ((h, w, 3) if fmt == OUT_RGB24 else (3, h, w))
 
 
@@ -305,9 +307,9 @@ class Decoder:
 
     def decode_host_ex(self, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0,
                        pixel_model=PIXELS_REFERENCE, scale=1):
-        """b2j_decode_host_ex: like decode_host with an output layout, a pixel model, a scale (1, 2, 4 or 8: the libjpeg
-        model's scaled decode) and host threads. files: bytes objects or addresses (then `lens`); outs: numpy arrays or
-        addresses."""
+        """b2j_decode_host_ex: like decode_host with an output layout (OUT_GRAY8 with PIXELS_LIBJPEG only), a pixel model,
+        a scale (1, 2, 4 or 8: the libjpeg model's scaled decode) and host threads. files: bytes objects or addresses (then
+        `lens`); outs: numpy arrays or addresses."""
         n = len(files)
         lens = lens if lens is not None else [len(f) for f in files]
         outs, fp, op = _host_call_args(files, outs, gate, out_format, scale)
@@ -419,7 +421,8 @@ class Batch:
         return out
 
     def set_output_format(self, fmt):
-        """OUT_BGRA (reference layout, default), OUT_RGB24 (H,W,3) or OUT_RGB_PLANAR (3,H,W) for the decodes that follow."""
+        """OUT_BGRA (reference layout, default), OUT_RGB24 (H,W,3), OUT_RGB_PLANAR (3,H,W) or OUT_GRAY8 (H,W: libjpeg's
+        grayscale output, the luma samples; decodes need PIXELS_LIBJPEG) for the decodes that follow."""
         _check(self.lib.b2j_batch_set_output_format(self._h, fmt), "b2j_batch_set_output_format")
         self.out_format = fmt
 
@@ -465,11 +468,7 @@ class Batch:
         self.small_factor = factor
 
     def downscaled(self, i, stream=None):
-        d, f = self.descs[i], self.small_factor
-        ow, oh = (d.width + f - 1) // f, (d.height + f - 1) // f
-        fmt = getattr(self, "out_format", OUT_BGRA)
-        shape = (oh, ow, 4) if fmt == OUT_BGRA else ((oh, ow, 3) if fmt == OUT_RGB24 else (3, oh, ow))
-        out = np.zeros(shape, np.uint8)
+        out = np.zeros(_out_shape(self.descs[i], getattr(self, "out_format", OUT_BGRA), self.small_factor), np.uint8)
         _check(self.lib.b2j_batch_read_downscaled(self._h, stream, i, out.ctypes.data), "b2j_batch_read_downscaled")
         return out
 

@@ -20,6 +20,8 @@
 //   k_idct_libjpeg, k_upsample_libjpeg
 //       the libjpeg pixel model (B2J_PIXELS_LIBJPEG) instead of k_idct_csc, at every scale (1, 1/2, 1/4, 1/8):
 //       libjpeg-turbo's ISLOW or reduced IDCTs into a sample plane, then its chroma upsampling and fixed-point colour.
+//   k_idct_gray
+//       the libjpeg pixel model in B2J_OUT_GRAY8 (libjpeg's JCS_GRAYSCALE): the luma blocks only, straight into the pixels.
 //   k_expand_coefs
 //       the reference's coefficient tap (int32, dequantised) from the int16 plane, for parity.
 #include <cuda.h>
@@ -1962,6 +1964,73 @@ k_upsample_libjpeg(const uint8_t *__restrict__ samples, const ImgDev *__restrict
     }
 }
 
+// B2J_OUT_GRAY8 in the libjpeg model: libjpeg's JCS_GRAYSCALE output, the luma component's samples as they are. No
+// sample plane and no second kernel: the luma blocks of the tile are transformed into a staging strip in shared memory
+// behind TileSmem (the tile's MCUs side by side, MINS * yh x MINS * yv samples each, so that the *_block helpers store
+// whole aligned rows), then the strip is copied into the ceil(W / s) x ceil(H / s) image.
+constexpr size_t kGrayStageBytes = (size_t)kTileBlocks * 64;
+static_assert(kTileSmemBytes + kGrayStageBytes <= 48 * 1024, "k_idct_gray would need its dynamic shared memory limit raised");
+
+// `len` bytes from shared memory at src to global memory at dst (any alignment), by the lanes of one warp: the 4-byte
+// words dst covers completely are stored whole, the bytes of the partial words at its ends one by one, so that the
+// neighbouring bytes (another tile's, another image's) are never written.
+__device__ __forceinline__ void warp_copy_out(uint8_t *__restrict__ dst, const uint8_t *src, uint32_t len, uint32_t lane)
+{
+    const uint32_t head = min((uint32_t)(-(uintptr_t)dst) & 3u, len);   // bytes before the first whole word
+    const uint32_t words = (len - head) >> 2;
+    for (uint32_t w = lane; w < words; w += 32u)
+    {
+        const uint8_t *p = src + head + 4u * w;
+        *reinterpret_cast<uint32_t *>(dst + head + 4u * w) = (uint32_t)p[0] | (uint32_t)p[1] << 8 | (uint32_t)p[2] << 16 | (uint32_t)p[3] << 24;
+    }
+    const uint32_t tail = head + 4u * words;
+    if (lane < head) dst[lane] = src[lane];
+    else if (lane >= 4u && lane - 4u < len - tail) dst[tail + lane - 4u] = src[tail + lane - 4u];
+}
+
+// One launch over every tile kind. Only the luma blocks get a thread (n_mcus * yh * yv). The luma component has the largest
+// factors, so jdmaster.c never doubles its DCT size: it is MINS, and each instantiation carries one transform.
+template <uint32_t MINS>
+__global__ void __launch_bounds__(kTileBlocks)
+k_idct_gray(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
+            const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ pix, int32_t *__restrict__ status)
+{
+    constexpr uint32_t s = 8u / MINS;
+    TileSmem &sm = *tile_smem();
+    uint8_t *strip = reinterpret_cast<uint8_t *>(&sm + 1);
+    const uint32_t tid = threadIdx.x;
+    const TileDev d = tile_load<false>(sm, &tmap, imgs, tiles, qtabs, pix, status);   // 32-bit quantisers; sd.pix = the image's output
+    const uint32_t sp = sm.side.samp, n = sm.side.n_mcus;
+    const uint32_t yh = sp & 15u, yv = (sp >> 4) & 15u, ny = yh * yv;
+    const uint32_t tot = ny + ((sp >> 8) & 15u) * ((sp >> 12) & 15u) + ((sp >> 16) & 15u) * ((sp >> 20) & 15u);
+    const uint32_t mw = yh * MINS, mh = yv * MINS, spitch = n * mw;   // an MCU's luma samples; the strip's pitch
+    if (tid < n * ny)
+    {
+        const uint32_t m = tid / ny, k = tid % ny;   // MCU m of the tile, luma block k in it
+        uint8_t *dst = strip + (k / yh) * MINS * spitch + m * mw + (k % yh) * MINS;
+        const uint32_t row = m * tot + k;           // the block's row in the tile (MCU-interleaved)
+        const uint32_t *q = sm.side.qt;
+        if (MINS == 8u) islow_block(sm.tile, row, q, dst, spitch);
+        else if (MINS == 4u) red4_block(sm.tile, row, q, dst, spitch);
+        else if (MINS == 2u) red2_block(sm.tile, row, q, dst, spitch);
+        else *dst = (uint8_t)islow_limit((tile_coef(sm.tile + row * 128u, row & 7u, q, 0, 0) + 4) >> 3);
+    }
+    __syncthreads();
+    // The tile's MCUs are consecutive in raster order, so the strip holds one run of MCUs per MCU row the tile touches.
+    // One warp per output row of a run; samples of padding MCUs (right of or below the output) are dropped.
+    const uint32_t ow = (sm.side.width + s - 1u) / s, oh = (sm.side.height + s - 1u) / s;
+    const uint32_t mcw = __ldg(&imgs[d.img].mcu_count_w), my0 = sm.side.mcu_xy[0].y;
+    const uint32_t rows = (sm.side.mcu_xy[n - 1u].y - my0 + 1u) * mh;
+    for (uint32_t i = tid >> 5; i < rows; i += kTileBlocks / 32)
+    {
+        const uint32_t my = my0 + i / mh, r = i % mh, y = my * mh + r;
+        if (y >= oh) break;
+        const uint32_t ma = max(my * mcw, d.mcu_first) - d.mcu_first, mb = min((my + 1u) * mcw, d.mcu_first + n) - d.mcu_first;
+        const uint32_t x0 = sm.side.mcu_xy[ma].x * mw, x1 = min(x0 + (mb - ma) * mw, ow);
+        if (x0 < x1) warp_copy_out(sm.side.pix + (size_t)y * ow + x0, strip + r * spitch + ma * mw, x1 - x0, tid & 31u);
+    }
+}
+
 // =====================================================================================
 // Coefficient tap: int16 quantised plane -> the reference's int32 dequantised mcu_data layout.
 __global__ void __launch_bounds__(256)
@@ -2105,10 +2174,17 @@ static void launch_libjpeg_format(const DecodeArgs &a, cudaStream_t s)
     else launch_libjpeg_scale<FMT, 1>(a, s);
 }
 
+// GRAY8 in the libjpeg model: one kernel straight into the pixel plane.
+template <uint32_t MINS>
+static void launch_gray_scale(const DecodeArgs &a, cudaStream_t s)
+{
+    k_idct_gray<MINS><<<a.n_tiles, kTileBlocks, kTileSmemBytes + kGrayStageBytes, s>>>(*a.tmap, a.imgs, a.tiles, a.qtabs, a.pixels, a.status);
+}
+
 int idct_launches(const DecodeArgs &a)
 {
     if (a.n_tiles == 0) return 0;
-    if (a.pixel_model == B2J_PIXELS_LIBJPEG) return 2;
+    if (a.pixel_model == B2J_PIXELS_LIBJPEG) return a.out_format == B2J_OUT_GRAY8 ? 1 : 2;
     return (a.gray_tile0 > 0 ? 1 : 0) + (a.generic_tile0 > a.gray_tile0 ? 1 : 0) + (a.n_tiles > a.generic_tile0 ? 1 : 0);
 }
 
@@ -2117,7 +2193,14 @@ void launch_idct(const DecodeArgs &a, cudaStream_t s)
     if (a.pixel_model == B2J_PIXELS_LIBJPEG)
     {
         if (a.n_tiles == 0) return;
-        if (a.out_format == B2J_OUT_RGB24) launch_libjpeg_format<B2J_OUT_RGB24>(a, s);
+        if (a.out_format == B2J_OUT_GRAY8)
+        {
+            if (a.scale == 1) launch_gray_scale<8>(a, s);   // MINS = 8 / scale
+            else if (a.scale == 2) launch_gray_scale<4>(a, s);
+            else if (a.scale == 4) launch_gray_scale<2>(a, s);
+            else launch_gray_scale<1>(a, s);
+        }
+        else if (a.out_format == B2J_OUT_RGB24) launch_libjpeg_format<B2J_OUT_RGB24>(a, s);
         else if (a.out_format == B2J_OUT_RGB_PLANAR) launch_libjpeg_format<B2J_OUT_RGB_PLANAR>(a, s);
         else launch_libjpeg_format<B2J_OUT_BGRA>(a, s);
         return;

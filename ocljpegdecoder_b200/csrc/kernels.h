@@ -44,7 +44,8 @@ struct DecodeArgs
     int out_format;          // B2J_OUT_*: layout of the pixel plane (b2j_batch_set_output_format)
     bool any_wide_q;         // some quantiser of the batch exceeds 255 (16-bit DQT): generic dequantisation
     int pixel_model;         // B2J_PIXELS_*: which pixels the IDCT/colour stage computes (b2j_batch_set_pixel_model)
-    uint8_t *samples;        // B2J_PIXELS_LIBJPEG: the sample plane, 64 B per block (allocated by the first decode in that model)
+    uint8_t *samples;        // B2J_PIXELS_LIBJPEG: the sample plane, 64 B per block (allocated by the first decode in that model
+                             // whose format is not B2J_OUT_GRAY8)
     uint32_t max_px_groups;  // largest ceil(OW / 4) * OH of the batch's output sizes: the grid of the libjpeg model's upsampling kernel
     uint32_t scale;          // B2J_PIXELS_LIBJPEG: the output is ceil(W / scale) x ceil(H / scale); 1, 2, 4 or 8 (b2j_batch_set_scale)
 };
@@ -56,7 +57,7 @@ void launch_prepass(const DecodeArgs &a, cudaStream_t s);   // 1 kernel
 void launch_huffman(const DecodeArgs &a, cudaStream_t s);   // 1 kernel
 void launch_huffman_sync(const DecodeArgs &a, cudaStream_t s);   // 4 kernels
 constexpr int kSyncLaunches = 4;
-void launch_idct(const DecodeArgs &a, cudaStream_t s);      // reference model: 1 kernel per tile kind present; libjpeg model: 2
+void launch_idct(const DecodeArgs &a, cudaStream_t s);      // reference model: 1 kernel per tile kind present; libjpeg model: 2, 1 in GRAY8
 int idct_launches(const DecodeArgs &a);                      // kernels launch_idct() enqueues
 void launch_downscale(const uint8_t *pix, const ImgDev *imgs, const uint64_t *out_off, uint8_t *out, uint32_t n_images, uint32_t max_out_samples,
                       uint32_t factor, int fmt, cudaStream_t s);   // box-filter reduction of the pixel plane

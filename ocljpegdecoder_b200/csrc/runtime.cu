@@ -241,7 +241,9 @@ int64_t device_bytes(const b2j_batch *b)
 const ImgDev *image_of(const b2j_batch *b, int image) { return b && image >= 0 && image < b->n ? &b->imgs[(size_t)image] : nullptr; }
 
 // Bytes per pixel of an output format (B2J_OUT_*).
-size_t format_bpp(int fmt) { return fmt == B2J_OUT_BGRA ? 4 : 3; }
+size_t format_bpp(int fmt) { return fmt == B2J_OUT_BGRA ? 4 : (fmt == B2J_OUT_GRAY8 ? 1 : 3); }
+
+bool format_ok(int fmt) { return fmt == B2J_OUT_BGRA || fmt == B2J_OUT_RGB24 || fmt == B2J_OUT_RGB_PLANAR || fmt == B2J_OUT_GRAY8; }
 
 // An image's output size at the batch's scale: ceil(W / scale) x ceil(H / scale).
 uint32_t out_width(const b2j_batch *b, const ImgDev &im) { return (im.width + b->args.scale - 1) / b->args.scale; }
@@ -682,7 +684,12 @@ static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStep
         t_last_error = "a scaled decode (b2j_batch_set_scale) needs the libjpeg pixel model: the reference has none";
         return B2J_E_ARG;
     }
-    if (b->args.pixel_model == B2J_PIXELS_LIBJPEG && !b->d_samples.p)
+    if (b->args.out_format == B2J_OUT_GRAY8 && b->args.pixel_model != B2J_PIXELS_LIBJPEG)
+    {
+        t_last_error = "B2J_OUT_GRAY8 (libjpeg's grayscale output) needs the libjpeg pixel model: the reference has none";
+        return B2J_E_ARG;
+    }
+    if (b->args.pixel_model == B2J_PIXELS_LIBJPEG && b->args.out_format != B2J_OUT_GRAY8 && !b->d_samples.p)
     {
         // the sample plane: 64 bytes per block, image by image at 64 * blk_first
         const cudaError_t e = grow(b->ctx, b->d_samples, (size_t)b->info.total_blocks * 64);
@@ -777,8 +784,10 @@ extern "C" int b2j_batch_sync_stats(b2j_batch *b, void *stream, uint32_t *out8)
 
 extern "C" int b2j_batch_set_output_format(b2j_batch *b, int format)
 {
-    if (!b || (format != B2J_OUT_BGRA && format != B2J_OUT_RGB24 && format != B2J_OUT_RGB_PLANAR)) return B2J_E_ARG;
+    if (!b || !format_ok(format)) return B2J_E_ARG;
+    b->info.kernel_launches -= idct_launches(b->args);
     b->args.out_format = format;   // the pixel plane is sized for 4 bytes per pixel: every format fits
+    b->info.kernel_launches += idct_launches(b->args);
     return B2J_OK;
 }
 
@@ -936,11 +945,12 @@ void destroy_batch_done(b2j_batch *b)
 }
 
 // Host feed only: the images of the batch packed as tightly in the pixel plane as the stores of the colour kernel allow
-// (16-byte aligned starts for BGRA, 4-byte aligned for the three-byte formats), so that the downloads of neighbouring
-// images merge into one copy when the caller's buffers are neighbours too. Before b2j_batch_upload().
+// (16-byte aligned starts for BGRA, 4-byte aligned for the three-byte formats, none for GRAY8, whose kernel stores bytes
+// at any alignment), so that the downloads of neighbouring images merge into one copy when the caller's buffers are
+// neighbours too. Before b2j_batch_upload().
 void pack_pixel_plane(b2j_batch *b, int fmt)
 {
-    const size_t a = fmt == B2J_OUT_BGRA ? 16 : 4;
+    const size_t a = fmt == B2J_OUT_BGRA ? 16 : (fmt == B2J_OUT_GRAY8 ? 1 : 4);
     b->args.out_format = fmt;
     size_t off = 0;
     for (ImgDev &im : b->imgs)
@@ -979,9 +989,14 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
 {
     if (!ctx || n <= 0 || !files || !lens || !out || !status || !opts) return B2J_E_ARG;
     const int fmt = opts->out_format;
-    if (fmt != B2J_OUT_BGRA && fmt != B2J_OUT_RGB24 && fmt != B2J_OUT_RGB_PLANAR) return B2J_E_ARG;
+    if (!format_ok(fmt)) return B2J_E_ARG;
     const int model = opts->pixel_model;
     if (model != B2J_PIXELS_REFERENCE && model != B2J_PIXELS_LIBJPEG) return B2J_E_ARG;
+    if (fmt == B2J_OUT_GRAY8 && model != B2J_PIXELS_LIBJPEG)
+    {
+        t_last_error = "B2J_OUT_GRAY8 (libjpeg's grayscale output) needs the libjpeg pixel model: the reference has none";
+        return B2J_E_ARG;
+    }
     const int scale = opts->scale ? opts->scale : 1;
     if (!scale_ok(scale)) return B2J_E_ARG;
     if (scale != 1 && model != B2J_PIXELS_LIBJPEG)
