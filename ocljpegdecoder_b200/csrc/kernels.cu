@@ -2063,35 +2063,38 @@ k_pack_coefs(const int32_t *__restrict__ in, int16_t *__restrict__ coef, size_t 
 // Output stage (SURVEY 8f rank 3, "optional resize"): box-filter reduction of the decoded pixels by an integer factor per
 // axis. One thread per output sample group: BGRA / RGB24 = one output pixel (all its channels), planar RGB = one output
 // sample of one plane. Every output value is the rounded mean of the input values it covers (at the right and bottom
-// edges: of those that exist). blockIdx.y = image.
+// edges: of those that exist). blockIdx.y (strided by gridDim.y) = image.
 __global__ void __launch_bounds__(256)
 k_downscale(const uint8_t *__restrict__ pix, const ImgDev *__restrict__ imgs, const uint64_t *__restrict__ out_off,
-            uint8_t *__restrict__ out, uint32_t factor, int fmt)
+            uint8_t *__restrict__ out, uint32_t n_images, uint32_t factor, int fmt)
 {
-    const ImgDev &im = imgs[blockIdx.y];
-    const uint32_t w = im.width, h = im.height, ow = (w + factor - 1) / factor, oh = (h + factor - 1) / factor;
-    const uint32_t planes = fmt == B2J_OUT_RGB_PLANAR ? 3u : 1u;
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= ow * oh * planes) return;
-    const uint32_t pl = i / (ow * oh), r = i % (ow * oh), oy = r / ow, ox = r % ow;
-    const uint32_t x0 = ox * factor, y0 = oy * factor, x1 = min(x0 + factor, w), y1 = min(y0 + factor, h);
-    const uint32_t bpp = fmt == B2J_OUT_BGRA ? 4u : (fmt == B2J_OUT_RGB24 ? 3u : 1u);
-    const uint8_t *src = pix + im.pix_off + (size_t)pl * w * h;
-    uint32_t acc[4] = {0u, 0u, 0u, 0u};
-    for (uint32_t y = y0; y < y1; y++)
-        for (uint32_t x = x0; x < x1; x++)
-        {
-            const uint8_t *p = src + ((size_t)y * w + x) * bpp;
-            if (bpp == 4u) { const uint32_t v = *reinterpret_cast<const uint32_t *>(p); acc[0] += v & 0xFFu; acc[1] += (v >> 8) & 0xFFu; acc[2] += (v >> 16) & 0xFFu; }
-            else if (bpp == 3u) { acc[0] += p[0]; acc[1] += p[1]; acc[2] += p[2]; }
-            else acc[0] += p[0];
-        }
-    const uint32_t n = (x1 - x0) * (y1 - y0), half = n / 2u;
-    uint8_t *dst = out + out_off[blockIdx.y] + (size_t)pl * ow * oh + ((size_t)oy * ow + ox) * bpp;
-    if (bpp == 4u)
-        *reinterpret_cast<uint32_t *>(dst) = (acc[0] + half) / n | ((acc[1] + half) / n) << 8 | ((acc[2] + half) / n) << 16;
-    else if (bpp == 3u) { dst[0] = (uint8_t)((acc[0] + half) / n); dst[1] = (uint8_t)((acc[1] + half) / n); dst[2] = (uint8_t)((acc[2] + half) / n); }
-    else dst[0] = (uint8_t)((acc[0] + half) / n);
+    for (uint32_t img = blockIdx.y; img < n_images; img += gridDim.y)
+    {
+        const ImgDev &im = imgs[img];
+        const uint32_t w = im.width, h = im.height, ow = (w + factor - 1) / factor, oh = (h + factor - 1) / factor;
+        const uint32_t planes = fmt == B2J_OUT_RGB_PLANAR ? 3u : 1u;
+        const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+        if (i >= ow * oh * planes) continue;
+        const uint32_t pl = i / (ow * oh), r = i % (ow * oh), oy = r / ow, ox = r % ow;
+        const uint32_t x0 = ox * factor, y0 = oy * factor, x1 = min(x0 + factor, w), y1 = min(y0 + factor, h);
+        const uint32_t bpp = fmt == B2J_OUT_BGRA ? 4u : (fmt == B2J_OUT_RGB24 ? 3u : 1u);
+        const uint8_t *src = pix + im.pix_off + (size_t)pl * w * h;
+        uint32_t acc[4] = {0u, 0u, 0u, 0u};
+        for (uint32_t y = y0; y < y1; y++)
+            for (uint32_t x = x0; x < x1; x++)
+            {
+                const uint8_t *p = src + ((size_t)y * w + x) * bpp;
+                if (bpp == 4u) { const uint32_t v = *reinterpret_cast<const uint32_t *>(p); acc[0] += v & 0xFFu; acc[1] += (v >> 8) & 0xFFu; acc[2] += (v >> 16) & 0xFFu; }
+                else if (bpp == 3u) { acc[0] += p[0]; acc[1] += p[1]; acc[2] += p[2]; }
+                else acc[0] += p[0];
+            }
+        const uint32_t n = (x1 - x0) * (y1 - y0), half = n / 2u;
+        uint8_t *dst = out + out_off[img] + (size_t)pl * ow * oh + ((size_t)oy * ow + ox) * bpp;
+        if (bpp == 4u)
+            *reinterpret_cast<uint32_t *>(dst) = (acc[0] + half) / n | ((acc[1] + half) / n) << 8 | ((acc[2] + half) / n) << 16;
+        else if (bpp == 3u) { dst[0] = (uint8_t)((acc[0] + half) / n); dst[1] = (uint8_t)((acc[1] + half) / n); dst[2] = (uint8_t)((acc[2] + half) / n); }
+        else dst[0] = (uint8_t)((acc[0] + half) / n);
+    }
 }
 
 // =====================================================================================
@@ -2214,8 +2217,8 @@ void launch_downscale(const uint8_t *pix, const ImgDev *imgs, const uint64_t *ou
                       uint32_t factor, int fmt, cudaStream_t s)
 {
     if (n_images == 0 || max_out_samples == 0) return;
-    const dim3 grid((max_out_samples + 255u) / 256u, n_images);
-    k_downscale<<<grid, 256, 0, s>>>(pix, imgs, out_off, out, factor, fmt);
+    const dim3 grid((max_out_samples + 255u) / 256u, n_images < 65535u ? n_images : 65535u);   // gridDim.y is at most 65535
+    k_downscale<<<grid, 256, 0, s>>>(pix, imgs, out_off, out, n_images, factor, fmt);
 }
 
 void launch_pack(const int32_t *in, int16_t *coef, size_t n_values, cudaStream_t s)

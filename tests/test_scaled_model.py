@@ -20,8 +20,11 @@ PIL = pytest.importorskip("PIL.Image")
 
 SCALES = (2, 4, 8)
 SIZES = [(1, 1), (3, 7), (9, 5), (17, 33), (131, 77), (203, 99), (640, 480)]
-# 4:2:2, 4:4:0, 4:1:1, 2x2, 1x4, 4x2, (22,12,12), (22,21,21)
-CRAFT_LAYOUTS = [(2, 1), (1, 2), (4, 1), (2, 2), (1, 4), (4, 2), ((2, 2), (1, 2), (1, 2)), ((2, 2), (2, 1), (2, 1))]
+# 4:2:2, 4:4:0, 4:1:1, 2x2, 1x4, 4x2, (22,12,12), (22,21,21);
+# then what else the extended gate admits: luma factors of 3 (chroma replicated by 3, a DCT size that never doubles),
+# 2x3, 2x4 (chroma h1v2 at 1/2), and Cb and Cr on layouts of their own, (41,21,21) and (22,21,12) (h2v1 beside h1v2)
+CRAFT_LAYOUTS = [(2, 1), (1, 2), (4, 1), (2, 2), (1, 4), (4, 2), ((2, 2), (1, 2), (1, 2)), ((2, 2), (2, 1), (2, 1)),
+                 (3, 1), (1, 3), (3, 2), (2, 3), (2, 4), ((4, 1), (2, 1), (2, 1)), ((2, 2), (2, 1), (1, 2))]
 
 
 def _gate():
