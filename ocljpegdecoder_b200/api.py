@@ -368,6 +368,7 @@ class Batch:
         self.files = list(files)   # keep the bytes alive
         self.descs = descs
         self.n = len(files)
+        self.out_format, self.pixel_model, self.scale = OUT_BGRA, PIXELS_REFERENCE, 1   # what b2j_batch_create sets
         fp = (ctypes.c_char_p * self.n)(*self.files)
         ln = (ctypes.c_size_t * self.n)(*[len(f) for f in self.files])
         self._h = ctypes.c_void_p()
@@ -440,7 +441,7 @@ class Batch:
 
     def pixel_shape(self, i):
         """Shape of image i's pixels in the batch's output format and scale."""
-        return _out_shape(self.descs[i], getattr(self, "out_format", OUT_BGRA), getattr(self, "scale", 1))
+        return _out_shape(self.descs[i], self.out_format, self.scale)
 
     def pixels(self, i, stream=None):
         out = np.zeros(self.pixel_shape(i), np.uint8)
@@ -468,7 +469,7 @@ class Batch:
         self.small_factor = factor
 
     def downscaled(self, i, stream=None):
-        out = np.zeros(_out_shape(self.descs[i], getattr(self, "out_format", OUT_BGRA), self.small_factor), np.uint8)
+        out = np.zeros(_out_shape(self.descs[i], self.out_format, self.small_factor), np.uint8)
         _check(self.lib.b2j_batch_read_downscaled(self._h, stream, i, out.ctypes.data), "b2j_batch_read_downscaled")
         return out
 

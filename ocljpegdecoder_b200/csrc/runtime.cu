@@ -140,6 +140,7 @@ struct b2j_batch
 
     CUtensorMap tmap;
     DecodeArgs args;
+    int fixed_launches;   // the kernels of a decode before the IDCT/colour stage: pre-pass and entropy stage
     bool uploaded = false;
     cudaStream_t last_stream = nullptr;   // the stream the batch was last uploaded / decoded / read on
 };
@@ -245,13 +246,47 @@ size_t format_bpp(int fmt) { return fmt == B2J_OUT_BGRA ? 4 : (fmt == B2J_OUT_GR
 
 bool format_ok(int fmt) { return fmt == B2J_OUT_BGRA || fmt == B2J_OUT_RGB24 || fmt == B2J_OUT_RGB_PLANAR || fmt == B2J_OUT_GRAY8; }
 
-// An image's output size at the batch's scale: ceil(W / scale) x ceil(H / scale).
-uint32_t out_width(const b2j_batch *b, const ImgDev &im) { return (im.width + b->args.scale - 1) / b->args.scale; }
-uint32_t out_height(const b2j_batch *b, const ImgDev &im) { return (im.height + b->args.scale - 1) / b->args.scale; }
-
-size_t image_bytes(const b2j_batch *b, const ImgDev &im) { return (size_t)out_width(b, im) * out_height(b, im) * format_bpp(b->args.out_format); }
+bool model_ok(int model) { return model == B2J_PIXELS_REFERENCE || model == B2J_PIXELS_LIBJPEG; }
 
 bool scale_ok(int denom) { return denom == 1 || denom == 2 || denom == 4 || denom == 8; }
+
+// Why a decode with these settings cannot run, or nullptr when it can. The setters store any valid value, so a batch
+// may hold such a combination; the decode refuses it.
+const char *output_refusal(int model, int fmt, int scale)
+{
+    if (model == B2J_PIXELS_LIBJPEG) return nullptr;
+    if (scale != 1) return "a scaled decode (b2j_batch_set_scale, b2j_host_opts.scale) needs the libjpeg pixel model: the reference has none";
+    if (fmt == B2J_OUT_GRAY8) return "B2J_OUT_GRAY8 (libjpeg's grayscale output) needs the libjpeg pixel model: the reference has none";
+    return nullptr;
+}
+
+// An image's size with each side divided by `div`, rounded up: the output of a decode at scale `div`, or the reduced
+// copy of b2j_batch_downscale() by factor `div`.
+struct Dims { uint32_t w, h; };
+Dims out_dims(const ImgDev &im, uint32_t div) { return {(im.width + div - 1) / div, (im.height + div - 1) / div}; }
+
+size_t image_bytes(const b2j_batch *b, const ImgDev &im)
+{
+    const Dims o = out_dims(im, b->args.scale);
+    return (size_t)o.w * o.h * format_bpp(b->args.out_format);
+}
+
+// The only writer of a batch's output settings and of what follows from them: the upsampling kernel's grid and the
+// launch count of a decode.
+void set_output(b2j_batch *b, int model, int fmt, int scale)
+{
+    b->args.pixel_model = model;   // the sample plane, once allocated, stays with the batch
+    b->args.out_format = fmt;      // the pixel plane is sized for BGRA at scale 1: every format and scale fits
+    b->args.scale = (uint32_t)scale;
+    uint32_t groups = 0;           // one thread per 4 output pixels of a row
+    for (const ImgDev &im : b->imgs)
+    {
+        const Dims o = out_dims(im, (uint32_t)scale);
+        groups = std::max(groups, (o.w + 3) / 4 * o.h);
+    }
+    b->args.max_px_groups = groups;
+    b->info.kernel_launches = b->fixed_launches + idct_launches(b->args);
+}
 
 // One device->host copy on the call's stream, waited for.
 int read_back(b2j_batch *b, void *stream, void *dst, const void *src, size_t bytes)
@@ -400,7 +435,6 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     static const uint8_t zz[64] = B2J_ZIGZAG_TABLE;
 
     size_t raw_total = 0, pix_total = 0, blk_total = 0;
-    uint32_t max_px_groups = 0;   // largest ceil(W / 4) * H
     uint32_t seg_total = 0, max_lut_len = 0, max_lut_dec_len = 0, max_lut_walk_len = 0;
     int64_t pixels = 0, scan_bytes = 0;
     int rc = B2J_OK;
@@ -474,7 +508,6 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
                 if (q > 255) im.wide_q = 1;
             }
         pixels += (int64_t)d.width * d.height;
-        max_px_groups = std::max(max_px_groups, (uint32_t)((d.width + 3) / 4) * (uint32_t)d.height);
         if (coef_only) continue;
         scan_bytes += (int64_t)d.scan_size;
         // decode tables, shared between images that carry identical DHT payloads
@@ -609,13 +642,9 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     a.max_lut_len = max_lut_len;
     a.max_lut_dec_len = max_lut_dec_len;
     a.max_lut_walk_len = max_lut_walk_len;
-    a.out_format = B2J_OUT_BGRA;
     a.any_wide_q = false;
     for (const ImgDev &im : b->imgs) a.any_wide_q = a.any_wide_q || im.wide_q != 0;
-    a.pixel_model = B2J_PIXELS_REFERENCE;
     a.samples = nullptr;
-    a.max_px_groups = max_px_groups;
-    a.scale = 1;
     {
         const char *sp = getenv("B2J_SYNC_PRE");
         a.sync_use_pre = !(sp && atoi(sp) == 0);
@@ -624,7 +653,6 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     b2j_batch_info &inf = b->info;
     memset(&inf, 0, sizeof(inf));
     inf.n_images = n;
-    inf.kernel_launches = idct_launches(a) + 1 + (ctas.empty() ? 0 : 1) + (sctas.empty() ? 0 : kSyncLaunches);
     inf.total_pixels = pixels;
     inf.total_blocks = (int64_t)blk_total;
     inf.scan_bytes = scan_bytes;
@@ -633,6 +661,8 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     inf.algorithmic_bytes = inf.scan_bytes + 2 * inf.coef_plane_bytes + inf.pixel_bytes;
     inf.device_bytes = device_bytes(b);
     inf.h2d_bytes = (int64_t)b->blob_bytes;
+    b->fixed_launches = 1 + (ctas.empty() ? 0 : 1) + (sctas.empty() ? 0 : kSyncLaunches);
+    set_output(b, B2J_PIXELS_REFERENCE, B2J_OUT_BGRA, 1);
     *out = b;
     return B2J_OK;
 }
@@ -679,16 +709,7 @@ constexpr size_t kStepEvents = 5;
 static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStepEvents or NULL */)
 {
     if (!b->uploaded) { t_last_error = "b2j_batch_decode before b2j_batch_upload"; return B2J_E_ARG; }
-    if (b->args.scale != 1 && b->args.pixel_model != B2J_PIXELS_LIBJPEG)
-    {
-        t_last_error = "a scaled decode (b2j_batch_set_scale) needs the libjpeg pixel model: the reference has none";
-        return B2J_E_ARG;
-    }
-    if (b->args.out_format == B2J_OUT_GRAY8 && b->args.pixel_model != B2J_PIXELS_LIBJPEG)
-    {
-        t_last_error = "B2J_OUT_GRAY8 (libjpeg's grayscale output) needs the libjpeg pixel model: the reference has none";
-        return B2J_E_ARG;
-    }
+    if (const char *why = output_refusal(b->args.pixel_model, b->args.out_format, (int)b->args.scale)) { t_last_error = why; return B2J_E_ARG; }
     if (b->args.pixel_model == B2J_PIXELS_LIBJPEG && b->args.out_format != B2J_OUT_GRAY8 && !b->d_samples.p)
     {
         // the sample plane: 64 bytes per block, image by image at 64 * blk_first
@@ -785,28 +806,21 @@ extern "C" int b2j_batch_sync_stats(b2j_batch *b, void *stream, uint32_t *out8)
 extern "C" int b2j_batch_set_output_format(b2j_batch *b, int format)
 {
     if (!b || !format_ok(format)) return B2J_E_ARG;
-    b->info.kernel_launches -= idct_launches(b->args);
-    b->args.out_format = format;   // the pixel plane is sized for 4 bytes per pixel: every format fits
-    b->info.kernel_launches += idct_launches(b->args);
+    set_output(b, b->args.pixel_model, format, (int)b->args.scale);
     return B2J_OK;
 }
 
 extern "C" int b2j_batch_set_pixel_model(b2j_batch *b, int model)
 {
-    if (!b || (model != B2J_PIXELS_REFERENCE && model != B2J_PIXELS_LIBJPEG)) return B2J_E_ARG;
-    b->info.kernel_launches -= idct_launches(b->args);
-    b->args.pixel_model = model;   // the sample plane, once allocated, stays with the batch
-    b->info.kernel_launches += idct_launches(b->args);
+    if (!b || !model_ok(model)) return B2J_E_ARG;
+    set_output(b, model, b->args.out_format, (int)b->args.scale);
     return B2J_OK;
 }
 
 extern "C" int b2j_batch_set_scale(b2j_batch *b, int denom)
 {
     if (!b || !scale_ok(denom)) return B2J_E_ARG;
-    b->args.scale = (uint32_t)denom;
-    uint32_t groups = 0;   // the upsampling kernel's grid: one thread per 4 output pixels of a row
-    for (const ImgDev &im : b->imgs) groups = std::max(groups, (out_width(b, im) + 3) / 4 * out_height(b, im));
-    b->args.max_px_groups = groups;
+    set_output(b, b->args.pixel_model, b->args.out_format, denom);
     return B2J_OK;
 }
 
@@ -867,12 +881,6 @@ extern "C" int b2j_batch_read_coefs(b2j_batch *b, void *stream, int image, int32
 
 // ---------------------------------------------------------------------------------------
 // Output stage: reduced copies of the decoded pixels (SURVEY.md 8f rank 3).
-static void small_dims(const ImgDev &im, int f, uint32_t *ow, uint32_t *oh)
-{
-    *ow = (im.width + (uint32_t)f - 1) / (uint32_t)f;
-    *oh = (im.height + (uint32_t)f - 1) / (uint32_t)f;
-}
-
 extern "C" int b2j_batch_downscale(b2j_batch *b, void *stream, int factor)
 {
     if (!b || (factor != 2 && factor != 4 && factor != 8)) return B2J_E_ARG;
@@ -887,10 +895,9 @@ extern "C" int b2j_batch_downscale(b2j_batch *b, void *stream, int factor)
         size_t off = align_up(8 * (size_t)b->n, 256);   // behind the offset table
         for (int i = 0; i < b->n; i++)
         {
-            uint32_t ow, oh;
-            small_dims(b->imgs[(size_t)i], factor, &ow, &oh);
+            const Dims o = out_dims(b->imgs[(size_t)i], (uint32_t)factor);
             b->small_off[(size_t)i] = off;
-            off += align_up((size_t)ow * oh * format_bpp(B2J_OUT_BGRA), 16);   // sized for BGRA: every format fits
+            off += align_up((size_t)o.w * o.h * format_bpp(B2J_OUT_BGRA), 16);   // sized for BGRA: every format fits
         }
         if (grow(b->ctx, b->d_small, off) != cudaSuccess) return B2J_E_NOMEM;
         CU_TRY(cudaMemcpyAsync(b->d_small.p, b->small_off.data(), 8 * (size_t)b->n, cudaMemcpyHostToDevice, s));
@@ -898,12 +905,10 @@ extern "C" int b2j_batch_downscale(b2j_batch *b, void *stream, int factor)
         b->small_factor = factor;
     }
     uint32_t max_samples = 0;
-    for (int i = 0; i < b->n; i++)
+    for (const ImgDev &im : b->imgs)
     {
-        uint32_t ow, oh;
-        small_dims(b->imgs[(size_t)i], factor, &ow, &oh);
-        const uint32_t ns = ow * oh * (fmt == B2J_OUT_RGB_PLANAR ? 3u : 1u);
-        if (ns > max_samples) max_samples = ns;
+        const Dims o = out_dims(im, (uint32_t)factor);
+        max_samples = std::max(max_samples, o.w * o.h * (fmt == B2J_OUT_RGB_PLANAR ? 3u : 1u));
     }
     launch_downscale(b->args.pixels, b->args.imgs, at<const uint64_t>(b->d_small, 0), at<uint8_t>(b->d_small, 0), (uint32_t)b->n, max_samples,
                      (uint32_t)factor, fmt, s);
@@ -915,12 +920,11 @@ extern "C" int b2j_batch_downscaled_device(const b2j_batch *b, int image, void *
 {
     const ImgDev *im = image_of(b, image);
     if (!im || !dptr || !b->small_factor) return B2J_E_ARG;
-    uint32_t ow, oh;
-    small_dims(*im, b->small_factor, &ow, &oh);
+    const Dims o = out_dims(*im, (uint32_t)b->small_factor);
     *dptr = at<uint8_t>(b->d_small, b->small_off[(size_t)image]);
-    if (nbytes) *nbytes = (size_t)ow * oh * format_bpp(b->args.out_format);
-    if (width) *width = (int)ow;
-    if (height) *height = (int)oh;
+    if (nbytes) *nbytes = (size_t)o.w * o.h * format_bpp(b->args.out_format);
+    if (width) *width = (int)o.w;
+    if (height) *height = (int)o.h;
     return B2J_OK;
 }
 
@@ -937,21 +941,14 @@ extern "C" int b2j_batch_read_downscaled(b2j_batch *b, void *stream, int image, 
 
 namespace {
 
-// Buffers back to the pools without a stream synchronisation: the caller has seen the event that closes the batch's work.
-void destroy_batch_done(b2j_batch *b)
-{
-    release_batch_buffers(b);
-    delete b;
-}
-
 // Host feed only: the images of the batch packed as tightly in the pixel plane as the stores of the colour kernel allow
 // (16-byte aligned starts for BGRA, 4-byte aligned for the three-byte formats, none for GRAY8, whose kernel stores bytes
 // at any alignment), so that the downloads of neighbouring images merge into one copy when the caller's buffers are
-// neighbours too. Before b2j_batch_upload().
-void pack_pixel_plane(b2j_batch *b, int fmt)
+// neighbours too. After set_output(), before b2j_batch_upload().
+void pack_pixel_plane(b2j_batch *b)
 {
+    const int fmt = b->args.out_format;
     const size_t a = fmt == B2J_OUT_BGRA ? 16 : (fmt == B2J_OUT_GRAY8 ? 1 : 4);
-    b->args.out_format = fmt;
     size_t off = 0;
     for (ImgDev &im : b->imgs)
     {
@@ -979,7 +976,6 @@ struct FeedGroup
     bool ready = false;                  // set by the worker under the feed mutex
     bool parsed = false;                 // the header verdicts of its files are in status[]
     cudaEvent_t decoded = nullptr, done = nullptr;
-    bool closed = false;
 };
 
 } // namespace
@@ -988,22 +984,9 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
                                   uint8_t *const *out, int32_t *status)
 {
     if (!ctx || n <= 0 || !files || !lens || !out || !status || !opts) return B2J_E_ARG;
-    const int fmt = opts->out_format;
-    if (!format_ok(fmt)) return B2J_E_ARG;
-    const int model = opts->pixel_model;
-    if (model != B2J_PIXELS_REFERENCE && model != B2J_PIXELS_LIBJPEG) return B2J_E_ARG;
-    if (fmt == B2J_OUT_GRAY8 && model != B2J_PIXELS_LIBJPEG)
-    {
-        t_last_error = "B2J_OUT_GRAY8 (libjpeg's grayscale output) needs the libjpeg pixel model: the reference has none";
-        return B2J_E_ARG;
-    }
-    const int scale = opts->scale ? opts->scale : 1;
-    if (!scale_ok(scale)) return B2J_E_ARG;
-    if (scale != 1 && model != B2J_PIXELS_LIBJPEG)
-    {
-        t_last_error = "a scaled decode (b2j_host_opts.scale) needs the libjpeg pixel model: the reference has none";
-        return B2J_E_ARG;
-    }
+    const int fmt = opts->out_format, model = opts->pixel_model, scale = opts->scale ? opts->scale : 1;
+    if (!format_ok(fmt) || !model_ok(model) || !scale_ok(scale)) return B2J_E_ARG;
+    if (const char *why = output_refusal(model, fmt, scale)) { t_last_error = why; return B2J_E_ARG; }
     CU_TRY(cudaSetDevice(ctx->device));
     const int gate = opts->gate;
     const int group = opts->group > 0 ? opts->group : 32;
@@ -1073,9 +1056,8 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
                 if (G.rc != B2J_OK) G.err = t_last_error;
                 else
                 {
-                    b2j_batch_set_scale(G.b, scale);   // before the packing: it sizes the images
-                    pack_pixel_plane(G.b, fmt);
-                    b2j_batch_set_pixel_model(G.b, model);
+                    set_output(G.b, model, fmt, scale);
+                    pack_pixel_plane(G.b);
                 }
             }
             {
@@ -1090,31 +1072,36 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
 
     int rc = B2J_OK;
     int oldest = 0;   // first group whose buffers are still held
+    // Hands a group's status words to the caller and its buffers back to the pools; a second call does nothing.
     auto close_group = [&](FeedGroup &G) {
-        if (G.closed) return;
-        G.closed = true;
         if (G.b)
         {
             for (size_t k = 0; k < G.idx.size(); k++) status[G.idx[k]] = h_status[G.idx[k]];
-            destroy_batch_done(G.b);
+            release_batch_buffers(G.b);   // no stream synchronisation: the group's work is over (its `done` event)
+            delete G.b;
             G.b = nullptr;
         }
         if (G.decoded) cudaEventDestroy(G.decoded);
         if (G.done) cudaEventDestroy(G.done);
         G.decoded = G.done = nullptr;
     };
+    // Closes the groups before `end`, oldest first, so that their buffers serve the groups still to come: with `wait`
+    // once each group's downloads have arrived, without it up to the first group whose downloads are still in flight.
+    auto retire = [&](int end, bool wait) {
+        for (; oldest < end; oldest++)
+        {
+            FeedGroup &O = groups[(size_t)oldest];
+            const cudaError_t q = !O.done ? cudaSuccess : (wait ? cudaEventSynchronize(O.done) : cudaEventQuery(O.done));
+            if (!wait && q != cudaSuccess) { if (q == cudaErrorNotReady) cudaGetLastError(); return; }
+            close_group(O);
+        }
+    };
     const int max_in_flight = window + 4;   // groups enqueued and not yet back: bounds the buffers the pools ever hold, so that
                                             // after the first call no group waits for a cudaMalloc / cudaHostAlloc
     for (int g = 0; g < ng && rc == B2J_OK; g++)
     {
         FeedGroup &G = groups[(size_t)g];
-        while (g - oldest >= max_in_flight)
-        {
-            FeedGroup &O = groups[(size_t)oldest];
-            if (!O.closed && O.done) cudaEventSynchronize(O.done);
-            close_group(O);
-            oldest++;
-        }
+        retire(g - max_in_flight + 1, true);
         {
             std::unique_lock<std::mutex> lk(mu);
             cv.wait(lk, [&] { return G.ready; });
@@ -1122,7 +1109,7 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
         }
         cv.notify_all();
         if (G.rc != B2J_OK) { rc = G.rc; t_last_error = G.err; break; }
-        if (!G.b) { G.closed = true; continue; }
+        if (!G.b) continue;
         if ((rc = b2j_batch_upload(G.b, ctx->stream)) != B2J_OK) break;
         if ((rc = b2j_batch_decode(G.b, ctx->stream)) != B2J_OK) break;
         cudaError_t e = cudaEventCreateWithFlags(&G.decoded, cudaEventDisableTiming);
@@ -1152,18 +1139,7 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
         }
         if (e == cudaSuccess) e = cudaEventRecord(G.done, ctx->stream2);
         if (e != cudaSuccess) { rc = fail_cuda(e, "b2j_decode_host_ex enqueue"); break; }
-        // groups whose pixels have arrived give their buffers back to the pools for the groups still to come
-        while (oldest < g)
-        {
-            FeedGroup &O = groups[(size_t)oldest];
-            if (!O.closed)
-            {
-                const cudaError_t q = cudaEventQuery(O.done);
-                if (q != cudaSuccess) { if (q == cudaErrorNotReady) cudaGetLastError(); break; }
-            }
-            close_group(O);
-            oldest++;
-        }
+        retire(g, false);
     }
     {
         std::lock_guard<std::mutex> lk(mu);

@@ -2,7 +2,7 @@
 test_gpu_libjpeg.py -- everyday, generic and gray tiles, restart-interval and self-synchronising streams, a 3x11 image, a
 1080p 4:2:0 and a 4K 4:4:4 frame and streams of extreme coefficients -- at scales 1, 2, 4 and 8, against the numpy model and
 Pillow's draft("L"); status and coefficients, the launch count, the sample plane that GRAY8 does not allocate, switching
-formats and scales, downscale, the host calls and the refusals."""
+formats, scales and pixel models against fresh batches, downscale, the host calls and the refusals."""
 import numpy as np
 import pytest
 
@@ -123,9 +123,49 @@ def test_alternating_formats_and_scales_gives_a_fresh_batch_pixels(decoder, batc
         for i in range(len(ITEMS)):
             got = batch.pixels(i)
             assert np.array_equal(got, want[i]) and np.array_equal(got, px[2][i][0]), ITEMS[i][0]
+
+        # Whatever the settings before it, a (model, format, scale) setting gives what a batch set straight to it gives:
+        # the launch count, the output sizes and, where the combination decodes, the pixels. The reference model has no
+        # scaled decode and no GRAY8: decode() refuses those, and the next decode is still right.
+        def straight(model, fmt, s):
+            b = decoder.batch([it[1] for it in ITEMS], gate=_gate())
+            b.upload()
+            b.set_pixel_model(model)
+            b.set_output_format(fmt)
+            b.set_scale(s)
+            return b
+
+        ref, lj = b2j.PIXELS_REFERENCE, b2j.PIXELS_LIBJPEG
+        walk = [(lj, b2j.OUT_RGB_PLANAR, 4), (ref, b2j.OUT_RGB_PLANAR, 4), (ref, b2j.OUT_BGRA, 1), (lj, b2j.OUT_GRAY8, 8),
+                (ref, b2j.OUT_GRAY8, 8), (lj, b2j.OUT_BGRA, 2), (ref, b2j.OUT_RGB24, 1), (ref, b2j.OUT_GRAY8, 1),
+                (lj, b2j.OUT_RGB24, 1), (ref, b2j.OUT_RGB_PLANAR, 1)]
+        setters = (batch.set_pixel_model, batch.set_output_format, batch.set_scale)
+        for k, setting in enumerate(walk):
+            for j in range(3):   # the setters in another order at every step
+                setters[(j + k) % 3](setting[(j + k) % 3])
+            model, fmt, s = setting
+            other = straight(model, fmt, s)
+            try:
+                assert batch.info().kernel_launches == other.info().kernel_launches, setting
+                for i in range(len(ITEMS)):
+                    assert batch.pixels_device(i)[1] == other.pixels_device(i)[1], (ITEMS[i][0], setting)
+                if model == lj or (fmt != b2j.OUT_GRAY8 and s == 1):
+                    for b in (batch, other):
+                        b.decode()
+                        assert not b.status().any(), setting
+                    for i in range(len(ITEMS)):
+                        assert np.array_equal(batch.pixels(i), other.pixels(i)), (ITEMS[i][0], setting)
+                else:
+                    for b in (batch, other):
+                        with pytest.raises(b2j.B2JError) as e:
+                            b.decode()
+                        assert e.value.code == -1 and "libjpeg pixel model" in str(e.value), setting
+            finally:
+                other.close()
     finally:
         batch.set_scale(1)
         batch.set_output_format(b2j.OUT_BGRA)
+        batch.set_pixel_model(b2j.PIXELS_LIBJPEG)
         fresh.close()
 
 
