@@ -36,6 +36,8 @@
  *   b2j_batch_downscale     (none)              reduced copies of the decoded pixels for consumers (SURVEY.md 8f rank 3)
  *   b2j_batch_set_scale     (none)              libjpeg's scaled decode (scale_num / scale_denom, Pillow's draft()):
  *                                               1/2, 1/4 or 1/8 size straight from the coefficients
+ *   b2j_parse_orientation,  (none)              EXIF orientation as OpenCV's imdecode, torchvision's decode_jpeg(...,
+ *   b2j_batch_set_orientations                  apply_exif_orientation=True) and Pillow's exif_transpose() apply it
  *   b2j_idct_*              idct.h:9-18         the device backend as the reference's own decoder.cpp drives it
  *                                               (coefficients in, pixels out): see "secondary boundary" below
  *   b2j_read_files          decoder.cpp:94-101  the 2 KiB fread() loop (and main.cpp's fopen): whole files read with
@@ -177,7 +179,8 @@ typedef struct b2j_stage_times
 {
     float prepass_ms;   /* marker scan + unstuff + restart-interval table                   */
     float huffman_ms;   /* entropy decode -> int16 coefficient plane                        */
-    float idct_ms;      /* dequant + IDCT + upsample + colour -> BGRA                       */
+    float idct_ms;      /* dequant + IDCT + upsample + colour -> BGRA, and the orientation pass
+                         * (b2j_batch_set_orientations) when it runs                         */
     float total_ms;
 } b2j_stage_times;
 
@@ -199,6 +202,14 @@ const char *b2j_last_error(void);
  * long pass the limit, e.g. three DC and two AC tables of that kind. The reference decodes such files. The check is per
  * file, so that such a file cannot make b2j_batch_create fail for the whole batch. */
 int b2j_parse_header(const uint8_t *file, size_t len, int gate, b2j_image_desc *out);
+
+/* EXIF orientation of a file held in memory: *orientation = the value of tag 0x0112 (Orientation) in IFD0 of the first
+ * APP1 segment whose payload starts with "Exif\0\0" (what Pillow reads: an XMP APP1 in front of it is skipped, a second
+ * Exif APP1 is not read), read as 16 bits in the TIFF header's byte order (II or MM). The length-prefixed segments from SOI
+ * to SOS are walked whatever the gate. *orientation = 1 when there is no such tag, when its value is outside 1..8, and
+ * when anything is cut or malformed; nothing outside [file, file + len) is read. B2J_E_ARG only for null pointers.
+ * b2j_batch_set_orientations() and b2j_host_opts.exif_orientation take these codes. */
+int b2j_parse_orientation(const uint8_t *file, size_t len, int32_t *orientation);
 
 /* ------------------------------------------------------------------ device -------------- */
 int b2j_device_count(void);
@@ -247,6 +258,19 @@ int b2j_batch_set_pixel_model(b2j_batch *batch, int model);
  * and so does b2j_batch_downscale() while denom != 1. The coefficients, the status words and b2j_batch_info do not
  * change; the sample plane keeps its size. */
 int b2j_batch_set_scale(b2j_batch *batch, int denom);
+/* EXIF orientation of every image for the decodes that follow: codes[i] in 1..8 (b2j_parse_orientation), NULL = 1 for
+ * every image (the default); B2J_E_ARG for any other code, and then nothing changes. An image of w x h pixels at the
+ * batch's scale is decoded as before, then transformed (numpy, a = the (h, w, ...) image): 1 a, 2 a[:, ::-1],
+ * 3 a[::-1, ::-1], 4 a[::-1], 5 a.swapaxes(0, 1), 6 a.swapaxes(0, 1)[:, ::-1], 7 a.swapaxes(0, 1)[::-1, ::-1],
+ * 8 a.swapaxes(0, 1)[::-1]; codes 5..8 give h x w pixels. Planar RGB: each plane. Scaled decode first, then orientation:
+ * what OpenCV's cv2.imdecode / cv2.imread give with their default flags (IMREAD_COLOR, IMREAD_GRAYSCALE,
+ * IMREAD_REDUCED_*; only IMREAD_IGNORE_ORIENTATION turns it off), torchvision's decode_jpeg(..., apply_exif_orientation=True)
+ * and Pillow's ImageOps.exif_transpose(). In both pixel models, every output format and every scale. The oriented
+ * pixels have tight pitch in the batch's format and as many bytes as the unoriented ones; b2j_batch_pixels_device and
+ * the reads return them. One more kernel runs after the IDCT/colour stage over the images whose code is not 1, into a
+ * buffer of their own (b2j_batch_info counts both); with every code 1 a decode is what it is without this call.
+ * b2j_batch_downscale() is refused (B2J_E_ARG) while a code is not 1. */
+int b2j_batch_set_orientations(b2j_batch *batch, const uint8_t *codes /* n or NULL */);
 
 /* Per-image status words (B2J_ST_* bits). Synchronises the stream. */
 int b2j_batch_status(b2j_batch *batch, void *stream, int32_t *status /* n */);
@@ -275,7 +299,8 @@ int b2j_batch_read_coefs(b2j_batch *batch, void *stream, int image, int32_t *dst
 /* Output stage for consumers that want smaller images (SURVEY.md 8f rank 3): box-filter reduction of the decoded pixels by
  * factor 2, 4 or 8 per axis, after b2j_batch_decode(), in the batch's output format. Reduced size: ceil(w/f) x ceil(h/f);
  * every value is the rounded mean (sum + n/2) / n of the n input values it covers (at the right / bottom edge: of those that
- * exist). The full-size pixels stay where they are. B2J_E_ARG while the batch's scale (b2j_batch_set_scale) is not 1. */
+ * exist). The full-size pixels stay where they are. B2J_E_ARG while the batch's scale (b2j_batch_set_scale) is not 1, and
+ * while an orientation code (b2j_batch_set_orientations) is not 1. */
 int b2j_batch_downscale(b2j_batch *batch, void *stream, int factor);
 int b2j_batch_downscaled_device(const b2j_batch *batch, int image, void **dptr, size_t *nbytes, int *width, int *height);
 int b2j_batch_read_downscaled(b2j_batch *batch, void *stream, int image, uint8_t *dst);   /* synchronises */
@@ -297,7 +322,8 @@ typedef struct b2j_host_opts
     int32_t group_mb;    /* and at most this many MiB of files per group (0 = 12): one host thread stages a group  */
     int32_t pixel_model; /* B2J_PIXELS_* (0 = the reference's pixels)                                             */
     int32_t scale;       /* 1, 2, 4 or 8 (0 = 1): b2j_batch_set_scale(); needs B2J_PIXELS_LIBJPEG                     */
-    int32_t reserved[1]; /* 0                                                                                     */
+    int32_t exif_orientation; /* 0: as decoded; 1: each file's b2j_parse_orientation() code applied
+                               * (b2j_batch_set_orientations()), so out[i] holds the oriented image, sides swapped for 5..8 */
 } b2j_host_opts;
 
 /* b2j_decode_host() with options: the pixels arrive in opts->out_format (RGB24 moves 25 % fewer bytes over PCIe,
@@ -305,7 +331,9 @@ typedef struct b2j_host_opts
  * staged by opts->n_threads host threads while the calling thread only enqueues uploads, decodes and downloads.
  * out[i]: w*h*4, w*h*3 or w*h (GRAY8) bytes, with w = ceil(width/scale) and h = ceil(height/scale) for opts->scale
  * (B2J_E_ARG for a scale other than 0, 1, 2, 4 and 8, and for a scale other than 1 or B2J_OUT_GRAY8 in the reference
- * pixel model). */
+ * pixel model). With opts->exif_orientation = 1 (B2J_E_ARG for a value other than 0 and 1) out[i] holds the image
+ * oriented by its EXIF code: h*w bytes per channel with the sides swapped for codes 5..8. b2j_decode_host() does not
+ * orient. */
 int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *files, const size_t *lens, const b2j_host_opts *opts,
                        uint8_t *const *out, int32_t *status);
 

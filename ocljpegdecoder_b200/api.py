@@ -19,9 +19,9 @@ B2J_E_NODEVICE = -7
 
 # every symbol include/b2j.h declares (tests check that the built library exports all of them)
 EXPORTED_SYMBOLS = [
-    "b2j_abi_version", "b2j_strerror", "b2j_last_error", "b2j_parse_header", "b2j_device_count",
+    "b2j_abi_version", "b2j_strerror", "b2j_last_error", "b2j_parse_header", "b2j_parse_orientation", "b2j_device_count",
     "b2j_create", "b2j_destroy", "b2j_batch_create", "b2j_batch_destroy", "b2j_batch_get_info",
-    "b2j_batch_upload", "b2j_batch_set_output_format", "b2j_batch_set_pixel_model", "b2j_batch_set_scale", "b2j_batch_decode", "b2j_batch_decode_timed", "b2j_batch_decode_steps", "b2j_batch_sync", "b2j_batch_status", "b2j_batch_sync_stats",
+    "b2j_batch_upload", "b2j_batch_set_output_format", "b2j_batch_set_pixel_model", "b2j_batch_set_scale", "b2j_batch_set_orientations", "b2j_batch_decode", "b2j_batch_decode_timed", "b2j_batch_decode_steps", "b2j_batch_sync", "b2j_batch_status", "b2j_batch_sync_stats",
     "b2j_batch_pixels_device", "b2j_batch_coefs_device", "b2j_batch_read_pixels", "b2j_batch_read_all_pixels",
     "b2j_batch_read_coefs", "b2j_decode_host", "b2j_decode_host_ex", "b2j_decode_host_multi", "b2j_host_alloc", "b2j_host_free",
     "b2j_read_files", "b2j_idct_create", "b2j_idct_blk_count", "b2j_idct_upload", "b2j_idct_run", "b2j_idct_read_pixels", "b2j_idct_read_coefs",
@@ -66,7 +66,7 @@ class BatchInfo(ctypes.Structure):
 class HostOpts(ctypes.Structure):
     """b2j_host_opts"""
     _fields_ = [("gate", ctypes.c_int32), ("out_format", ctypes.c_int32), ("n_threads", ctypes.c_int32), ("group", ctypes.c_int32),
-                ("group_mb", ctypes.c_int32), ("pixel_model", ctypes.c_int32), ("scale", ctypes.c_int32), ("reserved", ctypes.c_int32 * 1)]
+                ("group_mb", ctypes.c_int32), ("pixel_model", ctypes.c_int32), ("scale", ctypes.c_int32), ("exif_orientation", ctypes.c_int32)]
 
 
 class StageTimes(ctypes.Structure):
@@ -97,6 +97,7 @@ def load_library():
     L.b2j_strerror.argtypes = [ci]
     L.b2j_last_error.restype = ctypes.c_char_p
     L.b2j_parse_header.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ci, ctypes.POINTER(ImageDesc)]
+    L.b2j_parse_orientation.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.POINTER(ctypes.c_int32)]
     L.b2j_device_count.restype = ci
     L.b2j_create.argtypes = [ci, ctypes.POINTER(vp)]
     L.b2j_destroy.argtypes = [vp]
@@ -110,6 +111,7 @@ def load_library():
     L.b2j_batch_set_output_format.argtypes = [vp, ci]
     L.b2j_batch_set_pixel_model.argtypes = [vp, ci]
     L.b2j_batch_set_scale.argtypes = [vp, ci]
+    L.b2j_batch_set_orientations.argtypes = [vp, vp]
     L.b2j_batch_decode.argtypes = [vp, vp]
     L.b2j_batch_decode_timed.argtypes = [vp, vp, ctypes.POINTER(StageTimes)]
     L.b2j_batch_decode_steps.argtypes = [vp, vp, ci, ctypes.POINTER(StageTimes), ctypes.POINTER(ctypes.c_float)]
@@ -160,22 +162,34 @@ def parse_header(data, gate=GATE_EXTENDED):
     return rc, d
 
 
-def _out_shape(d, fmt, scale=1):
-    """Shape of an image's pixels in output format fmt, at 1/scale of its size (ceil(W/scale) x ceil(H/scale))."""
+def parse_orientation(data):
+    """b2j_parse_orientation: the file's EXIF orientation code, 1..8 (1 when it has none or it is out of range)."""
+    o = ctypes.c_int32()
+    _check(load_library().b2j_parse_orientation(data, len(data), ctypes.byref(o)), "b2j_parse_orientation")
+    return o.value
+
+
+def _out_shape(d, fmt, scale=1, orientation=1):
+    """Shape of an image's pixels in output format fmt, at 1/scale of its size (ceil(W/scale) x ceil(H/scale)), with the
+    sides swapped for the EXIF orientation codes 5..8."""
     w, h = -(-d.width // scale), -(-d.height // scale)
+    if orientation >= 5:
+        w, h = h, w
     if fmt == OUT_GRAY8:
         return (h, w)
     return (h, w, 4) if fmt == OUT_BGRA else ((h, w, 3) if fmt == OUT_RGB24 else (3, h, w))
 
 
-def _host_call_args(files, outs, gate, fmt, scale=1):
-    """Argument arrays of the b2j_decode_host* calls; allocates the outputs when none are given."""
+def _host_call_args(files, outs, gate, fmt, scale=1, exif_orientation=False):
+    """Argument arrays of the b2j_decode_host* calls; allocates the outputs when none are given (oriented with
+    exif_orientation)."""
     n = len(files)
     if outs is None:
         outs = []
         for f in files:
             rc, d = parse_header(f, gate)
-            outs.append(np.zeros(_out_shape(d, fmt, scale or 1), np.uint8) if rc == 0 else np.zeros((0, 0, 4), np.uint8))
+            o = parse_orientation(f) if exif_orientation else 1
+            outs.append(np.zeros(_out_shape(d, fmt, scale or 1, o), np.uint8) if rc == 0 else np.zeros((0, 0, 4), np.uint8))
     ptrs = [f if isinstance(f, int) else ctypes.cast(ctypes.c_char_p(f), ctypes.c_void_p).value for f in files]
     fp = ctypes.cast((ctypes.c_void_p * n)(*ptrs), ctypes.POINTER(ctypes.c_char_p))
     return outs, fp, (ctypes.c_void_p * n)(*[o if isinstance(o, int) else o.ctypes.data for o in outs])
@@ -186,14 +200,14 @@ class HostArgs:
     ctypes work per call otherwise): files / lens / outs as for Decoder.decode_host_ex."""
 
     def __init__(self, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0, group_mb=0,
-                 pixel_model=PIXELS_REFERENCE, scale=1):
+                 pixel_model=PIXELS_REFERENCE, scale=1, exif_orientation=False):
         self.n = len(files)
         self.files = files                      # keeps the bytes objects alive
         lens = lens if lens is not None else [len(f) for f in files]
-        self.outs, self.fp, self.op = _host_call_args(files, outs, gate, out_format, scale)
+        self.outs, self.fp, self.op = _host_call_args(files, outs, gate, out_format, scale, exif_orientation)
         self.ln = (ctypes.c_size_t * self.n)(*lens)
         self.opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, group_mb=group_mb, pixel_model=pixel_model,
-                             scale=scale)
+                             scale=scale, exif_orientation=int(exif_orientation))
         self.status = np.zeros(self.n, np.int32)
 
 
@@ -241,14 +255,15 @@ def host_free(address):
 
 
 def decode_host_multi(decoders, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0,
-                      pixel_model=PIXELS_REFERENCE, scale=1):
+                      pixel_model=PIXELS_REFERENCE, scale=1, exif_orientation=False):
     """b2j_decode_host_multi over the given Decoder objects (one per GPU). files: bytes objects or addresses (then `lens`)."""
     L = load_library()
     n = len(files)
     lens = lens if lens is not None else [len(f) for f in files]
-    outs, fp, op = _host_call_args(files, outs, gate, out_format, scale)
+    outs, fp, op = _host_call_args(files, outs, gate, out_format, scale, exif_orientation)
     ln = (ctypes.c_size_t * n)(*lens)
-    opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, pixel_model=pixel_model, scale=scale)
+    opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, pixel_model=pixel_model, scale=scale,
+                    exif_orientation=int(exif_orientation))
     cx = (ctypes.c_void_p * len(decoders))(*[d._h.value for d in decoders])
     status = np.zeros(n, np.int32)
     _check(L.b2j_decode_host_multi(cx, len(decoders), n, fp, ln, ctypes.byref(opts), op, status.ctypes.data), "b2j_decode_host_multi")
@@ -306,15 +321,16 @@ class Decoder:
         return args.outs, args.status
 
     def decode_host_ex(self, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0,
-                       pixel_model=PIXELS_REFERENCE, scale=1):
+                       pixel_model=PIXELS_REFERENCE, scale=1, exif_orientation=False):
         """b2j_decode_host_ex: like decode_host with an output layout (OUT_GRAY8 with PIXELS_LIBJPEG only), a pixel model,
-        a scale (1, 2, 4 or 8: the libjpeg model's scaled decode) and host threads. files: bytes objects or addresses (then
-        `lens`); outs: numpy arrays or addresses."""
+        a scale (1, 2, 4 or 8: the libjpeg model's scaled decode), each file's EXIF orientation applied (exif_orientation)
+        and host threads. files: bytes objects or addresses (then `lens`); outs: numpy arrays or addresses."""
         n = len(files)
         lens = lens if lens is not None else [len(f) for f in files]
-        outs, fp, op = _host_call_args(files, outs, gate, out_format, scale)
+        outs, fp, op = _host_call_args(files, outs, gate, out_format, scale, exif_orientation)
         ln = (ctypes.c_size_t * n)(*lens)
-        opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, pixel_model=pixel_model, scale=scale)
+        opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, pixel_model=pixel_model, scale=scale,
+                        exif_orientation=int(exif_orientation))
         status = np.zeros(n, np.int32)
         _check(self.lib.b2j_decode_host_ex(self._h, n, fp, ln, ctypes.byref(opts), op, status.ctypes.data), "b2j_decode_host_ex")
         return outs, status
@@ -369,6 +385,7 @@ class Batch:
         self.descs = descs
         self.n = len(files)
         self.out_format, self.pixel_model, self.scale = OUT_BGRA, PIXELS_REFERENCE, 1   # what b2j_batch_create sets
+        self.orientations = None
         fp = (ctypes.c_char_p * self.n)(*self.files)
         ln = (ctypes.c_size_t * self.n)(*[len(f) for f in self.files])
         self._h = ctypes.c_void_p()
@@ -439,9 +456,20 @@ class Batch:
         _check(self.lib.b2j_batch_set_scale(self._h, denom), "b2j_batch_set_scale")
         self.scale = denom
 
+    def set_orientations(self, codes=None):
+        """EXIF orientation codes (1..8, one per image, e.g. parse_orientation() of each file) for the decodes that follow:
+        each image is decoded at the batch's scale, then rotated / mirrored as OpenCV's imdecode, torchvision's
+        decode_jpeg(apply_exif_orientation=True) and Pillow's exif_transpose() do. None: every code 1 (the default)."""
+        arr = None if codes is None else np.ascontiguousarray(codes, np.uint8)
+        if arr is not None and arr.shape != (self.n,):
+            raise ValueError("one orientation code per image")
+        _check(self.lib.b2j_batch_set_orientations(self._h, None if arr is None else arr.ctypes.data), "b2j_batch_set_orientations")
+        self.orientations = None if arr is None or (arr == 1).all() else arr.copy()
+
     def pixel_shape(self, i):
-        """Shape of image i's pixels in the batch's output format and scale."""
-        return _out_shape(self.descs[i], self.out_format, self.scale)
+        """Shape of image i's pixels in the batch's output format, scale and orientation."""
+        o = 1 if self.orientations is None else int(self.orientations[i])
+        return _out_shape(self.descs[i], self.out_format, self.scale, o)
 
     def pixels(self, i, stream=None):
         out = np.zeros(self.pixel_shape(i), np.uint8)

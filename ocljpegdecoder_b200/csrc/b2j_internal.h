@@ -128,6 +128,16 @@ struct TileDev
     uint32_t info;        // SamplingMode | n_mcus << 8
 };
 
+// One tile of the orientation pass (k_orient): kOrientTile x kOrientTile pixels of one image whose EXIF orientation code
+// is not 1, at the batch's scale.
+constexpr uint32_t kOrientTile = 64;
+struct OrientTileDev
+{
+    uint64_t dst_off;     // byte offset of the image's oriented copy in the output buffer
+    uint32_t img;
+    uint32_t tile;        // tile column | tile row << 11 | orientation code << 22
+};
+
 // ---------------------------------------------------------------- host helpers ---------
 // Canonical Huffman table -> two-level LUT. Returns false when the table cannot be built
 // (code space overflow) or needs more than `max_entries` entries.

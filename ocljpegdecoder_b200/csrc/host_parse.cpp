@@ -12,6 +12,8 @@
 
 #include <string.h>
 
+#include <algorithm>
+
 namespace {
 
 struct Reader
@@ -255,4 +257,61 @@ extern "C" int b2j_parse_header(const uint8_t *file, size_t len, int gate_flags,
         if (!r.take(tag, 2)) return B2J_E_FORMAT;
     }
     return B2J_E_FORMAT;
+}
+
+namespace {
+
+// EXIF orientation (tag 0x0112 of IFD0) from the TIFF structure of an Exif APP1 payload behind "Exif\0\0": its 16-bit
+// value in the file's byte order, or 1 when there is none, it is outside 1..8, or the structure is cut or malformed.
+int32_t tiff_orientation(const uint8_t *t, size_t n)
+{
+    if (n < 8) return 1;
+    const bool le = t[0] == 'I' && t[1] == 'I' && t[2] == 42 && t[3] == 0;
+    if (!le && !(t[0] == 'M' && t[1] == 'M' && t[2] == 0 && t[3] == 42)) return 1;
+    auto u16 = [&](size_t o) { return le ? (uint32_t)t[o] | (uint32_t)t[o + 1] << 8 : (uint32_t)t[o] << 8 | t[o + 1]; };
+    const size_t ifd = le ? (size_t)(u16(4) | u16(6) << 16) : (size_t)(u16(4) << 16 | u16(6));
+    if (ifd > n - 2) return 1;
+    const size_t count = u16(ifd);
+    for (size_t k = 0; k < count; k++)
+    {
+        const size_t e = ifd + 2 + 12 * k;
+        if (n < 12 || e > n - 12) return 1;
+        if (u16(e) == 0x0112)
+        {
+            const uint32_t v = u16(e + 8);
+            return v >= 1 && v <= 8 ? (int32_t)v : 1;
+        }
+    }
+    return 1;
+}
+
+} // namespace
+
+extern "C" int b2j_parse_orientation(const uint8_t *file, size_t len, int32_t *orientation)
+{
+    if (!file || !orientation) return B2J_E_ARG;
+    *orientation = 1;
+    if (len < 2 || file[0] != 0xFF || file[1] != 0xD8) return B2J_OK;
+    // the length-prefixed segments from SOI to SOS, whatever the gate; the first APP1 that starts with "Exif\0\0" counts
+    // (what Pillow reads: an XMP APP1 in front of it is skipped, a second Exif APP1 is not read)
+    size_t pos = 2;
+    while (len - pos >= 4)
+    {
+        if (file[pos] != 0xFF) return B2J_OK;
+        const uint8_t m = file[pos + 1];
+        if (m == 0xFF) { pos++; continue; }   // fill byte in front of a marker
+        if (m == 0xDA || m == 0xD9) return B2J_OK;
+        if (m == 0x01 || (m >= 0xD0 && m <= 0xD7)) { pos += 2; continue; }   // stand-alone markers
+        const size_t l = be16(file + pos + 2);
+        if (l < 2) return B2J_OK;
+        const size_t body = pos + 4, end = std::min(pos + 2 + l, len);   // a segment cut by the end of the file: what is there
+        if (m == 0xE1 && end - body >= 6 && memcmp(file + body, "Exif\0\0", 6) == 0)
+        {
+            *orientation = tiff_orientation(file + body + 6, end - body - 6);
+            return B2J_OK;
+        }
+        pos += 2 + l;
+        if (pos > len) return B2J_OK;
+    }
+    return B2J_OK;
 }

@@ -24,6 +24,8 @@
 //       the libjpeg pixel model in B2J_OUT_GRAY8 (libjpeg's JCS_GRAYSCALE): the luma blocks only, straight into the pixels.
 //   k_expand_coefs
 //       the reference's coefficient tap (int32, dequantised) from the int16 plane, for parity.
+//   k_orient
+//       EXIF orientation after the IDCT/colour stage: tiled copies of the images whose code is not 1, rotated or mirrored.
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -2098,6 +2100,90 @@ k_downscale(const uint8_t *__restrict__ pix, const ImgDev *__restrict__ imgs, co
 }
 
 // =====================================================================================
+// EXIF orientation (b2j_batch_set_orientations): a copy of every image whose code is not 1, transformed. One CTA per tile
+// of kOrientTile x kOrientTile source pixels of one image, from a flat host-built list over every oriented image. The
+// tile's source rows are read as aligned 4-byte words into shared memory, each row keeping its misalignment; then the
+// destination rows the tile covers are written as aligned words, with single bytes where a row's bytes begin or end
+// inside a word. So the transposing codes 5..8 read and write whole rows too, and no byte outside an image's result is
+// written: the host feed packs GRAY8 and three-byte images at 1- and 4-byte alignment. Destination (X, Y) takes the
+// source pixel (x, y) with (u, v) = (Y, X) for codes 5..8, else (X, Y); x = u, or w - 1 - u for codes 2, 3, 7 and 8;
+// y = v, or h - 1 - v for codes 3, 4, 6 and 7.
+template <int FMT>
+__global__ void __launch_bounds__(256)
+k_orient(const uint8_t *__restrict__ pix, const ImgDev *__restrict__ imgs, const OrientTileDev *__restrict__ tiles, uint32_t scale,
+         uint8_t *__restrict__ out)
+{
+    constexpr uint32_t T = kOrientTile;
+    constexpr uint32_t bpp = FMT == B2J_OUT_BGRA ? 4u : (FMT == B2J_OUT_RGB24 ? 3u : 1u);
+    constexpr uint32_t planes = FMT == B2J_OUT_RGB_PLANAR ? 3u : 1u;
+    constexpr uint32_t pw = ((T * bpp + 3u) / 4u + 1u) | 1u;   // words per shared row: a row's bytes and its misalignment; odd,
+                                                                // so that the rows of one column fall into different banks
+    __shared__ uint32_t s_w[T * pw];
+    const uint8_t *s_b = reinterpret_cast<const uint8_t *>(s_w);
+    const OrientTileDev t = tiles[blockIdx.x];
+    const ImgDev &im = imgs[t.img];
+    const uint32_t w = (im.width + scale - 1u) / scale, h = (im.height + scale - 1u) / scale;
+    const uint32_t code = t.tile >> 22, x0 = (t.tile & 0x7FFu) * T, y0 = ((t.tile >> 11) & 0x7FFu) * T;
+    const uint32_t tw = min(T, w - x0), th = min(T, h - y0);
+    const bool swap = code >= 5u, mx = code == 2u || code == 3u || code == 7u || code == 8u, my = code == 3u || code == 4u || code == 6u || code == 7u;
+    const uint32_t u0 = mx ? w - x0 - tw : x0, v0 = my ? h - y0 - th : y0;   // the tile's (u, v) rectangle
+    const uint32_t dx0 = swap ? v0 : u0, dy0 = swap ? u0 : v0, dw = swap ? th : tw, dh = swap ? tw : th;
+    const size_t spitch = (size_t)w * bpp, dpitch = (size_t)(swap ? h : w) * bpp, plane = (size_t)w * h;
+    for (uint32_t p = 0; p < planes; p++)
+    {
+        const uint8_t *src = pix + im.pix_off + p * plane + (size_t)y0 * spitch + x0 * bpp;
+        uint8_t *dst = out + t.dst_off + p * plane + (size_t)dy0 * dpitch + dx0 * bpp;
+        if (p) __syncthreads();
+        for (uint32_t i = threadIdx.x; i < th * pw; i += blockDim.x)
+        {
+            const uint32_t r = i / pw, k = i % pw;
+            const uint8_t *row = src + r * spitch;
+            const uint32_t a = (uint32_t)(uintptr_t)row & 3u;
+            // a whole aligned word that holds a byte of the row lies inside the plane's allocation
+            if (4u * k < a + tw * bpp) s_w[r * pw + k] = __ldg(reinterpret_cast<const uint32_t *>(row - a) + k);
+        }
+        __syncthreads();
+        for (uint32_t i = threadIdx.x; i < dh * pw; i += blockDim.x)
+        {
+            const uint32_t r = i / pw, k = i % pw, len = dw * bpp;
+            uint8_t *row = dst + r * dpitch;
+            const uint32_t a = (uint32_t)(uintptr_t)row & 3u;
+            const int32_t b0 = (int32_t)(4u * k) - (int32_t)a;   // the word's first byte, counted from the row's first
+            if (b0 >= (int32_t)len) continue;
+            if constexpr (bpp == 4u)
+            {
+                // BGRA rows are 4-byte aligned: word k is destination pixel k
+                const uint32_t uu = swap ? r : k, vv = swap ? k : r;
+                const uint32_t lx = mx ? tw - 1u - uu : uu, ly = my ? th - 1u - vv : vv;
+                *reinterpret_cast<uint32_t *>(row + 4u * k) = s_w[ly * pw + lx];
+            }
+            else
+            {
+                uint32_t v = 0u;
+#pragma unroll
+                for (uint32_t j = 0; j < 4u; j++)
+                {
+                    const int32_t b = b0 + (int32_t)j;
+                    if (b < 0 || b >= (int32_t)len) continue;
+                    const uint32_t X = (uint32_t)b / bpp, c = (uint32_t)b % bpp;
+                    const uint32_t uu = swap ? r : X, vv = swap ? X : r;
+                    const uint32_t lx = mx ? tw - 1u - uu : uu, ly = my ? th - 1u - vv : vv;
+                    const uint32_t sa = (uint32_t)(uintptr_t)(src + ly * spitch) & 3u;
+                    v |= (uint32_t)s_b[ly * pw * 4u + sa + lx * bpp + c] << (8u * j);
+                }
+                if (b0 >= 0 && b0 + 4 <= (int32_t)len) *reinterpret_cast<uint32_t *>(row + b0) = v;
+                else
+                    for (uint32_t j = 0; j < 4u; j++)
+                    {
+                        const int32_t b = b0 + (int32_t)j;
+                        if (b >= 0 && b < (int32_t)len) row[b] = (uint8_t)(v >> (8u * j));
+                    }
+            }
+        }
+    }
+}
+
+// =====================================================================================
 // Launchers (host).
 size_t huff_smem_bytes(uint32_t max_lut_len) { return (size_t)kHuffThreads * 128 + kZzBytes + (size_t)max_lut_len * 2; }
 
@@ -2219,6 +2305,16 @@ void launch_downscale(const uint8_t *pix, const ImgDev *imgs, const uint64_t *ou
     if (n_images == 0 || max_out_samples == 0) return;
     const dim3 grid((max_out_samples + 255u) / 256u, n_images < 65535u ? n_images : 65535u);   // gridDim.y is at most 65535
     k_downscale<<<grid, 256, 0, s>>>(pix, imgs, out_off, out, n_images, factor, fmt);
+}
+
+void launch_orient(const uint8_t *pix, const ImgDev *imgs, const OrientTileDev *tiles, uint32_t n_tiles, uint32_t scale, int fmt, uint8_t *out,
+                   cudaStream_t s)
+{
+    if (n_tiles == 0) return;   // one CTA per tile: a flat grid, so any number of images fits
+    if (fmt == B2J_OUT_RGB24) k_orient<B2J_OUT_RGB24><<<n_tiles, 256, 0, s>>>(pix, imgs, tiles, scale, out);
+    else if (fmt == B2J_OUT_RGB_PLANAR) k_orient<B2J_OUT_RGB_PLANAR><<<n_tiles, 256, 0, s>>>(pix, imgs, tiles, scale, out);
+    else if (fmt == B2J_OUT_GRAY8) k_orient<B2J_OUT_GRAY8><<<n_tiles, 256, 0, s>>>(pix, imgs, tiles, scale, out);
+    else k_orient<B2J_OUT_BGRA><<<n_tiles, 256, 0, s>>>(pix, imgs, tiles, scale, out);
 }
 
 void launch_pack(const int32_t *in, int16_t *coef, size_t n_values, cudaStream_t s)

@@ -61,6 +61,8 @@ void launch_idct(const DecodeArgs &a, cudaStream_t s);      // reference model: 
 int idct_launches(const DecodeArgs &a);                      // kernels launch_idct() enqueues
 void launch_downscale(const uint8_t *pix, const ImgDev *imgs, const uint64_t *out_off, uint8_t *out, uint32_t n_images, uint32_t max_out_samples,
                       uint32_t factor, int fmt, cudaStream_t s);   // box-filter reduction of the pixel plane
+void launch_orient(const uint8_t *pix, const ImgDev *imgs, const OrientTileDev *tiles, uint32_t n_tiles, uint32_t scale, int fmt, uint8_t *out,
+                   cudaStream_t s);   // 1 kernel: EXIF orientation of the images the tiles cover, into `out`
 void launch_pack(const int32_t *in, int16_t *coef, size_t n_values, cudaStream_t s);   // int32 dequantised coefficients -> the int16 plane
 void launch_expand(const int16_t *coef, const uint16_t *qtab, uint32_t blk_count, uint32_t tot, uint32_t ny, uint32_t nu, int32_t *out, cudaStream_t s);
 

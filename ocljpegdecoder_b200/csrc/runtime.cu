@@ -137,6 +137,15 @@ struct b2j_batch
     PoolBuf d_samples;   // lazily allocated by the first decode in the libjpeg pixel model: its sample plane
     int small_factor = 0;                     // 0 = none
     std::vector<uint64_t> small_off;          // byte offset of every image's reduced pixels behind the offset table
+    // EXIF orientation (b2j_batch_set_orientations): d_orient holds the orientation pass's tile table, then the oriented
+    // copies of the images whose code is not 1, in image order; h_orient is the pinned staging of the table
+    std::vector<uint8_t> orient;              // one code per image; empty = every code 1
+    std::vector<uint64_t> orient_off;         // byte offset of an oriented image's copy in d_orient
+    PoolBuf d_orient, h_orient;
+    size_t orient_table_bytes = 0;            // room for the table at scale 1, where an image has the most tiles
+    uint32_t n_orient_tiles = 0;
+    bool orient_stale = false;                // the table on the device is not the one of the current settings
+    cudaEvent_t orient_copied = nullptr;      // the last copy out of h_orient
 
     CUtensorMap tmap;
     DecodeArgs args;
@@ -211,20 +220,33 @@ bool geometry_ok(const b2j_image_desc &d)
 
 cudaStream_t pick_stream(b2j_batch *b, void *stream) { return b->last_stream = (stream ? (cudaStream_t)stream : b->ctx->stream); }
 
-// Grows the device buffer `buf` to at least n bytes from the context's pool; its contents are not kept. On failure the
-// buffer is left empty and CUDA's last error is cleared, so that it cannot fail the next, unrelated call on this thread.
-cudaError_t grow(b2j_ctx *ctx, PoolBuf &buf, size_t n)
+// Grows the device (or, `pinned`, page-locked host) buffer `buf` to at least n bytes from the context's pool; its contents
+// are not kept. On failure the buffer is left empty and CUDA's last error is cleared, so that it cannot fail the next,
+// unrelated call on this thread.
+cudaError_t grow(b2j_ctx *ctx, PoolBuf &buf, size_t n, bool pinned = false)
 {
     if (buf.cap >= n) return cudaSuccess;
     std::lock_guard<std::mutex> lk(ctx->mu);
-    ctx->dev_pool.put(buf);
-    const cudaError_t e = ctx->dev_pool.get(n, buf);
+    Pool &pool = pinned ? ctx->pin_pool : ctx->dev_pool;
+    pool.put(buf);
+    const cudaError_t e = pool.get(n, buf);
     if (e != cudaSuccess) cudaGetLastError();
     return e;
 }
 
+void release_orient_buffers(b2j_batch *b)
+{
+    b2j_ctx *c = b->ctx;
+    std::lock_guard<std::mutex> lk(c->mu);
+    c->dev_pool.put(b->d_orient);
+    c->pin_pool.put(b->h_orient);
+}
+
 void release_batch_buffers(b2j_batch *b)
 {
+    release_orient_buffers(b);
+    if (b->orient_copied) cudaEventDestroy(b->orient_copied);
+    b->orient_copied = nullptr;
     b2j_ctx *c = b->ctx;
     std::lock_guard<std::mutex> lk(c->mu);
     c->pin_pool.put(b->h_blob);
@@ -235,7 +257,7 @@ void release_batch_buffers(b2j_batch *b)
 // b2j_batch_downscale() are not counted)
 int64_t device_bytes(const b2j_batch *b)
 {
-    return (int64_t)(b->d_blob.cap + b->d_scratch.cap + b->d_coef.cap + b->d_pix.cap + b->d_samples.cap);
+    return (int64_t)(b->d_blob.cap + b->d_scratch.cap + b->d_coef.cap + b->d_pix.cap + b->d_samples.cap + b->d_orient.cap);
 }
 
 // The image `image` of the batch, or nullptr when the batch has no such image.
@@ -271,8 +293,12 @@ size_t image_bytes(const b2j_batch *b, const ImgDev &im)
     return (size_t)o.w * o.h * format_bpp(b->args.out_format);
 }
 
-// The only writer of a batch's output settings and of what follows from them: the upsampling kernel's grid and the
-// launch count of a decode.
+// Alignment of an image's start when images are packed side by side in a format: what the stores of the kernels that
+// write them allow (16 bytes for BGRA, 4 for the three-byte formats, none for GRAY8, whose kernels store single bytes).
+size_t pack_align(int fmt) { return fmt == B2J_OUT_BGRA ? 16 : (fmt == B2J_OUT_GRAY8 ? 1 : 4); }
+
+// The only writer of a batch's output settings and of what follows from them: the upsampling kernel's grid, the places of
+// the oriented copies and the launch count of a decode.
 void set_output(b2j_batch *b, int model, int fmt, int scale)
 {
     b->args.pixel_model = model;   // the sample plane, once allocated, stays with the batch
@@ -285,7 +311,17 @@ void set_output(b2j_batch *b, int model, int fmt, int scale)
         groups = std::max(groups, (o.w + 3) / 4 * o.h);
     }
     b->args.max_px_groups = groups;
-    b->info.kernel_launches = b->fixed_launches + idct_launches(b->args);
+    // the oriented copies behind the tile table, neighbours in image order (d_orient is sized for BGRA at scale 1); the
+    // table itself follows the settings at the next decode
+    size_t off = b->orient_table_bytes;
+    for (size_t i = 0; i < b->orient.size(); i++)
+        if (b->orient[i] != 1)
+        {
+            b->orient_off[i] = off = align_up(off, pack_align(fmt));
+            off += image_bytes(b, b->imgs[i]);
+        }
+    b->orient_stale = !b->orient.empty();
+    b->info.kernel_launches = b->fixed_launches + idct_launches(b->args) + (b->orient.empty() ? 0 : 1);
 }
 
 // One device->host copy on the call's stream, waited for.
@@ -305,6 +341,13 @@ template <class T> const T *stage(const b2j_batch *b, size_t off, const std::vec
 {
     memcpy(at<T>(b->h_blob, off), v.data(), sizeof(T) * v.size());
     return at<const T>(b->d_blob, off);
+}
+
+// Where image i's pixels are read from: its oriented copy when its orientation code is not 1, else the pixel plane.
+uint8_t *result_of(const b2j_batch *b, size_t i)
+{
+    if (!b->orient.empty() && b->orient[i] != 1) return at<uint8_t>(b->d_orient, b->orient_off[i]);
+    return b->args.pixels + b->imgs[i].pix_off;
 }
 
 } // namespace
@@ -705,7 +748,32 @@ extern "C" int b2j_batch_upload(b2j_batch *b, void *stream)
 // after the IDCT/colour stage (= end of the step).
 constexpr size_t kStepEvents = 5;
 
-// One decode of the whole batch: the pre-pass, the entropy stage and the IDCT/colour stage, in order on `s`.
+// The orientation pass's tile table for the current settings, copied to the front of d_orient on `s`: one tile of
+// kOrientTile x kOrientTile pixels per piece of every image whose code is not 1, at the batch's scale.
+static int stage_orient_tiles(b2j_batch *b, cudaStream_t s)
+{
+    // the pinned table is rebuilt only once the copy out of it has left
+    if (!b->orient_copied) CU_TRY(cudaEventCreateWithFlags(&b->orient_copied, cudaEventDisableTiming));
+    else CU_TRY(cudaEventSynchronize(b->orient_copied));
+    OrientTileDev *t = at<OrientTileDev>(b->h_orient, 0);
+    uint32_t k = 0;
+    for (size_t i = 0; i < b->orient.size(); i++)
+    {
+        const uint32_t code = b->orient[i];
+        if (code == 1) continue;
+        const Dims o = out_dims(b->imgs[i], b->args.scale);
+        for (uint32_t ty = 0; ty * kOrientTile < o.h; ty++)
+            for (uint32_t tx = 0; tx * kOrientTile < o.w; tx++) t[k++] = {b->orient_off[i], (uint32_t)i, tx | ty << 11 | code << 22};
+    }
+    b->n_orient_tiles = k;
+    CU_TRY(cudaMemcpyAsync(b->d_orient.p, t, sizeof(OrientTileDev) * k, cudaMemcpyHostToDevice, s));
+    CU_TRY(cudaEventRecord(b->orient_copied, s));
+    b->orient_stale = false;
+    return B2J_OK;
+}
+
+// One decode of the whole batch: the pre-pass, the entropy stage and the IDCT/colour stage, in order on `s`, then the
+// orientation pass when some image's code is not 1.
 static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStepEvents or NULL */)
 {
     if (!b->uploaded) { t_last_error = "b2j_batch_decode before b2j_batch_upload"; return B2J_E_ARG; }
@@ -718,6 +786,8 @@ static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStep
         b->args.samples = at<uint8_t>(b->d_samples, 0);
         b->info.device_bytes = device_bytes(b);
     }
+    if (b->orient_stale)
+        if (const int rc = stage_orient_tiles(b, s)) return rc;
     const DecodeArgs &a = b->args;
     if (ev) CU_TRY(cudaEventRecord(ev[0], s));
     if (a.n_huff_ctas) CU_TRY(cudaMemsetAsync(a.seg_start, 0xFF, 4 * (size_t)b->n_segs_total, s));   // read by the restart-interval decoder only
@@ -729,6 +799,8 @@ static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStep
     launch_huffman_sync(a, s);
     if (ev) CU_TRY(cudaEventRecord(ev[3], s));
     launch_idct(a, s);
+    if (!b->orient.empty())
+        launch_orient(a.pixels, a.imgs, at<const OrientTileDev>(b->d_orient, 0), b->n_orient_tiles, a.scale, a.out_format, at<uint8_t>(b->d_orient, 0), s);
     if (ev) CU_TRY(cudaEventRecord(ev[4], s));
     CU_TRY(cudaGetLastError());
     return B2J_OK;
@@ -824,11 +896,56 @@ extern "C" int b2j_batch_set_scale(b2j_batch *b, int denom)
     return B2J_OK;
 }
 
+extern "C" int b2j_batch_set_orientations(b2j_batch *b, const uint8_t *codes)
+{
+    if (!b) return B2J_E_ARG;
+    bool any = false;
+    for (int i = 0; codes && i < b->n; i++)
+    {
+        if (codes[i] < 1 || codes[i] > 8) return B2J_E_ARG;
+        any = any || codes[i] != 1;
+    }
+    CU_TRY(cudaSetDevice(b->ctx->device));
+    // the buffers go back to the pool or grow: work in flight may still read the table or write the copies
+    if (b->last_stream && (b->d_orient.p || any)) CU_TRY(cudaStreamSynchronize(b->last_stream));
+    b->orient.clear();
+    b->orient_off.clear();
+    b->orient_table_bytes = 0;
+    int rc = B2J_OK;
+    if (any)
+    {
+        size_t tiles = 0, bytes = 0;   // at scale 1 in BGRA, the most any setting needs
+        for (int i = 0; i < b->n; i++)
+            if (codes[i] != 1)
+            {
+                const Dims o = out_dims(b->imgs[(size_t)i], 1);
+                tiles += (size_t)((o.w + kOrientTile - 1) / kOrientTile) * ((o.h + kOrientTile - 1) / kOrientTile);
+                bytes += (size_t)o.w * o.h * 4 + pack_align(B2J_OUT_BGRA) - 1;
+            }
+        const size_t table = align_up(sizeof(OrientTileDev) * tiles, 256);
+        if (grow(b->ctx, b->d_orient, table + bytes) != cudaSuccess || grow(b->ctx, b->h_orient, table, true) != cudaSuccess)
+        {
+            t_last_error = "orientation buffer allocation";
+            rc = B2J_E_NOMEM;   // every code is 1 then
+        }
+        else
+        {
+            b->orient.assign(codes, codes + b->n);
+            b->orient_off.assign((size_t)b->n, 0);
+            b->orient_table_bytes = table;
+        }
+    }
+    if (b->orient.empty()) release_orient_buffers(b);
+    b->info.device_bytes = device_bytes(b);
+    set_output(b, b->args.pixel_model, b->args.out_format, (int)b->args.scale);
+    return rc;
+}
+
 extern "C" int b2j_batch_pixels_device(const b2j_batch *b, int image, void **dptr, size_t *nbytes)
 {
     const ImgDev *im = image_of(b, image);
     if (!im || !dptr) return B2J_E_ARG;
-    *dptr = b->args.pixels + im->pix_off;
+    *dptr = result_of(b, (size_t)image);
     if (nbytes) *nbytes = image_bytes(b, *im);
     return B2J_OK;
 }
@@ -846,7 +963,7 @@ extern "C" int b2j_batch_read_pixels(b2j_batch *b, void *stream, int image, uint
 {
     const ImgDev *im = image_of(b, image);
     if (!im || !dst) return B2J_E_ARG;
-    return read_back(b, stream, dst, b->args.pixels + im->pix_off, image_bytes(b, *im));
+    return read_back(b, stream, dst, result_of(b, (size_t)image), image_bytes(b, *im));
 }
 
 extern "C" int b2j_batch_read_all_pixels(b2j_batch *b, void *stream, uint8_t *const *dsts)
@@ -858,7 +975,7 @@ extern "C" int b2j_batch_read_all_pixels(b2j_batch *b, void *stream, uint8_t *co
     {
         const ImgDev &im = b->imgs[(size_t)i];
         if (!dsts[i]) continue;
-        CU_TRY(cudaMemcpyAsync(dsts[i], b->args.pixels + im.pix_off, image_bytes(b, im), cudaMemcpyDeviceToHost, s));
+        CU_TRY(cudaMemcpyAsync(dsts[i], result_of(b, (size_t)i), image_bytes(b, im), cudaMemcpyDeviceToHost, s));
     }
     CU_TRY(cudaStreamSynchronize(s));
     return B2J_OK;
@@ -885,6 +1002,8 @@ extern "C" int b2j_batch_downscale(b2j_batch *b, void *stream, int factor)
 {
     if (!b || (factor != 2 && factor != 4 && factor != 8)) return B2J_E_ARG;
     if (b->args.scale != 1) { t_last_error = "b2j_batch_downscale of a scaled decode"; return B2J_E_ARG; }
+    // k_downscale takes each image's size from its unoriented descriptor
+    if (!b->orient.empty()) { t_last_error = "b2j_batch_downscale of oriented images (b2j_batch_set_orientations)"; return B2J_E_ARG; }
     CU_TRY(cudaSetDevice(b->ctx->device));
     cudaStream_t s = pick_stream(b, stream);
     const int fmt = b->args.out_format;
@@ -942,13 +1061,11 @@ extern "C" int b2j_batch_read_downscaled(b2j_batch *b, void *stream, int image, 
 namespace {
 
 // Host feed only: the images of the batch packed as tightly in the pixel plane as the stores of the colour kernel allow
-// (16-byte aligned starts for BGRA, 4-byte aligned for the three-byte formats, none for GRAY8, whose kernel stores bytes
-// at any alignment), so that the downloads of neighbouring images merge into one copy when the caller's buffers are
+// (pack_align), so that the downloads of neighbouring images merge into one copy when the caller's buffers are
 // neighbours too. After set_output(), before b2j_batch_upload().
 void pack_pixel_plane(b2j_batch *b)
 {
-    const int fmt = b->args.out_format;
-    const size_t a = fmt == B2J_OUT_BGRA ? 16 : (fmt == B2J_OUT_GRAY8 ? 1 : 4);
+    const size_t a = pack_align(b->args.out_format);
     size_t off = 0;
     for (ImgDev &im : b->imgs)
     {
@@ -985,7 +1102,8 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
 {
     if (!ctx || n <= 0 || !files || !lens || !out || !status || !opts) return B2J_E_ARG;
     const int fmt = opts->out_format, model = opts->pixel_model, scale = opts->scale ? opts->scale : 1;
-    if (!format_ok(fmt) || !model_ok(model) || !scale_ok(scale)) return B2J_E_ARG;
+    const bool orient = opts->exif_orientation == 1;
+    if (!format_ok(fmt) || !model_ok(model) || !scale_ok(scale) || (opts->exif_orientation & ~1)) return B2J_E_ARG;
     if (const char *why = output_refusal(model, fmt, scale)) { t_last_error = why; return B2J_E_ARG; }
     CU_TRY(cudaSetDevice(ctx->device));
     const int gate = opts->gate;
@@ -1031,6 +1149,7 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
         std::vector<b2j_image_desc> d;
         std::vector<const uint8_t *> f;
         std::vector<size_t> l;
+        std::vector<uint8_t> codes;   // orientation codes of the accepted files
         for (;;)
         {
             const int g = next_group.fetch_add(1);
@@ -1041,24 +1160,29 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
                 if (stop) { groups[(size_t)g].ready = true; cv.notify_all(); continue; }
             }
             FeedGroup &G = groups[(size_t)g];
-            d.clear(); f.clear(); l.clear();
+            d.clear(); f.clear(); l.clear(); codes.clear();
             for (int i = G.first; i < G.first + G.count; i++)
             {
                 b2j_image_desc desc;
                 const int prc = b2j_parse_header(files[i], lens[i], gate, &desc);
                 status[i] = prc;
-                if (prc == B2J_OK) { G.idx.push_back(i); d.push_back(desc); f.push_back(files[i]); l.push_back(lens[i]); }
+                if (prc != B2J_OK) continue;
+                G.idx.push_back(i); d.push_back(desc); f.push_back(files[i]); l.push_back(lens[i]);
+                int32_t code = 1;
+                if (orient) b2j_parse_orientation(files[i], lens[i], &code);
+                codes.push_back((uint8_t)code);
             }
             G.parsed = true;
             if (!d.empty())
             {
                 G.rc = b2j_batch_create(ctx, (int)d.size(), d.data(), f.data(), l.data(), &G.b);
-                if (G.rc != B2J_OK) G.err = t_last_error;
-                else
+                if (G.rc == B2J_OK)
                 {
                     set_output(G.b, model, fmt, scale);
+                    if (orient) G.rc = b2j_batch_set_orientations(G.b, codes.data());
                     pack_pixel_plane(G.b);
                 }
+                if (G.rc != B2J_OK) G.err = t_last_error;
             }
             {
                 std::lock_guard<std::mutex> lk(mu);
@@ -1116,17 +1240,18 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&G.done, cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaEventRecord(G.decoded, ctx->stream);
         if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->stream2, G.decoded, 0);
-        // one download per run of images that are neighbours in the pixel plane and in the caller's memory (a copy costs
-        // a few microseconds whatever its size: 8192 small images one by one spend a third of the time on that)
+        // one download per run of images that are neighbours on the device (in the pixel plane, or as oriented copies)
+        // and in the caller's memory (a copy costs a few microseconds whatever its size: 8192 small images one by one
+        // spend a third of the time on that)
         for (size_t k = 0; k < G.idx.size() && e == cudaSuccess;)
         {
-            const ImgDev &im = G.b->imgs[k];
             uint8_t *dst = out[G.idx[k]];
-            size_t bytes = image_bytes(G.b, im), k1 = k + 1;
+            const uint8_t *src = result_of(G.b, k);
+            size_t bytes = image_bytes(G.b, G.b->imgs[k]), k1 = k + 1;
             if (!dst) { k = k1; continue; }
-            while (k1 < G.idx.size() && out[G.idx[k1]] == dst + bytes && G.b->imgs[k1].pix_off == im.pix_off + bytes)
+            while (k1 < G.idx.size() && out[G.idx[k1]] == dst + bytes && result_of(G.b, k1) == src + bytes)
                 bytes += image_bytes(G.b, G.b->imgs[k1++]);
-            e = cudaMemcpyAsync(dst, G.b->args.pixels + im.pix_off, bytes, cudaMemcpyDeviceToHost, ctx->stream2);
+            e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, ctx->stream2);
             k = k1;
         }
         // the status words of the group's images land at their file indices (consecutive only when no file was refused)
