@@ -78,6 +78,11 @@ extern "C" {
 #define B2J_ST_DC_RANGE 0x10      /* DC category > 16 or DC predictor outside int16          */
 #define B2J_ST_SEGMENT_END 0x20   /* a restart interval did not end at its marker            */
 #define B2J_ST_INTERNAL 0x4000    /* a TMA tile load did not complete (never observed; guards against a hang) */
+/* A restart marker that starts no restart interval ends the image's entropy-coded data: any RSTn in a file without DRI,
+ * and in a file of n intervals (n - 1 markers) the n-th marker and every later one. The reference keeps such a marker's
+ * Dn byte as data and decodes on, so its coefficients differ from the file's without the marker; here a decode that needs
+ * bytes behind the marker flags B2J_ST_OVERRUN instead. A stray marker behind the last block (right before EOI) changes
+ * nothing, as in the reference. */
 
 /* ---- accept gate ---- */
 #define B2J_GATE_REFERENCE 0 /* exactly decoder.cpp:58-69: 4:2:0 (22,11,11) and 4:4:4        */

@@ -57,7 +57,8 @@ cudaError_t init_constants()
 //   b != FF : dropped iff p == FF and b is 00 (stuffing) or D0..D7 (RSTn, recorded as a marker);
 //             kept otherwise.
 // The reference keeps the Dn byte in its stream and consumes it at the interval switch
-// (decoder.cpp:136-141, 296-297); here it is dropped and becomes a segment boundary instead.
+// (decoder.cpp:136-141, 296-297); here it is dropped and becomes a segment boundary instead, or, when it starts no
+// interval, the end of the data the decoders may read (mark_group).
 //
 // The classification runs on 4 bytes at a time in a "flag" domain: bit 7 of every byte of a 32-bit
 // word is the predicate for that byte (byte j of the thread = bits 8(j&3).. of word j>>2).
@@ -261,8 +262,11 @@ __device__ __forceinline__ void squeeze_group(uint8_t *__restrict__ s_out, uint3
 
 // Phase B of a 16-byte group: the restart-interval starts of its RSTn markers (clean_pos = position of the
 // group's first kept byte in the image's clean stream, rank = ordinal of the next marker of the image).
+// A marker that starts no interval (any RSTn without DRI; the n_segs-th and later ones with DRI) ends the data the
+// decoders may read (scan_cut, b2j.h): the reference keeps its Dn byte as data, so a decode past it would differ.
 __device__ __forceinline__ void mark_group(const uint32_t w[4], const ScanFlags &f, uint32_t &rank, uint32_t clean_pos, const ImgDev &im,
-                                           uint32_t img_idx, uint32_t *__restrict__ seg_start, int32_t *__restrict__ status)
+                                           uint32_t img_idx, uint32_t *__restrict__ seg_start, uint32_t *__restrict__ scan_cut,
+                                           int32_t *__restrict__ status)
 {
     if (!(f.mark[0] | f.mark[1] | f.mark[2] | f.mark[3])) return;
     uint32_t keep16 = 0, mark16 = 0;
@@ -276,13 +280,16 @@ __device__ __forceinline__ void mark_group(const uint32_t w[4], const ScanFlags 
     {
         const uint32_t j = (uint32_t)__ffs(mark16) - 1u;
         mark16 &= mark16 - 1u;
+        const uint32_t at = clean_pos + __popc(keep16 & ((1u << j) - 1u));
         if (im.has_dri && rank + 1 < im.n_segs)
         {
-            seg_start[im.seg_first + rank + 1] = clean_pos + __popc(keep16 & ((1u << j) - 1u));
+            seg_start[im.seg_first + rank + 1] = at;
             const uint32_t wj = j < 4u ? w[0] : (j < 8u ? w[1] : (j < 12u ? w[2] : w[3]));
             const uint32_t bj = (wj >> (8 * (j & 3u))) & 0xFFu;
             if (bj != 0xD0u + (rank & 7u)) atomicOr(&status[img_idx], B2J_ST_RST_MISMATCH);   // decoder.cpp:298
         }
+        else
+            atomicMax(&scan_cut[img_idx], ~at);   // zeroed before the decode: the first such marker wins
         rank++;
     }
 }
@@ -291,7 +298,7 @@ constexpr int kScanMinCtas = 4;   // 64 registers (92 B of spills), 4 CTAs per S
 __global__ void __launch_bounds__(kScanThreads, kScanMinCtas)
 k_unstuff_fused(const uint8_t *__restrict__ raw, uint8_t *__restrict__ clean, const ImgDev *__restrict__ imgs,
                 const uint32_t *__restrict__ chunk_img, uint64_t *__restrict__ chunk_state, uint32_t *__restrict__ clean_len,
-                uint32_t *__restrict__ seg_start, int32_t *__restrict__ status)
+                uint32_t *__restrict__ seg_start, uint32_t *__restrict__ scan_cut, int32_t *__restrict__ status)
 {
     __shared__ uint32_t s_min;
     __shared__ uint32_t s_warp[kScanThreads / 32];
@@ -429,7 +436,7 @@ k_unstuff_fused(const uint8_t *__restrict__ raw, uint8_t *__restrict__ clean, co
 #pragma unroll
         for (int g = 0; g < kScanGroups; g++)
         {
-            mark_group(st.w[g], st.f[g], rank, base_keep + lo, im, img_idx, seg_start, status);
+            mark_group(st.w[g], st.f[g], rank, base_keep + lo, im, img_idx, seg_start, scan_cut, status);
             lo += nkeep[g];
         }
     }
@@ -552,6 +559,13 @@ __device__ __forceinline__ int32_t extend_sz(uint32_t v, uint32_t size)
     return (int32_t)(u - __funnelshift_l(neg, 0u, size));            // negative: u - (2^size - 1)
 }
 
+// Clean bytes of an image the decoders may read: its clean stream, up to the first restart marker that starts no
+// interval (mark_group; scan_cut holds its complement, 0 = none). Reading past the end flags B2J_ST_OVERRUN.
+__device__ __forceinline__ uint32_t stream_len(const uint32_t *__restrict__ clean_len, const uint32_t *__restrict__ scan_cut, uint32_t img)
+{
+    return min(clean_len[img], ~scan_cut[img]);
+}
+
 // SYNC = false: a lane is a restart interval (byte-aligned start from seg_start[], DC predictors 0, the
 //   block-in-MCU phase is 0 and therefore uniform across the warp).
 // SYNC = true : a lane is a sub-sequence of a stream without restart markers; its first block, bit
@@ -561,7 +575,7 @@ constexpr uint32_t kZzBytes = 192;   // 128 zig-zag offsets + 64 bytes of scratc
 template <bool SYNC>
 __global__ void __launch_bounds__(kHuffThreads)
 k_huff_decode(const uint8_t *__restrict__ clean, const ImgDev *__restrict__ imgs, const HuffCtaDev *__restrict__ ctas,
-              const uint32_t *__restrict__ seg_start, const uint32_t *__restrict__ clean_len,
+              const uint32_t *__restrict__ seg_start, const uint32_t *__restrict__ clean_len, const uint32_t *__restrict__ scan_cut,
               const uint16_t *__restrict__ luts, int16_t *__restrict__ coef, int32_t *__restrict__ status,
               const SubRec *__restrict__ recs, const uint4 *__restrict__ cta_base)
 {
@@ -604,14 +618,14 @@ k_huff_decode(const uint8_t *__restrict__ clean, const ImgDev *__restrict__ imgs
             nblk = nmcu * tot;
             blk0 = im.blk_first + mcu0 * tot;
             if (seg + 1 < im.n_segs) { end = seg_start[im.seg_first + seg + 1]; check_end = (end != kSegInvalid); }
-            if (!check_end) end = clean_len[cta.img];
+            if (!check_end) end = stream_len(clean_len, scan_cut, cta.img);
         }
         // a lane whose start is unknown (missing RSTn) still emits zero blocks so the plane is defined
         decodable = active && start != kSegInvalid;
     }
     else
     {
-        const uint32_t bits = clean_len[cta.img] * 8u;
+        const uint32_t bits = stream_len(clean_len, scan_cut, cta.img) * 8u;
         const uint32_t n_sub = (bits + kSubBytes * 8 - 1) / (kSubBytes * 8);
         active = seg < n_sub && tid < (uint32_t)kSyncLanes;   // a decode CTA covers one chunk of the synchronisation
         SubRec rec;
@@ -639,19 +653,16 @@ k_huff_decode(const uint8_t *__restrict__ clean, const ImgDev *__restrict__ imgs
             pre.blk = acc.x + ib - rec.nblk;
             pre.dc[0] = (int32_t)acc.y + i0 - rec.dc[0]; pre.dc[1] = (int32_t)acc.z + i1 - rec.dc[1]; pre.dc[2] = (int32_t)acc.w + i2 - rec.dc[2];
         }
-        if (active)
+        if (active && rec.fs != kSubNone && pre.blk < im.blk_count)
         {
-            if (rec.fs != kSubNone && pre.blk < im.blk_count)
-            {
-                nblk = min(rec.nblk, im.blk_count - pre.blk);           // bits behind the last block decode to junk blocks: dropped
-                blk0 = im.blk_first + pre.blk;
-                start_bit = rec.fs;
-                bi = rec.fc;
-                dc0 = pre.dc[0]; dc1 = pre.dc[1]; dc2 = pre.dc[2];
-            }
-            if (seg + 1 == n_sub && pre.blk + rec.nblk < im.blk_count) err |= B2J_ST_OVERRUN;   // the stream ends before the last block
-            end = clean_len[cta.img];
+            nblk = min(rec.nblk, im.blk_count - pre.blk);           // bits behind the last block decode to junk blocks: dropped
+            blk0 = im.blk_first + pre.blk;
+            start_bit = rec.fs;
+            bi = rec.fc;
+            dc0 = pre.dc[0]; dc1 = pre.dc[1]; dc2 = pre.dc[2];
         }
+        // the stream ends before the last block (an empty stream has no sub-sequence: lane 0 of the first CTA reports it)
+        if (tid < (uint32_t)kSyncLanes && seg + 1 == max(n_sub, 1u) && pre.blk + rec.nblk < im.blk_count) err |= B2J_ST_OVERRUN;
         decodable = active && nblk > 0;
         // Lanes change places: sorted by the phase of their first block inside the MCU, then by falling block count.
         // The decode loop below runs block by block in warp lockstep, so a warp costs (longest lane in blocks) x
@@ -940,8 +951,8 @@ __device__ __forceinline__ void sync_stage_lut(uint16_t *s_lut, const uint16_t *
 // but the first starts from the bare guess, so that every border is repaired by the sweep -- a test knob).
 __global__ void __launch_bounds__(kHuffThreads)
 k_sync_chunks(const uint8_t *__restrict__ clean, const ImgDev *__restrict__ imgs, const HuffCtaDev *__restrict__ ctas,
-              const uint32_t *__restrict__ clean_len, const uint16_t *__restrict__ luts, SubRec *__restrict__ recs,
-              uint4 *__restrict__ chunk_state, uint4 *__restrict__ cta_tot, uint32_t *__restrict__ stats, uint32_t use_pre)
+              const uint32_t *__restrict__ clean_len, const uint32_t *__restrict__ scan_cut, const uint16_t *__restrict__ luts,
+              SubRec *__restrict__ recs, uint4 *__restrict__ chunk_state, uint4 *__restrict__ cta_tot, uint32_t *__restrict__ stats, uint32_t use_pre)
 {
     extern __shared__ __align__(16) uint8_t smem[];
     __shared__ uint4 s_wtot[kHuffThreads / 32];
@@ -950,7 +961,7 @@ k_sync_chunks(const uint8_t *__restrict__ clean, const ImgDev *__restrict__ imgs
     uint16_t *s_lut = reinterpret_cast<uint16_t *>(smem + kSyncSharedBytes);
     const HuffCtaDev cta = ctas[blockIdx.x];
     const ImgDev &im = imgs[cta.img];
-    const uint32_t bits = clean_len[cta.img] * 8u;
+    const uint32_t bits = stream_len(clean_len, scan_cut, cta.img) * 8u;
     const uint32_t n_sub = (bits + kSubBytes * 8 - 1) / (kSubBytes * 8);
     if (cta.seg_first >= n_sub)
     {
@@ -979,8 +990,8 @@ k_sync_chunks(const uint8_t *__restrict__ clean, const ImgDev *__restrict__ imgs
 // may have changed). With pre-lanes this finds nothing in almost every image and costs one pass over the chunk states.
 __global__ void __launch_bounds__(kHuffThreads)
 k_sync_sweep(const uint8_t *__restrict__ clean, const ImgDev *__restrict__ imgs, const uint32_t *__restrict__ sync_imgs,
-             const uint32_t *__restrict__ clean_len, const uint16_t *__restrict__ luts, SubRec *__restrict__ recs,
-             uint4 *chunk_state, uint4 *cta_tot, uint32_t *__restrict__ stats)
+             const uint32_t *__restrict__ clean_len, const uint32_t *__restrict__ scan_cut, const uint16_t *__restrict__ luts,
+             SubRec *__restrict__ recs, uint4 *chunk_state, uint4 *cta_tot, uint32_t *__restrict__ stats)
 {
     extern __shared__ __align__(16) uint8_t smem[];
     __shared__ __align__(16) WalkCtab s_ctab[16];
@@ -989,7 +1000,7 @@ k_sync_sweep(const uint8_t *__restrict__ clean, const ImgDev *__restrict__ imgs,
     const uint32_t tid = threadIdx.x;
     const uint32_t img = sync_imgs[blockIdx.x];
     const ImgDev &im = imgs[img];
-    const uint32_t bits = clean_len[img] * 8u;
+    const uint32_t bits = stream_len(clean_len, scan_cut, img) * 8u;
     const uint32_t n_sub = (bits + kSubBytes * 8 - 1) / (kSubBytes * 8);
     const uint32_t nc = (n_sub + (uint32_t)kSyncLanes - 1u) / (uint32_t)kSyncLanes;
     uint4 *state = chunk_state + im.scta_first;
@@ -2202,14 +2213,15 @@ cudaError_t configure_kernels(uint32_t max_lut_len)
 void launch_prepass(const DecodeArgs &a, cudaStream_t s)
 {
     if (a.n_chunks == 0) return;
-    k_unstuff_fused<<<a.n_chunks, kScanThreads, 0, s>>>(a.raw, a.clean, a.imgs, a.chunk_img, a.chunk_state, a.clean_len, a.seg_start, a.status);
+    k_unstuff_fused<<<a.n_chunks, kScanThreads, 0, s>>>(a.raw, a.clean, a.imgs, a.chunk_img, a.chunk_state, a.clean_len, a.seg_start, a.scan_cut,
+                                                              a.status);
 }
 
 void launch_huffman(const DecodeArgs &a, cudaStream_t s)
 {
     if (a.n_huff_ctas == 0) return;
     k_huff_decode<false><<<a.n_huff_ctas, kHuffThreads, huff_smem_bytes(a.max_lut_dec_len), s>>>(a.clean, a.imgs, a.huff_ctas, a.seg_start, a.clean_len,
-                                                                                                a.luts, a.coef, a.status, nullptr, nullptr);
+                                                                                                a.scan_cut, a.luts, a.coef, a.status, nullptr, nullptr);
 }
 
 // Streams without restart markers: chunk-wise synchronisation, the sweep, the scan, then the decode.
@@ -2218,12 +2230,12 @@ void launch_huffman_sync(const DecodeArgs &a, cudaStream_t s)
     const uint32_t n = a.n_sync_ctas, ni = a.n_sync_imgs;
     if (n == 0 || ni == 0) return;
     const size_t sync_bytes = kSyncSharedBytes + (size_t)a.max_lut_walk_len * 2;
-    k_sync_chunks<<<n, kHuffThreads, sync_bytes, s>>>(a.clean, a.imgs, a.sync_ctas, a.clean_len, a.luts, a.recs, a.sync_chunk_state, a.sync_cta_base,
+    k_sync_chunks<<<n, kHuffThreads, sync_bytes, s>>>(a.clean, a.imgs, a.sync_ctas, a.clean_len, a.scan_cut, a.luts, a.recs, a.sync_chunk_state, a.sync_cta_base,
                                                       a.sync_stats, a.sync_use_pre ? 1u : 0u);
-    k_sync_sweep<<<ni, kHuffThreads, sync_bytes, s>>>(a.clean, a.imgs, a.sync_imgs, a.clean_len, a.luts, a.recs, a.sync_chunk_state, a.sync_cta_base,
+    k_sync_sweep<<<ni, kHuffThreads, sync_bytes, s>>>(a.clean, a.imgs, a.sync_imgs, a.clean_len, a.scan_cut, a.luts, a.recs, a.sync_chunk_state, a.sync_cta_base,
                                                      a.sync_stats);
     k_sync_cta_scan<<<ni, 32, 0, s>>>(a.imgs, a.sync_imgs, a.sync_cta_base);
-    k_huff_decode<true><<<n, kHuffThreads, huff_smem_bytes(a.max_lut_dec_len), s>>>(a.clean, a.imgs, a.sync_ctas, a.seg_start, a.clean_len, a.luts,
+    k_huff_decode<true><<<n, kHuffThreads, huff_smem_bytes(a.max_lut_dec_len), s>>>(a.clean, a.imgs, a.sync_ctas, a.seg_start, a.clean_len, a.scan_cut, a.luts,
                                                                                     a.coef, a.status, a.recs, a.sync_cta_base);
 }
 

@@ -27,6 +27,7 @@ struct DecodeArgs
     uint8_t *clean;
     uint64_t *chunk_state;   // pre-pass: look-back words, zeroed before every decode
     uint32_t *clean_len, *seg_start;
+    uint32_t *scan_cut;      // pre-pass: per image, ~(clean position of the first restart marker that starts no interval), zeroed before every decode
     SubRec *recs;           // self-synchronising path: one record per sub-sequence
     uint4 *sync_cta_base;   // per chunk (= decode CTA) of the self-synchronising path: (blocks started, DC sums), then their prefix
     uint4 *sync_chunk_state;   // per chunk: entry state it assumed (x, y), exit state (z, w)

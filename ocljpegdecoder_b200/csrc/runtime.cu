@@ -617,6 +617,7 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     const size_t o_chunk_states = place(sizeof(uint4) * (sctas.size() + 1));
     // what every decode starts from zero, side by side: one memset
     const size_t o_status = place(4 * (size_t)n);
+    const size_t o_scan_cut = place(4 * (size_t)n);
     const size_t o_sync_stats = place(4 * 8);
     const size_t o_chunk_state = place(8 * chunk_img.size());
     b->zero_bytes = off - o_status;
@@ -669,6 +670,7 @@ static int batch_create_impl(b2j_ctx *ctx, int n, const b2j_image_desc *descs, c
     a.sync_cta_base = at<uint4>(b->d_scratch, o_pres);
     a.sync_chunk_state = at<uint4>(b->d_scratch, o_chunk_states);
     a.status = at<int32_t>(b->d_scratch, o_status);
+    a.scan_cut = at<uint32_t>(b->d_scratch, o_scan_cut);
     a.sync_stats = at<uint32_t>(b->d_scratch, o_sync_stats);
     a.chunk_state = at<uint64_t>(b->d_scratch, o_chunk_state);
     a.tmap = &b->tmap;

@@ -56,6 +56,7 @@ def canonical_codes(bits, vals):
 class BitWriter:
     def __init__(self):
         self.out = bytearray()
+        self.plain = bytearray()   # the same bytes before stuffing
         self.acc = 0
         self.n = 0
 
@@ -67,6 +68,7 @@ class BitWriter:
         while self.n >= 8:
             b = (self.acc >> (self.n - 8)) & 0xFF
             self.out.append(b)
+            self.plain.append(b)
             if b == 0xFF:
                 self.out.append(0x00)   # byte stuffing
             self.n -= 8
@@ -126,18 +128,46 @@ def _seg(marker, payload):
     return bytes([0xFF, marker]) + (len(payload) + 2).to_bytes(2, "big") + bytes(payload)
 
 
-def build_jpeg(width, height, sampling, blocks, qtabs, restart_interval=0, fill_before_rst=0,
+def build_jpeg(width, height, sampling, blocks, qtabs, restart_interval=0, fill_before_rst=0, fill_before_eoi=0,
                tables=None, comp_tables=((0, 0), (1, 1), (1, 1)), with_app0=True, trailing=b"", dqt16=False,
                comp_quant=(0, 1, 1)):
-    """sampling: luma (h, v) with 1x1 chroma, or ((hy, vy), (hu, vu), (hv, vv)). blocks: int array [n_blocks, 64] in MCU order and
-    SCAN (zig-zag) coefficient order, blocks[:,0] = absolute DC. qtabs: one to four 64-lists (zig-zag order), written as
-    DQT tables 0, 1, ...; comp_quant: the table of each component (Y, Cb, Cr). tables: dict like STD_TABLES, keyed
-    (class, id); comp_tables: the (DC id, AC id) of each component. Returns the file bytes."""
+    """sampling: luma (h, v) with 1x1 chroma, ((hy, vy), (hu, vu), (hv, vv)), or "gray" (one 1x1 component). blocks: int
+    array [n_blocks, 64] in MCU order and SCAN (zig-zag) coefficient order, blocks[:,0] = absolute DC. qtabs: one to four
+    64-lists (zig-zag order), written as DQT tables 0, 1, ...; comp_quant: the table of each component (Y, Cb, Cr).
+    tables: dict like STD_TABLES, keyed (class, id); comp_tables: the (DC id, AC id) of each component.
+    fill_before_rst: FF fill bytes in front of every RSTn, or a sequence of one count per marker; fill_before_eoi: in
+    front of EOI. Returns the file bytes."""
+    head, intervals, _ = build_parts(width, height, sampling, blocks, qtabs, restart_interval, tables, comp_tables, with_app0,
+                                     dqt16, comp_quant)
+    n_rst = len(intervals) - 1
+    fills = [fill_before_rst] * n_rst if isinstance(fill_before_rst, int) else list(fill_before_rst)
+    assert len(fills) == n_rst, (len(fills), n_rst)
+    return head + join_scan(intervals, fills, fill_before_eoi) + trailing
+
+
+def join_scan(intervals, fills, fill_before_eoi=0):
+    """The entropy-coded segment and EOI: the (stuffed) restart intervals, fills[r] FF bytes and RSTn in front of interval
+    r + 1, fill_before_eoi FF bytes, FF D9."""
+    out = bytearray(intervals[0])
+    for r, (f, iv) in enumerate(zip(fills, intervals[1:])):
+        out += b"\xFF" * f + bytes([0xFF, 0xD0 + (r & 7)]) + iv
+    return bytes(out) + b"\xFF" * fill_before_eoi + b"\xFF\xD9"
+
+
+def build_parts(width, height, sampling, blocks, qtabs, restart_interval=0, tables=None, comp_tables=((0, 0), (1, 1), (1, 1)),
+                with_app0=True, dqt16=False, comp_quant=(0, 1, 1)):
+    """build_jpeg's pieces: (the file up to and including SOS, [each restart interval's bytes as written], [the same
+    bytes before stuffing])."""
     tables = tables or STD_TABLES
-    if isinstance(sampling[0], (tuple, list)):
+    gray = isinstance(sampling, str)
+    if gray:
+        assert sampling == "gray"
+        samp = [(1, 1)]
+    elif isinstance(sampling[0], (tuple, list)):
         samp = [tuple(x) for x in sampling]          # ((hy, vy), (hu, vu), (hv, vv))
     else:
         samp = [tuple(sampling), (1, 1), (1, 1)]
+    nc = len(samp)
     h, v = samp[0]
     nblk = [a * b for a, b in samp]
     tot = sum(nblk)
@@ -154,40 +184,41 @@ def build_jpeg(width, height, sampling, blocks, qtabs, restart_interval=0, fill_
             out += _seg(0xDB, bytes([0x10 | k]) + b"".join(int(q).to_bytes(2, "big") for q in qt))
         else:
             out += _seg(0xDB, bytes([k]) + bytes(qt))
-    sof = bytes([8]) + height.to_bytes(2, "big") + width.to_bytes(2, "big") + bytes([3])
-    for c in range(3):
+    sof = bytes([8]) + height.to_bytes(2, "big") + width.to_bytes(2, "big") + bytes([nc])
+    for c in range(nc):
         sof += bytes([c + 1, (samp[c][0] << 4) | samp[c][1], comp_quant[c]])
     out += _seg(0xC0, sof)
     for (tc, th), (bits, vals) in sorted(tables.items()):
         out += _seg(0xC4, bytes([(tc << 4) | th]) + bytes(bits) + bytes(vals))
     if restart_interval:
         out += _seg(0xDD, restart_interval.to_bytes(2, "big"))
-    sos = bytes([3])
-    for c in range(3):
+    sos = bytes([nc])
+    for c in range(nc):
         sos += bytes([c + 1, (comp_tables[c][0] << 4) | comp_tables[c][1]])
     sos += bytes([0, 0x3F, 0])
     out += _seg(0xDA, sos)
     codes = {k: canonical_codes(*tv) for k, tv in tables.items()}
     bw = BitWriter()
+    intervals, plain = [], []
     pred = [0, 0, 0]
-    rst = 0
     bi = 0
     for m in range(n_mcu):
         if restart_interval and m and m % restart_interval == 0:
             bw.flush()
-            bw.raw(b"\xFF" * fill_before_rst + bytes([0xFF, 0xD0 + (rst & 7)]))
-            rst += 1
+            intervals.append(bytes(bw.out))
+            plain.append(bytes(bw.plain))
+            bw = BitWriter()
             pred = [0, 0, 0]
-        for c in range(3):
+        for c in range(nc):
             for _ in range(nblk[c]):
                 dc_codes = codes[(0, comp_tables[c][0])]
                 ac_codes = codes[(1, comp_tables[c][1])]
                 pred[c] = encode_block(bw, blocks[bi], pred[c], dc_codes, ac_codes)
                 bi += 1
     bw.flush()
-    out += bw.out
-    out += b"\xFF\xD9" + trailing
-    return bytes(out)
+    intervals.append(bytes(bw.out))
+    plain.append(bytes(bw.plain))
+    return bytes(out), intervals, plain
 
 
 # ---- tables whose codes reach the long-code paths of a decoder ------------------------------------------------------
