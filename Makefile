@@ -33,7 +33,10 @@ $(BINDIR)/b2jdec: $(CSRC)/refshim/b2jdec_main.cpp $(CSRC)/refshim/decoder_b2j.cp
 	    -L$(LIBDIR) -lb2j -Wl,-rpath,'$$ORIGIN/../lib' -o $@
 
 # host-side unit-check helper: the device arithmetic header + the LUT builder compiled with g++
-mathcheck: tests/native/libb2jcheck.so tests/native/libb2jsync.so
+mathcheck: tests/native/libb2jcheck.so tests/native/libb2jsync.so tests/native/libb2jcrop.so
+# the host side of a cropped decode (box mapping, crop tile list)
+tests/native/libb2jcrop.so: tests/native/cropcheck.cpp $(CSRC)/crop_plan.h $(CSRC)/b2j_internal.h include/b2j.h
+	$(CXX) -O2 -std=c++17 -fPIC -shared -Wall -I$(CSRC) -Iinclude tests/native/cropcheck.cpp -o $@
 # host emulation of the self-synchronising path (walk + chunk rounds of b2j_sync.h) against a table-free sequential walk
 tests/native/libb2jsync.so: tests/native/synccheck.cpp $(CSRC)/b2j_sync.h $(CSRC)/huff_lut.cpp $(CSRC)/host_parse.cpp $(CSRC)/b2j_internal.h include/b2j.h
 	$(CXX) -O2 -std=c++17 -fPIC -shared -Wall -I$(CSRC) -Iinclude tests/native/synccheck.cpp $(CSRC)/huff_lut.cpp $(CSRC)/host_parse.cpp -o $@

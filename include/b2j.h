@@ -38,6 +38,8 @@
  *                                               1/2, 1/4 or 1/8 size straight from the coefficients
  *   b2j_parse_orientation,  (none)              EXIF orientation as OpenCV's imdecode, torchvision's decode_jpeg(...,
  *   b2j_batch_set_orientations                  apply_exif_orientation=True) and Pillow's exif_transpose() apply it
+ *   b2j_batch_set_crops,    (none)              a crop window per image (SURVEY.md 8f rank 3), decoded from the MCUs
+ *   b2j_decode_host_crop                        it touches: a training loader's RandomResizedCrop / CenterCrop input
  *   b2j_idct_*              idct.h:9-18         the device backend as the reference's own decoder.cpp drives it
  *                                               (coefficients in, pixels out): see "secondary boundary" below
  *   b2j_read_files          decoder.cpp:94-101  the 2 KiB fread() loop (and main.cpp's fopen): whole files read with
@@ -276,6 +278,21 @@ int b2j_batch_set_scale(b2j_batch *batch, int denom);
  * buffer of their own (b2j_batch_info counts both); with every code 1 a decode is what it is without this call.
  * b2j_batch_downscale() is refused (B2J_E_ARG) while a code is not 1. */
 int b2j_batch_set_orientations(b2j_batch *batch, const uint8_t *codes /* n or NULL */);
+/* A crop box per image for the decodes that follow: boxes[4*i .. 4*i+3] = x, y, w, h of image i, NULL = the whole images
+ * (the default); B2J_E_ARG for a negative value or w or h < 1, and then nothing changes. A box is given in the frame the
+ * decode would otherwise deliver: the image at the batch's scale (b2j_batch_set_scale), then oriented by its code
+ * (b2j_batch_set_orientations; codes 5..8 swap the sides). The result is exactly that image's [y:y+h, x:x+w] (numpy;
+ * planar RGB: each plane), w x h pixels with tight pitch in the batch's format, in every format and at every scale:
+ * Pillow's draft(), exif_transpose(), then crop((x, y, x+w, y+h)); torchvision's decode_jpeg(..., apply_exif_orientation=
+ * True)[..., y:y+h, x:x+w]. b2j_batch_pixels_device and the reads return it. The box is checked at each decode, since the
+ * scale and the codes may change after this call: a box that does not lie inside its frame fails the decode, and the
+ * reads, with B2J_E_ARG, and b2j_last_error() names the image. Needs B2J_PIXELS_LIBJPEG: a decode with crops in the
+ * reference model fails with B2J_E_ARG. b2j_batch_downscale() is refused (B2J_E_ARG) while crops are set.
+ * Only the MCUs the window touches, with one MCU around them for fancy upsampling (none in GRAY8 and at scale 8), are
+ * transformed, and only the window is upsampled and coloured; the pre-pass and the entropy stage decode the whole scan,
+ * so the status words and the coefficients are those of the uncropped decode. The windows and their tile list live in a
+ * buffer of their own (b2j_batch_info counts it); with NULL a decode is what it is without this call. */
+int b2j_batch_set_crops(b2j_batch *batch, const int32_t *boxes /* 4*n or NULL */);
 
 /* Per-image status words (B2J_ST_* bits). Synchronises the stream. */
 int b2j_batch_status(b2j_batch *batch, void *stream, int32_t *status /* n */);
@@ -286,14 +303,15 @@ int b2j_batch_status(b2j_batch *batch, void *stream, int32_t *status /* n */);
 int b2j_batch_sync_stats(b2j_batch *batch, void *stream, uint32_t *out8);
 
 /* Device-resident results. Pixels: top-down, tight pitch, in the batch's output format (BGRA: width*4 per row, A = 0),
- * at the batch's scale (b2j_batch_set_scale: width and height are then the reduced ones). */
+ * at the batch's scale (b2j_batch_set_scale: width and height are then the reduced ones), oriented, cropped
+ * (b2j_batch_set_crops: w x h). */
 int b2j_batch_pixels_device(const b2j_batch *batch, int image, void **dptr, size_t *nbytes);
 /* Coefficient plane: int16[blk_count][64], natural order, QUANTISED (dequantisation happens
  * at IDCT load), MCU-interleaved block order. */
 int b2j_batch_coefs_device(const b2j_batch *batch, int image, void **dptr, size_t *nbytes);
 
 /* D2H of one image (synchronises). dst: width*height*4 bytes (BGRA), width*height*3 (RGB24, planar RGB) or width*height
- * (GRAY8), of the size at the batch's scale. */
+ * (GRAY8), of the size at the batch's scale, oriented; a crop box's w*h pixels with crops. */
 int b2j_batch_read_pixels(b2j_batch *batch, void *stream, int image, uint8_t *dst);
 /* D2H of every image into dsts[i] (pinned staging, one copy per image; synchronises). */
 int b2j_batch_read_all_pixels(b2j_batch *batch, void *stream, uint8_t *const *dsts);
@@ -304,8 +322,8 @@ int b2j_batch_read_coefs(b2j_batch *batch, void *stream, int image, int32_t *dst
 /* Output stage for consumers that want smaller images (SURVEY.md 8f rank 3): box-filter reduction of the decoded pixels by
  * factor 2, 4 or 8 per axis, after b2j_batch_decode(), in the batch's output format. Reduced size: ceil(w/f) x ceil(h/f);
  * every value is the rounded mean (sum + n/2) / n of the n input values it covers (at the right / bottom edge: of those that
- * exist). The full-size pixels stay where they are. B2J_E_ARG while the batch's scale (b2j_batch_set_scale) is not 1, and
- * while an orientation code (b2j_batch_set_orientations) is not 1. */
+ * exist). The full-size pixels stay where they are. B2J_E_ARG while the batch's scale (b2j_batch_set_scale) is not 1,
+ * while an orientation code (b2j_batch_set_orientations) is not 1, and while crops (b2j_batch_set_crops) are set. */
 int b2j_batch_downscale(b2j_batch *batch, void *stream, int factor);
 int b2j_batch_downscaled_device(const b2j_batch *batch, int image, void **dptr, size_t *nbytes, int *width, int *height);
 int b2j_batch_read_downscaled(b2j_batch *batch, void *stream, int image, uint8_t *dst);   /* synchronises */
@@ -338,9 +356,16 @@ typedef struct b2j_host_opts
  * (B2J_E_ARG for a scale other than 0, 1, 2, 4 and 8, and for a scale other than 1 or B2J_OUT_GRAY8 in the reference
  * pixel model). With opts->exif_orientation = 1 (B2J_E_ARG for a value other than 0 and 1) out[i] holds the image
  * oriented by its EXIF code: h*w bytes per channel with the sides swapped for codes 5..8. b2j_decode_host() does not
- * orient. */
+ * orient. b2j_decode_host_ex() is b2j_decode_host_crop() with crops = NULL. */
 int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *files, const size_t *lens, const b2j_host_opts *opts,
                        uint8_t *const *out, int32_t *status);
+/* b2j_decode_host_ex() with a crop box per file (crops[4*i .. 4*i+3] = x, y, w, h; NULL = none), as
+ * b2j_batch_set_crops() takes it: in the file's frame at opts->scale, oriented when opts->exif_orientation = 1.
+ * out[i] holds the box's w*h pixels (w*h*4, w*h*3 or w*h bytes). A file whose box does not lie inside its frame (a
+ * negative value, w or h < 1 included) gets status[i] = B2J_E_ARG and is skipped; the others are decoded. Needs
+ * B2J_PIXELS_LIBJPEG when crops is not NULL (B2J_E_ARG for the whole call otherwise). */
+int b2j_decode_host_crop(b2j_ctx *ctx, int n, const uint8_t *const *files, const size_t *lens, const b2j_host_opts *opts,
+                         const int32_t *crops /* 4*n or NULL */, uint8_t *const *out, int32_t *status);
 
 /* The same over several devices: ctxs[k] = a context on the k-th device to use (b2j_create(device)); image i goes to
  * exactly one of them (contiguous index ranges of about equal compressed size). One host thread per context runs

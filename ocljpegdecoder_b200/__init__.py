@@ -6,7 +6,7 @@ for bench.py; it contains no decode logic and no fallback: if the library is mis
 fails, and if no B200 is visible, ``Decoder()`` raises.
 """
 from .api import (  # noqa: F401
-    B2JError, BatchInfo, Decoder, Batch, Idct, ImageDesc, StageTimes, HostOpts, HostArgs, PinnedBuffer, parse_header, parse_orientation, read_files, host_free, decode_host_multi, library_path, load_library,
+    B2JError, BatchInfo, Decoder, Batch, Idct, ImageDesc, StageTimes, HostOpts, HostArgs, PinnedBuffer, parse_header, parse_orientation, crop_frame, read_files, host_free, decode_host_multi, library_path, load_library,
     GATE_REFERENCE, GATE_EXTENDED, PARSE_ROBUST, GATE_GRAY, OUT_BGRA, OUT_RGB24, OUT_RGB_PLANAR, OUT_GRAY8, PIXELS_REFERENCE, PIXELS_LIBJPEG,
     EXPORTED_SYMBOLS,
 )

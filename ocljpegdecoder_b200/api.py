@@ -21,9 +21,9 @@ B2J_E_NODEVICE = -7
 EXPORTED_SYMBOLS = [
     "b2j_abi_version", "b2j_strerror", "b2j_last_error", "b2j_parse_header", "b2j_parse_orientation", "b2j_device_count",
     "b2j_create", "b2j_destroy", "b2j_batch_create", "b2j_batch_destroy", "b2j_batch_get_info",
-    "b2j_batch_upload", "b2j_batch_set_output_format", "b2j_batch_set_pixel_model", "b2j_batch_set_scale", "b2j_batch_set_orientations", "b2j_batch_decode", "b2j_batch_decode_timed", "b2j_batch_decode_steps", "b2j_batch_sync", "b2j_batch_status", "b2j_batch_sync_stats",
+    "b2j_batch_upload", "b2j_batch_set_output_format", "b2j_batch_set_pixel_model", "b2j_batch_set_scale", "b2j_batch_set_orientations", "b2j_batch_set_crops", "b2j_batch_decode", "b2j_batch_decode_timed", "b2j_batch_decode_steps", "b2j_batch_sync", "b2j_batch_status", "b2j_batch_sync_stats",
     "b2j_batch_pixels_device", "b2j_batch_coefs_device", "b2j_batch_read_pixels", "b2j_batch_read_all_pixels",
-    "b2j_batch_read_coefs", "b2j_decode_host", "b2j_decode_host_ex", "b2j_decode_host_multi", "b2j_host_alloc", "b2j_host_free",
+    "b2j_batch_read_coefs", "b2j_decode_host", "b2j_decode_host_ex", "b2j_decode_host_crop", "b2j_decode_host_multi", "b2j_host_alloc", "b2j_host_free",
     "b2j_read_files", "b2j_idct_create", "b2j_idct_blk_count", "b2j_idct_upload", "b2j_idct_run", "b2j_idct_read_pixels", "b2j_idct_read_coefs",
     "b2j_idct_destroy", "b2j_batch_downscale", "b2j_batch_downscaled_device", "b2j_batch_read_downscaled",
 ]
@@ -112,6 +112,7 @@ def load_library():
     L.b2j_batch_set_pixel_model.argtypes = [vp, ci]
     L.b2j_batch_set_scale.argtypes = [vp, ci]
     L.b2j_batch_set_orientations.argtypes = [vp, vp]
+    L.b2j_batch_set_crops.argtypes = [vp, vp]
     L.b2j_batch_decode.argtypes = [vp, vp]
     L.b2j_batch_decode_timed.argtypes = [vp, vp, ctypes.POINTER(StageTimes)]
     L.b2j_batch_decode_steps.argtypes = [vp, vp, ci, ctypes.POINTER(StageTimes), ctypes.POINTER(ctypes.c_float)]
@@ -127,6 +128,8 @@ def load_library():
                                   ctypes.POINTER(vp), vp]
     L.b2j_decode_host_ex.argtypes = [vp, ci, ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(ctypes.c_size_t), ctypes.POINTER(HostOpts),
                                      ctypes.POINTER(vp), vp]
+    L.b2j_decode_host_crop.argtypes = [vp, ci, ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(ctypes.c_size_t), ctypes.POINTER(HostOpts), vp,
+                                       ctypes.POINTER(vp), vp]
     L.b2j_decode_host_multi.argtypes = [ctypes.POINTER(vp), ci, ci, ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(ctypes.c_size_t),
                                         ctypes.POINTER(HostOpts), ctypes.POINTER(vp), vp]
     L.b2j_host_alloc.argtypes = [ctypes.POINTER(vp), ctypes.c_size_t]
@@ -169,27 +172,44 @@ def parse_orientation(data):
     return o.value
 
 
-def _out_shape(d, fmt, scale=1, orientation=1):
-    """Shape of an image's pixels in output format fmt, at 1/scale of its size (ceil(W/scale) x ceil(H/scale)), with the
-    sides swapped for the EXIF orientation codes 5..8."""
+def crop_frame(d, scale=1, orientation=1):
+    """(width, height) of the frame a crop box refers to (Batch.set_crops, crops=): the image described by d (ImageDesc) at
+    1/scale of its size, then oriented by its EXIF code (sides swapped for 5..8). Boxes are drawn inside it."""
     w, h = -(-d.width // scale), -(-d.height // scale)
-    if orientation >= 5:
-        w, h = h, w
+    return (h, w) if orientation >= 5 else (w, h)
+
+
+def _crop_boxes(boxes, n):
+    """boxes (N x 4 array-like of x, y, w, h, or None) as a contiguous int32 array, or None."""
+    if boxes is None:
+        return None
+    arr = np.ascontiguousarray(boxes, np.int32)
+    if arr.shape != (n, 4):
+        raise ValueError("one crop box (x, y, w, h) per image")
+    return arr
+
+
+def _out_shape(d, fmt, scale=1, orientation=1, box=None):
+    """Shape of an image's pixels in output format fmt, at 1/scale of its size (ceil(W/scale) x ceil(H/scale)), with the
+    sides swapped for the EXIF orientation codes 5..8; box (x, y, w, h): the crop's w x h."""
+    w, h = crop_frame(d, scale, orientation) if box is None else (int(box[2]), int(box[3]))
     if fmt == OUT_GRAY8:
         return (h, w)
     return (h, w, 4) if fmt == OUT_BGRA else ((h, w, 3) if fmt == OUT_RGB24 else (3, h, w))
 
 
-def _host_call_args(files, outs, gate, fmt, scale=1, exif_orientation=False):
+def _host_call_args(files, outs, gate, fmt, scale=1, exif_orientation=False, crops=None):
     """Argument arrays of the b2j_decode_host* calls; allocates the outputs when none are given (oriented with
-    exif_orientation)."""
+    exif_orientation, of the crop's size with crops)."""
     n = len(files)
     if outs is None:
         outs = []
-        for f in files:
+        for i, f in enumerate(files):
             rc, d = parse_header(f, gate)
             o = parse_orientation(f) if exif_orientation else 1
-            outs.append(np.zeros(_out_shape(d, fmt, scale or 1, o), np.uint8) if rc == 0 else np.zeros((0, 0, 4), np.uint8))
+            box = None if crops is None else crops[i]
+            ok = rc == 0 and (box is None or (min(box) >= 0 and min(box[2:]) >= 1))
+            outs.append(np.zeros(_out_shape(d, fmt, scale or 1, o, box), np.uint8) if ok else np.zeros((0, 0, 4), np.uint8))
     ptrs = [f if isinstance(f, int) else ctypes.cast(ctypes.c_char_p(f), ctypes.c_void_p).value for f in files]
     fp = ctypes.cast((ctypes.c_void_p * n)(*ptrs), ctypes.POINTER(ctypes.c_char_p))
     return outs, fp, (ctypes.c_void_p * n)(*[o if isinstance(o, int) else o.ctypes.data for o in outs])
@@ -321,18 +341,25 @@ class Decoder:
         return args.outs, args.status
 
     def decode_host_ex(self, files, lens=None, outs=None, gate=GATE_EXTENDED, out_format=OUT_BGRA, n_threads=0, group=0,
-                       pixel_model=PIXELS_REFERENCE, scale=1, exif_orientation=False):
+                       pixel_model=PIXELS_REFERENCE, scale=1, exif_orientation=False, crops=None):
         """b2j_decode_host_ex: like decode_host with an output layout (OUT_GRAY8 with PIXELS_LIBJPEG only), a pixel model,
         a scale (1, 2, 4 or 8: the libjpeg model's scaled decode), each file's EXIF orientation applied (exif_orientation)
-        and host threads. files: bytes objects or addresses (then `lens`); outs: numpy arrays or addresses."""
+        and host threads. files: bytes objects or addresses (then `lens`); outs: numpy arrays or addresses.
+        crops: an N x 4 array-like of boxes (x, y, w, h in the crop_frame() of each file, PIXELS_LIBJPEG only) through
+        b2j_decode_host_crop; a file whose box does not fit gets status B2J_E_ARG (-1)."""
         n = len(files)
         lens = lens if lens is not None else [len(f) for f in files]
-        outs, fp, op = _host_call_args(files, outs, gate, out_format, scale, exif_orientation)
+        boxes = _crop_boxes(crops, n)
+        outs, fp, op = _host_call_args(files, outs, gate, out_format, scale, exif_orientation, boxes)
         ln = (ctypes.c_size_t * n)(*lens)
         opts = HostOpts(gate=gate, out_format=out_format, n_threads=n_threads, group=group, pixel_model=pixel_model, scale=scale,
                         exif_orientation=int(exif_orientation))
         status = np.zeros(n, np.int32)
-        _check(self.lib.b2j_decode_host_ex(self._h, n, fp, ln, ctypes.byref(opts), op, status.ctypes.data), "b2j_decode_host_ex")
+        if boxes is None:
+            _check(self.lib.b2j_decode_host_ex(self._h, n, fp, ln, ctypes.byref(opts), op, status.ctypes.data), "b2j_decode_host_ex")
+        else:
+            _check(self.lib.b2j_decode_host_crop(self._h, n, fp, ln, ctypes.byref(opts), boxes.ctypes.data, op, status.ctypes.data),
+                   "b2j_decode_host_crop")
         return outs, status
 
 
@@ -386,6 +413,7 @@ class Batch:
         self.n = len(files)
         self.out_format, self.pixel_model, self.scale = OUT_BGRA, PIXELS_REFERENCE, 1   # what b2j_batch_create sets
         self.orientations = None
+        self.crops = None
         fp = (ctypes.c_char_p * self.n)(*self.files)
         ln = (ctypes.c_size_t * self.n)(*[len(f) for f in self.files])
         self._h = ctypes.c_void_p()
@@ -466,10 +494,23 @@ class Batch:
         _check(self.lib.b2j_batch_set_orientations(self._h, None if arr is None else arr.ctypes.data), "b2j_batch_set_orientations")
         self.orientations = None if arr is None or (arr == 1).all() else arr.copy()
 
-    def pixel_shape(self, i):
-        """Shape of image i's pixels in the batch's output format, scale and orientation."""
+    def set_crops(self, boxes=None):
+        """A crop box (x, y, w, h) per image for the decodes that follow (N x 4 array-like, PIXELS_LIBJPEG only), in the
+        frame the decode would otherwise deliver (crop_frame(): scaled, then oriented): each image's pixels become
+        that image's [y:y+h, x:x+w]. None: the whole images (the default). Checked against the frame at each decode."""
+        arr = _crop_boxes(boxes, self.n)
+        _check(self.lib.b2j_batch_set_crops(self._h, None if arr is None else arr.ctypes.data), "b2j_batch_set_crops")
+        self.crops = None if arr is None else arr.copy()
+
+    def crop_frame(self, i):
+        """(width, height) of the frame image i's crop box refers to at the batch's scale and orientation."""
         o = 1 if self.orientations is None else int(self.orientations[i])
-        return _out_shape(self.descs[i], self.out_format, self.scale, o)
+        return crop_frame(self.descs[i], self.scale, o)
+
+    def pixel_shape(self, i):
+        """Shape of image i's pixels in the batch's output format, scale, orientation and crop."""
+        o = 1 if self.orientations is None else int(self.orientations[i])
+        return _out_shape(self.descs[i], self.out_format, self.scale, o, None if self.crops is None else self.crops[i])
 
     def pixels(self, i, stream=None):
         out = np.zeros(self.pixel_shape(i), np.uint8)

@@ -138,6 +138,11 @@ struct OrientTileDev
     uint32_t tile;        // tile column | tile row << 11 | orientation code << 22
 };
 
+// The window a cropped decode delivers of one image (b2j_batch_set_crops), in its unoriented frame at the batch's scale:
+// the caller's box mapped back through the image's orientation code. The kernels of a cropped decode write it at the
+// image's pix_off with pitch w.
+struct CropDev { uint32_t x0, y0, w, h; };
+
 // ---------------------------------------------------------------- host helpers ---------
 // Canonical Huffman table -> two-level LUT. Returns false when the table cannot be built
 // (code space overflow) or needs more than `max_entries` entries.

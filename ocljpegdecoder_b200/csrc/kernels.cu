@@ -1934,6 +1934,44 @@ __device__ __forceinline__ uint32_t ycc_rgb_libjpeg(int32_t y, int32_t cb, int32
     return (uint32_t)min(max(r, 0), 255) | (uint32_t)min(max(g, 0), 255) << 8 | (uint32_t)min(max(b, 0), 255) << 16;
 }
 
+// 4-pixel group i of the width x height window at (x0, y0) of an image's ceil(W / s) x ceil(H / s) output, s = 8 / MINS,
+// into the window's pixels at the image's pix_off (pitch: the window's width). The samples are read in the image's whole
+// sample plane, so the fancy filters at the window's edges see the neighbours outside it, clamped at the image's edges.
+template <int FMT, uint32_t MINS>
+__device__ __forceinline__ void upsample_group(const uint8_t *__restrict__ samples, const ImgDev &im, uint32_t x0, uint32_t y0, uint32_t width,
+                                               uint32_t height, uint32_t i, uint8_t *__restrict__ pix)
+{
+    constexpr bool fancy = MINS > 1u;
+    const uint32_t gw = (width + 3u) / 4u;
+    if (i >= gw * height) return;
+    const uint32_t py = i / gw, px = (i % gw) * 4u;
+    const uint32_t sp = im.samp, mcw = im.mcu_count_w;
+    const uint32_t yh = sp & 15u, yv = (sp >> 4) & 15u, uh = (sp >> 8) & 15u, uv = (sp >> 12) & 15u, vh = (sp >> 16) & 15u, vv = (sp >> 20) & 15u;
+    const uint8_t *p0 = samples + 64ull * im.blk_first;
+    const bool gray = im.mode == kModeGray;
+    // the chroma factors divide the luma's (geometry_ok), so the luma's are the maxima
+    const UpComp cy = up_comp(p0, yh, yv, yh, yv, mcw, im.width, im.height, MINS);
+    UpComp cu = cy, cv = cy;
+    if (!gray)
+    {
+        cu = up_comp(p0 + 64ull * im.mcu_count * (yh * yv), uh, uv, yh, yv, mcw, im.width, im.height, MINS);
+        cv = up_comp(p0 + 64ull * im.mcu_count * (yh * yv + uh * uv), vh, vv, yh, yv, mcw, im.width, im.height, MINS);
+    }
+    uint32_t R[2] = {0u, 0u}, Gc[2] = {0u, 0u}, B[2] = {0u, 0u};
+#pragma unroll
+    for (uint32_t k = 0; k < 4u; k++)
+    {
+        const uint32_t x = x0 + min(px + k, width - 1u), y = y0 + py;   // the stores skip pixels behind the last column
+        const uint32_t Y = up_sample(cy, x, y, fancy);
+        const uint32_t rgb = gray ? Y * 0x10101u
+                                  : ycc_rgb_libjpeg((int32_t)Y, (int32_t)up_sample(cu, x, y, fancy), (int32_t)up_sample(cv, x, y, fancy));
+        const uint32_t sh = 16u * (k & 1u);
+        R[k >> 1] |= (rgb & 0xFFu) << sh; Gc[k >> 1] |= ((rgb >> 8) & 0xFFu) << sh; B[k >> 1] |= (rgb >> 16) << sh;
+    }
+    constexpr uint32_t bpp = FMT == B2J_OUT_BGRA ? 4u : (FMT == B2J_OUT_RGB24 ? 3u : 1u);
+    store_pixels4<FMT>(pix + im.pix_off + ((size_t)py * width + px) * bpp, (size_t)width * height, px, width, (width & 3u) == 0u, R, Gc, B);
+}
+
 // One thread per 4-pixel group of a row of the ceil(W / s) x ceil(H / s) output, s = 8 / MINS; blockIdx.y (strided by
 // gridDim.y) = image.
 template <int FMT, uint32_t MINS>
@@ -1941,39 +1979,24 @@ __global__ void __launch_bounds__(256)
 k_upsample_libjpeg(const uint8_t *__restrict__ samples, const ImgDev *__restrict__ imgs, uint32_t n_images, uint8_t *__restrict__ pix)
 {
     constexpr uint32_t s = 8u / MINS;
-    constexpr bool fancy = MINS > 1u;
     for (uint32_t img = blockIdx.y; img < n_images; img += gridDim.y)
     {
         const ImgDev &im = imgs[img];
-        const uint32_t width = (im.width + s - 1u) / s, height = (im.height + s - 1u) / s, gw = (width + 3u) / 4u;
-        const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-        if (i >= gw * height) continue;
-        const uint32_t py = i / gw, px = (i % gw) * 4u;
-        const uint32_t sp = im.samp, mcw = im.mcu_count_w;
-        const uint32_t yh = sp & 15u, yv = (sp >> 4) & 15u, uh = (sp >> 8) & 15u, uv = (sp >> 12) & 15u, vh = (sp >> 16) & 15u, vv = (sp >> 20) & 15u;
-        const uint8_t *p0 = samples + 64ull * im.blk_first;
-        const bool gray = im.mode == kModeGray;
-        // the chroma factors divide the luma's (geometry_ok), so the luma's are the maxima
-        const UpComp cy = up_comp(p0, yh, yv, yh, yv, mcw, im.width, im.height, MINS);
-        UpComp cu = cy, cv = cy;
-        if (!gray)
-        {
-            cu = up_comp(p0 + 64ull * im.mcu_count * (yh * yv), uh, uv, yh, yv, mcw, im.width, im.height, MINS);
-            cv = up_comp(p0 + 64ull * im.mcu_count * (yh * yv + uh * uv), vh, vv, yh, yv, mcw, im.width, im.height, MINS);
-        }
-        uint32_t R[2] = {0u, 0u}, Gc[2] = {0u, 0u}, B[2] = {0u, 0u};
-#pragma unroll
-        for (uint32_t k = 0; k < 4u; k++)
-        {
-            const uint32_t x = min(px + k, width - 1u);   // the stores skip pixels behind the last column
-            const uint32_t Y = up_sample(cy, x, py, fancy);
-            const uint32_t rgb = gray ? Y * 0x10101u
-                                      : ycc_rgb_libjpeg((int32_t)Y, (int32_t)up_sample(cu, x, py, fancy), (int32_t)up_sample(cv, x, py, fancy));
-            const uint32_t sh = 16u * (k & 1u);
-            R[k >> 1] |= (rgb & 0xFFu) << sh; Gc[k >> 1] |= ((rgb >> 8) & 0xFFu) << sh; B[k >> 1] |= (rgb >> 16) << sh;
-        }
-        constexpr uint32_t bpp = FMT == B2J_OUT_BGRA ? 4u : (FMT == B2J_OUT_RGB24 ? 3u : 1u);
-        store_pixels4<FMT>(pix + im.pix_off + ((size_t)py * width + px) * bpp, (size_t)width * height, px, width, (width & 3u) == 0u, R, Gc, B);
+        upsample_group<FMT, MINS>(samples, im, 0u, 0u, (im.width + s - 1u) / s, (im.height + s - 1u) / s, blockIdx.x * blockDim.x + threadIdx.x, pix);
+    }
+}
+
+// A cropped decode (CROP): one thread per 4-pixel group of a row of each image's window crops[image].
+template <int FMT, uint32_t MINS, bool CROP>
+__global__ void __launch_bounds__(256)
+k_upsample_libjpeg(const uint8_t *__restrict__ samples, const ImgDev *__restrict__ imgs, const CropDev *__restrict__ crops, uint32_t n_images,
+                   uint8_t *__restrict__ pix)
+{
+    static_assert(CROP, "the whole image is k_upsample_libjpeg<FMT, MINS>");
+    for (uint32_t img = blockIdx.y; img < n_images; img += gridDim.y)
+    {
+        const CropDev c = crops[img];
+        upsample_group<FMT, MINS>(samples, imgs[img], c.x0, c.y0, c.w, c.h, blockIdx.x * blockDim.x + threadIdx.x, pix);
     }
 }
 
@@ -2003,10 +2026,12 @@ __device__ __forceinline__ void warp_copy_out(uint8_t *__restrict__ dst, const u
 
 // One launch over every tile kind. Only the luma blocks get a thread (n_mcus * yh * yv). The luma component has the largest
 // factors, so jdmaster.c never doubles its DCT size: it is MINS, and each instantiation carries one transform.
-template <uint32_t MINS>
-__global__ void __launch_bounds__(kTileBlocks)
-k_idct_gray(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
-            const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ pix, int32_t *__restrict__ status)
+// CROP: only the rows and columns inside the image's window crops[img] are copied out, to the window's pixels at the
+// image's pix_off (pitch: the window's width).
+template <uint32_t MINS, bool CROP>
+__device__ __forceinline__ void idct_gray(const CUtensorMap &tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
+                                          const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ pix, int32_t *__restrict__ status,
+                                          const CropDev *__restrict__ crops)
 {
     constexpr uint32_t s = 8u / MINS;
     TileSmem &sm = *tile_smem();
@@ -2034,14 +2059,45 @@ k_idct_gray(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__
     const uint32_t ow = (sm.side.width + s - 1u) / s, oh = (sm.side.height + s - 1u) / s;
     const uint32_t mcw = __ldg(&imgs[d.img].mcu_count_w), my0 = sm.side.mcu_xy[0].y;
     const uint32_t rows = (sm.side.mcu_xy[n - 1u].y - my0 + 1u) * mh;
-    for (uint32_t i = tid >> 5; i < rows; i += kTileBlocks / 32)
+    if constexpr (CROP)
     {
-        const uint32_t my = my0 + i / mh, r = i % mh, y = my * mh + r;
-        if (y >= oh) break;
-        const uint32_t ma = max(my * mcw, d.mcu_first) - d.mcu_first, mb = min((my + 1u) * mcw, d.mcu_first + n) - d.mcu_first;
-        const uint32_t x0 = sm.side.mcu_xy[ma].x * mw, x1 = min(x0 + (mb - ma) * mw, ow);
-        if (x0 < x1) warp_copy_out(sm.side.pix + (size_t)y * ow + x0, strip + r * spitch + ma * mw, x1 - x0, tid & 31u);
+        const CropDev c = crops[d.img];   // inside the ow x oh frame (checked by the host)
+        for (uint32_t i = tid >> 5; i < rows; i += kTileBlocks / 32)
+        {
+            const uint32_t my = my0 + i / mh, r = i % mh, y = my * mh + r;
+            if (y >= c.y0 + c.h) break;
+            if (y < c.y0) continue;
+            const uint32_t ma = max(my * mcw, d.mcu_first) - d.mcu_first, mb = min((my + 1u) * mcw, d.mcu_first + n) - d.mcu_first;
+            const uint32_t x0 = sm.side.mcu_xy[ma].x * mw, xa = max(x0, c.x0), xb = min(x0 + (mb - ma) * mw, c.x0 + c.w);
+            if (xa < xb) warp_copy_out(sm.side.pix + (size_t)(y - c.y0) * c.w + (xa - c.x0), strip + r * spitch + ma * mw + (xa - x0), xb - xa, tid & 31u);
+        }
     }
+    else
+        for (uint32_t i = tid >> 5; i < rows; i += kTileBlocks / 32)
+        {
+            const uint32_t my = my0 + i / mh, r = i % mh, y = my * mh + r;
+            if (y >= oh) break;
+            const uint32_t ma = max(my * mcw, d.mcu_first) - d.mcu_first, mb = min((my + 1u) * mcw, d.mcu_first + n) - d.mcu_first;
+            const uint32_t x0 = sm.side.mcu_xy[ma].x * mw, x1 = min(x0 + (mb - ma) * mw, ow);
+            if (x0 < x1) warp_copy_out(sm.side.pix + (size_t)y * ow + x0, strip + r * spitch + ma * mw, x1 - x0, tid & 31u);
+        }
+}
+
+template <uint32_t MINS>
+__global__ void __launch_bounds__(kTileBlocks)
+k_idct_gray(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
+            const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ pix, int32_t *__restrict__ status)
+{
+    idct_gray<MINS, false>(tmap, imgs, tiles, qtabs, pix, status, nullptr);
+}
+
+template <uint32_t MINS, bool CROP>
+__global__ void __launch_bounds__(kTileBlocks)
+k_idct_gray(const __grid_constant__ CUtensorMap tmap, const ImgDev *__restrict__ imgs, const TileDev *__restrict__ tiles,
+            const uint16_t *__restrict__ qtabs, uint8_t *__restrict__ pix, int32_t *__restrict__ status, const CropDev *__restrict__ crops)
+{
+    static_assert(CROP, "the whole image is k_idct_gray<MINS>");
+    idct_gray<MINS, true>(tmap, imgs, tiles, qtabs, pix, status, crops);
 }
 
 // =====================================================================================
@@ -2258,10 +2314,18 @@ static void launch_idct_format(const DecodeArgs &a, cudaStream_t s)
 }
 
 // The libjpeg model: the IDCT over every tile into the sample plane, then the upsampling / colour pass over every image.
+// A cropped decode (a.crops) transforms the tiles of its crop tile list (every window has one at least) and upsamples
+// the windows only.
 template <int FMT, uint32_t MINS>
 static void launch_libjpeg_scale(const DecodeArgs &a, cudaStream_t s)
 {
     const dim3 grid((a.max_px_groups + 255u) / 256u, a.n_images < 65535u ? a.n_images : 65535u);
+    if (a.crops)
+    {
+        k_idct_libjpeg<MINS><<<a.n_crop_tiles, kTileBlocks, kTileSmemBytes, s>>>(*a.tmap, a.imgs, a.crop_tiles, a.qtabs, a.samples, a.status);
+        k_upsample_libjpeg<FMT, MINS, true><<<grid, 256, 0, s>>>(a.samples, a.imgs, a.crops, a.n_images, a.pixels);
+        return;
+    }
     k_idct_libjpeg<MINS><<<a.n_tiles, kTileBlocks, kTileSmemBytes, s>>>(*a.tmap, a.imgs, a.tiles, a.qtabs, a.samples, a.status);
     k_upsample_libjpeg<FMT, MINS><<<grid, 256, 0, s>>>(a.samples, a.imgs, a.n_images, a.pixels);
 }
@@ -2279,6 +2343,12 @@ static void launch_libjpeg_format(const DecodeArgs &a, cudaStream_t s)
 template <uint32_t MINS>
 static void launch_gray_scale(const DecodeArgs &a, cudaStream_t s)
 {
+    if (a.crops)
+    {
+        k_idct_gray<MINS, true><<<a.n_crop_tiles, kTileBlocks, kTileSmemBytes + kGrayStageBytes, s>>>(*a.tmap, a.imgs, a.crop_tiles, a.qtabs, a.pixels,
+                                                                                                    a.status, a.crops);
+        return;
+    }
     k_idct_gray<MINS><<<a.n_tiles, kTileBlocks, kTileSmemBytes + kGrayStageBytes, s>>>(*a.tmap, a.imgs, a.tiles, a.qtabs, a.pixels, a.status);
 }
 

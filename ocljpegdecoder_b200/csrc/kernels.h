@@ -49,6 +49,11 @@ struct DecodeArgs
                              // whose format is not B2J_OUT_GRAY8)
     uint32_t max_px_groups;  // largest ceil(OW / 4) * OH of the batch's output sizes: the grid of the libjpeg model's upsampling kernel
     uint32_t scale;          // B2J_PIXELS_LIBJPEG: the output is ceil(W / scale) x ceil(H / scale); 1, 2, 4 or 8 (b2j_batch_set_scale)
+    // B2J_PIXELS_LIBJPEG, b2j_batch_set_crops: every image's window, nullptr = the whole images; the IDCT then runs over
+    // the crop tile list (the windows' MCUs and their halo) instead of `tiles`
+    const CropDev *crops;
+    const TileDev *crop_tiles;
+    uint32_t n_crop_tiles;
 };
 
 cudaError_t init_constants();

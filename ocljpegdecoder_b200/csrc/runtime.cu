@@ -31,6 +31,7 @@
 
 #include "b2j_internal.h"
 #include "b2j_math.h"
+#include "crop_plan.h"
 #include "kernels.h"
 
 using namespace b2j;
@@ -146,6 +147,15 @@ struct b2j_batch
     uint32_t n_orient_tiles = 0;
     bool orient_stale = false;                // the table on the device is not the one of the current settings
     cudaEvent_t orient_copied = nullptr;      // the last copy out of h_orient
+    // crop windows (b2j_batch_set_crops): d_crop holds every image's window, the window views that the orientation pass
+    // reads as its image table (an image the size of its window), then the crop tile list; h_crop is their pinned staging
+    std::vector<int32_t> crops;               // x, y, w, h per image, in the oriented frame at the batch's scale; empty = none
+    std::vector<CropDev> win;                 // every image's window in its unoriented frame (set_output)
+    int crop_misfit = -1;                     // the first image whose box does not fit its frame (set_output); -1 = none
+    PoolBuf d_crop, h_crop;
+    size_t crop_views_off = 0, crop_tiles_off = 0;
+    bool crop_stale = false;                  // the windows and tiles on the device are not those of the current settings
+    cudaEvent_t crop_copied = nullptr;        // the last copy out of h_crop
 
     CUtensorMap tmap;
     DecodeArgs args;
@@ -234,6 +244,8 @@ cudaError_t grow(b2j_ctx *ctx, PoolBuf &buf, size_t n, bool pinned = false)
     return e;
 }
 
+template <class T> T *at(const PoolBuf &buf, size_t off) { return reinterpret_cast<T *>((uint8_t *)buf.p + off); }
+
 void release_orient_buffers(b2j_batch *b)
 {
     b2j_ctx *c = b->ctx;
@@ -242,11 +254,23 @@ void release_orient_buffers(b2j_batch *b)
     c->pin_pool.put(b->h_orient);
 }
 
+void release_crop_buffers(b2j_batch *b)
+{
+    b2j_ctx *c = b->ctx;
+    std::lock_guard<std::mutex> lk(c->mu);
+    c->dev_pool.put(b->d_crop);
+    c->pin_pool.put(b->h_crop);
+}
+
 void release_batch_buffers(b2j_batch *b)
 {
     release_orient_buffers(b);
-    if (b->orient_copied) cudaEventDestroy(b->orient_copied);
-    b->orient_copied = nullptr;
+    release_crop_buffers(b);
+    for (cudaEvent_t *e : {&b->orient_copied, &b->crop_copied})
+    {
+        if (*e) cudaEventDestroy(*e);
+        *e = nullptr;
+    }
     b2j_ctx *c = b->ctx;
     std::lock_guard<std::mutex> lk(c->mu);
     c->pin_pool.put(b->h_blob);
@@ -257,7 +281,7 @@ void release_batch_buffers(b2j_batch *b)
 // b2j_batch_downscale() are not counted)
 int64_t device_bytes(const b2j_batch *b)
 {
-    return (int64_t)(b->d_blob.cap + b->d_scratch.cap + b->d_coef.cap + b->d_pix.cap + b->d_samples.cap + b->d_orient.cap);
+    return (int64_t)(b->d_blob.cap + b->d_scratch.cap + b->d_coef.cap + b->d_pix.cap + b->d_samples.cap + b->d_orient.cap + b->d_crop.cap);
 }
 
 // The image `image` of the batch, or nullptr when the batch has no such image.
@@ -274,11 +298,12 @@ bool scale_ok(int denom) { return denom == 1 || denom == 2 || denom == 4 || deno
 
 // Why a decode with these settings cannot run, or nullptr when it can. The setters store any valid value, so a batch
 // may hold such a combination; the decode refuses it.
-const char *output_refusal(int model, int fmt, int scale)
+const char *output_refusal(int model, int fmt, int scale, bool cropped)
 {
     if (model == B2J_PIXELS_LIBJPEG) return nullptr;
     if (scale != 1) return "a scaled decode (b2j_batch_set_scale, b2j_host_opts.scale) needs the libjpeg pixel model: the reference has none";
     if (fmt == B2J_OUT_GRAY8) return "B2J_OUT_GRAY8 (libjpeg's grayscale output) needs the libjpeg pixel model: the reference has none";
+    if (cropped) return "a cropped decode (b2j_batch_set_crops, b2j_decode_host_crop) needs the libjpeg pixel model";
     return nullptr;
 }
 
@@ -287,28 +312,70 @@ const char *output_refusal(int model, int fmt, int scale)
 struct Dims { uint32_t w, h; };
 Dims out_dims(const ImgDev &im, uint32_t div) { return {(im.width + div - 1) / div, (im.height + div - 1) / div}; }
 
-size_t image_bytes(const b2j_batch *b, const ImgDev &im)
+// What a decode delivers of image i: scale, then crop, then orientation. `win` is the window the IDCT/colour stage
+// writes, in the image's unoriented frame at the batch's scale (the whole frame without crops); `dims` is the size of the
+// result the reads return (the window, sides swapped for orientation codes 5..8).
+struct ImageOut { CropDev win; Dims dims; };
+ImageOut image_out(const b2j_batch *b, size_t i)
 {
-    const Dims o = out_dims(im, b->args.scale);
+    const Dims f = out_dims(b->imgs[i], b->args.scale);
+    const CropDev win = b->crops.empty() ? CropDev{0, 0, f.w, f.h} : b->win[i];
+    const bool swap = !b->orient.empty() && b->orient[i] >= 5;
+    return {win, swap ? Dims{win.h, win.w} : Dims{win.w, win.h}};
+}
+
+size_t image_bytes(const b2j_batch *b, size_t i)
+{
+    const Dims o = image_out(b, i).dims;
     return (size_t)o.w * o.h * format_bpp(b->args.out_format);
+}
+
+// B2J_E_ARG, naming the image, while a crop box does not lie inside its image's frame at the batch's scale and orientation.
+int crop_refusal(const b2j_batch *b)
+{
+    if (b->crop_misfit < 0) return B2J_OK;
+    const ImgDev &im = b->imgs[(size_t)b->crop_misfit];
+    const Dims f = out_dims(im, b->args.scale);
+    const bool swap = !b->orient.empty() && b->orient[(size_t)b->crop_misfit] >= 5;
+    const int32_t *c = &b->crops[4 * (size_t)b->crop_misfit];
+    char buf[256];
+    snprintf(buf, sizeof(buf), "the crop box (%d, %d, %d, %d) of image %d does not lie inside its %u x %u frame (at the batch's scale, oriented)", c[0], c[1],
+             c[2], c[3], b->crop_misfit, swap ? f.h : f.w, swap ? f.w : f.h);
+    t_last_error = buf;
+    return B2J_E_ARG;
 }
 
 // Alignment of an image's start when images are packed side by side in a format: what the stores of the kernels that
 // write them allow (16 bytes for BGRA, 4 for the three-byte formats, none for GRAY8, whose kernels store single bytes).
 size_t pack_align(int fmt) { return fmt == B2J_OUT_BGRA ? 16 : (fmt == B2J_OUT_GRAY8 ? 1 : 4); }
 
-// The only writer of a batch's output settings and of what follows from them: the upsampling kernel's grid, the places of
-// the oriented copies and the launch count of a decode.
+// The only writer of a batch's output settings and of what follows from them: the crop windows, the upsampling kernel's
+// grid, the places of the oriented copies and the launch count of a decode.
 void set_output(b2j_batch *b, int model, int fmt, int scale)
 {
     b->args.pixel_model = model;   // the sample plane, once allocated, stays with the batch
-    b->args.out_format = fmt;      // the pixel plane is sized for BGRA at scale 1: every format and scale fits
+    b->args.out_format = fmt;      // the pixel plane is sized for BGRA at scale 1: every format, scale and crop fits
     b->args.scale = (uint32_t)scale;
-    uint32_t groups = 0;           // one thread per 4 output pixels of a row
-    for (const ImgDev &im : b->imgs)
+    // the windows of the crop boxes; a box that does not fit the frame stands for the whole frame until the settings
+    // change, and decodes and reads are refused (crop_refusal)
+    b->crop_misfit = -1;
+    for (size_t i = 0; i < b->crops.size() / 4; i++)
     {
-        const Dims o = out_dims(im, (uint32_t)scale);
-        groups = std::max(groups, (o.w + 3) / 4 * o.h);
+        const Dims f = out_dims(b->imgs[i], (uint32_t)scale);
+        if (!crop_window(f.w, f.h, b->orient.empty() ? 1u : b->orient[i], &b->crops[4 * i], b->win[i]))
+        {
+            b->win[i] = {0, 0, f.w, f.h};
+            if (b->crop_misfit < 0) b->crop_misfit = (int)i;
+        }
+    }
+    b->crop_stale = !b->crops.empty();
+    b->args.crops = b->crops.empty() ? nullptr : at<const CropDev>(b->d_crop, 0);
+    b->args.crop_tiles = b->crops.empty() ? nullptr : at<const TileDev>(b->d_crop, b->crop_tiles_off);
+    uint32_t groups = 0;           // one thread per 4 output pixels of a row
+    for (size_t i = 0; i < b->imgs.size(); i++)
+    {
+        const CropDev w = image_out(b, i).win;
+        groups = std::max(groups, (w.w + 3) / 4 * w.h);
     }
     b->args.max_px_groups = groups;
     // the oriented copies behind the tile table, neighbours in image order (d_orient is sized for BGRA at scale 1); the
@@ -318,7 +385,7 @@ void set_output(b2j_batch *b, int model, int fmt, int scale)
         if (b->orient[i] != 1)
         {
             b->orient_off[i] = off = align_up(off, pack_align(fmt));
-            off += image_bytes(b, b->imgs[i]);
+            off += image_bytes(b, i);
         }
     b->orient_stale = !b->orient.empty();
     b->info.kernel_launches = b->fixed_launches + idct_launches(b->args) + (b->orient.empty() ? 0 : 1);
@@ -333,8 +400,6 @@ int read_back(b2j_batch *b, void *stream, void *dst, const void *src, size_t byt
     CU_TRY(cudaStreamSynchronize(s));
     return B2J_OK;
 }
-
-template <class T> T *at(const PoolBuf &buf, size_t off) { return reinterpret_cast<T *>((uint8_t *)buf.p + off); }
 
 // Copies a host-built array to its place in the pinned blob; returns where it lands on the device.
 template <class T> const T *stage(const b2j_batch *b, size_t off, const std::vector<T> &v)
@@ -751,7 +816,8 @@ extern "C" int b2j_batch_upload(b2j_batch *b, void *stream)
 constexpr size_t kStepEvents = 5;
 
 // The orientation pass's tile table for the current settings, copied to the front of d_orient on `s`: one tile of
-// kOrientTile x kOrientTile pixels per piece of every image whose code is not 1, at the batch's scale.
+// kOrientTile x kOrientTile pixels per piece of every image whose code is not 1 (of its window when it is cropped), at
+// the batch's scale.
 static int stage_orient_tiles(b2j_batch *b, cudaStream_t s)
 {
     // the pinned table is rebuilt only once the copy out of it has left
@@ -763,7 +829,7 @@ static int stage_orient_tiles(b2j_batch *b, cudaStream_t s)
     {
         const uint32_t code = b->orient[i];
         if (code == 1) continue;
-        const Dims o = out_dims(b->imgs[i], b->args.scale);
+        const CropDev o = image_out(b, i).win;
         for (uint32_t ty = 0; ty * kOrientTile < o.h; ty++)
             for (uint32_t tx = 0; tx * kOrientTile < o.w; tx++) t[k++] = {b->orient_off[i], (uint32_t)i, tx | ty << 11 | code << 22};
     }
@@ -774,12 +840,41 @@ static int stage_orient_tiles(b2j_batch *b, cudaStream_t s)
     return B2J_OK;
 }
 
+// The crop windows, the window views and the crop tile list for the current settings, copied to d_crop on `s`. GRAY8
+// and scale 1/8 have no fancy upsampling, so their tiles need no halo. A tile's TMA box is always kTileBlocks rows from
+// its first block, which lies inside the plane: it ends inside the plane's kTileBlocks rows of slack (coef_rows).
+static int stage_crop_tiles(b2j_batch *b, cudaStream_t s)
+{
+    // the pinned copy is rebuilt only once the copy out of it has left
+    if (!b->crop_copied) CU_TRY(cudaEventCreateWithFlags(&b->crop_copied, cudaEventDisableTiming));
+    else CU_TRY(cudaEventSynchronize(b->crop_copied));
+    const uint32_t halo = (b->args.out_format == B2J_OUT_GRAY8 || b->args.scale == 8) ? 0u : 1u;
+    CropDev *w = at<CropDev>(b->h_crop, 0);
+    ImgDev *v = at<ImgDev>(b->h_crop, b->crop_views_off);
+    std::vector<TileDev> tiles;
+    for (size_t i = 0; i < b->imgs.size(); i++)
+    {
+        w[i] = b->win[i];
+        v[i] = b->imgs[i];
+        v[i].width = w[i].w;
+        v[i].height = w[i].h;
+        crop_tiles(b->imgs[i], (uint32_t)i, w[i], b->args.scale, halo, tiles);
+    }
+    memcpy(at<TileDev>(b->h_crop, b->crop_tiles_off), tiles.data(), sizeof(TileDev) * tiles.size());
+    b->args.n_crop_tiles = (uint32_t)tiles.size();
+    CU_TRY(cudaMemcpyAsync(b->d_crop.p, b->h_crop.p, b->crop_tiles_off + sizeof(TileDev) * tiles.size(), cudaMemcpyHostToDevice, s));
+    CU_TRY(cudaEventRecord(b->crop_copied, s));
+    b->crop_stale = false;
+    return B2J_OK;
+}
+
 // One decode of the whole batch: the pre-pass, the entropy stage and the IDCT/colour stage, in order on `s`, then the
 // orientation pass when some image's code is not 1.
 static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStepEvents or NULL */)
 {
     if (!b->uploaded) { t_last_error = "b2j_batch_decode before b2j_batch_upload"; return B2J_E_ARG; }
-    if (const char *why = output_refusal(b->args.pixel_model, b->args.out_format, (int)b->args.scale)) { t_last_error = why; return B2J_E_ARG; }
+    if (const char *why = output_refusal(b->args.pixel_model, b->args.out_format, (int)b->args.scale, !b->crops.empty())) { t_last_error = why; return B2J_E_ARG; }
+    if (const int rc = crop_refusal(b)) return rc;
     if (b->args.pixel_model == B2J_PIXELS_LIBJPEG && b->args.out_format != B2J_OUT_GRAY8 && !b->d_samples.p)
     {
         // the sample plane: 64 bytes per block, image by image at 64 * blk_first
@@ -790,6 +885,8 @@ static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStep
     }
     if (b->orient_stale)
         if (const int rc = stage_orient_tiles(b, s)) return rc;
+    if (b->crop_stale)
+        if (const int rc = stage_crop_tiles(b, s)) return rc;
     const DecodeArgs &a = b->args;
     if (ev) CU_TRY(cudaEventRecord(ev[0], s));
     if (a.n_huff_ctas) CU_TRY(cudaMemsetAsync(a.seg_start, 0xFF, 4 * (size_t)b->n_segs_total, s));   // read by the restart-interval decoder only
@@ -801,8 +898,10 @@ static int enqueue_decode(b2j_batch *b, cudaStream_t s, cudaEvent_t *ev /* kStep
     launch_huffman_sync(a, s);
     if (ev) CU_TRY(cudaEventRecord(ev[3], s));
     launch_idct(a, s);
+    // a cropped image is oriented as an image of its window's size: the window views at scale 1
     if (!b->orient.empty())
-        launch_orient(a.pixels, a.imgs, at<const OrientTileDev>(b->d_orient, 0), b->n_orient_tiles, a.scale, a.out_format, at<uint8_t>(b->d_orient, 0), s);
+        launch_orient(a.pixels, a.crops ? at<const ImgDev>(b->d_crop, b->crop_views_off) : a.imgs, at<const OrientTileDev>(b->d_orient, 0), b->n_orient_tiles,
+                      a.crops ? 1u : a.scale, a.out_format, at<uint8_t>(b->d_orient, 0), s);
     if (ev) CU_TRY(cudaEventRecord(ev[4], s));
     CU_TRY(cudaGetLastError());
     return B2J_OK;
@@ -943,12 +1042,47 @@ extern "C" int b2j_batch_set_orientations(b2j_batch *b, const uint8_t *codes)
     return rc;
 }
 
+extern "C" int b2j_batch_set_crops(b2j_batch *b, const int32_t *boxes)
+{
+    if (!b) return B2J_E_ARG;
+    for (int i = 0; boxes && i < b->n; i++)
+        if (boxes[4 * i] < 0 || boxes[4 * i + 1] < 0 || boxes[4 * i + 2] < 1 || boxes[4 * i + 3] < 1) return B2J_E_ARG;
+    CU_TRY(cudaSetDevice(b->ctx->device));
+    // the buffers go back to the pool or grow: work in flight may still read the windows or the tiles
+    if (b->last_stream && (b->d_crop.p || boxes)) CU_TRY(cudaStreamSynchronize(b->last_stream));
+    b->crops.clear();
+    b->win.clear();
+    int rc = B2J_OK;
+    if (boxes)
+    {
+        size_t tiles = 0;   // at any window and scale
+        for (const ImgDev &im : b->imgs) tiles += crop_tiles_max(im);
+        b->crop_views_off = align_up(sizeof(CropDev) * (size_t)b->n, 256);
+        b->crop_tiles_off = b->crop_views_off + align_up(sizeof(ImgDev) * (size_t)b->n, 256);
+        const size_t bytes = b->crop_tiles_off + sizeof(TileDev) * tiles;
+        if (grow(b->ctx, b->d_crop, bytes) != cudaSuccess || grow(b->ctx, b->h_crop, bytes, true) != cudaSuccess)
+        {
+            t_last_error = "crop buffer allocation";
+            rc = B2J_E_NOMEM;   // no crops then
+        }
+        else
+        {
+            b->crops.assign(boxes, boxes + 4 * (size_t)b->n);
+            b->win.assign((size_t)b->n, CropDev{});
+        }
+    }
+    if (b->crops.empty()) release_crop_buffers(b);
+    b->info.device_bytes = device_bytes(b);
+    set_output(b, b->args.pixel_model, b->args.out_format, (int)b->args.scale);
+    return rc;
+}
+
 extern "C" int b2j_batch_pixels_device(const b2j_batch *b, int image, void **dptr, size_t *nbytes)
 {
-    const ImgDev *im = image_of(b, image);
-    if (!im || !dptr) return B2J_E_ARG;
+    if (!image_of(b, image) || !dptr) return B2J_E_ARG;
+    if (const int rc = crop_refusal(b)) return rc;
     *dptr = result_of(b, (size_t)image);
-    if (nbytes) *nbytes = image_bytes(b, *im);
+    if (nbytes) *nbytes = image_bytes(b, (size_t)image);
     return B2J_OK;
 }
 
@@ -963,21 +1097,21 @@ extern "C" int b2j_batch_coefs_device(const b2j_batch *b, int image, void **dptr
 
 extern "C" int b2j_batch_read_pixels(b2j_batch *b, void *stream, int image, uint8_t *dst)
 {
-    const ImgDev *im = image_of(b, image);
-    if (!im || !dst) return B2J_E_ARG;
-    return read_back(b, stream, dst, result_of(b, (size_t)image), image_bytes(b, *im));
+    if (!image_of(b, image) || !dst) return B2J_E_ARG;
+    if (const int rc = crop_refusal(b)) return rc;
+    return read_back(b, stream, dst, result_of(b, (size_t)image), image_bytes(b, (size_t)image));
 }
 
 extern "C" int b2j_batch_read_all_pixels(b2j_batch *b, void *stream, uint8_t *const *dsts)
 {
     if (!b || !dsts) return B2J_E_ARG;
+    if (const int rc = crop_refusal(b)) return rc;
     CU_TRY(cudaSetDevice(b->ctx->device));
     cudaStream_t s = pick_stream(b, stream);
     for (int i = 0; i < b->n; i++)
     {
-        const ImgDev &im = b->imgs[(size_t)i];
         if (!dsts[i]) continue;
-        CU_TRY(cudaMemcpyAsync(dsts[i], result_of(b, (size_t)i), image_bytes(b, im), cudaMemcpyDeviceToHost, s));
+        CU_TRY(cudaMemcpyAsync(dsts[i], result_of(b, (size_t)i), image_bytes(b, (size_t)i), cudaMemcpyDeviceToHost, s));
     }
     CU_TRY(cudaStreamSynchronize(s));
     return B2J_OK;
@@ -1006,6 +1140,7 @@ extern "C" int b2j_batch_downscale(b2j_batch *b, void *stream, int factor)
     if (b->args.scale != 1) { t_last_error = "b2j_batch_downscale of a scaled decode"; return B2J_E_ARG; }
     // k_downscale takes each image's size from its unoriented descriptor
     if (!b->orient.empty()) { t_last_error = "b2j_batch_downscale of oriented images (b2j_batch_set_orientations)"; return B2J_E_ARG; }
+    if (!b->crops.empty()) { t_last_error = "b2j_batch_downscale of cropped images (b2j_batch_set_crops)"; return B2J_E_ARG; }
     CU_TRY(cudaSetDevice(b->ctx->device));
     cudaStream_t s = pick_stream(b, stream);
     const int fmt = b->args.out_format;
@@ -1069,10 +1204,10 @@ void pack_pixel_plane(b2j_batch *b)
 {
     const size_t a = pack_align(b->args.out_format);
     size_t off = 0;
-    for (ImgDev &im : b->imgs)
+    for (size_t i = 0; i < b->imgs.size(); i++)
     {
-        im.pix_off = off = align_up(off, a);
-        off += image_bytes(b, im);
+        b->imgs[i].pix_off = off = align_up(off, a);
+        off += image_bytes(b, i);
     }
     memcpy(b->h_imgs, b->imgs.data(), sizeof(ImgDev) * (size_t)b->n);
 }
@@ -1099,14 +1234,14 @@ struct FeedGroup
 
 } // namespace
 
-extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *files, const size_t *lens, const b2j_host_opts *opts,
-                                  uint8_t *const *out, int32_t *status)
+extern "C" int b2j_decode_host_crop(b2j_ctx *ctx, int n, const uint8_t *const *files, const size_t *lens, const b2j_host_opts *opts,
+                                    const int32_t *crops, uint8_t *const *out, int32_t *status)
 {
     if (!ctx || n <= 0 || !files || !lens || !out || !status || !opts) return B2J_E_ARG;
     const int fmt = opts->out_format, model = opts->pixel_model, scale = opts->scale ? opts->scale : 1;
     const bool orient = opts->exif_orientation == 1;
     if (!format_ok(fmt) || !model_ok(model) || !scale_ok(scale) || (opts->exif_orientation & ~1)) return B2J_E_ARG;
-    if (const char *why = output_refusal(model, fmt, scale)) { t_last_error = why; return B2J_E_ARG; }
+    if (const char *why = output_refusal(model, fmt, scale, crops != nullptr)) { t_last_error = why; return B2J_E_ARG; }
     CU_TRY(cudaSetDevice(ctx->device));
     const int gate = opts->gate;
     const int group = opts->group > 0 ? opts->group : 32;
@@ -1152,6 +1287,7 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
         std::vector<const uint8_t *> f;
         std::vector<size_t> l;
         std::vector<uint8_t> codes;   // orientation codes of the accepted files
+        std::vector<int32_t> boxes;   // their crop boxes
         for (;;)
         {
             const int g = next_group.fetch_add(1);
@@ -1162,16 +1298,24 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
                 if (stop) { groups[(size_t)g].ready = true; cv.notify_all(); continue; }
             }
             FeedGroup &G = groups[(size_t)g];
-            d.clear(); f.clear(); l.clear(); codes.clear();
+            d.clear(); f.clear(); l.clear(); codes.clear(); boxes.clear();
             for (int i = G.first; i < G.first + G.count; i++)
             {
                 b2j_image_desc desc;
                 const int prc = b2j_parse_header(files[i], lens[i], gate, &desc);
                 status[i] = prc;
                 if (prc != B2J_OK) continue;
-                G.idx.push_back(i); d.push_back(desc); f.push_back(files[i]); l.push_back(lens[i]);
                 int32_t code = 1;
                 if (orient) b2j_parse_orientation(files[i], lens[i], &code);
+                if (crops)
+                {
+                    // the box must lie inside the image's frame at the scale, oriented; else the image is skipped
+                    CropDev win;
+                    const uint32_t fw = ((uint32_t)desc.width + scale - 1) / scale, fh = ((uint32_t)desc.height + scale - 1) / scale;
+                    if (!crop_window(fw, fh, (uint32_t)code, crops + 4 * (size_t)i, win)) { status[i] = B2J_E_ARG; continue; }
+                    boxes.insert(boxes.end(), crops + 4 * (size_t)i, crops + 4 * (size_t)i + 4);
+                }
+                G.idx.push_back(i); d.push_back(desc); f.push_back(files[i]); l.push_back(lens[i]);
                 codes.push_back((uint8_t)code);
             }
             G.parsed = true;
@@ -1182,6 +1326,7 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
                 {
                     set_output(G.b, model, fmt, scale);
                     if (orient) G.rc = b2j_batch_set_orientations(G.b, codes.data());
+                    if (crops && G.rc == B2J_OK) G.rc = b2j_batch_set_crops(G.b, boxes.data());
                     pack_pixel_plane(G.b);
                 }
                 if (G.rc != B2J_OK) G.err = t_last_error;
@@ -1249,10 +1394,10 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
         {
             uint8_t *dst = out[G.idx[k]];
             const uint8_t *src = result_of(G.b, k);
-            size_t bytes = image_bytes(G.b, G.b->imgs[k]), k1 = k + 1;
+            size_t bytes = image_bytes(G.b, k), k1 = k + 1;
             if (!dst) { k = k1; continue; }
             while (k1 < G.idx.size() && out[G.idx[k1]] == dst + bytes && result_of(G.b, k1) == src + bytes)
-                bytes += image_bytes(G.b, G.b->imgs[k1++]);
+                bytes += image_bytes(G.b, k1++);
             e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, ctx->stream2);
             k = k1;
         }
@@ -1265,7 +1410,7 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
             k = k1;
         }
         if (e == cudaSuccess) e = cudaEventRecord(G.done, ctx->stream2);
-        if (e != cudaSuccess) { rc = fail_cuda(e, "b2j_decode_host_ex enqueue"); break; }
+        if (e != cudaSuccess) { rc = fail_cuda(e, "b2j_decode_host_crop enqueue"); break; }
         retire(g, false);
     }
     {
@@ -1292,6 +1437,12 @@ extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *fil
         ctx->pin_pool.put(h_status_buf);
     }
     return rc;
+}
+
+extern "C" int b2j_decode_host_ex(b2j_ctx *ctx, int n, const uint8_t *const *files, const size_t *lens, const b2j_host_opts *opts,
+                                  uint8_t *const *out, int32_t *status)
+{
+    return b2j_decode_host_crop(ctx, n, files, lens, opts, nullptr, out, status);
 }
 
 extern "C" int b2j_decode_host_multi(b2j_ctx *const *ctxs, int n_ctx, int n, const uint8_t *const *files, const size_t *lens,
